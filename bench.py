@@ -50,21 +50,42 @@ HORIZON = 4
 def parse_args():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=100)
+    ap.add_argument("--steps", type=int, default=100,
+                    help="timed steps of every leg except the batched leg of the latency workload (--batched-steps)")
     ap.add_argument("--warmup", type=int, default=10)
     ap.add_argument("--impl", choices=["ours", "reference"], default="ours")
     ap.add_argument("--workload", choices=["auto", "latency", "batched", "openvla"], default="auto",
                     help="headline measurement (see the module docstring)")
     ap.add_argument("--batch", type=int, default=1, help="episodes per GPU of the latency measurement")
     ap.add_argument("--batched", type=int, default=64, help="episodes per GPU of the batched measurement (0 = skip)")
-    ap.add_argument("--batched-steps", type=int, default=0, help="timed steps of the batched leg when it is not the headline (0 = 10)")
+    ap.add_argument("--batched-steps", type=int, default=0, help="timed steps of the batched leg when it is not the headline (0 = 10); --steps times it when it is")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-roofline", action="store_true")
     ap.add_argument("--no-raw-frames", action="store_true", help="skip the e2e leg that starts from raw camera frames")
     ap.add_argument("--flow-steps", type=int, default=1, help="num_inference_steps (1 = --preset blurr)")
     ap.add_argument("--robot", choices=["bridge", "fractal"], default="bridge", help="config family (BASELINE.json configs[2]: fractal)")
     ap.add_argument("--ring", type=int, default=50, help="distinct pre-staged control-step inputs (one episode)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step of each timed leg returned as DIR/<name>.npy; with N > 1 GPUs "
+                         "rank 0 writes its own episodes (its shard of the batched leg)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.batched_steps < 0:
+        ap.error("--batched-steps must not be negative")
+    return args
+
+
+def dump_outputs(out_dir, arrays):
+    """Save each output as float32 (float64 for integer ids, exact) .npy so that two builds can be compared output
+    for output; every input of the run is seeded, so the same arguments give the same inputs."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        t = t.detach().cpu()
+        t = t.double() if not t.is_floating_point() else t.float()
+        np.save(os.path.join(out_dir, f"{name}.npy"), t.numpy())
 
 
 def measured_peaks():
@@ -196,6 +217,7 @@ class Ctx:
         self.model = PiZeroInference.from_state_dict(self.cfg, sd, device=self.dev)
         del sd
         self.model.set_engine_options(reserve_batch=max(args.batch, args.batched))
+        self.outputs = {}           # leg name -> actions of its last timed step (--dump-outputs)
 
     def barrier(self):
         import torch
@@ -218,9 +240,10 @@ class Ctx:
         return self.model(**{k: r[k] for k in synth.CALL_KEYS}, noise=r["noise"])
 
 
-def timed_device_loop(ctx, ring, K, W, sample_clocks):
+def timed_device_loop(ctx, ring, K, W, sample_clocks, name):
     """W warm-up + K timed steps on device-resident inputs: CUDA events on the launching stream, barrier +
-    synchronize on both sides, max over ranks.  Returns (total_ms, per-step latencies, launches per step, clocks)."""
+    synchronize on both sides, max over ranks.  Returns (total_ms, per-step latencies, launches per step, clocks);
+    the actions of the last timed step go to `ctx.outputs[name + "_actions"]`."""
     import torch
     model, dev = ctx.model, ctx.dev
     clocks = None
@@ -238,9 +261,10 @@ def timed_device_loop(ctx, ring, K, W, sample_clocks):
         evs = [torch.cuda.Event(enable_timing=True) for _ in range(K + 1)]
         evs[0].record()
         for i in range(K):
-            ctx.step(ring[i % len(ring)])
+            actions = ctx.step(ring[i % len(ring)])
             evs[i + 1].record()
         ctx.barrier()
+        ctx.outputs[name + "_actions"] = actions
         if sampler:
             # a short timed region ends before nvidia-smi has sampled it a few times: keep the same load
             # running (untimed) until there are enough samples of the clocks under this workload
@@ -293,7 +317,7 @@ def leg_latency(ctx, K, W, headline):
     args, cfg, world, rank = ctx.args, ctx.cfg, ctx.world, ctx.rank
     B = args.batch
     ring = make_ring(cfg, B, min(args.ring, max(K, 1)), ctx.dev, seed=1234 + rank)
-    total_ms, lat, launches, clocks = timed_device_loop(ctx, ring, K, W, sample_clocks=headline)
+    total_ms, lat, launches, clocks = timed_device_loop(ctx, ring, K, W, sample_clocks=headline, name="latency")
     wl = "bridge_bs1_blurr_preset_50step_episode (BASELINE.json configs[1])"
     if args.robot == "fractal" or args.flow_steps != 1:
         wl = f"{args.robot}_bs1_{args.flow_steps}_flow_steps (BASELINE.json configs[2])"
@@ -421,7 +445,7 @@ def leg_batched(ctx, K, W, headline):
         ring.append({k: v.to(dev) for k, v in local.items()})
         if s == 0:
             check_inputs = glob
-    total_ms, lat, launches, clocks = timed_device_loop(ctx, ring, K, W, sample_clocks=headline)
+    total_ms, lat, launches, clocks = timed_device_loop(ctx, ring, K, W, sample_clocks=headline, name="batched")
     value = world * Bb * HORIZON * K / (total_ms / 1e3)
     flops = ALG_FLOPS_STEP * Bb * K / (total_ms / 1e3) / 1e12          # per GPU
     res = {"workload": "bridge_bs64_per_gpu_episode_sharded (BASELINE.json configs[3])", "episodes_per_gpu": Bb,
@@ -483,10 +507,8 @@ def run_ours(args):
             legs["batched"] = leg_batched(ctx, args.batched_steps or 10, 3, headline=False)
         head = legs["latency"]
     else:
-        # the batched step is ~80 ms: cap the timed steps so that the run stays within minutes at any --steps
-        Kb = min(K, 50)
-        legs["batched"] = leg_batched(ctx, Kb, W, headline=True)
-        legs["latency"] = leg_latency(ctx, min(K, 100), W, headline=False)
+        legs["batched"] = leg_batched(ctx, K, W, headline=True)
+        legs["latency"] = leg_latency(ctx, K, W, headline=False)
         head = legs["batched"]
 
     line = {
@@ -524,6 +546,8 @@ def run_ours(args):
     if rank == 0 and world == 1 and not args.no_cpu_baseline:
         line["cpu_baseline"] = cpu_baseline(ctx.cfg, ctx.model, warm=1, timed=2)
     if rank == 0:
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, ctx.outputs)
         print(json.dumps(line), flush=True)
     if world > 1:
         import torch.distributed as dist
@@ -544,7 +568,7 @@ def run_openvla(args):
     peaks = measured_peaks()
     cfg = openvla.openvla_7b_config()
     prompt, n_new = 1 + 256 + 24, 7
-    K, W = min(args.steps, 50), max(args.warmup, 3)
+    K, W = args.steps, max(args.warmup, 3)
     dec = openvla.LlamaDecoder(cfg, dev, max_batch=32)
     g = torch.Generator(device=dev)
     g.manual_seed(0)
@@ -574,7 +598,7 @@ def run_openvla(args):
                        torch.zeros(n_out, device=dev, dtype=torch.bfloat16))
     fused = openvla.FusedVisionBackbone(dino, sig, proj)
     n_text = prompt - 1 - 256
-    out = {}
+    out, outputs = {}, {}
     for B in (1, 32):
         ring = [(torch.randn((B, prompt, cfg.hidden), device=dev, generator=g) * 0.5).to(torch.bfloat16) for _ in range(4)]
         host = [r.cpu().pin_memory() for r in ring]
@@ -624,10 +648,11 @@ def run_openvla(args):
             evs = [torch.cuda.Event(enable_timing=True) for _ in range(K + 1)]
             evs[0].record()
             for i in range(K):
-                dec.generate(ring[i % 4], n)
+                ids = dec.generate(ring[i % 4], n)
                 evs[i + 1].record()
             torch.cuda.synchronize()
             dec.check()
+            outputs[f"bs{B}_{label}_token_ids"] = ids
             lat = sorted(evs[i].elapsed_time(evs[i + 1]) for i in range(K))
             res[label] = {"ms_p50": lat[len(lat) // 2], "ms_mean": evs[0].elapsed_time(evs[K]) / K, "launches": dec.last_launch_count}
             if sampler:
@@ -679,6 +704,8 @@ def run_openvla(args):
         "parity": "pinned against transformers 5.5 LlamaForCausalLM (tests/test_gpu_llm.py); unpinned against the reference's remote code",
         "openvla": out,
     }
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, outputs)
     print(json.dumps(line), flush=True)
     dec.close()
     return 0
@@ -833,7 +860,7 @@ def run_reference(args):
     `__graft_entry__.build()` ships in the git-ignored `baseline/_ref/` on the GPU box) it is the thing timed
     (`kind: "reference"`): `PiZeroInference` imported through `oracle/ref_harness.py`, called exactly like
     `scripts/benchmark_pi0.py:238-242`.  Otherwise its pinned restatement, the oracle (`kind: "port"`).
-    fp32 on all host cores, bs=1, the same synthetic inputs every step, mean over the timed steps (bounded to 150 s)."""
+    fp32 on all host cores, bs=1, the same synthetic inputs every step, mean over the timed steps."""
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
@@ -859,24 +886,20 @@ def run_reference(args):
         except Exception as exc:       # a broken shipped copy must not take the arm down: fall back to the port
             print(f"reference import failed ({type(exc).__name__}: {exc}); timing the port", file=sys.stderr)
     W = max(1, min(args.warmup, 2))
-    budget_s = 150.0
     ts = []
     with torch.inference_mode():
         for _ in range(W):
             call()
-        t_begin = time.perf_counter()
         for _ in range(args.steps):
             t0 = time.perf_counter()
-            call()
+            actions = call()
             ts.append(time.perf_counter() - t0)
-            if time.perf_counter() - t_begin > budget_s:
-                break
     sec = statistics.fmean(ts)
     value = HORIZON / sec
     what = ("the unmodified reference PiZeroInference (" + ref_harness.REF_ROOT + ")") if kind == "reference" else \
         "the oracle port of the reference's op sequence (reference tree not reachable)"
-    sample = (f"{what}: {len(ts)} of {args.steps} requested full-size Bridge control steps (bs=1, fp32, {args.flow_steps} flow "
-              f"step, identical inputs every step, mean) after {W} warm-up, bounded to {budget_s:.0f} s; torch {torch.__version__}, "
+    sample = (f"{what}: {len(ts)} full-size Bridge control steps (bs=1, fp32, {args.flow_steps} flow "
+              f"step, identical inputs every step, mean) after {W} warm-up; torch {torch.__version__}, "
               f"{cores} threads")
     line = {
         "impl": "reference", "metric": "pi0_bridge_actions_per_sec", "value": value, "unit": "actions/s",
@@ -890,6 +913,8 @@ def run_reference(args):
         "e2e": {"value": value, "unit": "actions/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
         "gpu_launches": 0,
     }
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"reference_actions": actions})
     print(json.dumps(line), flush=True)
 
 

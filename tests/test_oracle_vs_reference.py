@@ -1,6 +1,6 @@
-"""Pins the oracle (`oracle/pi0_oracle.py`) against the *unmodified reference* imported from
-/root/reference (only present in the build container; skipped elsewhere — the committed golden
-vectors in tests/golden/ carry the same check to other machines)."""
+"""Pins the oracle (`oracle/pi0_oracle.py`) against the *unmodified reference*, imported from the source tree
+that `oracle/ref_harness.py` finds (`BLURR_REF_ROOT`); skipped without it — the committed golden vectors in
+tests/golden/ carry the infer_action part of the check to other machines."""
 
 import pytest
 import torch
@@ -11,7 +11,7 @@ from oracle import pi0_oracle as O
 from oracle import ref_harness
 
 pytestmark = pytest.mark.skipif(not ref_harness.reference_available(),
-                                reason="/root/reference not present on this machine")
+                                reason="reference source not found (set BLURR_REF_ROOT)")
 
 
 def _ref_model(cfg, sd, dtype):
