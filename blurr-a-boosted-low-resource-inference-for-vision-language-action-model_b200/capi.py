@@ -159,6 +159,14 @@ _SIGNATURES = [
     ("blurr_mlp_destroy", None, [C.c_void_p]),
     ("blurr_mlp_set_weight", C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]),
     ("blurr_mlp_forward", C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_int, C.c_void_p, C.c_int]),
+    ("blurr_vla_preproc_create", C.c_int,
+     [C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_float),
+      C.POINTER(C.c_float), C.POINTER(C.c_void_p)]),
+    ("blurr_vla_preproc_destroy", None, [C.c_void_p]),
+    ("blurr_vla_preproc_frame", C.c_int,
+     [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int, C.c_int64, C.c_void_p, C.c_void_p]),
+    ("blurr_vla_preproc_build_coeffs", C.c_int,
+     [C.c_int, C.c_int, C.POINTER(C.c_int32), C.POINTER(C.c_int32), C.c_int]),
 ]
 DECLARED_SYMBOLS = [s[0] for s in _SIGNATURES]
 

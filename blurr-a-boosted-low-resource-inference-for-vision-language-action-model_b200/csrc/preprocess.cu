@@ -12,8 +12,15 @@
 //             one kernel (one CTA per output row, the 8 source rows staged in shared memory).
 //  * proprio: normalize_bound / normalize_gaussian in float64 (env_adapter/base.py:8-18,33-40),
 //             float32 (simpler.py:93-95), then bfloat16 (eval.py:194).
-// Both kernels are pure bandwidth/latency work (a 640x480 frame is 0.9 MB): no tensor cores.
+//  * OpenVLA frame: uint8 HWC camera frame -> Pillow `Image.resize(BICUBIC)` (what torchvision's resize does to a
+//             PIL image) -> center crop -> per-tower fp32 `to_tensor` / `normalize` -> bf16, written as the
+//             [3 * n_norms][crop_h][crop_w] pixel_values of the fused DINOv2 + SigLIP backbone.  The resize is
+//             Pillow's fixed-point resample (libImaging/Resample.c: precompute_coeffs in double,
+//             normalize_coeffs_8bpc with PRECISION_BITS = 22, a horizontal then a vertical pass, each only when
+//             its dimension changes, each rounding to uint8); only the cropped window is computed.
+// All three kernels are pure bandwidth/latency work (a 640x480 frame is 0.9 MB): no tensor cores.
 #include "blurr_pi0.h"
+#include "blurr_vit.h"
 #include "common.cuh"
 
 #include <algorithm>
@@ -167,7 +174,165 @@ __global__ void normalize_proprio_kernel(const double* raw, const double* lo, co
     out[i] = __float2bfloat16_rn(static_cast<float>(y));      // float64 -> float32 -> bf16, as the reference
 }
 
+// ------------------------------------------------------------------------------------------------------------------
+// OpenVLA: Pillow bicubic resize + center crop + per-tower normalisation
+// ------------------------------------------------------------------------------------------------------------------
+constexpr int kPrecisionBits = 22;                 // Resample.c PRECISION_BITS
+constexpr int kVlaMaxSize = 1 << 15;               // any side of the source or the resize
+constexpr int kVlaMaxNorms = 2;
+constexpr int kVlaBandRows = 8;                    // output rows per CTA (fewer when the staged rows would not fit)
+constexpr int kVlaMaxSmem = 200 * 1024;
+constexpr int kVlaThreads = 256;
+
+// Resample.c bicubic_filter, a = -0.5
+double bicubic_filter(double x) {
+    const double a = -0.5;
+    if (x < 0.0) x = -x;
+    if (x < 1.0) return ((a + 2.0) * x - (a + 3.0)) * x * x + 1;
+    if (x < 2.0) return (((x - 5) * x + 8) * x - 4) * a;
+    return 0.0;
+}
+
+// Resample.c precompute_coeffs (box = the whole axis) + normalize_coeffs_8bpc, operation for operation in double.
+// bounds: [out][2] = (first source index, tap count); weights: [out][ksize], zero past the tap count.  Returns ksize.
+int pillow_bicubic_coeffs(int in_size, int out_size, std::vector<int32_t>* bounds, std::vector<int32_t>* weights) {
+    const double scale = static_cast<double>(in_size) / out_size;
+    const double filterscale = scale < 1.0 ? 1.0 : scale;
+    const double support = 2.0 * filterscale;
+    const int ksize = static_cast<int>(std::ceil(support)) * 2 + 1;
+    bounds->assign(static_cast<size_t>(out_size) * 2, 0);
+    weights->assign(static_cast<size_t>(out_size) * ksize, 0);
+    std::vector<double> k(ksize);
+    for (int xx = 0; xx < out_size; ++xx) {
+        const double center = (xx + 0.5) * scale;
+        const double ss = 1.0 / filterscale;
+        int xmin = static_cast<int>(center - support + 0.5);
+        if (xmin < 0) xmin = 0;
+        int xmax = static_cast<int>(center + support + 0.5);
+        if (xmax > in_size) xmax = in_size;
+        xmax -= xmin;
+        double ww = 0.0;
+        for (int x = 0; x < xmax; ++x) {
+            const double w = bicubic_filter((x + xmin - center + 0.5) * ss);
+            k[x] = w;
+            ww += w;
+        }
+        for (int x = 0; x < xmax; ++x) {
+            if (ww != 0.0) k[x] /= ww;
+            (*weights)[static_cast<size_t>(xx) * ksize + x] = k[x] < 0 ? static_cast<int32_t>(-0.5 + k[x] * (1 << kPrecisionBits))
+                                                                       : static_cast<int32_t>(0.5 + k[x] * (1 << kPrecisionBits));
+        }
+        (*bounds)[2 * xx] = xmin;
+        (*bounds)[2 * xx + 1] = xmax;
+    }
+    return ksize;
+}
+
+// The kernel's table for one axis: Pillow's coefficients for output indices [first, first + count) of an `in -> out`
+// resize, or, when in == out (Pillow skips that pass), the identity: one tap of weight 1.0, which reproduces the
+// source byte exactly ((v << 22) + (1 << 21)) >> 22 = v.
+int axis_table(int in_size, int out_size, int first, int count, std::vector<int32_t>* bounds, std::vector<int32_t>* weights) {
+    if (in_size == out_size) {
+        bounds->resize(static_cast<size_t>(count) * 2);
+        weights->assign(count, 1 << kPrecisionBits);
+        for (int i = 0; i < count; ++i) { (*bounds)[2 * i] = first + i; (*bounds)[2 * i + 1] = 1; }
+        return 1;
+    }
+    std::vector<int32_t> b, w;
+    const int ksize = pillow_bicubic_coeffs(in_size, out_size, &b, &w);
+    bounds->assign(b.begin() + 2 * static_cast<size_t>(first), b.begin() + 2 * static_cast<size_t>(first + count));
+    weights->assign(w.begin() + static_cast<size_t>(first) * ksize, w.begin() + static_cast<size_t>(first + count) * ksize);
+    return ksize;
+}
+
+struct VlaArgs {
+    const uint8_t* frame; long long row_stride, frame_stride;
+    int crop_h, crop_w, kx, ky, band_rows, n_norms;
+    const int32_t *x_bounds, *x_weights, *y_bounds, *y_weights;    // crop-window slices of the two axis tables
+    float mean[3 * kVlaMaxNorms], stdev[3 * kVlaMaxNorms];
+    bf16* pixel_values;        // [batch][3 * n_norms][crop_h][crop_w]
+    uint8_t* resized;          // [batch][crop_h][crop_w][3] or nullptr
+};
+
+__device__ __forceinline__ int clip8(int acc) {
+    acc >>= kPrecisionBits;
+    return acc < 0 ? 0 : (acc > 255 ? 255 : acc);
+}
+
+// One CTA = one band of output rows of one frame.  The horizontal pass runs over the source rows the band's vertical
+// windows cover, for the crop's columns only, into shared memory as uint8 (Pillow rounds between the passes); the
+// vertical pass then reads those rows.  Pillow accumulates in int32 from 1 << 21; the sums stay below 2^31 (255 times
+// the absolute weight sum, at most ~1.2 * 2^22).
+__global__ void __launch_bounds__(kVlaThreads) resize_bicubic_crop_normalize_kernel(const VlaArgs a) {
+    extern __shared__ __align__(16) uint8_t hrows[];      // [span][crop_w * 3]
+    const int b = blockIdx.y;
+    const int r0 = blockIdx.x * a.band_rows;
+    const int r1 = min(r0 + a.band_rows, a.crop_h);
+    const int y0 = __ldg(a.y_bounds + 2 * r0);
+    const int span = __ldg(a.y_bounds + 2 * (r1 - 1)) + __ldg(a.y_bounds + 2 * (r1 - 1) + 1) - y0;   // windows are monotonic
+    const int row_bytes = a.crop_w * 3;
+    const uint8_t* src = a.frame + static_cast<long long>(b) * a.frame_stride;
+    for (int i = threadIdx.x; i < span * a.crop_w; i += blockDim.x) {
+        const int j = i / a.crop_w, c = i - j * a.crop_w;
+        const int xmin = __ldg(a.x_bounds + 2 * c), n = __ldg(a.x_bounds + 2 * c + 1);
+        const int32_t* w = a.x_weights + static_cast<size_t>(c) * a.kx;
+        const uint8_t* p = src + static_cast<long long>(y0 + j) * a.row_stride + xmin * 3;
+        int s0 = 1 << (kPrecisionBits - 1), s1 = s0, s2 = s0;
+        for (int k = 0; k < n; ++k) {
+            const int wk = __ldg(w + k);
+            s0 += static_cast<int>(__ldg(p + 3 * k)) * wk;
+            s1 += static_cast<int>(__ldg(p + 3 * k + 1)) * wk;
+            s2 += static_cast<int>(__ldg(p + 3 * k + 2)) * wk;
+        }
+        uint8_t* d = hrows + j * row_bytes + c * 3;
+        d[0] = static_cast<uint8_t>(clip8(s0));
+        d[1] = static_cast<uint8_t>(clip8(s1));
+        d[2] = static_cast<uint8_t>(clip8(s2));
+    }
+    __syncthreads();
+    const size_t plane = static_cast<size_t>(a.crop_h) * a.crop_w;
+    for (int i = threadIdx.x; i < (r1 - r0) * a.crop_w; i += blockDim.x) {
+        const int r = r0 + i / a.crop_w, c = i % a.crop_w;
+        const int ymin = __ldg(a.y_bounds + 2 * r) - y0, n = __ldg(a.y_bounds + 2 * r + 1);
+        const int32_t* w = a.y_weights + static_cast<size_t>(r) * a.ky;
+        const uint8_t* p = hrows + ymin * row_bytes + c * 3;
+        int s0 = 1 << (kPrecisionBits - 1), s1 = s0, s2 = s0;
+        for (int k = 0; k < n; ++k) {
+            const int wk = __ldg(w + k);
+            s0 += static_cast<int>(p[k * row_bytes]) * wk;
+            s1 += static_cast<int>(p[k * row_bytes + 1]) * wk;
+            s2 += static_cast<int>(p[k * row_bytes + 2]) * wk;
+        }
+        const int v[3] = {clip8(s0), clip8(s1), clip8(s2)};
+        if (a.resized != nullptr) {
+            uint8_t* d = a.resized + ((static_cast<size_t>(b) * a.crop_h + r) * a.crop_w + c) * 3;
+            d[0] = static_cast<uint8_t>(v[0]); d[1] = static_cast<uint8_t>(v[1]); d[2] = static_cast<uint8_t>(v[2]);
+        }
+        // TVF.to_tensor: fp32 v / 255 (a true division); TVF.normalize: (x - mean) / std in fp32; then .to(bfloat16)
+        float f[3];
+#pragma unroll
+        for (int ch = 0; ch < 3; ++ch) f[ch] = __fdiv_rn(static_cast<float>(v[ch]), 255.0f);
+        bf16* out = a.pixel_values + static_cast<size_t>(b) * 3 * a.n_norms * plane + static_cast<size_t>(r) * a.crop_w + c;
+#pragma unroll
+        for (int m = 0; m < kVlaMaxNorms; ++m) {
+            if (m >= a.n_norms) break;
+#pragma unroll
+            for (int ch = 0; ch < 3; ++ch)
+                out[(3 * m + ch) * plane] = __float2bfloat16_rn(__fdiv_rn(__fsub_rn(f[ch], a.mean[3 * m + ch]), a.stdev[3 * m + ch]));
+        }
+    }
+}
+
 }  // namespace
+
+struct blurr_vla_preproc {
+    int device = 0;
+    int src_h = 0, src_w = 0, crop_h = 0, crop_w = 0, n_norms = 0;
+    int kx = 0, ky = 0, band_rows = 0, smem = 0;
+    int32_t* tables = nullptr;                        // device: x_bounds | x_weights | y_bounds | y_weights
+    size_t x_weights_at = 0, y_bounds_at = 0, y_weights_at = 0;
+    float mean[3 * kVlaMaxNorms] = {}, stdev[3 * kVlaMaxNorms] = {};
+};
 
 extern "C" int blurr_preproc_create(int device, int src_h, int src_w, int dst_h, int dst_w, blurr_preproc_t** out) {
     if (!out) return blurr::fail(BLURR_ERR_INVALID, "preproc_create: null out");
@@ -245,6 +410,107 @@ extern "C" int blurr_preproc_frame(blurr_preproc_t* p, void* cuda_stream, const 
     resize_lanczos4_normalize_kernel<<<dim3(p->dst_h, batch), 256, smem, static_cast<cudaStream_t>(cuda_stream)>>>(a);
     const cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return blurr::fail(BLURR_ERR_CUDA, std::string("preproc_frame launch failed: ") + cudaGetErrorString(e));
+    return 0;
+}
+
+extern "C" int blurr_vla_preproc_build_coeffs(int in_size, int out_size, int32_t* bounds, int32_t* weights, int max_taps) {
+    if (in_size < 1 || out_size < 1 || in_size > kVlaMaxSize || out_size > kVlaMaxSize)
+        return blurr::fail(BLURR_ERR_INVALID, "vla_preproc_build_coeffs: sizes must be in 1..32768");
+    std::vector<int32_t> b, w;
+    const int ksize = pillow_bicubic_coeffs(in_size, out_size, &b, &w);
+    if (bounds == nullptr && weights == nullptr) return ksize;              // query the tap count
+    if (bounds == nullptr || weights == nullptr || max_taps < ksize)
+        return blurr::fail(BLURR_ERR_INVALID, "vla_preproc_build_coeffs: null table or max_taps below the tap count");
+    std::copy(b.begin(), b.end(), bounds);
+    for (int o = 0; o < out_size; ++o)
+        for (int k = 0; k < max_taps; ++k)
+            weights[static_cast<size_t>(o) * max_taps + k] = k < ksize ? w[static_cast<size_t>(o) * ksize + k] : 0;
+    return ksize;
+}
+
+extern "C" int blurr_vla_preproc_create(int device, int src_h, int src_w, int resize_h, int resize_w, int crop_top,
+                                        int crop_left, int crop_h, int crop_w, int n_norms, const float* mean,
+                                        const float* stdev, blurr_vla_preproc_t** out) {
+    if (!out) return blurr::fail(BLURR_ERR_INVALID, "vla_preproc_create: null out");
+    *out = nullptr;
+    for (int s : {src_h, src_w, resize_h, resize_w, crop_h, crop_w})
+        if (s < 1 || s > kVlaMaxSize) return blurr::fail(BLURR_ERR_INVALID, "vla_preproc_create: sizes must be in 1..32768");
+    if (crop_top < 0 || crop_left < 0 || crop_top + crop_h > resize_h || crop_left + crop_w > resize_w)
+        return blurr::fail(BLURR_ERR_INVALID, "vla_preproc_create: the crop lies outside the resized image");
+    if (n_norms < 1 || n_norms > kVlaMaxNorms)
+        return blurr::fail(BLURR_ERR_INVALID, "vla_preproc_create: n_norms must be 1 or 2");
+    if (!mean || !stdev) return blurr::fail(BLURR_ERR_INVALID, "vla_preproc_create: null mean or std");
+    for (int i = 0; i < 3 * n_norms; ++i)
+        if (!(stdev[i] != 0.0f) || !std::isfinite(stdev[i]) || !std::isfinite(mean[i]))
+            return blurr::fail(BLURR_ERR_INVALID, "vla_preproc_create: mean and std must be finite and std non-zero");
+    std::vector<int32_t> xb, xw, yb, yw;
+    const int kx = axis_table(src_w, resize_w, crop_left, crop_w, &xb, &xw);
+    const int ky = axis_table(src_h, resize_h, crop_top, crop_h, &yb, &yw);
+    // staged source rows of the widest band: the first row of its first window to the last row of its last window
+    int band_rows = kVlaBandRows;
+    long long smem = 0;
+    for (; band_rows >= 1; band_rows /= 2) {
+        long long span = 0;
+        for (int r0 = 0; r0 < crop_h; r0 += band_rows) {
+            const int r1 = std::min(r0 + band_rows, crop_h) - 1;
+            span = std::max<long long>(span, yb[2 * r1] + yb[2 * r1 + 1] - yb[2 * r0]);
+        }
+        smem = span * crop_w * 3;
+        if (smem <= kVlaMaxSmem) break;
+    }
+    if (band_rows < 1)
+        return blurr::fail(BLURR_ERR_INVALID, "vla_preproc_create: one output row's source window is too large for shared memory");
+    int n_dev = 0;
+    if (cudaGetDeviceCount(&n_dev) != cudaSuccess || n_dev <= 0)
+        return blurr::fail(BLURR_ERR_CUDA, "no CUDA device: the preprocessing path has no CPU fallback");
+    if (device < 0 || device >= n_dev) return blurr::fail(BLURR_ERR_INVALID, "vla_preproc_create: bad device index");
+    if (cudaSetDevice(device) != cudaSuccess) return blurr::fail(BLURR_ERR_CUDA, "cudaSetDevice failed");
+    blurr_vla_preproc* p = new blurr_vla_preproc();
+    p->device = device; p->src_h = src_h; p->src_w = src_w; p->crop_h = crop_h; p->crop_w = crop_w; p->n_norms = n_norms;
+    p->kx = kx; p->ky = ky; p->band_rows = band_rows; p->smem = static_cast<int>(smem);
+    std::copy(mean, mean + 3 * n_norms, p->mean);
+    std::copy(stdev, stdev + 3 * n_norms, p->stdev);
+    std::vector<int32_t> all(xb);
+    p->x_weights_at = all.size(); all.insert(all.end(), xw.begin(), xw.end());
+    p->y_bounds_at = all.size(); all.insert(all.end(), yb.begin(), yb.end());
+    p->y_weights_at = all.size(); all.insert(all.end(), yw.begin(), yw.end());
+    bool ok = cudaMalloc(&p->tables, all.size() * sizeof(int32_t)) == cudaSuccess &&
+              cudaMemcpy(p->tables, all.data(), all.size() * sizeof(int32_t), cudaMemcpyHostToDevice) == cudaSuccess;
+    if (ok && smem > 48 * 1024)
+        ok = cudaFuncSetAttribute(resize_bicubic_crop_normalize_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, p->smem) == cudaSuccess;
+    if (!ok) {
+        blurr_vla_preproc_destroy(p);
+        return blurr::fail(BLURR_ERR_CUDA, "vla_preproc_create: device allocation failed");
+    }
+    *out = p;
+    return 0;
+}
+
+extern "C" void blurr_vla_preproc_destroy(blurr_vla_preproc_t* p) {
+    if (!p) return;
+    cudaFree(p->tables);
+    delete p;
+}
+
+extern "C" int blurr_vla_preproc_frame(blurr_vla_preproc_t* p, void* cuda_stream, const void* frames_u8,
+                                       int64_t row_stride_bytes, int batch, int64_t frame_stride_bytes,
+                                       void* pixel_values_bf16, void* resized_u8) {
+    if (!p || !frames_u8 || !pixel_values_bf16) return blurr::fail(BLURR_ERR_INVALID, "vla_preproc_frame: null argument");
+    if (batch < 1 || batch > 65535 || row_stride_bytes < static_cast<int64_t>(p->src_w) * 3)
+        return blurr::fail(BLURR_ERR_INVALID, "vla_preproc_frame: batch must be in 1..65535 and the row stride >= 3 * width");
+    if (cudaSetDevice(p->device) != cudaSuccess) return blurr::fail(BLURR_ERR_CUDA, "cudaSetDevice failed");
+    VlaArgs a{};
+    a.frame = static_cast<const uint8_t*>(frames_u8); a.row_stride = row_stride_bytes; a.frame_stride = frame_stride_bytes;
+    a.crop_h = p->crop_h; a.crop_w = p->crop_w; a.kx = p->kx; a.ky = p->ky; a.band_rows = p->band_rows; a.n_norms = p->n_norms;
+    a.x_bounds = p->tables; a.x_weights = p->tables + p->x_weights_at;
+    a.y_bounds = p->tables + p->y_bounds_at; a.y_weights = p->tables + p->y_weights_at;
+    std::copy(p->mean, p->mean + 3 * kVlaMaxNorms, a.mean);
+    std::copy(p->stdev, p->stdev + 3 * kVlaMaxNorms, a.stdev);
+    a.pixel_values = static_cast<bf16*>(pixel_values_bf16); a.resized = static_cast<uint8_t*>(resized_u8);
+    const dim3 grid((p->crop_h + p->band_rows - 1) / p->band_rows, batch);
+    resize_bicubic_crop_normalize_kernel<<<grid, kVlaThreads, p->smem, static_cast<cudaStream_t>(cuda_stream)>>>(a);
+    const cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) return blurr::fail(BLURR_ERR_CUDA, std::string("vla_preproc_frame launch failed: ") + cudaGetErrorString(e));
     return 0;
 }
 

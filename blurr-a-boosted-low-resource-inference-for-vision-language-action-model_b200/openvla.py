@@ -1,4 +1,4 @@
-"""OpenVLA-7B-shaped path (SURVEY.md §8(f) row 3, BASELINE.json configs[4]): the language-model half.
+"""OpenVLA-7B-shaped path (SURVEY.md §8(f) row 3, BASELINE.json configs[4]), from the camera frame to the actions.
 
 The reference has no source for this model — `scripts/benchmark_hf_vla.py:100-109` loads `openvla/openvla-7b` with
 `trust_remote_code=True` and times `model.predict_action(**inputs, unnorm_key=..., do_sample=False)` (:141-197).
@@ -6,18 +6,24 @@ That call (public Prismatic/OpenVLA architecture) runs the fused SigLIP+DINOv2 b
 `[BOS] + 256 patch embeddings + prompt tokens`, and lets a `LlamaForCausalLM` generate `action_dim` = 7 tokens greedily
 with a KV cache; each token is mapped to one of 256 uniform bins on [-1, 1] and de-normalised with q01/q99.
 
-Built here: the Llama-2-7B-shaped decoder (`LlamaDecoder`, csrc/llm_engine.cu behind include/blurr_llm.h) — prefill of
-the multimodal prompt embeddings + greedy decode — and the action de-tokeniser (`ActionDetokenizer`).  NOT built: the
-fused vision backbone and projector (the caller supplies the projected patch embeddings; the benchmark uses random ones
-of the right shape — at 7B the vision tower is ~5 % of the step's weight bytes).  PARITY: the decoder is pinned against
-transformers' `LlamaForCausalLM` (eager attention) in tests/test_gpu_llm.py; against the reference's remote code it is
-UNPINNED (not vendored, not downloadable)."""
+Built here, all on the device:
+  * `ImagePreprocessor` — the processor's bicubic resize, center crop and the two per-tower normalisations
+    (csrc/preprocess.cu behind include/blurr_vit.h), bit-exact against Pillow + torchvision;
+  * `VitEncoder` x 2 + `MlpProjector` = `FusedVisionBackbone` — DINOv2 and SigLIP towers and the projector
+    (csrc/vit_engine.cu behind include/blurr_vit.h);
+  * `LlamaDecoder` — the Llama-2-7B-shaped decoder (csrc/llm_engine.cu behind include/blurr_llm.h): prefill of the
+    multimodal prompt embeddings + greedy decode;
+  * `ActionDetokenizer` (host) and `OpenVlaPolicy`, which chains them: `predict_action(frames, input_ids, q01, q99)`.
+Not built: tokenisation of the instruction (the caller passes `input_ids`).  PARITY: the towers are pinned against
+transformers (tests/test_gpu_vit.py), the decoder against `LlamaForCausalLM` with eager attention
+(tests/test_gpu_llm.py), the preprocessing against Pillow + torchvision (tests/test_openvla_preprocess.py); against
+the reference's remote code all of it is UNPINNED (not vendored, not downloadable)."""
 
 from __future__ import annotations
 
 import ctypes as C
 from dataclasses import dataclass
-from typing import Dict, Optional, Tuple
+from typing import Dict, Optional, Sequence, Tuple, Union
 
 import numpy as np
 import torch
@@ -453,3 +459,147 @@ class FusedVisionBackbone:
             pixel_values_siglip.record_stream(self._side)
             feats.record_stream(self._side)
         return self.projector.forward(feats)
+
+
+# ---------------------------------------------------------------------------------------------------------------------
+# Image preprocessing (include/blurr_vit.h: blurr_vla_preproc_*) and the whole policy
+# ---------------------------------------------------------------------------------------------------------------------
+DINOV2_MEAN, DINOV2_STD = (0.485, 0.456, 0.406), (0.229, 0.224, 0.225)     # ImageNet, timm's DINOv2 data config
+SIGLIP_MEAN, SIGLIP_STD = (0.5, 0.5, 0.5), (0.5, 0.5, 0.5)
+
+
+def resize_geometry(h: int, w: int, size: Union[int, Sequence[int]] = 224,
+                    crop: Union[int, Sequence[int]] = 224) -> Tuple[int, int, int, int]:
+    """(resize_h, resize_w, crop_top, crop_left) of `TVF.center_crop(TVF.resize(img, size), crop)` on an h x w image.
+    An int `size` becomes the shorter side, the longer one `int(size * long / short)`; an `(h, w)` tuple is the exact
+    output shape (OpenVLA's "resize-naive").  Crop offsets are `int(round((H - crop) / 2.0))`, half to even."""
+    if isinstance(size, int):
+        short, long = (w, h) if w <= h else (h, w)
+        new_short, new_long = size, int(size * long / short)
+        rw, rh = (new_short, new_long) if w <= h else (new_long, new_short)
+    else:
+        rh, rw = int(size[0]), int(size[1])
+    ch, cw = (crop, crop) if isinstance(crop, int) else (int(crop[0]), int(crop[1]))
+    if ch > rh or cw > rw:
+        raise ValueError(f"crop {(ch, cw)} is larger than the resized image {(rh, rw)} (torchvision would pad: not supported)")
+    return rh, rw, int(round((rh - ch) / 2.0)), int(round((rw - cw) / 2.0))
+
+
+def pillow_bicubic_coefficients(in_size: int, out_size: int) -> Tuple[np.ndarray, np.ndarray]:
+    """Pillow's bicubic tables for one axis, from the library's host-side builder: bounds int32 [out, 2] = (first
+    source index, tap count) and weights int32 [out, ksize] in Q22."""
+    lib = capi.load_library()
+    ksize = capi.check(lib.blurr_vla_preproc_build_coeffs(in_size, out_size, None, None, 0))
+    bounds = np.zeros((out_size, 2), np.int32)
+    weights = np.zeros((out_size, ksize), np.int32)
+    capi.check(lib.blurr_vla_preproc_build_coeffs(in_size, out_size, bounds.ctypes.data_as(C.POINTER(C.c_int32)),
+                                                  weights.ctypes.data_as(C.POINTER(C.c_int32)), ksize))
+    return bounds, weights
+
+
+class ImagePreprocessor:
+    """OpenVLA's `PrismaticImageProcessor` for one frame geometry, on the device: Pillow bicubic resize, center crop,
+    and one `to_tensor` + `normalize` per tower, stacked channel-wise ([DINOv2 RGB, SigLIP RGB]) in bf16."""
+
+    def __init__(self, src_h: int, src_w: int, size: Union[int, Sequence[int]] = 224, crop: Union[int, Sequence[int]] = 224,
+                 means: Sequence[Sequence[float]] = (DINOV2_MEAN, SIGLIP_MEAN),
+                 stds: Sequence[Sequence[float]] = (DINOV2_STD, SIGLIP_STD), device="cuda:0"):
+        self.device = torch.device(device)
+        if self.device.type != "cuda":
+            raise RuntimeError("ImagePreprocessor runs on a CUDA device only (no CPU fallback)")
+        if len(means) != len(stds) or any(len(m) != 3 for m in means) or any(len(s) != 3 for s in stds):
+            raise ValueError("means and stds must be equally many RGB triples")
+        self.src_h, self.src_w = int(src_h), int(src_w)
+        self.resize_h, self.resize_w, self.crop_top, self.crop_left = resize_geometry(self.src_h, self.src_w, size, crop)
+        self.crop_h, self.crop_w = (crop, crop) if isinstance(crop, int) else (int(crop[0]), int(crop[1]))
+        self.n_norms = len(means)
+        mean = (C.c_float * (3 * self.n_norms))(*[float(v) for m in means for v in m])
+        std = (C.c_float * (3 * self.n_norms))(*[float(v) for s in stds for v in s])
+        self.lib = capi.load_library()
+        index = self.device.index if self.device.index is not None else torch.cuda.current_device()
+        handle = C.c_void_p()
+        capi.check(self.lib.blurr_vla_preproc_create(index, self.src_h, self.src_w, self.resize_h, self.resize_w,
+                                                     self.crop_top, self.crop_left, self.crop_h, self.crop_w, self.n_norms,
+                                                     mean, std, C.byref(handle)))
+        self.handle = handle
+
+    def coefficients(self):
+        """((x_bounds, x_weights), (y_bounds, y_weights)): Pillow's tables for the whole resize of each axis.  An axis
+        whose size does not change is not resampled (Pillow skips that pass), whatever its table says."""
+        return (pillow_bicubic_coefficients(self.src_w, self.resize_w), pillow_bicubic_coefficients(self.src_h, self.resize_h))
+
+    def __call__(self, frames_u8: torch.Tensor, out: Optional[torch.Tensor] = None, return_resized: bool = False):
+        """frames_u8: CUDA uint8 [H, W, 3] or [B, H, W, 3]; rows and frames may be strided.  Returns bf16 pixel_values
+        [B, 3 * n_norms, crop_h, crop_w]; with `return_resized` also the cropped uint8 resize [B, crop_h, crop_w, 3]."""
+        if frames_u8.dtype != torch.uint8 or frames_u8.device != self.device:
+            raise ValueError("frames must be uint8 tensors on the preprocessor's device")
+        if frames_u8.dim() == 3:
+            frames_u8 = frames_u8[None]
+        if frames_u8.dim() != 4 or tuple(frames_u8.shape[1:]) != (self.src_h, self.src_w, 3):
+            raise ValueError(f"frame geometry {tuple(frames_u8.shape)} != [B, {self.src_h}, {self.src_w}, 3]")
+        if frames_u8.stride(3) != 1 or frames_u8.stride(2) != 3:
+            frames_u8 = frames_u8.contiguous()
+        B = frames_u8.shape[0]
+        shape = (B, 3 * self.n_norms, self.crop_h, self.crop_w)
+        if out is None:
+            out = torch.empty(shape, device=self.device, dtype=torch.bfloat16)
+        elif tuple(out.shape) != shape or out.dtype != torch.bfloat16 or out.device != self.device or not out.is_contiguous():
+            raise ValueError(f"out must be a contiguous bf16 tensor {shape} on the preprocessor's device")
+        resized = (torch.empty((B, self.crop_h, self.crop_w, 3), device=self.device, dtype=torch.uint8)
+                   if return_resized else None)
+        capi.check(self.lib.blurr_vla_preproc_frame(
+            self.handle, C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream), C.c_void_p(frames_u8.data_ptr()),
+            frames_u8.stride(1), B, frames_u8.stride(0), C.c_void_p(out.data_ptr()),
+            C.c_void_p(resized.data_ptr()) if resized is not None else None))
+        return (out, resized) if return_resized else out
+
+    def close(self):
+        if getattr(self, "handle", None):
+            self.lib.blurr_vla_preproc_destroy(self.handle)
+            self.handle = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+
+class OpenVlaPolicy:
+    """OpenVLA's `predict_action` from raw camera frames: device preprocessing -> DINOv2 + SigLIP towers (fed the two
+    halves of one 6-channel pixel tensor as strided views) -> projector -> `[BOS] + patches + prompt` -> greedy
+    decode of `action_dim` tokens -> de-tokenised, de-normalised actions."""
+
+    def __init__(self, preprocessor: ImagePreprocessor, backbone: FusedVisionBackbone, decoder: LlamaDecoder,
+                 detokenizer: Optional[ActionDetokenizer] = None, action_dim: int = 7):
+        if preprocessor.n_norms != 2:
+            raise ValueError("the fused backbone needs two normalisations (DINOv2's, then SigLIP's)")
+        if (preprocessor.crop_h, preprocessor.crop_w) != (backbone.dino.cfg.image_size,) * 2:
+            raise ValueError("the preprocessor's crop must match the towers' image size")
+        self.preprocessor, self.backbone, self.decoder = preprocessor, backbone, decoder
+        self.detokenizer = detokenizer if detokenizer is not None else ActionDetokenizer()
+        self.action_dim = action_dim
+
+    def pixel_values(self, frames) -> torch.Tensor:
+        """uint8 frame(s) [H, W, 3] / [B, H, W, 3], on the device or on the host (copied over as they are) ->
+        bf16 [B, 6, 224, 224]."""
+        f = torch.as_tensor(frames)
+        if f.dim() == 3:
+            f = f[None]
+        if not f.is_cuda:
+            f = f.to(self.preprocessor.device)
+        return self.preprocessor(f)
+
+    def predict_action_from_pixels(self, pixel_values: torch.Tensor, input_ids: torch.Tensor, q01, q99, mask=None,
+                                   return_token_ids: bool = False):
+        """The same as `predict_action`, from prepared bf16 pixel values [B, 6, 224, 224]."""
+        patch = self.backbone.forward(pixel_values[:, :3], pixel_values[:, 3:])
+        ids = self.decoder.generate(build_prompt_embeds(self.decoder, input_ids, patch), self.action_dim)
+        tokens = ids.cpu().numpy()
+        actions = torch.from_numpy(self.detokenizer.actions(tokens[:, -self.action_dim:], q01, q99, mask))
+        return (actions, ids) if return_token_ids else actions
+
+    def predict_action(self, frames, input_ids: torch.Tensor, q01, q99, mask=None, return_token_ids: bool = False):
+        """frames: uint8 [H, W, 3] or [B, H, W, 3] RGB; input_ids [B, S] (first column BOS).  Returns float64 actions
+        [B, action_dim] on the host (and the int64 token ids [B, action_dim] on the device with `return_token_ids`)."""
+        return self.predict_action_from_pixels(self.pixel_values(frames), input_ids, q01, q99, mask, return_token_ids)

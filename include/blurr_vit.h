@@ -67,6 +67,29 @@ void blurr_mlp_destroy(blurr_mlp_t* h);
 int blurr_mlp_set_weight(blurr_mlp_t* h, int layer, const void* weight_dev, const void* bias_dev);   /* [out][in], [out] */
 int blurr_mlp_forward(blurr_mlp_t* h, void* cuda_stream, int rows, const void* x, int ldx, void* y, int ldy);
 
+/* Image preprocessing of OpenVLA's `PrismaticImageProcessor`, on the device: uint8 RGB frame -> Pillow
+ * `Image.resize((resize_w, resize_h), BICUBIC)` (torchvision's resize of a PIL image) -> crop of crop_h x crop_w at
+ * (crop_top, crop_left) -> for each of `n_norms` normalisations: fp32 v / 255, (x - mean) / std -> bf16.  Bit-exact
+ * against Pillow + torchvision (tests/test_openvla_preprocess.py).  Only the cropped window is computed.
+ * mean / std: host float[3 * n_norms], one RGB triple per normalisation (DINOv2's, then SigLIP's).  Sizes are 1..32768;
+ * create rejects a crop outside the resize, n_norms outside 1..2, a zero std, and geometries whose source rows for one
+ * output row do not fit in shared memory. */
+typedef struct blurr_vla_preproc blurr_vla_preproc_t;
+int blurr_vla_preproc_create(int device, int src_h, int src_w, int resize_h, int resize_w, int crop_top, int crop_left,
+                             int crop_h, int crop_w, int n_norms, const float* mean, const float* std,
+                             blurr_vla_preproc_t** out);
+void blurr_vla_preproc_destroy(blurr_vla_preproc_t* h);
+/* frames_u8: [batch] frames of src_h rows of src_w RGB pixels, `row_stride_bytes` (>= 3 * src_w) between rows and
+ * `frame_stride_bytes` between frames.  pixel_values_bf16: [batch][3 * n_norms][crop_h][crop_w]; resized_u8 (or NULL):
+ * [batch][crop_h][crop_w][3], the cropped uint8 resize.  Asynchronous on `cuda_stream`. */
+int blurr_vla_preproc_frame(blurr_vla_preproc_t* h, void* cuda_stream, const void* frames_u8, int64_t row_stride_bytes,
+                            int batch, int64_t frame_stride_bytes, void* pixel_values_bf16, void* resized_u8);
+/* Host only, no device needed: Pillow's bicubic coefficients for one axis of an in_size -> out_size resize.
+ * Returns ksize, the taps per output index, or a negative status.  With bounds and weights both NULL it only returns
+ * ksize; otherwise bounds gets int32 [out_size][2] = (first source index, tap count) and weights int32
+ * [out_size][max_taps] in Q22 (zero past the tap count), and max_taps must be >= ksize. */
+int blurr_vla_preproc_build_coeffs(int in_size, int out_size, int32_t* bounds, int32_t* weights, int max_taps);
+
 #ifdef __cplusplus
 }
 #endif
