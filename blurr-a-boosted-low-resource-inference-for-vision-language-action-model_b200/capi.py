@@ -142,6 +142,8 @@ _SIGNATURES = [
     ("blurr_llm_embed", C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p]),
     ("blurr_llm_generate", C.c_int,
      [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]),
+    ("blurr_llm_generate_ragged", C.c_int,
+     [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.POINTER(C.c_int32), C.c_int, C.c_void_p, C.c_void_p]),
     ("blurr_llm_set_option", C.c_int, [C.c_void_p, C.c_char_p, C.c_int64]),
     ("blurr_llm_check", C.c_int, [C.c_void_p, C.c_void_p]),
     ("blurr_llm_trace_report", C.c_int, [C.c_void_p, C.c_char_p, C.c_size_t]),

@@ -182,6 +182,9 @@ struct MhaAttnArgs {
     float scale;              // head_dim ** -0.5
     bf16* out;                // [B * q_per_sample][n_heads * head_dim]
     unsigned long long* trace;
+    // decode of prompts of different lengths (q_per_sample 1): non-null -> sequence b attends keys 0 .. seq_len[b] + len_off - 1
+    // (n_keys is then the batch's largest count); nullptr -> every sequence attends n_keys keys
+    const int* seq_len; int len_off;
 };
 struct RopeMhaArgs;
 // decode steps of <= 2 waves of (sequence, head) CTAs can do the new token's RoPE + cache append themselves
@@ -199,13 +202,19 @@ struct RopeMhaArgs {
     bf16* q_out;                        // [T][n_heads * head_dim]
     bf16* k_cache; bf16* v_cache; int n_slots;      // [B][n_slots][n_kv_heads * head_dim]
     unsigned long long* trace;
+    // non-null: token t sits at position (and cache slot) seq_len[s] + len_off + t % tokens_per_seq instead (ragged decode)
+    const int* seq_len; int len_off;
 };
 cudaError_t launch_rope_mha(cudaStream_t stream, const RopeMhaArgs& a);
 // rows[i] = table[ids[i]] (token embedding); ids outside [0, vocab) set *err_flag and read row 0
 cudaError_t launch_embed_rows(cudaStream_t stream, const int64_t* ids, int n, const bf16* table, long long vocab, int width,
                               bf16* out, int* err_flag);
-// dst[b] = src[(b * rows_per_seq + row) ] (the last prompt position of every sequence)
-cudaError_t launch_gather_rows(cudaStream_t stream, const bf16* src, int batch, int rows_per_seq, int row, int width, bf16* dst);
+// dst[b] = src[(b * rows_per_seq + row) ] (the last prompt position of every sequence); with `seq_len` the row of sequence b
+// is seq_len[b] - 1 instead of `row`
+cudaError_t launch_gather_rows(cudaStream_t stream, const bf16* src, int batch, int rows_per_seq, int row, int width, bf16* dst,
+                               const int* seq_len = nullptr);
+// x[b][t][:] = 0 for seq_len[b] <= t < rows_per_seq: the pad rows of a ragged prompt batch (device lengths, read at run time)
+cudaError_t launch_zero_pad_rows(cudaStream_t stream, bf16* x, int batch, int rows_per_seq, int width, const int* seq_len);
 // ids[b] = argmax over logits[b][0..vocab) (lowest index among equal maxima, like torch.argmax on CPU)
 cudaError_t launch_argmax_rows(cudaStream_t stream, const bf16* logits, int batch, int ld, int vocab, int64_t* ids,
                                int64_t* ids_copy, int copy_stride);

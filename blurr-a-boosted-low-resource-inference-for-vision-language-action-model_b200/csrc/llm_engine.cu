@@ -79,12 +79,16 @@ struct blurr_llm {
     bf16 *kcache = nullptr, *vcache = nullptr;
     int64_t *ids = nullptr, *out_ids = nullptr;
     int* d_err = nullptr;
+    // per-sequence prompt lengths of a ragged call: the captured kernels read d_lens at replay, so one graph serves every
+    // length vector; h_lens is its pinned staging copy, reused once `lens_copied` says the last upload has left it
+    int *d_lens = nullptr, *h_lens = nullptr;
+    cudaEvent_t lens_copied = nullptr;
     std::set<std::string> seen;
     size_t expected_keys = 0;
     bool finalized = false, use_graph = true;
     int64_t launches = 0, weight_bytes = 0;
     struct GraphEntry { cudaGraph_t graph; cudaGraphExec_t exec; int64_t launches; };
-    std::map<std::tuple<int, int, int, int>, GraphEntry> graphs;
+    std::map<std::tuple<int, int, int, int, int>, GraphEntry> graphs;     // (batch, prompt_len, n_new, logits, ragged)
     // in-graph timeline (option "trace"): every kernel stamps %globaltimer at entry / after its dependency wait / at exit
     bool trace = false;
     unsigned long long* trace_buf = nullptr;
@@ -106,6 +110,8 @@ extern "C" void blurr_llm_destroy(blurr_llm_t* h) {
     cudaDeviceSynchronize();
     for (auto& kv : h->graphs) { cudaGraphExecDestroy(kv.second.exec); cudaGraphDestroy(kv.second.graph); }
     for (void* p : h->allocs) cudaFree(p);
+    if (h->h_lens) cudaFreeHost(h->h_lens);
+    if (h->lens_copied) cudaEventDestroy(h->lens_copied);
     gemm_forget_tensor_maps();
     delete h;
 }
@@ -171,6 +177,10 @@ extern "C" int blurr_llm_create(const blurr_llm_config* cfg, int device, int max
     h->ids = static_cast<int64_t*>(dalloc(h, static_cast<size_t>(max_batch) * 8));
     h->out_ids = static_cast<int64_t*>(dalloc(h, static_cast<size_t>(max_batch) * c.max_positions * 8));
     h->d_err = static_cast<int*>(dalloc(h, 16));
+    h->d_lens = static_cast<int*>(dalloc(h, static_cast<size_t>(max_batch) * 4));
+    if (cudaMallocHost(&h->h_lens, static_cast<size_t>(max_batch) * 4) != cudaSuccess) h->h_lens = nullptr;
+    if (cudaEventCreateWithFlags(&h->lens_copied, cudaEventDisableTiming) != cudaSuccess) h->lens_copied = nullptr;
+    ok &= h->d_lens && h->h_lens && h->lens_copied;
     ok &= h->embed && h->final_norm && h->IN && h->X && h->XN && h->Q && h->AO && h->HM && h->LIN && h->LAST && h->LOGITS &&
           h->LOGITS_ALL && h->ws && h->kcache && h->vcache && h->ids && h->out_ids && h->d_err;
     if (!ok) { blurr_llm_destroy(h); return fail(BLURR_ERR_CUDA, "blurr_llm_create: device allocation failed"); }
@@ -342,8 +352,10 @@ struct Run {
         launched(launch_consumer(st, a), "consumer");
     }
 
-    // One decoder layer over B sequences x Tq new tokens at positions pos0..pos0+Tq-1 (modeling_llama.py LlamaDecoderLayer)
-    void layer(int l, int B, int Tq, int pos0, const bf16* next_norm) {
+    // One decoder layer over B sequences x Tq new tokens at positions pos0..pos0+Tq-1 (modeling_llama.py LlamaDecoderLayer).
+    // `lens` (decode of a ragged batch, Tq == 1): sequence b's token sits at position lens[b] + step - 1 instead and
+    // attends lens[b] + step keys; pos0 is then the batch's largest position.
+    void layer(int l, int B, int Tq, int pos0, const bf16* next_norm, const int* lens = nullptr, int step = 0) {
         const auto& c = h->cfg;
         Layer& L = h->layers[l];
         const int T = B * Tq, QW = c.num_heads * c.head_dim, KVW = c.num_kv_heads * c.head_dim;
@@ -357,11 +369,13 @@ struct Run {
         r.T = T; r.ldp = L.qkv.Nw; r.n_heads = c.num_heads; r.n_kv_heads = c.num_kv_heads; r.head_dim = c.head_dim;
         r.tokens_per_seq = Tq; r.pos0 = pos0; r.cos_table = h->cos_t; r.sin_table = h->sin_t; r.n_pos = h->n_pos;
         r.q_out = h->Q; r.k_cache = h->kcache + cache_off; r.v_cache = h->vcache + cache_off; r.n_slots = c.max_positions;
+        r.seq_len = lens; r.len_off = step - 1;
         // causal multi-head attention over the cache
         MhaAttnArgs m{};
         m.q = h->Q; m.q_per_sample = Tq; m.q_pos0 = pos0; m.k_cache = r.k_cache; m.v_cache = r.v_cache;
         m.n_slots = c.max_positions; m.n_keys = pos0 + Tq; m.batch = B; m.n_heads = c.num_heads; m.n_kv_heads = c.num_kv_heads;
         m.head_dim = c.head_dim; m.scale = static_cast<float>(std::pow(static_cast<double>(c.head_dim), -0.5)); m.out = h->AO;
+        m.seq_len = lens; m.len_off = step;
         const bool fuse = few && Tq == 1 && mha_decode_fuses_rope(m);       // decode: RoPE + append inside the attention kernel
         if (!fuse) {
             r.trace = slot("rope_mha");
@@ -399,7 +413,10 @@ struct Run {
     }
 };
 
-void run_generate(Run& R, int B, int T, int n_new, bool keep_logits) {
+// `ragged`: sequence b's prompt is rows 0 .. d_lens[b] - 1 of its T rows; the rest are pads.  Prefill runs over all T rows
+// unchanged (pads come after the real rows, so the causal mask hides them from every real query); the pads are zeroed
+// first, the first token is read from row d_lens[b] - 1, and decode step i places sequence b's token at d_lens[b] + i - 1.
+void run_generate(Run& R, int B, int T, int n_new, bool keep_logits, bool ragged) {
     blurr_llm* h = R.h;
     const auto& c = h->cfg;
     const int L = c.num_layers;
@@ -408,16 +425,18 @@ void run_generate(Run& R, int B, int T, int n_new, bool keep_logits) {
         if (cudaMemsetAsync(h->trace_buf, 0xFF, static_cast<size_t>(kTraceMax) * 4 * sizeof(unsigned long long), R.st) != cudaSuccess)
             R.rc = fail(BLURR_ERR_CUDA, "trace reset failed");
     }
+    const int* lens = ragged ? h->d_lens : nullptr;
+    if (ragged && !R.rc) R.launched(launch_zero_pad_rows(R.st, h->IN, B, T, c.hidden, lens), "zero_pad_rows");
     // ---- prefill: X <- inputs_embeds, XN <- input norm of layer 0 ----
     R.consumer(0, nullptr, B * T, c.hidden, c.hidden, h->IN, h->X, h->layers[0].in_ln, h->XN);
     for (int l = 0; l < L; ++l) R.layer(l, B, T, 0, l + 1 < L ? h->layers[l + 1].in_ln : h->final_norm);
-    if (!R.rc) R.launched(launch_gather_rows(R.st, h->XN, B, T, T - 1, c.hidden, h->LAST), "gather_last");
+    if (!R.rc) R.launched(launch_gather_rows(R.st, h->XN, B, T, T - 1, c.hidden, h->LAST, lens), "gather_last");
     R.head(h->LAST, B, 0, n_new, keep_logits);
     // ---- greedy decode: one token per sequence per step ----
     for (int i = 1; i < n_new; ++i) {
         if (!R.rc) R.launched(launch_embed_rows(R.st, h->ids, B, h->embed, c.vocab, c.hidden, h->X, h->d_err), "embed");
         R.consumer(0, nullptr, B, c.hidden, c.hidden, h->X, nullptr, h->layers[0].in_ln, h->XN);
-        for (int l = 0; l < L; ++l) R.layer(l, B, 1, T + i - 1, l + 1 < L ? h->layers[l + 1].in_ln : h->final_norm);
+        for (int l = 0; l < L; ++l) R.layer(l, B, 1, T + i - 1, l + 1 < L ? h->layers[l + 1].in_ln : h->final_norm, lens, i);
         R.head(h->XN, B, i, n_new, keep_logits);
     }
 }
@@ -433,29 +452,31 @@ extern "C" int blurr_llm_embed(blurr_llm_t* h, void* cuda_stream, const int64_t*
     return 0;
 }
 
-extern "C" int blurr_llm_generate(blurr_llm_t* h, void* cuda_stream, int batch, int prompt_len, const void* inputs_embeds,
-                                  int n_new, int64_t* out_ids, void* out_logits) {
-    if (!h || !inputs_embeds || !out_ids) return fail(BLURR_ERR_INVALID, "blurr_llm_generate: null argument");
-    if (!h->finalized) return fail(BLURR_ERR_STATE, "blurr_llm_generate: call blurr_llm_finalize first");
+// The body of blurr_llm_generate / blurr_llm_generate_ragged; `lens` (host, validated) selects the ragged schedule.
+static int generate(blurr_llm_t* h, void* cuda_stream, int batch, int prompt_len, const void* inputs_embeds, const int32_t* lens,
+                    int n_new, int64_t* out_ids, void* out_logits) {
     const auto& c = h->cfg;
-    if (batch < 1 || batch > h->max_batch) return fail(BLURR_ERR_INVALID, "blurr_llm_generate: batch out of range");
-    if (prompt_len < 1 || n_new < 1 || prompt_len + n_new > c.max_positions)
-        return fail(BLURR_ERR_INVALID, "blurr_llm_generate: prompt_len + n_new exceeds max_positions");
     LLM_CUDA_TRY(cudaSetDevice(h->device));
     cudaStream_t st = static_cast<cudaStream_t>(cuda_stream);
     const bool keep = out_logits != nullptr;
-    if (keep && n_new > kMaxKeptLogits) return fail(BLURR_ERR_INVALID, "blurr_llm_generate: logits are kept for at most 16 new tokens");
+    const bool ragged = lens != nullptr;
     LLM_CUDA_TRY(cudaMemcpyAsync(h->IN, inputs_embeds, static_cast<size_t>(batch) * prompt_len * c.hidden * 2, cudaMemcpyDeviceToDevice, st));
+    if (ragged) {
+        LLM_CUDA_TRY(cudaEventSynchronize(h->lens_copied));         // the previous upload has read the staging buffer
+        memcpy(h->h_lens, lens, static_cast<size_t>(batch) * 4);
+        LLM_CUDA_TRY(cudaMemcpyAsync(h->d_lens, h->h_lens, static_cast<size_t>(batch) * 4, cudaMemcpyHostToDevice, st));
+        LLM_CUDA_TRY(cudaEventRecord(h->lens_copied, st));
+    }
     h->launches = 0;
     Run R{h, st};
     if (!h->use_graph) {
-        run_generate(R, batch, prompt_len, n_new, keep);
+        run_generate(R, batch, prompt_len, n_new, keep, ragged);
         if (R.rc) return R.rc;
     } else {
-        const auto key = std::make_tuple(batch, prompt_len, n_new, keep ? 1 : 0);
+        const auto key = std::make_tuple(batch, prompt_len, n_new, keep ? 1 : 0, ragged ? 1 : 0);
         auto it = h->graphs.find(key);
         if (it == h->graphs.end()) {
-            run_generate(R, batch, prompt_len, n_new, keep);         // warm run: attribute setup, tensor maps
+            run_generate(R, batch, prompt_len, n_new, keep, ragged);         // warm run: attribute setup, tensor maps
             if (R.rc) return R.rc;
             LLM_CUDA_TRY(cudaStreamSynchronize(st));
             h->launches = 0;
@@ -464,7 +485,7 @@ extern "C" int blurr_llm_generate(blurr_llm_t* h, void* cuda_stream, int batch, 
             Run C{h, cs};
             cudaError_t e = cudaStreamBeginCapture(cs, cudaStreamCaptureModeThreadLocal);
             if (e != cudaSuccess) { cudaStreamDestroy(cs); return fail(BLURR_ERR_CUDA, "graph capture begin failed"); }
-            run_generate(C, batch, prompt_len, n_new, keep);
+            run_generate(C, batch, prompt_len, n_new, keep, ragged);
             cudaGraph_t g = nullptr;
             e = cudaStreamEndCapture(cs, &g);
             cudaStreamDestroy(cs);
@@ -482,6 +503,36 @@ extern "C" int blurr_llm_generate(blurr_llm_t* h, void* cuda_stream, int batch, 
     if (keep)
         LLM_CUDA_TRY(cudaMemcpyAsync(out_logits, h->LOGITS_ALL, static_cast<size_t>(batch) * n_new * c.vocab * 2, cudaMemcpyDeviceToDevice, st));
     return 0;
+}
+
+extern "C" int blurr_llm_generate(blurr_llm_t* h, void* cuda_stream, int batch, int prompt_len, const void* inputs_embeds,
+                                  int n_new, int64_t* out_ids, void* out_logits) {
+    if (!h || !inputs_embeds || !out_ids) return fail(BLURR_ERR_INVALID, "blurr_llm_generate: null argument");
+    if (!h->finalized) return fail(BLURR_ERR_STATE, "blurr_llm_generate: call blurr_llm_finalize first");
+    const auto& c = h->cfg;
+    if (batch < 1 || batch > h->max_batch) return fail(BLURR_ERR_INVALID, "blurr_llm_generate: batch out of range");
+    if (prompt_len < 1 || n_new < 1 || prompt_len + n_new > c.max_positions)
+        return fail(BLURR_ERR_INVALID, "blurr_llm_generate: prompt_len + n_new exceeds max_positions");
+    if (out_logits != nullptr && n_new > kMaxKeptLogits) return fail(BLURR_ERR_INVALID, "blurr_llm_generate: logits are kept for at most 16 new tokens");
+    return generate(h, cuda_stream, batch, prompt_len, inputs_embeds, nullptr, n_new, out_ids, out_logits);
+}
+
+extern "C" int blurr_llm_generate_ragged(blurr_llm_t* h, void* cuda_stream, int batch, int max_prompt_len, const void* inputs_embeds,
+                                         const int32_t* prompt_lens, int n_new, int64_t* out_ids, void* out_logits) {
+    if (!h || !inputs_embeds || !out_ids) return fail(BLURR_ERR_INVALID, "blurr_llm_generate_ragged: null argument");
+    if (!prompt_lens) return fail(BLURR_ERR_INVALID, "blurr_llm_generate_ragged: prompt_lens is null");
+    if (!h->finalized) return fail(BLURR_ERR_STATE, "blurr_llm_generate_ragged: call blurr_llm_finalize first");
+    const auto& c = h->cfg;
+    if (batch < 1 || batch > h->max_batch) return fail(BLURR_ERR_INVALID, "blurr_llm_generate_ragged: batch out of range");
+    if (max_prompt_len < 1 || n_new < 1 || max_prompt_len + n_new > c.max_positions)
+        return fail(BLURR_ERR_INVALID, "blurr_llm_generate_ragged: max_prompt_len + n_new exceeds max_positions");
+    for (int b = 0; b < batch; ++b)
+        if (prompt_lens[b] < 1 || prompt_lens[b] > max_prompt_len)
+            return fail(BLURR_ERR_INVALID, "blurr_llm_generate_ragged: prompt_lens[" + std::to_string(b) + "] = " +
+                                               std::to_string(prompt_lens[b]) + " is outside 1.." + std::to_string(max_prompt_len));
+    if (out_logits != nullptr && n_new > kMaxKeptLogits)
+        return fail(BLURR_ERR_INVALID, "blurr_llm_generate_ragged: logits are kept for at most 16 new tokens");
+    return generate(h, cuda_stream, batch, max_prompt_len, inputs_embeds, prompt_lens, n_new, out_ids, out_logits);
 }
 
 extern "C" int blurr_llm_set_option(blurr_llm_t* h, const char* name, int64_t value) {

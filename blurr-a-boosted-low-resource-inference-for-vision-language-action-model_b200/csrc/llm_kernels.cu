@@ -10,15 +10,16 @@ namespace blurr {
 // HF Llama (modeling_llama.py apply_rotary_pos_emb / rotate_half): with d = head_dim, for j < d/2
 //   y[j]       = bf16(bf16(x[j] * cos[j])       + bf16(-x[j + d/2] * sin[j]))
 //   y[j + d/2] = bf16(bf16(x[j + d/2] * cos[j]) + bf16( x[j]       * sin[j]))
-// (cos/sin are cat(freqs, freqs), cast to the activation dtype).  One thread per 4 rotation pairs.
-__global__ void __launch_bounds__(256) rope_mha_kernel(const RopeMhaArgs a) {
+// (cos/sin are cat(freqs, freqs), cast to the activation dtype).  One thread per 4 rotation pairs.  Three CTAs per SM:
+// left free, ptxas settles at 48 registers and spills loop invariants of the split-K sums to local memory.
+__global__ void __launch_bounds__(256, 3) rope_mha_kernel(const RopeMhaArgs a) {
     trace_stamp(a.trace, 0);
     pdl_wait();
     pdl_trigger();
     trace_stamp(a.trace, 1);
     const int t = blockIdx.x;
     const int seq = t / a.tokens_per_seq, i = t - seq * a.tokens_per_seq;
-    int pos = a.pos0 + i;
+    int pos = (a.seq_len != nullptr ? a.seq_len[seq] + a.len_off : a.pos0) + i;
     if (pos >= a.n_pos) pos = a.n_pos - 1;               // the host validates the range
     const int half = a.head_dim >> 1;
     const int gpr = half >> 2;                            // 4-wide groups per rotated head
@@ -74,7 +75,10 @@ __global__ void __launch_bounds__(256) rope_mha_kernel(const RopeMhaArgs a) {
 // one (sequence, head): with multi-head attention nothing a CTA needs lives in another head), so a decode step has one
 // kernel less per layer: q, k, v of the new token come from the q/k/v GEMM's split-K partials, the new K/V row is written
 // to the cache and used from shared memory as key n - 1.
-template <int HD, bool FUSED>
+// RAGGED: prompts of different lengths - the key count (and with FUSED the new token's position / cache slot) comes from
+// the device length array per sequence.  A template parameter, not a runtime test, so that the equal-length kernels keep
+// their register allocation (the FUSED head_dim-128 kernel sits at ~242 of 255 registers).
+template <int HD, bool FUSED, bool RAGGED>
 __global__ void __launch_bounds__(256, 1) mha_decode_kernel(const MhaAttnArgs a, const RopeMhaArgs r) {
     constexpr int LPK = HD / 8;                 // lanes per key
     constexpr int GROUPS = 256 / LPK;           // keys in flight per pass
@@ -94,7 +98,7 @@ __global__ void __launch_bounds__(256, 1) mha_decode_kernel(const MhaAttnArgs a,
     const size_t row0 = static_cast<size_t>(b) * a.n_slots;
     const bf16* kbase = a.k_cache + row0 * width + h * HD + gl * 8;
     const bf16* vbase = a.v_cache + row0 * width + h * HD + gl * 8;
-    const int n = a.n_keys;
+    const int n = RAGGED ? a.seq_len[b] + a.len_off : a.n_keys;
     const int nload = FUSED ? n - 1 : n;        // FUSED: key n - 1 is the token this step appends
     // every K and V row of this group is requested up front (<= 320 / GROUPS keys per group, 16 bytes each per lane): the
     // kernel is two HBM round trips long instead of one per 4 keys (measured 15 -> 4 us per layer at one sequence)
@@ -124,7 +128,7 @@ __global__ void __launch_bounds__(256, 1) mha_decode_kernel(const MhaAttnArgs a,
             raw[which][d] = bf16_round(acc);
         }
         __syncthreads();
-        int pos = r.pos0;
+        int pos = RAGGED ? r.seq_len[b] + r.len_off : r.pos0;
         if (pos >= r.n_pos) pos = r.n_pos - 1;
         const size_t cache_row = (row0 + pos) * width + h * HD;
         for (int i = threadIdx.x; i < 2 * half + HD; i += 256) {
@@ -228,7 +232,7 @@ __global__ void __launch_bounds__(256, 1) mha_decode_kernel(const MhaAttnArgs a,
 
 // Many sequences (grid > 2 CTAs per SM): the same kernel with 4 keys in flight per group and ~60 registers, so that
 // several CTAs share an SM and hide each other's round trips (measured at 32 sequences: 4.75 vs 5.34 ms per token).
-template <int HD>
+template <int HD, bool RAGGED>
 __global__ void __launch_bounds__(256) mha_decode_loop_kernel(const MhaAttnArgs a) {
     constexpr int LPK = HD / 8;                 // lanes per key
     constexpr int GROUPS = 256 / LPK;           // keys in flight per pass
@@ -254,7 +258,7 @@ __global__ void __launch_bounds__(256) mha_decode_loop_kernel(const MhaAttnArgs 
     const size_t row0 = static_cast<size_t>(b) * a.n_slots;
     const bf16* kbase = a.k_cache + row0 * width + h * HD + gl * 8;
     const bf16* vbase = a.v_cache + row0 * width + h * HD + gl * 8;
-    const int n = a.n_keys;
+    const int n = RAGGED ? a.seq_len[b] + a.len_off : a.n_keys;
     // ---- scores ----
     for (int kfirst = 0; kfirst < n; kfirst += 4 * GROUPS) {      // warp-uniform trip count: the groups of a warp shuffle together
         const int k0 = kfirst + group;
@@ -342,22 +346,29 @@ bool mha_decode_fuses_rope(const MhaAttnArgs& a) {
     return a.q_per_sample == 1 && a.n_heads * a.batch <= 2 * 148 && (a.head_dim == 128 || a.head_dim == 64);
 }
 
-// `rope` != nullptr (only when mha_decode_fuses_rope): the kernel also rotates / appends this step's token (no rope_mha launch)
+template <int HD, bool RAGGED>
+static cudaError_t launch_mha_decode_hd(cudaStream_t stream, const MhaAttnArgs& a, const RopeMhaArgs* rope, bool wide) {
+    const dim3 grid(a.n_heads, a.batch);
+    if (rope != nullptr) return launch_kernel(mha_decode_kernel<HD, true, RAGGED>, grid, dim3(256), 0, stream, a, *rope);
+    const RopeMhaArgs none{};
+    return wide ? launch_kernel(mha_decode_kernel<HD, false, RAGGED>, grid, dim3(256), 0, stream, a, none)
+                : launch_kernel(mha_decode_loop_kernel<HD, RAGGED>, grid, dim3(256), 0, stream, a);
+}
+
+// `rope` != nullptr (only when mha_decode_fuses_rope): the kernel also rotates / appends this step's token (no rope_mha launch).
+// a.seq_len != nullptr selects the ragged kernels; a fused `rope` must then carry the same lengths.
 cudaError_t launch_mha_decode(cudaStream_t stream, const MhaAttnArgs& a, const RopeMhaArgs* rope) {
     if (a.q_per_sample != 1 || a.n_keys > 320 || a.n_kv_heads != a.n_heads) return cudaErrorInvalidValue;
     const bool wide = a.n_heads * a.batch <= 2 * 148;       // few CTAs: every load of a CTA in flight at once
+    const bool ragged = a.seq_len != nullptr;
     if (rope != nullptr) {
         if (!mha_decode_fuses_rope(a) || rope->lin != nullptr || rope->tokens_per_seq != 1) return cudaErrorInvalidValue;
-        if (a.head_dim == 128) return launch_kernel(mha_decode_kernel<128, true>, dim3(a.n_heads, a.batch), dim3(256), 0, stream, a, *rope);
-        return launch_kernel(mha_decode_kernel<64, true>, dim3(a.n_heads, a.batch), dim3(256), 0, stream, a, *rope);
+        if ((rope->seq_len != nullptr) != ragged) return cudaErrorInvalidValue;
     }
-    const RopeMhaArgs none{};
     if (a.head_dim == 128)
-        return wide ? launch_kernel(mha_decode_kernel<128, false>, dim3(a.n_heads, a.batch), dim3(256), 0, stream, a, none)
-                    : launch_kernel(mha_decode_loop_kernel<128>, dim3(a.n_heads, a.batch), dim3(256), 0, stream, a);
+        return ragged ? launch_mha_decode_hd<128, true>(stream, a, rope, wide) : launch_mha_decode_hd<128, false>(stream, a, rope, wide);
     if (a.head_dim == 64)
-        return wide ? launch_kernel(mha_decode_kernel<64, false>, dim3(a.n_heads, a.batch), dim3(256), 0, stream, a, none)
-                    : launch_kernel(mha_decode_loop_kernel<64>, dim3(a.n_heads, a.batch), dim3(256), 0, stream, a);
+        return ragged ? launch_mha_decode_hd<64, true>(stream, a, rope, wide) : launch_mha_decode_hd<64, false>(stream, a, rope, wide);
     return cudaErrorInvalidValue;
 }
 
@@ -390,18 +401,41 @@ cudaError_t launch_embed_rows(cudaStream_t stream, const int64_t* ids, int n, co
     return launch_kernel(embed_rows_kernel, dim3(n), dim3(256), 0, stream, ids, n, table, vocab, width, out, err_flag);
 }
 
-__global__ void __launch_bounds__(256) gather_rows_kernel(const bf16* src, int rows_per_seq, int row, int width, bf16* dst) {
+__global__ void __launch_bounds__(256) gather_rows_kernel(const bf16* src, int rows_per_seq, int row, int width, bf16* dst,
+                                                          const int* seq_len) {
     pdl_wait();
     pdl_trigger();
     const int b = blockIdx.x;
+    if (seq_len != nullptr) row = seq_len[b] - 1;
     const uint4* s = reinterpret_cast<const uint4*>(src + (static_cast<size_t>(b) * rows_per_seq + row) * width);
     uint4* d = reinterpret_cast<uint4*>(dst + static_cast<size_t>(b) * width);
     for (int i = threadIdx.x; i < width / 8; i += blockDim.x) d[i] = s[i];
 }
 
-cudaError_t launch_gather_rows(cudaStream_t stream, const bf16* src, int batch, int rows_per_seq, int row, int width, bf16* dst) {
+cudaError_t launch_gather_rows(cudaStream_t stream, const bf16* src, int batch, int rows_per_seq, int row, int width, bf16* dst,
+                               const int* seq_len) {
     if (width & 7) return cudaErrorInvalidValue;
-    return launch_kernel(gather_rows_kernel, dim3(batch), dim3(256), 0, stream, src, rows_per_seq, row, width, dst);
+    return launch_kernel(gather_rows_kernel, dim3(batch), dim3(256), 0, stream, src, rows_per_seq, row, width, dst, seq_len);
+}
+
+// Pad rows of a ragged prompt batch -> 0 before prefill.  The prefill attention multiplies whole key blocks by P, and a
+// masked key's P = 0 still turns a NaN / Inf value into NaN; with zero inputs every pad row stays a finite function of
+// its sequence's real rows, so nothing the caller left in the pads reaches a real row.  One CTA column per sequence.
+__global__ void __launch_bounds__(256) zero_pad_rows_kernel(bf16* x, int rows_per_seq, int width, const int* seq_len) {
+    pdl_wait();
+    pdl_trigger();
+    const int b = blockIdx.x;
+    int len = seq_len[b];
+    len = len < 0 ? 0 : (len > rows_per_seq ? rows_per_seq : len);      // the host validates the range
+    const size_t n = static_cast<size_t>(rows_per_seq - len) * (width >> 3);
+    uint4* p = reinterpret_cast<uint4*>(x + (static_cast<size_t>(b) * rows_per_seq + len) * width);
+    for (size_t i = static_cast<size_t>(blockIdx.y) * blockDim.x + threadIdx.x; i < n; i += static_cast<size_t>(gridDim.y) * blockDim.x)
+        p[i] = make_uint4(0u, 0u, 0u, 0u);
+}
+
+cudaError_t launch_zero_pad_rows(cudaStream_t stream, bf16* x, int batch, int rows_per_seq, int width, const int* seq_len) {
+    if ((width & 7) || seq_len == nullptr) return cudaErrorInvalidValue;
+    return launch_kernel(zero_pad_rows_kernel, dim3(batch, 4), dim3(256), 0, stream, x, rows_per_seq, width, seq_len);
 }
 
 // One CTA per sequence.  Greedy decoding compares the bf16 logits as fp32 (HF casts the last row to fp32 first); the

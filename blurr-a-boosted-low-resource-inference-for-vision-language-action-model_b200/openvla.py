@@ -14,6 +14,10 @@ Built here, all on the device:
   * `LlamaDecoder` — the Llama-2-7B-shaped decoder (csrc/llm_engine.cu behind include/blurr_llm.h): prefill of the
     multimodal prompt embeddings + greedy decode;
   * `ActionDetokenizer` (host) and `OpenVlaPolicy`, which chains them: `predict_action(frames, input_ids, q01, q99)`.
+A batch may carry instructions of different lengths (`input_ids` as a list, or `[B, S]` with a tokenizer's
+`attention_mask`): `ragged_prompt_ids` packs them, `build_prompt_embeds_ragged` lays out `[BOS] + patches + text_b` with
+pad rows behind it, and `LlamaDecoder.generate(..., prompt_lens=...)` generates every sequence at its own positions, so
+each row gets what it would get alone.
 Not built: tokenisation of the instruction (the caller passes `input_ids`).  PARITY: the towers are pinned against
 transformers (tests/test_gpu_vit.py), the decoder against `LlamaForCausalLM` with eager attention
 (tests/test_gpu_llm.py), the preprocessing against Pillow + torchvision (tests/test_openvla_preprocess.py); against
@@ -117,8 +121,13 @@ class LlamaDecoder:
                                             C.c_void_p(out.data_ptr())))
         return out
 
-    def generate(self, inputs_embeds: torch.Tensor, n_new: int, return_logits: bool = False):
-        """inputs_embeds: bf16 [B, T, hidden] on the device -> int64 [B, n_new] (and bf16 logits [B, n_new, vocab])."""
+    def generate(self, inputs_embeds: torch.Tensor, n_new: int, return_logits: bool = False, prompt_lens=None):
+        """inputs_embeds: bf16 [B, T, hidden] on the device -> int64 [B, n_new] (and bf16 logits [B, n_new, vocab]).
+
+        `prompt_lens` (B ints, 1..T): prompts of different lengths.  Sequence b's prompt is rows 0 .. prompt_lens[b] - 1
+        of `inputs_embeds[b]`; the rows after it are padding and never influence any output.  Its token i is generated
+        at position prompt_lens[b] + i, so each sequence gets what it would get alone.  One CUDA graph per
+        (B, T, n_new) serves every length vector.  None: every sequence is T rows long."""
         if inputs_embeds.dim() != 3 or inputs_embeds.shape[2] != self.cfg.hidden:
             raise ValueError(f"inputs_embeds must be [B, T, {self.cfg.hidden}]")
         if inputs_embeds.dtype != torch.bfloat16 or inputs_embeds.device.type != "cuda":
@@ -128,9 +137,17 @@ class LlamaDecoder:
         ids = torch.empty((B, n_new), device=self.device, dtype=torch.int64)
         logits = torch.empty((B, n_new, self.cfg.vocab), device=self.device, dtype=torch.bfloat16) if return_logits else None
         stream = torch.cuda.current_stream(self.device).cuda_stream
-        capi.check(self.lib.blurr_llm_generate(self.handle, C.c_void_p(stream), B, T, C.c_void_p(x.data_ptr()), n_new,
-                                               C.c_void_p(ids.data_ptr()),
-                                               C.c_void_p(logits.data_ptr()) if logits is not None else None))
+        out_logits = C.c_void_p(logits.data_ptr()) if logits is not None else None
+        if prompt_lens is None:
+            capi.check(self.lib.blurr_llm_generate(self.handle, C.c_void_p(stream), B, T, C.c_void_p(x.data_ptr()), n_new,
+                                                   C.c_void_p(ids.data_ptr()), out_logits))
+        else:
+            lens = np.ascontiguousarray(torch.as_tensor(prompt_lens).cpu().numpy(), dtype=np.int32)
+            if lens.shape != (B,):
+                raise ValueError(f"prompt_lens must hold one length per sequence ({B}), got shape {lens.shape}")
+            capi.check(self.lib.blurr_llm_generate_ragged(self.handle, C.c_void_p(stream), B, T, C.c_void_p(x.data_ptr()),
+                                                          lens.ctypes.data_as(C.POINTER(C.c_int32)), n_new,
+                                                          C.c_void_p(ids.data_ptr()), out_logits))
         return (ids, logits) if return_logits else ids
 
     def check(self):
@@ -166,7 +183,9 @@ class LlamaDecoder:
 
 class ActionDetokenizer:
     """OpenVLA's `predict_action` tail (public modeling_prismatic.py): the last `action_dim` generated ids ->
-    `vocab_size - id` -> bin index -> bin centre on [-1, 1] -> de-normalised with the dataset's q01 / q99 where `mask`."""
+    `vocab_size - id` -> bin index -> bin centre on [-1, 1] -> de-normalised with the dataset's q01 / q99 where `mask`.
+    q01 / q99 / mask are `[action_dim]` (one dataset for the batch) or `[B, action_dim]` (one dataset's statistics per
+    row); they broadcast against the `[B, action_dim]` ids."""
 
     def __init__(self, vocab_size: int = 32000, n_bins: int = 256):
         self.vocab_size = vocab_size
@@ -190,6 +209,67 @@ def build_prompt_embeds(decoder: LlamaDecoder, input_ids: torch.Tensor, patch_em
     input_ids [B, S] (first column BOS), patch_embeds bf16 [B, P, hidden] -> bf16 [B, 1 + P + S - 1, hidden]."""
     tok = decoder.embed(input_ids)
     return torch.cat([tok[:, :1], patch_embeds.to(tok.dtype), tok[:, 1:]], dim=1).contiguous()
+
+
+def ragged_prompt_ids(input_ids, attention_mask: Optional[torch.Tensor] = None) -> Tuple[torch.Tensor, torch.Tensor]:
+    """Prompts of different lengths -> (ids int64 [B, S_max], lengths int64 [B]): row b holds its S_b tokens in columns
+    0 .. S_b - 1 and pad id 0 after them.  `input_ids` is either a list of 1-D id tensors (each starting with BOS) or
+    `[B, S]` with an `attention_mask` whose ones form one contiguous run per row, left- or right-padded (a HF tokenizer's
+    padded batch).  Raises ValueError for an empty row or a mask with a gap.  Runs on the host; the ids keep the
+    device of the input."""
+    if isinstance(input_ids, (list, tuple)):
+        if attention_mask is not None:
+            raise ValueError("attention_mask goes with a [B, S] input_ids tensor, not with a list")
+        if len(input_ids) == 0:
+            raise ValueError("input_ids is an empty list")
+        rows = [torch.as_tensor(r) for r in input_ids]
+        if any(r.dim() != 1 for r in rows):
+            raise ValueError("every prompt in the list must be a 1-D id tensor")
+        lens = torch.tensor([r.numel() for r in rows], dtype=torch.int64)
+        if int(lens.min()) < 1:
+            raise ValueError("empty prompt in input_ids")
+        ids = torch.zeros((len(rows), int(lens.max())), dtype=torch.int64, device=rows[0].device)
+        for b, r in enumerate(rows):
+            ids[b, :r.numel()] = r.to(device=ids.device, dtype=torch.int64)
+        return ids, lens
+    ids = torch.as_tensor(input_ids)
+    if ids.dim() != 2:
+        raise ValueError("input_ids must be a list of 1-D tensors or a [B, S] tensor")
+    if attention_mask is None:
+        if ids.shape[1] < 1:
+            raise ValueError("empty prompt in input_ids")
+        return ids.to(torch.int64), torch.full((ids.shape[0],), ids.shape[1], dtype=torch.int64)
+    m = torch.as_tensor(attention_mask).to("cpu")
+    if tuple(m.shape) != tuple(ids.shape):
+        raise ValueError(f"attention_mask shape {tuple(m.shape)} != input_ids shape {tuple(ids.shape)}")
+    if ((m != 0) & (m != 1)).any():
+        raise ValueError("attention_mask must hold only 0 and 1")
+    m = m.bool()
+    lens = m.sum(dim=1).to(torch.int64)
+    if int(lens.min()) < 1:
+        raise ValueError("empty prompt in input_ids (a row of attention_mask has no ones)")
+    first = m.to(torch.int64).argmax(dim=1)
+    col = torch.arange(ids.shape[1], dtype=torch.int64)
+    run = (col[None] >= first[:, None]) & (col[None] < (first + lens)[:, None])
+    if not torch.equal(run, m):
+        raise ValueError("every row of attention_mask must be one contiguous run of ones (left or right padding)")
+    S = int(lens.max())
+    src = (first[:, None] + col[None, :S]).clamp(max=ids.shape[1] - 1)
+    keep = col[None, :S] < lens[:, None]
+    out = torch.where(keep, ids.to("cpu", torch.int64).gather(1, src), torch.zeros((), dtype=torch.int64))
+    return out.to(ids.device), lens
+
+
+def build_prompt_embeds_ragged(decoder: LlamaDecoder, input_ids: torch.Tensor, text_lens, patch_embeds: torch.Tensor
+                               ) -> Tuple[torch.Tensor, torch.Tensor]:
+    """`build_prompt_embeds` for prompts of different lengths.  input_ids [B, S_max] with row b's S_b tokens first (as
+    `ragged_prompt_ids` returns them, first column BOS), text_lens [B], patch_embeds bf16 [B, P, hidden] ->
+    (bf16 [B, 1 + P + S_max - 1, hidden], int64 prompt lengths 1 + P + (S_b - 1) [B] on the host).  Row b is
+    `[BOS] + patches + text_b`, followed by pad rows, the layout `LlamaDecoder.generate(..., prompt_lens=...)` takes."""
+    lens = torch.as_tensor(text_lens, dtype=torch.int64).cpu()
+    if lens.shape != (input_ids.shape[0],) or int(lens.min()) < 1 or int(lens.max()) > input_ids.shape[1]:
+        raise ValueError("text_lens must hold one length in 1..S_max per row of input_ids")
+    return build_prompt_embeds(decoder, input_ids, patch_embeds), lens + patch_embeds.shape[1]
 
 
 def synthetic_llama_state_dict(cfg: LlamaShapedConfig, device, seed: int = 0, dtype=torch.bfloat16) -> Dict[str, torch.Tensor]:
@@ -590,16 +670,27 @@ class OpenVlaPolicy:
             f = f.to(self.preprocessor.device)
         return self.preprocessor(f)
 
-    def predict_action_from_pixels(self, pixel_values: torch.Tensor, input_ids: torch.Tensor, q01, q99, mask=None,
-                                   return_token_ids: bool = False):
+    def predict_action_from_pixels(self, pixel_values: torch.Tensor, input_ids, q01, q99, mask=None,
+                                   return_token_ids: bool = False, attention_mask: Optional[torch.Tensor] = None):
         """The same as `predict_action`, from prepared bf16 pixel values [B, 6, 224, 224]."""
         patch = self.backbone.forward(pixel_values[:, :3], pixel_values[:, 3:])
-        ids = self.decoder.generate(build_prompt_embeds(self.decoder, input_ids, patch), self.action_dim)
+        if isinstance(input_ids, (list, tuple)) or attention_mask is not None:
+            text, text_lens = ragged_prompt_ids(input_ids, attention_mask)
+            x, lens = build_prompt_embeds_ragged(self.decoder, text.to(self.decoder.device), text_lens, patch)
+            ids = self.decoder.generate(x, self.action_dim, prompt_lens=lens)
+        else:
+            ids = self.decoder.generate(build_prompt_embeds(self.decoder, input_ids, patch), self.action_dim)
         tokens = ids.cpu().numpy()
         actions = torch.from_numpy(self.detokenizer.actions(tokens[:, -self.action_dim:], q01, q99, mask))
         return (actions, ids) if return_token_ids else actions
 
-    def predict_action(self, frames, input_ids: torch.Tensor, q01, q99, mask=None, return_token_ids: bool = False):
-        """frames: uint8 [H, W, 3] or [B, H, W, 3] RGB; input_ids [B, S] (first column BOS).  Returns float64 actions
-        [B, action_dim] on the host (and the int64 token ids [B, action_dim] on the device with `return_token_ids`)."""
-        return self.predict_action_from_pixels(self.pixel_values(frames), input_ids, q01, q99, mask, return_token_ids)
+    def predict_action(self, frames, input_ids, q01, q99, mask=None, return_token_ids: bool = False,
+                       attention_mask: Optional[torch.Tensor] = None):
+        """frames: uint8 [H, W, 3] or [B, H, W, 3] RGB.  input_ids: [B, S] (first column BOS), every row S tokens; or
+        instructions of different lengths, as a list of B 1-D id tensors (each starting with BOS) or as [B, S] with a
+        tokenizer's left- or right-padded `attention_mask` (see `ragged_prompt_ids`).  `mask` is the action mask of
+        the de-normalisation, not a prompt mask.  q01 / q99 / mask: [action_dim], or [B, action_dim] for one dataset's
+        statistics per row.  Returns float64 actions [B, action_dim] on the host (and the int64 token ids
+        [B, action_dim] on the device with `return_token_ids`)."""
+        return self.predict_action_from_pixels(self.pixel_values(frames), input_ids, q01, q99, mask, return_token_ids,
+                                               attention_mask)

@@ -13,6 +13,10 @@
  * PARITY: pinned against transformers 5.5.0 `LlamaForCausalLM` (a library present in this image, not reference source);
  * against the reference itself it is UNPINNED (the remote code is neither vendored nor downloadable), see DESIGN.md.
  *
+ * A batch may mix prompts of different lengths (blurr_llm_generate_ragged): each sequence's prompt sits at the front of
+ * its rows, pads behind it, and its tokens are generated at its own positions, so each sequence gets what it would get
+ * alone; one CUDA graph per batch shape serves every vector of lengths.
+ *
  * All pointers are device pointers unless stated.  Errors: negative blurr_status (blurr_pi0.h), message from
  * blurr_last_error().  One handle per GPU and per host thread.  Weights are bf16.
  */
@@ -58,12 +62,22 @@ int blurr_llm_finalize(blurr_llm_t* h);
 /* rows[i] = embed_tokens[ids[i]]  (bf16 [n][hidden]) */
 int blurr_llm_embed(blurr_llm_t* h, void* cuda_stream, const int64_t* ids, int n, void* rows_out);
 
-/* Greedy generation.  inputs_embeds: bf16 [batch][prompt_len][hidden] (every sequence has the same length, no padding -
- * the benchmark replicates one prompt).  Writes out_ids int64 [batch][n_new]; if out_logits != NULL also the bf16 logits
- * each token was chosen from, [batch][n_new][vocab].  prompt_len + n_new <= max_positions.  The whole call (prefill,
- * n_new - 1 decode steps, argmax) is replayed as one CUDA graph per (batch, prompt_len, n_new). */
+/* Greedy generation.  inputs_embeds: bf16 [batch][prompt_len][hidden] (every sequence has the same length, no padding;
+ * prompts of different lengths go through blurr_llm_generate_ragged).  Writes out_ids int64 [batch][n_new]; if out_logits
+ * != NULL also the bf16 logits each token was chosen from, [batch][n_new][vocab] (n_new <= 16).  prompt_len + n_new <=
+ * max_positions.  The whole call (prefill, n_new - 1 decode steps, argmax) is replayed as one CUDA graph per
+ * (batch, prompt_len, n_new, logits). */
 int blurr_llm_generate(blurr_llm_t* h, void* cuda_stream, int batch, int prompt_len, const void* inputs_embeds, int n_new,
                        int64_t* out_ids, void* out_logits);
+/* Greedy generation over prompts of different lengths, right-aligned: sequence b's prompt is rows 0 .. prompt_lens[b] - 1.
+ * inputs_embeds: bf16 [batch][max_prompt_len][hidden]; rows t >= prompt_lens[b] are ignored (never influence any output:
+ * they are zeroed on the device before the prefill, which runs over all max_prompt_len rows).
+ * prompt_lens: HOST int32 [batch], 1 <= prompt_lens[b] <= max_prompt_len; max_prompt_len + n_new <= max_positions.
+ * Token i of sequence b is generated at position prompt_lens[b] + i, so each sequence gets what it would get alone.
+ * Outputs as blurr_llm_generate.  One CUDA graph per (batch, max_prompt_len, n_new, logits) serves every length vector:
+ * the lengths are uploaded before the launch and read by the kernels at run time. */
+int blurr_llm_generate_ragged(blurr_llm_t* h, void* cuda_stream, int batch, int max_prompt_len, const void* inputs_embeds,
+                              const int32_t* prompt_lens, int n_new, int64_t* out_ids, void* out_logits);
 /* Options: "use_cuda_graph" (default 1), "trace" (default 0: every kernel stamps %globaltimer, see blurr_llm_trace_report). */
 int blurr_llm_set_option(blurr_llm_t* h, const char* name, int64_t value);
 /* Synchronises the stream; reports and clears device-side sticky errors (token id outside the table, expired pipeline wait). */
