@@ -58,6 +58,12 @@ class LlmConfigC(C.Structure):
 LLM_ABI_VERSION = 1
 
 
+class LlmSamplingC(C.Structure):
+    """`blurr_llm_sampling` (include/blurr_llm.h): 24 bytes, seed at 0, temperature 8, top_k 12, top_p 16."""
+
+    _fields_ = [("seed", C.c_uint64), ("temperature", C.c_float), ("top_k", C.c_int32), ("top_p", C.c_float)]
+
+
 class VitConfigC(C.Structure):
     """`blurr_vit_config` (include/blurr_vit.h)."""
 
@@ -144,6 +150,11 @@ _SIGNATURES = [
      [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]),
     ("blurr_llm_generate_ragged", C.c_int,
      [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.POINTER(C.c_int32), C.c_int, C.c_void_p, C.c_void_p]),
+    ("blurr_llm_generate_sampled", C.c_int,
+     [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.POINTER(C.c_int32), C.POINTER(LlmSamplingC), C.c_int, C.c_void_p,
+      C.c_void_p]),
+    ("blurr_llm_sample", C.c_int,
+     [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.POINTER(LlmSamplingC), C.c_int, C.c_void_p, C.c_void_p]),
     ("blurr_llm_set_option", C.c_int, [C.c_void_p, C.c_char_p, C.c_int64]),
     ("blurr_llm_check", C.c_int, [C.c_void_p, C.c_void_p]),
     ("blurr_llm_trace_report", C.c_int, [C.c_void_p, C.c_char_p, C.c_size_t]),

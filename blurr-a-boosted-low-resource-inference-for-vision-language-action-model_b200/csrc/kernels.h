@@ -218,6 +218,19 @@ cudaError_t launch_zero_pad_rows(cudaStream_t stream, bf16* x, int batch, int ro
 // ids[b] = argmax over logits[b][0..vocab) (lowest index among equal maxima, like torch.argmax on CPU)
 cudaError_t launch_argmax_rows(cudaStream_t stream, const bf16* logits, int batch, int ld, int vocab, int64_t* ids,
                                int64_t* ids_copy, int copy_stride);
+// Per-row parameters of the sampler; the layout of `blurr_llm_sampling` (include/blurr_llm.h, checked in llm_engine.cu).
+struct SampleParams {
+    uint64_t seed;
+    float temperature;      // > 0, finite
+    int32_t top_k;          // 0: off
+    float top_p;            // in [0, 1]; 1: off
+};
+// ids[b] = one draw from softmax(top-p(top-k(logits[b][0..vocab) * (1 / T)))), HF's warper order, with Philox4x32-10
+// (key = seed, counter = (step, 0, 0, 0)).  probs != nullptr: probs[b][0..vocab) = the probability each token was drawn
+// with (0 outside the kept set).  A row with no finite positive mass takes the greedy argmax and sets *err_flag |= 2.
+cudaError_t launch_sample_rows(cudaStream_t stream, const bf16* logits, int batch, int ld, int vocab, const SampleParams* params,
+                               int step, int64_t* ids, int64_t* ids_copy, int copy_stride, float* probs, int* err_flag,
+                               unsigned long long* trace);
 // few-token GLU from the split-K partials of a gate/up projection with interleaved rows; act: 0 tanh GELU, 1 SiLU
 cudaError_t launch_glu_partial(cudaStream_t stream, const float* partial, int splitk, int T, int Nw, int act, bf16* out, int ldo,
                                unsigned long long* trace = nullptr);

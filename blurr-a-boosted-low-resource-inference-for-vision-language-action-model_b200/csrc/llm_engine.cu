@@ -14,6 +14,7 @@
 #include "launch.cuh"
 
 #include <cmath>
+#include <cstddef>
 #include <cstdio>
 #include <cstring>
 #include <map>
@@ -30,6 +31,13 @@ int gemm_take_timeout_flag();
 int attn_take_timeout_flag();
 }
 using namespace blurr;
+
+// the device array the sampler reads is the host ABI struct, byte for byte
+static_assert(sizeof(blurr_llm_sampling) == sizeof(SampleParams) && offsetof(blurr_llm_sampling, seed) == offsetof(SampleParams, seed) &&
+                  offsetof(blurr_llm_sampling, temperature) == offsetof(SampleParams, temperature) &&
+                  offsetof(blurr_llm_sampling, top_k) == offsetof(SampleParams, top_k) &&
+                  offsetof(blurr_llm_sampling, top_p) == offsetof(SampleParams, top_p),
+              "blurr_llm_sampling and SampleParams must share one layout");
 
 static int fail(int code, const std::string& msg) { return record_error(code, msg); }
 #define LLM_CUDA_TRY(expr)                                                                       \
@@ -79,16 +87,19 @@ struct blurr_llm {
     bf16 *kcache = nullptr, *vcache = nullptr;
     int64_t *ids = nullptr, *out_ids = nullptr;
     int* d_err = nullptr;
-    // per-sequence prompt lengths of a ragged call: the captured kernels read d_lens at replay, so one graph serves every
-    // length vector; h_lens is its pinned staging copy, reused once `lens_copied` says the last upload has left it
-    int *d_lens = nullptr, *h_lens = nullptr;
-    cudaEvent_t lens_copied = nullptr;
+    // per-row inputs the captured kernels read at replay, so one graph serves every vector of them: the prompt lengths of
+    // a ragged call (d_lens) and the sampling parameters of a sampled one (d_sampling).  h_stage is their pinned staging
+    // copy ([max_batch] parameters, then [max_batch] lengths), reused once `staged` says the last upload has left it.
+    int* d_lens = nullptr;
+    SampleParams* d_sampling = nullptr;
+    unsigned char* h_stage = nullptr;
+    cudaEvent_t staged = nullptr;
     std::set<std::string> seen;
     size_t expected_keys = 0;
     bool finalized = false, use_graph = true;
     int64_t launches = 0, weight_bytes = 0;
     struct GraphEntry { cudaGraph_t graph; cudaGraphExec_t exec; int64_t launches; };
-    std::map<std::tuple<int, int, int, int, int>, GraphEntry> graphs;     // (batch, prompt_len, n_new, logits, ragged)
+    std::map<std::tuple<int, int, int, int, int, int>, GraphEntry> graphs;     // (batch, prompt_len, n_new, logits, ragged, sampled)
     // in-graph timeline (option "trace"): every kernel stamps %globaltimer at entry / after its dependency wait / at exit
     bool trace = false;
     unsigned long long* trace_buf = nullptr;
@@ -110,8 +121,8 @@ extern "C" void blurr_llm_destroy(blurr_llm_t* h) {
     cudaDeviceSynchronize();
     for (auto& kv : h->graphs) { cudaGraphExecDestroy(kv.second.exec); cudaGraphDestroy(kv.second.graph); }
     for (void* p : h->allocs) cudaFree(p);
-    if (h->h_lens) cudaFreeHost(h->h_lens);
-    if (h->lens_copied) cudaEventDestroy(h->lens_copied);
+    if (h->h_stage) cudaFreeHost(h->h_stage);
+    if (h->staged) cudaEventDestroy(h->staged);
     gemm_forget_tensor_maps();
     delete h;
 }
@@ -178,9 +189,10 @@ extern "C" int blurr_llm_create(const blurr_llm_config* cfg, int device, int max
     h->out_ids = static_cast<int64_t*>(dalloc(h, static_cast<size_t>(max_batch) * c.max_positions * 8));
     h->d_err = static_cast<int*>(dalloc(h, 16));
     h->d_lens = static_cast<int*>(dalloc(h, static_cast<size_t>(max_batch) * 4));
-    if (cudaMallocHost(&h->h_lens, static_cast<size_t>(max_batch) * 4) != cudaSuccess) h->h_lens = nullptr;
-    if (cudaEventCreateWithFlags(&h->lens_copied, cudaEventDisableTiming) != cudaSuccess) h->lens_copied = nullptr;
-    ok &= h->d_lens && h->h_lens && h->lens_copied;
+    h->d_sampling = static_cast<SampleParams*>(dalloc(h, static_cast<size_t>(max_batch) * sizeof(SampleParams)));
+    if (cudaMallocHost(&h->h_stage, static_cast<size_t>(max_batch) * (sizeof(SampleParams) + 4)) != cudaSuccess) h->h_stage = nullptr;
+    if (cudaEventCreateWithFlags(&h->staged, cudaEventDisableTiming) != cudaSuccess) h->staged = nullptr;
+    ok &= h->d_lens && h->d_sampling && h->h_stage && h->staged;
     ok &= h->embed && h->final_norm && h->IN && h->X && h->XN && h->Q && h->AO && h->HM && h->LIN && h->LAST && h->LOGITS &&
           h->LOGITS_ALL && h->ws && h->kcache && h->vcache && h->ids && h->out_ids && h->d_err;
     if (!ok) { blurr_llm_destroy(h); return fail(BLURR_ERR_CUDA, "blurr_llm_create: device allocation failed"); }
@@ -398,12 +410,19 @@ struct Run {
         (void)QW;
     }
 
-    // final-normed rows [B][hidden] -> logits -> greedy token `step` of every sequence
-    void head(const bf16* xn_rows, int B, int step, int n_new, bool keep_logits) {
+    // final-normed rows [B][hidden] -> logits -> token `step` of every sequence: greedy, or (`sampled`) drawn with the
+    // per-row parameters in d_sampling
+    void head(const bf16* xn_rows, int B, int step, int n_new, bool keep_logits, bool sampled) {
         const auto& c = h->cfg;
         const int s = gemm(h->lm_head, xn_rows, B, EPI_PARTIAL, nullptr, 0);
         if (!rc) launched(launch_bias_act(st, h->ws, s, B, h->lm_head.Nw, h->lm_head.Nw, nullptr, ACT_NONE, 1.0f, h->LOGITS, h->lm_head.Nw), "logits");
-        if (!rc) launched(launch_argmax_rows(st, h->LOGITS, B, h->lm_head.Nw, c.vocab, h->ids, h->out_ids + step, n_new), "argmax");
+        if (sampled) {
+            unsigned long long* tr = slot("sample_rows");
+            if (!rc) launched(launch_sample_rows(st, h->LOGITS, B, h->lm_head.Nw, c.vocab, h->d_sampling, step, h->ids, h->out_ids + step,
+                                                 n_new, nullptr, h->d_err, tr), "sample_rows");
+        } else if (!rc) {
+            launched(launch_argmax_rows(st, h->LOGITS, B, h->lm_head.Nw, c.vocab, h->ids, h->out_ids + step, n_new), "argmax");
+        }
         if (keep_logits && !rc) {
             const cudaError_t e = cudaMemcpy2DAsync(h->LOGITS_ALL + static_cast<size_t>(step) * c.vocab, static_cast<size_t>(n_new) * c.vocab * 2,
                                                     h->LOGITS, static_cast<size_t>(h->lm_head.Nw) * 2, static_cast<size_t>(c.vocab) * 2, B,
@@ -416,7 +435,7 @@ struct Run {
 // `ragged`: sequence b's prompt is rows 0 .. d_lens[b] - 1 of its T rows; the rest are pads.  Prefill runs over all T rows
 // unchanged (pads come after the real rows, so the causal mask hides them from every real query); the pads are zeroed
 // first, the first token is read from row d_lens[b] - 1, and decode step i places sequence b's token at d_lens[b] + i - 1.
-void run_generate(Run& R, int B, int T, int n_new, bool keep_logits, bool ragged) {
+void run_generate(Run& R, int B, int T, int n_new, bool keep_logits, bool ragged, bool sampled) {
     blurr_llm* h = R.h;
     const auto& c = h->cfg;
     const int L = c.num_layers;
@@ -431,13 +450,13 @@ void run_generate(Run& R, int B, int T, int n_new, bool keep_logits, bool ragged
     R.consumer(0, nullptr, B * T, c.hidden, c.hidden, h->IN, h->X, h->layers[0].in_ln, h->XN);
     for (int l = 0; l < L; ++l) R.layer(l, B, T, 0, l + 1 < L ? h->layers[l + 1].in_ln : h->final_norm);
     if (!R.rc) R.launched(launch_gather_rows(R.st, h->XN, B, T, T - 1, c.hidden, h->LAST, lens), "gather_last");
-    R.head(h->LAST, B, 0, n_new, keep_logits);
-    // ---- greedy decode: one token per sequence per step ----
+    R.head(h->LAST, B, 0, n_new, keep_logits, sampled);
+    // ---- decode: one token per sequence per step ----
     for (int i = 1; i < n_new; ++i) {
         if (!R.rc) R.launched(launch_embed_rows(R.st, h->ids, B, h->embed, c.vocab, c.hidden, h->X, h->d_err), "embed");
         R.consumer(0, nullptr, B, c.hidden, c.hidden, h->X, nullptr, h->layers[0].in_ln, h->XN);
         for (int l = 0; l < L; ++l) R.layer(l, B, 1, T + i - 1, l + 1 < L ? h->layers[l + 1].in_ln : h->final_norm, lens, i);
-        R.head(h->XN, B, i, n_new, keep_logits);
+        R.head(h->XN, B, i, n_new, keep_logits, sampled);
     }
 }
 
@@ -452,31 +471,47 @@ extern "C" int blurr_llm_embed(blurr_llm_t* h, void* cuda_stream, const int64_t*
     return 0;
 }
 
-// The body of blurr_llm_generate / blurr_llm_generate_ragged; `lens` (host, validated) selects the ragged schedule.
+// Uploads the per-row inputs a graph reads at replay (host arrays of `rows` entries, either may be null) through the pinned
+// staging buffer, on `st` ahead of the launch.
+static int stage_rows(blurr_llm_t* h, cudaStream_t st, int rows, const int32_t* lens, const blurr_llm_sampling* params) {
+    if (!lens && !params) return 0;
+    LLM_CUDA_TRY(cudaEventSynchronize(h->staged));              // the previous upload has read the staging buffer
+    unsigned char* stage_params = h->h_stage;
+    unsigned char* stage_lens = h->h_stage + static_cast<size_t>(h->max_batch) * sizeof(SampleParams);
+    if (params) {
+        memcpy(stage_params, params, static_cast<size_t>(rows) * sizeof(SampleParams));
+        LLM_CUDA_TRY(cudaMemcpyAsync(h->d_sampling, stage_params, static_cast<size_t>(rows) * sizeof(SampleParams), cudaMemcpyHostToDevice, st));
+    }
+    if (lens) {
+        memcpy(stage_lens, lens, static_cast<size_t>(rows) * 4);
+        LLM_CUDA_TRY(cudaMemcpyAsync(h->d_lens, stage_lens, static_cast<size_t>(rows) * 4, cudaMemcpyHostToDevice, st));
+    }
+    LLM_CUDA_TRY(cudaEventRecord(h->staged, st));
+    return 0;
+}
+
+// The body of blurr_llm_generate / _ragged / _sampled; `lens` (host, validated) selects the ragged schedule, `params`
+// (host, validated) the sampler.
 static int generate(blurr_llm_t* h, void* cuda_stream, int batch, int prompt_len, const void* inputs_embeds, const int32_t* lens,
-                    int n_new, int64_t* out_ids, void* out_logits) {
+                    const blurr_llm_sampling* params, int n_new, int64_t* out_ids, void* out_logits) {
     const auto& c = h->cfg;
     LLM_CUDA_TRY(cudaSetDevice(h->device));
     cudaStream_t st = static_cast<cudaStream_t>(cuda_stream);
     const bool keep = out_logits != nullptr;
     const bool ragged = lens != nullptr;
+    const bool sampled = params != nullptr;
     LLM_CUDA_TRY(cudaMemcpyAsync(h->IN, inputs_embeds, static_cast<size_t>(batch) * prompt_len * c.hidden * 2, cudaMemcpyDeviceToDevice, st));
-    if (ragged) {
-        LLM_CUDA_TRY(cudaEventSynchronize(h->lens_copied));         // the previous upload has read the staging buffer
-        memcpy(h->h_lens, lens, static_cast<size_t>(batch) * 4);
-        LLM_CUDA_TRY(cudaMemcpyAsync(h->d_lens, h->h_lens, static_cast<size_t>(batch) * 4, cudaMemcpyHostToDevice, st));
-        LLM_CUDA_TRY(cudaEventRecord(h->lens_copied, st));
-    }
+    if (const int rc = stage_rows(h, st, batch, lens, params)) return rc;
     h->launches = 0;
     Run R{h, st};
     if (!h->use_graph) {
-        run_generate(R, batch, prompt_len, n_new, keep, ragged);
+        run_generate(R, batch, prompt_len, n_new, keep, ragged, sampled);
         if (R.rc) return R.rc;
     } else {
-        const auto key = std::make_tuple(batch, prompt_len, n_new, keep ? 1 : 0, ragged ? 1 : 0);
+        const auto key = std::make_tuple(batch, prompt_len, n_new, keep ? 1 : 0, ragged ? 1 : 0, sampled ? 1 : 0);
         auto it = h->graphs.find(key);
         if (it == h->graphs.end()) {
-            run_generate(R, batch, prompt_len, n_new, keep, ragged);         // warm run: attribute setup, tensor maps
+            run_generate(R, batch, prompt_len, n_new, keep, ragged, sampled);         // warm run: attribute setup, tensor maps
             if (R.rc) return R.rc;
             LLM_CUDA_TRY(cudaStreamSynchronize(st));
             h->launches = 0;
@@ -485,7 +520,7 @@ static int generate(blurr_llm_t* h, void* cuda_stream, int batch, int prompt_len
             Run C{h, cs};
             cudaError_t e = cudaStreamBeginCapture(cs, cudaStreamCaptureModeThreadLocal);
             if (e != cudaSuccess) { cudaStreamDestroy(cs); return fail(BLURR_ERR_CUDA, "graph capture begin failed"); }
-            run_generate(C, batch, prompt_len, n_new, keep, ragged);
+            run_generate(C, batch, prompt_len, n_new, keep, ragged, sampled);
             cudaGraph_t g = nullptr;
             e = cudaStreamEndCapture(cs, &g);
             cudaStreamDestroy(cs);
@@ -514,7 +549,7 @@ extern "C" int blurr_llm_generate(blurr_llm_t* h, void* cuda_stream, int batch, 
     if (prompt_len < 1 || n_new < 1 || prompt_len + n_new > c.max_positions)
         return fail(BLURR_ERR_INVALID, "blurr_llm_generate: prompt_len + n_new exceeds max_positions");
     if (out_logits != nullptr && n_new > kMaxKeptLogits) return fail(BLURR_ERR_INVALID, "blurr_llm_generate: logits are kept for at most 16 new tokens");
-    return generate(h, cuda_stream, batch, prompt_len, inputs_embeds, nullptr, n_new, out_ids, out_logits);
+    return generate(h, cuda_stream, batch, prompt_len, inputs_embeds, nullptr, nullptr, n_new, out_ids, out_logits);
 }
 
 extern "C" int blurr_llm_generate_ragged(blurr_llm_t* h, void* cuda_stream, int batch, int max_prompt_len, const void* inputs_embeds,
@@ -532,7 +567,59 @@ extern "C" int blurr_llm_generate_ragged(blurr_llm_t* h, void* cuda_stream, int 
                                                std::to_string(prompt_lens[b]) + " is outside 1.." + std::to_string(max_prompt_len));
     if (out_logits != nullptr && n_new > kMaxKeptLogits)
         return fail(BLURR_ERR_INVALID, "blurr_llm_generate_ragged: logits are kept for at most 16 new tokens");
-    return generate(h, cuda_stream, batch, max_prompt_len, inputs_embeds, prompt_lens, n_new, out_ids, out_logits);
+    return generate(h, cuda_stream, batch, max_prompt_len, inputs_embeds, prompt_lens, nullptr, n_new, out_ids, out_logits);
+}
+
+// HF's checks of the warpers' arguments (TemperatureLogitsWarper, TopKLogitsWarper, TopPLogitsWarper) on the host
+static int check_sampling(const char* fn, const blurr_llm_sampling* params, int rows) {
+    if (!params) return fail(BLURR_ERR_INVALID, std::string(fn) + ": params is null");
+    for (int b = 0; b < rows; ++b) {
+        const blurr_llm_sampling& p = params[b];
+        const std::string at = std::string(fn) + ": params[" + std::to_string(b) + "].";
+        if (!std::isfinite(p.temperature) || !(p.temperature > 0.0f))
+            return fail(BLURR_ERR_INVALID, at + "temperature = " + std::to_string(p.temperature) + " must be finite and > 0");
+        if (p.top_k < 0) return fail(BLURR_ERR_INVALID, at + "top_k = " + std::to_string(p.top_k) + " must be >= 0");
+        if (!std::isfinite(p.top_p) || p.top_p < 0.0f || p.top_p > 1.0f)
+            return fail(BLURR_ERR_INVALID, at + "top_p = " + std::to_string(p.top_p) + " must be in [0, 1]");
+    }
+    return 0;
+}
+
+extern "C" int blurr_llm_generate_sampled(blurr_llm_t* h, void* cuda_stream, int batch, int max_prompt_len, const void* inputs_embeds,
+                                          const int32_t* prompt_lens, const blurr_llm_sampling* params, int n_new, int64_t* out_ids,
+                                          void* out_logits) {
+    const char* fn = "blurr_llm_generate_sampled";
+    if (!h || !inputs_embeds || !out_ids) return fail(BLURR_ERR_INVALID, std::string(fn) + ": null argument");
+    if (!h->finalized) return fail(BLURR_ERR_STATE, std::string(fn) + ": call blurr_llm_finalize first");
+    const auto& c = h->cfg;
+    if (batch < 1 || batch > h->max_batch) return fail(BLURR_ERR_INVALID, std::string(fn) + ": batch out of range");
+    if (max_prompt_len < 1 || n_new < 1 || max_prompt_len + n_new > c.max_positions)
+        return fail(BLURR_ERR_INVALID, std::string(fn) + ": max_prompt_len + n_new exceeds max_positions");
+    if (prompt_lens)
+        for (int b = 0; b < batch; ++b)
+            if (prompt_lens[b] < 1 || prompt_lens[b] > max_prompt_len)
+                return fail(BLURR_ERR_INVALID, std::string(fn) + ": prompt_lens[" + std::to_string(b) + "] = " +
+                                                   std::to_string(prompt_lens[b]) + " is outside 1.." + std::to_string(max_prompt_len));
+    if (out_logits != nullptr && n_new > kMaxKeptLogits)
+        return fail(BLURR_ERR_INVALID, std::string(fn) + ": logits are kept for at most 16 new tokens");
+    if (const int rc = check_sampling(fn, params, batch)) return rc;
+    return generate(h, cuda_stream, batch, max_prompt_len, inputs_embeds, prompt_lens, params, n_new, out_ids, out_logits);
+}
+
+extern "C" int blurr_llm_sample(blurr_llm_t* h, void* cuda_stream, const void* logits, int rows, int ld, const blurr_llm_sampling* params,
+                                int step, int64_t* out_ids, float* out_probs) {
+    const char* fn = "blurr_llm_sample";
+    if (!h || !logits || !out_ids) return fail(BLURR_ERR_INVALID, std::string(fn) + ": null argument");
+    if (rows < 1 || rows > h->max_batch) return fail(BLURR_ERR_INVALID, std::string(fn) + ": rows out of range 1..max_batch");
+    if (ld < h->cfg.vocab) return fail(BLURR_ERR_INVALID, std::string(fn) + ": ld < vocab");
+    if (step < 0) return fail(BLURR_ERR_INVALID, std::string(fn) + ": step < 0");
+    if (const int rc = check_sampling(fn, params, rows)) return rc;
+    LLM_CUDA_TRY(cudaSetDevice(h->device));
+    cudaStream_t st = static_cast<cudaStream_t>(cuda_stream);
+    if (const int rc = stage_rows(h, st, rows, nullptr, params)) return rc;
+    LLM_CUDA_TRY(launch_sample_rows(st, static_cast<const bf16*>(logits), rows, ld, h->cfg.vocab, h->d_sampling, step, out_ids, nullptr, 0,
+                                    out_probs, h->d_err, nullptr));
+    return 0;
 }
 
 extern "C" int blurr_llm_set_option(blurr_llm_t* h, const char* name, int64_t value) {
@@ -560,7 +647,9 @@ extern "C" int blurr_llm_check(blurr_llm_t* h, void* cuda_stream) {
     LLM_CUDA_TRY(cudaMemcpy(&flag, h->d_err, sizeof(int), cudaMemcpyDeviceToHost));
     if (flag) {
         LLM_CUDA_TRY(cudaMemset(h->d_err, 0, sizeof(int)));
-        return fail(BLURR_ERR_INPUT, "a generated token id fell outside the embedding table");
+        if (flag & 1) return fail(BLURR_ERR_INPUT, "a generated token id fell outside the embedding table");
+        return fail(BLURR_ERR_INPUT, "sampling: a logits row had no finite positive mass (all -inf / NaN, a +inf logit, or a scaled "
+                                     "score that overflows); that row took the greedy argmax");
     }
     const int g = gemm_take_timeout_flag(), a = attn_take_timeout_flag();
     if (g > 0 || a > 0) return fail(BLURR_ERR_CUDA, "a bounded pipeline wait expired inside a GEMM / attention kernel");

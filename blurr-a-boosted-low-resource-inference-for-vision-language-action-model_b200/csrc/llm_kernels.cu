@@ -389,7 +389,7 @@ __global__ void __launch_bounds__(256) embed_rows_kernel(const int64_t* ids, int
     pdl_trigger();
     const int r = blockIdx.x;
     long long id = ids[r];
-    if (id < 0 || id >= vocab) { if (threadIdx.x == 0 && err_flag) atomicExch(err_flag, 1); id = 0; }
+    if (id < 0 || id >= vocab) { if (threadIdx.x == 0 && err_flag) atomicOr(err_flag, 1); id = 0; }
     const uint4* src = reinterpret_cast<const uint4*>(table + static_cast<size_t>(id) * width);
     uint4* dst = reinterpret_cast<uint4*>(out + static_cast<size_t>(r) * width);
     for (int i = threadIdx.x; i < width / 8; i += blockDim.x) dst[i] = src[i];
@@ -498,6 +498,403 @@ __global__ void __launch_bounds__(1024) argmax_rows_kernel(const bf16* logits, i
 cudaError_t launch_argmax_rows(cudaStream_t stream, const bf16* logits, int batch, int ld, int vocab, int64_t* ids,
                                int64_t* ids_copy, int copy_stride) {
     return launch_kernel(argmax_rows_kernel, dim3(batch), dim3(1024), 0, stream, logits, ld, vocab, ids, ids_copy, copy_stride);
+}
+
+// ---- sampled decoding (HF `_sample`: fp32 scores, Temperature -> TopK -> TopP warpers, softmax, one draw) ----
+// One CTA per row, deterministic: no float atomics, nothing that depends on scheduling.  For T > 0 the scaled score
+// __fmul_rn(logit, 1 / T) is monotone in the bf16 logit, so the top-k threshold and the top-p cut are found by two
+// 8-bit radix passes over a 16-bit key of the bf16 bits with exact integer counts; masses are exp(s - s_max) rounded
+// to 64-bit fixed point (2^shift per unit, vocab * 2^shift < 2^63), so every histogram and prefix sum is an integer sum
+// whose value does not depend on the order of the atomics.  The row is read from L2 once per pass (at most six passes).
+namespace {
+
+constexpr int kSampleThreads = 1024;
+
+struct SampleShared {
+    unsigned cnt_hi[256], cnt_lo[256], cnt_cut[256];
+    unsigned long long mass_hi[256], mass_cut[256];
+    unsigned long long scan[32];
+    unsigned long long best, z, total, above, z_kept, target;
+    unsigned above_cnt, n_group, n_keep;
+    int bin, thr_key, cut_key, found;
+};
+
+// bf16 bits -> 16-bit key whose unsigned order is the float order; -0 -> +0 (HF counts them as one score); NaN -> -1
+__device__ __forceinline__ int sample_key(uint32_t b) {
+    b &= 0xffffu;
+    if ((b & 0x7fffu) > 0x7f80u) return -1;
+    if (b == 0x8000u) b = 0u;
+    return static_cast<int>((b & 0x8000u) ? (~b & 0xffffu) : (b | 0x8000u));
+}
+
+__device__ __forceinline__ float key_logit(int key) {
+    const uint32_t b = (key & 0x8000) ? (key & 0x7fff) : (~key & 0xffff);
+    return __uint_as_float(b << 16);
+}
+
+// keys of columns 8c .. 8c + 7 (-1 past the end of the row)
+__device__ __forceinline__ void load_keys8(const bf16* row, int vocab, bool vec, int c, int (&k)[8]) {
+    const int i0 = c * 8;
+    if (vec && i0 + 8 <= vocab) {
+        const uint4 q = __ldcg(reinterpret_cast<const uint4*>(row) + c);
+        const uint32_t w[4] = {q.x, q.y, q.z, q.w};
+#pragma unroll
+        for (int e = 0; e < 8; ++e) k[e] = sample_key((e & 1) ? (w[e >> 1] >> 16) : w[e >> 1]);
+    } else {
+        const unsigned short* r = reinterpret_cast<const unsigned short*>(row);
+#pragma unroll
+        for (int e = 0; e < 8; ++e) k[e] = i0 + e < vocab ? sample_key(__ldcg(r + i0 + e)) : -1;
+    }
+}
+
+// Philox4x32-10 (Salmon et al., SC'11; Random123's constants), counter (step, 0, 0, 0), key (seed lo, seed hi): word 0
+__device__ __forceinline__ uint32_t philox_word0(uint64_t seed, uint32_t step) {
+    uint32_t c0 = step, c1 = 0u, c2 = 0u, c3 = 0u;
+    uint32_t k0 = static_cast<uint32_t>(seed), k1 = static_cast<uint32_t>(seed >> 32);
+#pragma unroll
+    for (int r = 0; r < 10; ++r) {
+        const uint32_t hi0 = __umulhi(0xD2511F53u, c0), lo0 = 0xD2511F53u * c0;
+        const uint32_t hi1 = __umulhi(0xCD9E8D57u, c2), lo1 = 0xCD9E8D57u * c2;
+        c0 = hi1 ^ c1 ^ k0; c1 = lo1; c2 = hi0 ^ c3 ^ k1; c3 = lo0;
+        k0 += 0x9E3779B9u; k1 += 0xBB67AE85u;
+    }
+    return c0;
+}
+
+// Warp 0, lane l: bins 8l .. 8l + 7 of a 256-bin histogram; above[e] = base + the sum of every bin above bin 8l + e
+template <typename T>
+__device__ __forceinline__ void bins_above(const T* h, T base, int lane, T (&v)[8], T (&above)[8]) {
+    T sum = 0;
+#pragma unroll
+    for (int e = 0; e < 8; ++e) { v[e] = h[8 * lane + e]; sum += v[e]; }
+    T incl = sum;                                         // over lanes >= lane
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+        const T x = __shfl_down_sync(0xffffffffu, incl, o);
+        if (lane + o < 32) incl += x;
+    }
+    T run = base + incl - sum;
+#pragma unroll
+    for (int e = 7; e >= 0; --e) { above[e] = run; run += v[e]; }
+}
+
+// Warp 0: the largest bin j with above[j] + v[j] >= k (where the k-th largest key lies); `above` of it -> *above_out
+__device__ __forceinline__ int bin_of_kth(const unsigned* h, unsigned base, unsigned k, int lane, unsigned* above_out) {
+    unsigned v[8], above[8];
+    bins_above<unsigned>(h, base, lane, v, above);
+    int cand = -1;
+#pragma unroll
+    for (int e = 0; e < 8; ++e) if (above[e] + v[e] >= k) cand = 8 * lane + e;
+    const int bin = __reduce_max_sync(0xffffffffu, cand);
+#pragma unroll
+    for (int e = 0; e < 8; ++e) if (8 * lane + e == bin) *above_out = above[e];
+    return bin;
+}
+
+// Warp 0: the smallest bin j whose mass above it is < target (the lowest bin top-p keeps anything of)
+__device__ __forceinline__ int bin_of_cut(const unsigned long long* h, unsigned long long base, unsigned long long target, int lane,
+                                          unsigned long long* above_out) {
+    unsigned long long v[8], above[8];
+    bins_above<unsigned long long>(h, base, lane, v, above);
+    int cand = 0x7fffffff;
+#pragma unroll
+    for (int e = 7; e >= 0; --e) if (above[e] < target) cand = 8 * lane + e;
+    const int bin = __reduce_min_sync(0xffffffffu, cand);
+#pragma unroll
+    for (int e = 0; e < 8; ++e) if (8 * lane + e == bin) *above_out = above[e];
+    return bin;
+}
+
+// The first column i (index order) with  sum_{j <= i} w(key_j, j) > target, or -1.  Called by the whole CTA.
+template <class W>
+__device__ int select_first(const bf16* row, int vocab, bool vec, const W& w, unsigned long long target, SampleShared& sh) {
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const int nchunk = (vocab + 7) >> 3;
+    unsigned long long base = 0;
+    if (threadIdx.x == 0) sh.found = -1;
+    for (int r0 = 0; r0 < nchunk; r0 += kSampleThreads) {
+        const int c = r0 + static_cast<int>(threadIdx.x);
+        int k[8];
+        if (c < nchunk) {
+            load_keys8(row, vocab, vec, c, k);
+        } else {
+#pragma unroll
+            for (int e = 0; e < 8; ++e) k[e] = -1;
+        }
+        unsigned long long wv[8], local = 0;
+#pragma unroll
+        for (int e = 0; e < 8; ++e) { wv[e] = k[e] >= 0 ? w(k[e], c * 8 + e) : 0ull; local += wv[e]; }
+        unsigned long long incl = local;
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) {
+            const unsigned long long x = __shfl_up_sync(0xffffffffu, incl, o);
+            if (lane >= o) incl += x;
+        }
+        if (lane == 31) sh.scan[warp] = incl;
+        __syncthreads();
+        if (warp == 0) {
+            const unsigned long long v = sh.scan[lane];
+            unsigned long long s = v;
+#pragma unroll
+            for (int o = 1; o < 32; o <<= 1) {
+                const unsigned long long x = __shfl_up_sync(0xffffffffu, s, o);
+                if (lane >= o) s += x;
+            }
+            sh.scan[lane] = s - v;                        // exclusive prefix of warp `lane`
+            if (lane == 31) sh.total = s;
+        }
+        __syncthreads();
+        const unsigned long long excl = base + sh.scan[warp] + incl - local;
+        if (local > 0 && excl <= target && target - excl < local) {
+            unsigned long long acc = excl;
+            int found = -1;
+#pragma unroll
+            for (int e = 0; e < 8; ++e) { acc += wv[e]; if (found < 0 && acc > target) found = c * 8 + e; }
+            sh.found = found;
+        }
+        base += sh.total;
+        __syncthreads();
+        if (sh.found >= 0) break;
+    }
+    const int f = sh.found;
+    __syncthreads();                                      // the caller may reuse `sh`
+    return f;
+}
+
+}  // namespace
+
+__global__ void __launch_bounds__(kSampleThreads) sample_rows_kernel(const bf16* logits, int ld, int vocab, const SampleParams* params,
+                                                                     int step, int64_t* ids, int64_t* ids_copy, int copy_stride,
+                                                                     float* probs, int* err_flag, unsigned long long* trace) {
+    __shared__ SampleShared sh;
+    trace_stamp(trace, 0);
+    pdl_wait();
+    pdl_trigger();
+    trace_stamp(trace, 1);
+    const int b = blockIdx.x, lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const bf16* row = logits + static_cast<size_t>(b) * ld;
+    const bool vec = (reinterpret_cast<uintptr_t>(row) & 15) == 0;
+    const int nchunk = (vocab + 7) >> 3;
+    const SampleParams prm = params[b];
+    const float inv_t = 1.0f / prm.temperature;          // ATen's `scores / T`: a multiplication by the fp32 reciprocal
+    const int shift = 63 - (32 - __clz(vocab));           // vocab * 2^shift < 2^63: the kept mass fits 63 bits
+    const float unit = __uint_as_float(static_cast<uint32_t>(127 + shift) << 23);      // 2^shift
+    for (int i = threadIdx.x; i < 256; i += kSampleThreads) {
+        sh.cnt_hi[i] = sh.cnt_lo[i] = sh.cnt_cut[i] = 0u;
+        sh.mass_hi[i] = sh.mass_cut[i] = 0ull;
+    }
+    if (threadIdx.x == 0) { sh.best = 0ull; sh.z = 0ull; }
+    __syncthreads();
+
+    // ---- pass 1: the largest key (lowest column among equal ones: the greedy token) and the count of each high byte ----
+    {
+        unsigned long long best = 0ull;
+        int run_bin = -1;
+        unsigned run_n = 0u;
+        for (int c = threadIdx.x; c < nchunk; c += kSampleThreads) {
+            int k[8];
+            load_keys8(row, vocab, vec, c, k);
+#pragma unroll
+            for (int e = 0; e < 8; ++e) {
+                if (k[e] < 0) continue;
+                const unsigned long long packed = (static_cast<unsigned long long>(k[e] + 1) << 32) | static_cast<uint32_t>(~(c * 8 + e));
+                best = packed > best ? packed : best;
+                const int bin = k[e] >> 8;                // adjacent logits mostly share it: one atomic per run
+                if (bin != run_bin) {
+                    if (run_n) atomicAdd(&sh.cnt_hi[run_bin], run_n);
+                    run_bin = bin; run_n = 0u;
+                }
+                ++run_n;
+            }
+        }
+        if (run_n) atomicAdd(&sh.cnt_hi[run_bin], run_n);
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) {
+            const unsigned long long x = __shfl_xor_sync(0xffffffffu, best, o);
+            best = x > best ? x : best;
+        }
+        if (lane == 0) atomicMax(&sh.best, best);
+    }
+    __syncthreads();
+    const int key_max = static_cast<int>(sh.best >> 32) - 1;
+    const int idx_max = key_max < 0 ? 0 : static_cast<int>(~static_cast<uint32_t>(sh.best));
+    const float s_max = key_max < 0 ? __int_as_float(0x7fc00000) : __fmul_rn(key_logit(key_max), inv_t);
+    if (!isfinite(s_max)) {
+        // all NaN / -inf, a +inf logit, or a scaled score that overflows: softmax is undefined -> the greedy token
+        if (threadIdx.x == 0) {
+            ids[b] = idx_max;
+            if (ids_copy != nullptr) ids_copy[static_cast<size_t>(b) * copy_stride] = idx_max;
+            if (err_flag != nullptr) atomicOr(err_flag, 2);
+        }
+        if (probs != nullptr)
+            for (int i = threadIdx.x; i < vocab; i += kSampleThreads) probs[static_cast<size_t>(b) * vocab + i] = 0.f;
+        trace_stamp(trace, 2);
+        return;
+    }
+    auto mass_of = [&](float s) { return __float2ull_rn(expf(__fsub_rn(s, s_max)) * unit); };
+
+    // ---- top-k: the k-th largest key, counting repeats (pass 2: low bytes inside its high byte) ----
+    if (warp == 0) {
+        unsigned v[8], above[8];
+        bins_above<unsigned>(sh.cnt_hi, 0u, lane, v, above);
+        const unsigned n_valid = __shfl_sync(0xffffffffu, above[0] + v[0], 0);
+        const unsigned k = static_cast<unsigned>(prm.top_k);
+        int bin = -1;
+        unsigned ab = 0u;
+        if (prm.top_k > 0 && k < n_valid) bin = bin_of_kth(sh.cnt_hi, 0u, k, lane, &ab);
+        if (bin >= 0 && (lane == (bin >> 3))) sh.above_cnt = ab;
+        if (lane == 0) sh.bin = bin;
+    }
+    __syncthreads();
+    int thr_key = -1;
+    if (sh.bin >= 0) {
+        const int bin = sh.bin;
+        for (int c = threadIdx.x; c < nchunk; c += kSampleThreads) {
+            int k[8];
+            load_keys8(row, vocab, vec, c, k);
+#pragma unroll
+            for (int e = 0; e < 8; ++e)
+                if (k[e] >= 0 && (k[e] >> 8) == bin) atomicAdd(&sh.cnt_lo[k[e] & 255], 1u);
+        }
+        __syncthreads();
+        if (warp == 0) {
+            unsigned ab = 0u;
+            const int lo = bin_of_kth(sh.cnt_lo, sh.above_cnt, static_cast<unsigned>(prm.top_k), lane, &ab);
+            if (lane == 0) sh.thr_key = (bin << 8) | lo;
+        }
+        __syncthreads();
+        thr_key = sh.thr_key;
+    }
+    // every score >= the k-th largest survives (ties at the threshold included; the scaled threshold also admits keys
+    // that scale to the same fp32 value)
+    const float s_thr = thr_key < 0 ? -INFINITY : __fmul_rn(key_logit(thr_key), inv_t);
+
+    // ---- pass 3: the mass Z of the top-k set, and (top-p) the mass of each high byte ----
+    const bool top_p = prm.top_p < 1.0f;
+    {
+        unsigned long long z = 0ull, run_m = 0ull;
+        int run_bin = -1;
+        for (int c = threadIdx.x; c < nchunk; c += kSampleThreads) {
+            int k[8];
+            load_keys8(row, vocab, vec, c, k);
+#pragma unroll
+            for (int e = 0; e < 8; ++e) {
+                if (k[e] < 0) continue;
+                const float s = __fmul_rn(key_logit(k[e]), inv_t);
+                if (!(s >= s_thr)) continue;
+                const unsigned long long m = mass_of(s);
+                z += m;
+                if (top_p) {
+                    const int bin = k[e] >> 8;
+                    if (bin != run_bin) {
+                        if (run_m) atomicAdd(&sh.mass_hi[run_bin], run_m);
+                        run_bin = bin; run_m = 0ull;
+                    }
+                    run_m += m;
+                }
+            }
+        }
+        if (run_m) atomicAdd(&sh.mass_hi[run_bin], run_m);
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) z += __shfl_xor_sync(0xffffffffu, z, o);
+        if (lane == 0) atomicAdd(&sh.z, z);
+    }
+    __syncthreads();
+
+    // ---- top-p: HF keeps a token iff the mass strictly ahead of it in (score, column) descending order is < p * Z, and
+    // always the first one.  The cut group (one key) is found by radix over the masses (pass 4); inside it the columns
+    // are kept from the highest down (torch's stable ascending sort removes the lower columns first) ----
+    int cut_key = -1, idx_cut = 0;
+    unsigned long long z_kept = sh.z;
+    if (top_p) {
+        if (warp == 0) {
+            const unsigned long long target = static_cast<unsigned long long>(ceil(static_cast<double>(prm.top_p) * static_cast<double>(z_kept)));
+            int bin = key_max >> 8;                       // p * Z rounds to 0: only the first token
+            unsigned long long ab = 0ull;
+            if (target > 0ull) bin = bin_of_cut(sh.mass_hi, 0ull, target, lane, &ab);
+            if (target > 0ull && lane == (bin >> 3)) sh.above = ab;
+            if (lane == 0) { sh.bin = bin; sh.target = target; }
+        }
+        __syncthreads();
+        const int bin = sh.bin;
+        for (int c = threadIdx.x; c < nchunk; c += kSampleThreads) {
+            int k[8];
+            load_keys8(row, vocab, vec, c, k);
+#pragma unroll
+            for (int e = 0; e < 8; ++e) {
+                if (k[e] < 0 || (k[e] >> 8) != bin) continue;
+                const float s = __fmul_rn(key_logit(k[e]), inv_t);
+                if (!(s >= s_thr)) continue;
+                atomicAdd(&sh.mass_cut[k[e] & 255], mass_of(s));
+                atomicAdd(&sh.cnt_cut[k[e] & 255], 1u);
+            }
+        }
+        __syncthreads();
+        if (warp == 0) {
+            const unsigned long long target = sh.target;
+            int lo = key_max & 255;
+            unsigned long long ab = 0ull;
+            if (target > 0ull) lo = bin_of_cut(sh.mass_cut, sh.above, target, lane, &ab);
+            if (target > 0ull && lane == (lo >> 3)) sh.above = ab;
+            __syncwarp();
+            if (lane == 0) {
+                const int cut = (bin << 8) | lo;
+                const unsigned long long above = target > 0ull ? sh.above : 0ull;
+                const unsigned long long m = mass_of(__fmul_rn(key_logit(cut), inv_t));
+                const unsigned g = sh.cnt_cut[lo];
+                unsigned keep = 1u;
+                if (target > 0ull) {                      // columns r = 0, 1, .. of the group have above + r * m ahead
+                    const unsigned long long r = m == 0ull ? g : (target - above + m - 1ull) / m;
+                    keep = r < g ? static_cast<unsigned>(r) : g;
+                }
+                sh.cut_key = cut; sh.n_group = g; sh.n_keep = keep;
+                sh.z_kept = above + keep * m;
+            }
+        }
+        __syncthreads();
+        cut_key = sh.cut_key;
+        z_kept = sh.z_kept;
+        const unsigned g = sh.n_group, keep = sh.n_keep;
+        if (keep < g) {                                   // pass 5: the first kept column of the cut group
+            const auto member = [cut_key](int k, int) { return k == cut_key ? 1ull : 0ull; };
+            idx_cut = select_first(row, vocab, vec, member, static_cast<unsigned long long>(g - keep), sh);
+        }
+    }
+
+    // ---- pass 6: the draw, an inverse CDF over the kept set in column order: target = floor(u * Z_kept), u = x / 2^24 ----
+    const uint32_t x = philox_word0(prm.seed, static_cast<uint32_t>(step));
+    const unsigned long long target = __umul64hi(z_kept, static_cast<unsigned long long>(x >> 8) << 40);
+    const auto kept = [&](int k, int i, float s) { return s >= s_thr && k >= cut_key && (k != cut_key || i >= idx_cut); };
+    const auto kept_mass = [&](int k, int i) -> unsigned long long {
+        const float s = __fmul_rn(key_logit(k), inv_t);
+        return kept(k, i, s) ? mass_of(s) : 0ull;
+    };
+    int id = select_first(row, vocab, vec, kept_mass, target, sh);
+    if (id < 0) id = idx_max;                             // unreachable: the kept mass z_kept > target
+    if (threadIdx.x == 0) {
+        ids[b] = id;
+        if (ids_copy != nullptr) ids_copy[static_cast<size_t>(b) * copy_stride] = id;
+    }
+    if (probs != nullptr) {
+        const float zf = static_cast<float>(static_cast<double>(z_kept) * exp2(-static_cast<double>(shift)));
+        const unsigned short* r16 = reinterpret_cast<const unsigned short*>(row);
+        for (int i = threadIdx.x; i < vocab; i += kSampleThreads) {
+            const int k = sample_key(__ldcg(r16 + i));
+            const float s = k >= 0 ? __fmul_rn(key_logit(k), inv_t) : 0.f;
+            float p = 0.f;                                // (a kept token whose fixed-point mass rounds to 0 is never drawn)
+            if (k >= 0 && kept(k, i, s)) p = expf(__fsub_rn(s, s_max)) / zf;
+            probs[static_cast<size_t>(b) * vocab + i] = p;
+        }
+    }
+    trace_stamp(trace, 2);
+}
+
+cudaError_t launch_sample_rows(cudaStream_t stream, const bf16* logits, int batch, int ld, int vocab, const SampleParams* params,
+                               int step, int64_t* ids, int64_t* ids_copy, int copy_stride, float* probs, int* err_flag,
+                               unsigned long long* trace) {
+    if (batch < 1 || vocab < 1 || ld < vocab || params == nullptr || ids == nullptr) return cudaErrorInvalidValue;
+    return launch_kernel(sample_rows_kernel, dim3(batch), dim3(kSampleThreads), 0, stream, logits, ld, vocab, params, step, ids,
+                         ids_copy, copy_stride, probs, err_flag, trace);
 }
 
 // GLU over split-K partials of a few-token gate/up projection whose weight rows alternate gate_j, up_j (the layout of

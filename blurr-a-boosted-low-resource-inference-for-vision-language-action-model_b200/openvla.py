@@ -12,13 +12,16 @@ Built here, all on the device:
   * `VitEncoder` x 2 + `MlpProjector` = `FusedVisionBackbone` — DINOv2 and SigLIP towers and the projector
     (csrc/vit_engine.cu behind include/blurr_vit.h);
   * `LlamaDecoder` — the Llama-2-7B-shaped decoder (csrc/llm_engine.cu behind include/blurr_llm.h): prefill of the
-    multimodal prompt embeddings + greedy decode;
+    multimodal prompt embeddings + greedy decode, or sampled decode (`do_sample=True` with HF's `temperature`, `top_k`,
+    `top_p`; defaults 1.0 / 50 / 1.0 as in `generate`) drawn on the device inside the same CUDA graph, Philox-seeded
+    per row so that a row's tokens depend only on its seed;
   * `ActionDetokenizer` (host) and `OpenVlaPolicy`, which chains them: `predict_action(frames, input_ids, q01, q99)`.
 A batch may carry instructions of different lengths (`input_ids` as a list, or `[B, S]` with a tokenizer's
 `attention_mask`): `ragged_prompt_ids` packs them, `build_prompt_embeds_ragged` lays out `[BOS] + patches + text_b` with
 pad rows behind it, and `LlamaDecoder.generate(..., prompt_lens=...)` generates every sequence at its own positions, so
 each row gets what it would get alone.
-Not built: tokenisation of the instruction (the caller passes `input_ids`).  PARITY: the towers are pinned against
+`predict_action(..., do_sample=True, temperature=, top_k=, top_p=, seed=)` samples the action tokens for every prompt
+form.  Not built: tokenisation of the instruction (the caller passes `input_ids`).  PARITY: the towers are pinned against
 transformers (tests/test_gpu_vit.py), the decoder against `LlamaForCausalLM` with eager attention
 (tests/test_gpu_llm.py), the preprocessing against Pillow + torchvision (tests/test_openvla_preprocess.py); against
 the reference's remote code all of it is UNPINNED (not vendored, not downloadable)."""
@@ -26,6 +29,7 @@ the reference's remote code all of it is UNPINNED (not vendored, not downloadabl
 from __future__ import annotations
 
 import ctypes as C
+import math
 from dataclasses import dataclass
 from typing import Dict, Optional, Sequence, Tuple, Union
 
@@ -67,8 +71,52 @@ def default_inv_freq(head_dim: int, theta: float, device) -> torch.Tensor:
     return 1.0 / (theta ** (torch.arange(0, head_dim, 2, dtype=torch.int64, device=device).float() / head_dim))
 
 
+def _per_row(value, rows: int, name: str) -> list:
+    if isinstance(value, torch.Tensor):
+        value = value.detach().cpu().tolist()
+    elif isinstance(value, np.ndarray):
+        value = value.tolist()
+    if isinstance(value, (list, tuple)):
+        if len(value) != rows:
+            raise ValueError(f"{name} must be a scalar or hold one value per row ({rows}), got {len(value)}")
+        return list(value)
+    return [value] * rows
+
+
+def sampling_params(rows: int, temperature=1.0, top_k=50, top_p=1.0, seed=None) -> "C.Array":
+    """`blurr_llm_sampling[rows]` for `rows` sequences; each argument is a scalar or one value per row.  Checks HF's
+    rules (temperature finite and > 0, top_k an int >= 0, top_p in [0, 1]) and raises ValueError.  `seed`: None draws
+    one 63-bit seed per row from torch's default CPU generator (so `torch.manual_seed` makes a run repeatable); an int
+    `s` gives row b the seed s + b; a sequence gives each row its own seed (ints in [0, 2^64))."""
+    temps = [float(t) for t in _per_row(temperature, rows, "temperature")]
+    ks = _per_row(top_k, rows, "top_k")
+    ps = [float(p) for p in _per_row(top_p, rows, "top_p")]
+    if seed is None:
+        seeds = torch.randint(0, 2 ** 63 - 1, (rows,), dtype=torch.int64).tolist()
+    elif isinstance(seed, (int, np.integer)) and not isinstance(seed, bool):
+        seeds = [int(seed) + b for b in range(rows)]
+    else:
+        seeds = _per_row(seed, rows, "seed")
+    for t in temps:
+        if not math.isfinite(t) or t <= 0.0:
+            raise ValueError(f"temperature must be finite and > 0, got {t}")
+    for k in ks:
+        if isinstance(k, bool) or not isinstance(k, (int, np.integer)) or k < 0 or k > 2 ** 31 - 1:
+            raise ValueError(f"top_k must be an int >= 0, got {k!r}")
+    for p in ps:
+        if not math.isfinite(p) or p < 0.0 or p > 1.0:
+            raise ValueError(f"top_p must be in [0, 1], got {p}")
+    for sd in seeds:
+        if isinstance(sd, bool) or not isinstance(sd, (int, np.integer)) or not 0 <= int(sd) < 2 ** 64:
+            raise ValueError(f"seeds must be ints in [0, 2^64), got {sd!r}")
+    arr = (capi.LlmSamplingC * rows)()
+    for b in range(rows):
+        arr[b] = capi.LlmSamplingC(int(seeds[b]), temps[b], int(ks[b]), ps[b])
+    return arr
+
+
 class LlamaDecoder:
-    """Greedy generation of a Llama-shaped decoder on one B200 through `include/blurr_llm.h`."""
+    """Greedy or sampled generation of a Llama-shaped decoder on one B200 through `include/blurr_llm.h`."""
 
     def __init__(self, cfg: LlamaShapedConfig, device, max_batch: int = 1):
         self.lib = capi.load_library()
@@ -121,13 +169,18 @@ class LlamaDecoder:
                                             C.c_void_p(out.data_ptr())))
         return out
 
-    def generate(self, inputs_embeds: torch.Tensor, n_new: int, return_logits: bool = False, prompt_lens=None):
+    def generate(self, inputs_embeds: torch.Tensor, n_new: int, return_logits: bool = False, prompt_lens=None,
+                 do_sample: bool = False, temperature=1.0, top_k=50, top_p=1.0, seed=None):
         """inputs_embeds: bf16 [B, T, hidden] on the device -> int64 [B, n_new] (and bf16 logits [B, n_new, vocab]).
 
         `prompt_lens` (B ints, 1..T): prompts of different lengths.  Sequence b's prompt is rows 0 .. prompt_lens[b] - 1
         of `inputs_embeds[b]`; the rows after it are padding and never influence any output.  Its token i is generated
         at position prompt_lens[b] + i, so each sequence gets what it would get alone.  One CUDA graph per
-        (B, T, n_new) serves every length vector.  None: every sequence is T rows long."""
+        (B, T, n_new) serves every length vector.  None: every sequence is T rows long.
+
+        `do_sample`: draw every token as HF's `generate(do_sample=True, temperature=, top_k=, top_p=)` does instead of
+        taking the argmax (see `sampling_params` for the arguments and seeds).  Token i of row b depends only on the
+        row's logits, its seed and i; one CUDA graph serves every seed and parameter vector."""
         if inputs_embeds.dim() != 3 or inputs_embeds.shape[2] != self.cfg.hidden:
             raise ValueError(f"inputs_embeds must be [B, T, {self.cfg.hidden}]")
         if inputs_embeds.dtype != torch.bfloat16 or inputs_embeds.device.type != "cuda":
@@ -138,7 +191,17 @@ class LlamaDecoder:
         logits = torch.empty((B, n_new, self.cfg.vocab), device=self.device, dtype=torch.bfloat16) if return_logits else None
         stream = torch.cuda.current_stream(self.device).cuda_stream
         out_logits = C.c_void_p(logits.data_ptr()) if logits is not None else None
-        if prompt_lens is None:
+        if do_sample:
+            params = sampling_params(B, temperature, top_k, top_p, seed)
+            lens_p = None
+            if prompt_lens is not None:
+                lens = np.ascontiguousarray(torch.as_tensor(prompt_lens).cpu().numpy(), dtype=np.int32)
+                if lens.shape != (B,):
+                    raise ValueError(f"prompt_lens must hold one length per sequence ({B}), got shape {lens.shape}")
+                lens_p = lens.ctypes.data_as(C.POINTER(C.c_int32))
+            capi.check(self.lib.blurr_llm_generate_sampled(self.handle, C.c_void_p(stream), B, T, C.c_void_p(x.data_ptr()), lens_p,
+                                                           params, n_new, C.c_void_p(ids.data_ptr()), out_logits))
+        elif prompt_lens is None:
             capi.check(self.lib.blurr_llm_generate(self.handle, C.c_void_p(stream), B, T, C.c_void_p(x.data_ptr()), n_new,
                                                    C.c_void_p(ids.data_ptr()), out_logits))
         else:
@@ -149,6 +212,23 @@ class LlamaDecoder:
                                                           lens.ctypes.data_as(C.POINTER(C.c_int32)), n_new,
                                                           C.c_void_p(ids.data_ptr()), out_logits))
         return (ids, logits) if return_logits else ids
+
+    def sample(self, logits: torch.Tensor, temperature=1.0, top_k=50, top_p=1.0, seed=None, step: int = 0,
+               return_probs: bool = False):
+        """The device sampler alone: bf16 logits [rows, ld >= vocab] on the device (rows <= max_batch; the first vocab
+        columns are used) -> int64 ids [rows] (and fp32 [rows, vocab]: the probability each token was drawn with, 0
+        outside the kept set).  `step` is the Philox counter: `generate` draws its token i with step i."""
+        if logits.dim() != 2 or logits.dtype != torch.bfloat16 or logits.device.type != "cuda" or logits.stride(1) != 1:
+            raise ValueError("logits must be a bf16 CUDA tensor [rows, ld] with contiguous rows")
+        rows = logits.shape[0]
+        params = sampling_params(rows, temperature, top_k, top_p, seed)
+        ids = torch.empty(rows, device=self.device, dtype=torch.int64)
+        probs = torch.empty((rows, self.cfg.vocab), device=self.device, dtype=torch.float32) if return_probs else None
+        stream = torch.cuda.current_stream(self.device).cuda_stream
+        capi.check(self.lib.blurr_llm_sample(self.handle, C.c_void_p(stream), C.c_void_p(logits.data_ptr()), rows, logits.stride(0),
+                                             params, int(step), C.c_void_p(ids.data_ptr()),
+                                             C.c_void_p(probs.data_ptr()) if probs is not None else None))
+        return (ids, probs) if return_probs else ids
 
     def check(self):
         capi.check(self.lib.blurr_llm_check(self.handle, C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)))
@@ -647,8 +727,8 @@ class ImagePreprocessor:
 
 class OpenVlaPolicy:
     """OpenVLA's `predict_action` from raw camera frames: device preprocessing -> DINOv2 + SigLIP towers (fed the two
-    halves of one 6-channel pixel tensor as strided views) -> projector -> `[BOS] + patches + prompt` -> greedy
-    decode of `action_dim` tokens -> de-tokenised, de-normalised actions."""
+    halves of one 6-channel pixel tensor as strided views) -> projector -> `[BOS] + patches + prompt` -> greedy or
+    sampled decode of `action_dim` tokens -> de-tokenised, de-normalised actions."""
 
     def __init__(self, preprocessor: ImagePreprocessor, backbone: FusedVisionBackbone, decoder: LlamaDecoder,
                  detokenizer: Optional[ActionDetokenizer] = None, action_dim: int = 7):
@@ -671,26 +751,31 @@ class OpenVlaPolicy:
         return self.preprocessor(f)
 
     def predict_action_from_pixels(self, pixel_values: torch.Tensor, input_ids, q01, q99, mask=None,
-                                   return_token_ids: bool = False, attention_mask: Optional[torch.Tensor] = None):
+                                   return_token_ids: bool = False, attention_mask: Optional[torch.Tensor] = None,
+                                   do_sample: bool = False, temperature=1.0, top_k=50, top_p=1.0, seed=None):
         """The same as `predict_action`, from prepared bf16 pixel values [B, 6, 224, 224]."""
         patch = self.backbone.forward(pixel_values[:, :3], pixel_values[:, 3:])
+        sample = dict(do_sample=True, temperature=temperature, top_k=top_k, top_p=top_p, seed=seed) if do_sample else {}
         if isinstance(input_ids, (list, tuple)) or attention_mask is not None:
             text, text_lens = ragged_prompt_ids(input_ids, attention_mask)
             x, lens = build_prompt_embeds_ragged(self.decoder, text.to(self.decoder.device), text_lens, patch)
-            ids = self.decoder.generate(x, self.action_dim, prompt_lens=lens)
+            ids = self.decoder.generate(x, self.action_dim, prompt_lens=lens, **sample)
         else:
-            ids = self.decoder.generate(build_prompt_embeds(self.decoder, input_ids, patch), self.action_dim)
+            ids = self.decoder.generate(build_prompt_embeds(self.decoder, input_ids, patch), self.action_dim, **sample)
         tokens = ids.cpu().numpy()
         actions = torch.from_numpy(self.detokenizer.actions(tokens[:, -self.action_dim:], q01, q99, mask))
         return (actions, ids) if return_token_ids else actions
 
     def predict_action(self, frames, input_ids, q01, q99, mask=None, return_token_ids: bool = False,
-                       attention_mask: Optional[torch.Tensor] = None):
+                       attention_mask: Optional[torch.Tensor] = None, do_sample: bool = False, temperature=1.0, top_k=50,
+                       top_p=1.0, seed=None):
         """frames: uint8 [H, W, 3] or [B, H, W, 3] RGB.  input_ids: [B, S] (first column BOS), every row S tokens; or
         instructions of different lengths, as a list of B 1-D id tensors (each starting with BOS) or as [B, S] with a
         tokenizer's left- or right-padded `attention_mask` (see `ragged_prompt_ids`).  `mask` is the action mask of
         the de-normalisation, not a prompt mask.  q01 / q99 / mask: [action_dim], or [B, action_dim] for one dataset's
         statistics per row.  Returns float64 actions [B, action_dim] on the host (and the int64 token ids
-        [B, action_dim] on the device with `return_token_ids`)."""
+        [B, action_dim] on the device with `return_token_ids`).  `do_sample=True` draws the action tokens with HF's
+        `temperature`, `top_k` (default 50, as `generate` has it) and `top_p` instead of decoding greedily; `seed` as in
+        `sampling_params` (None: drawn from torch's default generator)."""
         return self.predict_action_from_pixels(self.pixel_values(frames), input_ids, q01, q99, mask, return_token_ids,
-                                               attention_mask)
+                                               attention_mask, do_sample, temperature, top_k, top_p, seed)

@@ -17,12 +17,18 @@
  * its rows, pads behind it, and its tokens are generated at its own positions, so each sequence gets what it would get
  * alone; one CUDA graph per batch shape serves every vector of lengths.
  *
+ * Sampled decoding (blurr_llm_generate_sampled) draws each token as transformers' `generate(do_sample=True)` does: the
+ * fp32 logits go through TemperatureLogitsWarper, TopKLogitsWarper and TopPLogitsWarper, then softmax and one draw.  The
+ * draw of sequence b at step i uses Philox4x32-10 with key = params[b].seed and counter = (i, 0, 0, 0), so it depends
+ * on nothing but the seed, the step and the logits; the result is bitwise repeatable.
+ *
  * All pointers are device pointers unless stated.  Errors: negative blurr_status (blurr_pi0.h), message from
  * blurr_last_error().  One handle per GPU and per host thread.  Weights are bf16.
  */
 #ifndef BLURR_LLM_H_
 #define BLURR_LLM_H_
 
+#include <stddef.h>
 #include <stdint.h>
 
 #ifdef __cplusplus
@@ -44,6 +50,27 @@ typedef struct blurr_llm_config {
     float rms_eps;                /* 1e-6 (OpenVLA) / 1e-5 (Llama-2) */
 } blurr_llm_config;
 #define BLURR_LLM_ABI_VERSION 1
+
+/* Per-sequence sampling parameters (HF names and rules):
+ *   temperature  finite, > 0: scores * (1.0f / temperature) (ATen's fp32 reciprocal);
+ *   top_k        >= 0; 0 = off, >= vocab = all; ties at the k-th largest score are all kept;
+ *   top_p        in [0, 1]; 1 = off; keeps the smallest set of highest scores whose mass reaches top_p (always the top
+ *                token; among equal scores at the cut the higher token ids are kept, as torch's stable sort does). */
+typedef struct blurr_llm_sampling {
+    uint64_t seed;
+    float temperature;
+    int32_t top_k;
+    float top_p;
+} blurr_llm_sampling;
+#ifdef __cplusplus
+static_assert(sizeof(blurr_llm_sampling) == 24 && offsetof(blurr_llm_sampling, temperature) == 8 &&
+                  offsetof(blurr_llm_sampling, top_k) == 12 && offsetof(blurr_llm_sampling, top_p) == 16,
+              "blurr_llm_sampling layout");
+#else
+_Static_assert(sizeof(blurr_llm_sampling) == 24 && offsetof(blurr_llm_sampling, temperature) == 8 &&
+                   offsetof(blurr_llm_sampling, top_k) == 12 && offsetof(blurr_llm_sampling, top_p) == 16,
+               "blurr_llm_sampling layout");
+#endif
 
 int blurr_llm_create(const blurr_llm_config* cfg, int device, int max_batch, blurr_llm_t** out);
 void blurr_llm_destroy(blurr_llm_t* h);
@@ -78,9 +105,24 @@ int blurr_llm_generate(blurr_llm_t* h, void* cuda_stream, int batch, int prompt_
  * the lengths are uploaded before the launch and read by the kernels at run time. */
 int blurr_llm_generate_ragged(blurr_llm_t* h, void* cuda_stream, int batch, int max_prompt_len, const void* inputs_embeds,
                               const int32_t* prompt_lens, int n_new, int64_t* out_ids, void* out_logits);
+/* Sampled generation over equal (prompt_lens == NULL: every sequence is max_prompt_len rows) or ragged prompts (as
+ * blurr_llm_generate_ragged).  params: HOST [batch], checked on the host (BLURR_ERR_INVALID for a bad value; the
+ * handle keeps working).  Outputs as blurr_llm_generate; out_logits holds the raw logits each token was drawn from.
+ * A row with no finite positive mass (all -inf / NaN, a +inf logit, or a scaled score that overflows) takes the greedy
+ * argmax and sets a sticky error that blurr_llm_check reports.  One CUDA graph per (batch, max_prompt_len, n_new,
+ * logits, ragged) serves every vector of seeds and parameters; a sampled call launches as many kernels as a greedy one. */
+int blurr_llm_generate_sampled(blurr_llm_t* h, void* cuda_stream, int batch, int max_prompt_len, const void* inputs_embeds,
+                               const int32_t* prompt_lens, const blurr_llm_sampling* params, int n_new, int64_t* out_ids,
+                               void* out_logits);
+/* The sampler alone, on caller-made logits (usable before blurr_llm_finalize): logits bf16 [rows][ld], first `vocab`
+ * columns used, rows <= max_batch, ld >= vocab; params HOST [rows]; `step` is the Philox counter.  Writes out_ids int64
+ * [rows]; out_probs (may be NULL) fp32 [rows][vocab]: the probability each token was drawn with, 0 outside the kept set. */
+int blurr_llm_sample(blurr_llm_t* h, void* cuda_stream, const void* logits, int rows, int ld, const blurr_llm_sampling* params,
+                     int step, int64_t* out_ids, float* out_probs);
 /* Options: "use_cuda_graph" (default 1), "trace" (default 0: every kernel stamps %globaltimer, see blurr_llm_trace_report). */
 int blurr_llm_set_option(blurr_llm_t* h, const char* name, int64_t value);
-/* Synchronises the stream; reports and clears device-side sticky errors (token id outside the table, expired pipeline wait). */
+/* Synchronises the stream; reports and clears device-side sticky errors (token id outside the table, a sampled row with
+ * no finite positive mass, expired pipeline wait). */
 int blurr_llm_check(blurr_llm_t* h, void* cuda_stream);
 /* Text timeline of the last generate call under option "trace": one line per kernel, microseconds. */
 int blurr_llm_trace_report(blurr_llm_t* h, char* buf, size_t buf_bytes);
