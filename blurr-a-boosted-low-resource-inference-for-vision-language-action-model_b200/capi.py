@@ -55,7 +55,7 @@ class LlmConfigC(C.Structure):
     ]
 
 
-LLM_ABI_VERSION = 1
+LLM_ABI_VERSION = 2
 
 
 class LlmSamplingC(C.Structure):
@@ -147,10 +147,6 @@ _SIGNATURES = [
     ("blurr_llm_finalize", C.c_int, [C.c_void_p]),
     ("blurr_llm_embed", C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p]),
     ("blurr_llm_generate", C.c_int,
-     [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]),
-    ("blurr_llm_generate_ragged", C.c_int,
-     [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.POINTER(C.c_int32), C.c_int, C.c_void_p, C.c_void_p]),
-    ("blurr_llm_generate_sampled", C.c_int,
      [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.POINTER(C.c_int32), C.POINTER(LlmSamplingC), C.c_int, C.c_void_p,
       C.c_void_p]),
     ("blurr_llm_sample", C.c_int,

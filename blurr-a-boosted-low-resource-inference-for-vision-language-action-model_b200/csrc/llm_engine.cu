@@ -115,11 +115,16 @@ static void* dalloc(blurr_llm* h, size_t bytes) {
     return p;
 }
 
+static void drop_graphs(blurr_llm* h) {
+    for (auto& kv : h->graphs) { cudaGraphExecDestroy(kv.second.exec); cudaGraphDestroy(kv.second.graph); }
+    h->graphs.clear();
+}
+
 extern "C" void blurr_llm_destroy(blurr_llm_t* h) {
     if (!h) return;
     cudaSetDevice(h->device);
     cudaDeviceSynchronize();
-    for (auto& kv : h->graphs) { cudaGraphExecDestroy(kv.second.exec); cudaGraphDestroy(kv.second.graph); }
+    drop_graphs(h);
     for (void* p : h->allocs) cudaFree(p);
     if (h->h_stage) cudaFreeHost(h->h_stage);
     if (h->staged) cudaEventDestroy(h->staged);
@@ -282,8 +287,7 @@ extern "C" int blurr_llm_finalize(blurr_llm_t* h) {
     if (!h->cos_t) return fail(BLURR_ERR_STATE, "blurr_llm_finalize: call blurr_llm_set_rope_table first");
     LLM_CUDA_TRY(cudaSetDevice(h->device));
     LLM_CUDA_TRY(cudaDeviceSynchronize());
-    for (auto& kv : h->graphs) { cudaGraphExecDestroy(kv.second.exec); cudaGraphDestroy(kv.second.graph); }
-    h->graphs.clear();
+    drop_graphs(h);
     h->finalized = true;
     return 0;
 }
@@ -490,28 +494,57 @@ static int stage_rows(blurr_llm_t* h, cudaStream_t st, int rows, const int32_t* 
     return 0;
 }
 
-// The body of blurr_llm_generate / _ragged / _sampled; `lens` (host, validated) selects the ragged schedule, `params`
-// (host, validated) the sampler.
-static int generate(blurr_llm_t* h, void* cuda_stream, int batch, int prompt_len, const void* inputs_embeds, const int32_t* lens,
-                    const blurr_llm_sampling* params, int n_new, int64_t* out_ids, void* out_logits) {
+// HF's checks of the warpers' arguments (TemperatureLogitsWarper, TopKLogitsWarper, TopPLogitsWarper) on the host
+static int check_sampling(const char* fn, const blurr_llm_sampling* params, int rows) {
+    if (!params) return fail(BLURR_ERR_INVALID, std::string(fn) + ": params is null");
+    for (int b = 0; b < rows; ++b) {
+        const blurr_llm_sampling& p = params[b];
+        const std::string at = std::string(fn) + ": params[" + std::to_string(b) + "].";
+        if (!std::isfinite(p.temperature) || !(p.temperature > 0.0f))
+            return fail(BLURR_ERR_INVALID, at + "temperature = " + std::to_string(p.temperature) + " must be finite and > 0");
+        if (p.top_k < 0) return fail(BLURR_ERR_INVALID, at + "top_k = " + std::to_string(p.top_k) + " must be >= 0");
+        if (!std::isfinite(p.top_p) || p.top_p < 0.0f || p.top_p > 1.0f)
+            return fail(BLURR_ERR_INVALID, at + "top_p = " + std::to_string(p.top_p) + " must be in [0, 1]");
+    }
+    return 0;
+}
+
+// `prompt_lens` (host) selects the ragged schedule, even when every length is max_prompt_len; `params` (host) the sampler.
+extern "C" int blurr_llm_generate(blurr_llm_t* h, void* cuda_stream, int batch, int max_prompt_len, const void* inputs_embeds,
+                                  const int32_t* prompt_lens, const blurr_llm_sampling* params, int n_new, int64_t* out_ids,
+                                  void* out_logits) {
+    const char* fn = "blurr_llm_generate";
+    if (!h || !inputs_embeds || !out_ids) return fail(BLURR_ERR_INVALID, std::string(fn) + ": null argument");
+    if (!h->finalized) return fail(BLURR_ERR_STATE, std::string(fn) + ": call blurr_llm_finalize first");
     const auto& c = h->cfg;
+    if (batch < 1 || batch > h->max_batch) return fail(BLURR_ERR_INVALID, std::string(fn) + ": batch out of range");
+    if (max_prompt_len < 1 || n_new < 1 || max_prompt_len + n_new > c.max_positions)
+        return fail(BLURR_ERR_INVALID, std::string(fn) + ": max_prompt_len + n_new exceeds max_positions");
+    if (prompt_lens)
+        for (int b = 0; b < batch; ++b)
+            if (prompt_lens[b] < 1 || prompt_lens[b] > max_prompt_len)
+                return fail(BLURR_ERR_INVALID, std::string(fn) + ": prompt_lens[" + std::to_string(b) + "] = " +
+                                                   std::to_string(prompt_lens[b]) + " is outside 1.." + std::to_string(max_prompt_len));
+    if (out_logits != nullptr && n_new > kMaxKeptLogits)
+        return fail(BLURR_ERR_INVALID, std::string(fn) + ": logits are kept for at most 16 new tokens");
+    if (const int rc = params ? check_sampling(fn, params, batch) : 0) return rc;
     LLM_CUDA_TRY(cudaSetDevice(h->device));
     cudaStream_t st = static_cast<cudaStream_t>(cuda_stream);
     const bool keep = out_logits != nullptr;
-    const bool ragged = lens != nullptr;
+    const bool ragged = prompt_lens != nullptr;
     const bool sampled = params != nullptr;
-    LLM_CUDA_TRY(cudaMemcpyAsync(h->IN, inputs_embeds, static_cast<size_t>(batch) * prompt_len * c.hidden * 2, cudaMemcpyDeviceToDevice, st));
-    if (const int rc = stage_rows(h, st, batch, lens, params)) return rc;
+    LLM_CUDA_TRY(cudaMemcpyAsync(h->IN, inputs_embeds, static_cast<size_t>(batch) * max_prompt_len * c.hidden * 2, cudaMemcpyDeviceToDevice, st));
+    if (const int rc = stage_rows(h, st, batch, prompt_lens, params)) return rc;
     h->launches = 0;
     Run R{h, st};
     if (!h->use_graph) {
-        run_generate(R, batch, prompt_len, n_new, keep, ragged, sampled);
+        run_generate(R, batch, max_prompt_len, n_new, keep, ragged, sampled);
         if (R.rc) return R.rc;
     } else {
-        const auto key = std::make_tuple(batch, prompt_len, n_new, keep ? 1 : 0, ragged ? 1 : 0, sampled ? 1 : 0);
+        const auto key = std::make_tuple(batch, max_prompt_len, n_new, keep ? 1 : 0, ragged ? 1 : 0, sampled ? 1 : 0);
         auto it = h->graphs.find(key);
         if (it == h->graphs.end()) {
-            run_generate(R, batch, prompt_len, n_new, keep, ragged, sampled);         // warm run: attribute setup, tensor maps
+            run_generate(R, batch, max_prompt_len, n_new, keep, ragged, sampled);         // warm run: attribute setup, tensor maps
             if (R.rc) return R.rc;
             LLM_CUDA_TRY(cudaStreamSynchronize(st));
             h->launches = 0;
@@ -520,7 +553,7 @@ static int generate(blurr_llm_t* h, void* cuda_stream, int batch, int prompt_len
             Run C{h, cs};
             cudaError_t e = cudaStreamBeginCapture(cs, cudaStreamCaptureModeThreadLocal);
             if (e != cudaSuccess) { cudaStreamDestroy(cs); return fail(BLURR_ERR_CUDA, "graph capture begin failed"); }
-            run_generate(C, batch, prompt_len, n_new, keep, ragged, sampled);
+            run_generate(C, batch, max_prompt_len, n_new, keep, ragged, sampled);
             cudaGraph_t g = nullptr;
             e = cudaStreamEndCapture(cs, &g);
             cudaStreamDestroy(cs);
@@ -538,72 +571,6 @@ static int generate(blurr_llm_t* h, void* cuda_stream, int batch, int prompt_len
     if (keep)
         LLM_CUDA_TRY(cudaMemcpyAsync(out_logits, h->LOGITS_ALL, static_cast<size_t>(batch) * n_new * c.vocab * 2, cudaMemcpyDeviceToDevice, st));
     return 0;
-}
-
-extern "C" int blurr_llm_generate(blurr_llm_t* h, void* cuda_stream, int batch, int prompt_len, const void* inputs_embeds,
-                                  int n_new, int64_t* out_ids, void* out_logits) {
-    if (!h || !inputs_embeds || !out_ids) return fail(BLURR_ERR_INVALID, "blurr_llm_generate: null argument");
-    if (!h->finalized) return fail(BLURR_ERR_STATE, "blurr_llm_generate: call blurr_llm_finalize first");
-    const auto& c = h->cfg;
-    if (batch < 1 || batch > h->max_batch) return fail(BLURR_ERR_INVALID, "blurr_llm_generate: batch out of range");
-    if (prompt_len < 1 || n_new < 1 || prompt_len + n_new > c.max_positions)
-        return fail(BLURR_ERR_INVALID, "blurr_llm_generate: prompt_len + n_new exceeds max_positions");
-    if (out_logits != nullptr && n_new > kMaxKeptLogits) return fail(BLURR_ERR_INVALID, "blurr_llm_generate: logits are kept for at most 16 new tokens");
-    return generate(h, cuda_stream, batch, prompt_len, inputs_embeds, nullptr, nullptr, n_new, out_ids, out_logits);
-}
-
-extern "C" int blurr_llm_generate_ragged(blurr_llm_t* h, void* cuda_stream, int batch, int max_prompt_len, const void* inputs_embeds,
-                                         const int32_t* prompt_lens, int n_new, int64_t* out_ids, void* out_logits) {
-    if (!h || !inputs_embeds || !out_ids) return fail(BLURR_ERR_INVALID, "blurr_llm_generate_ragged: null argument");
-    if (!prompt_lens) return fail(BLURR_ERR_INVALID, "blurr_llm_generate_ragged: prompt_lens is null");
-    if (!h->finalized) return fail(BLURR_ERR_STATE, "blurr_llm_generate_ragged: call blurr_llm_finalize first");
-    const auto& c = h->cfg;
-    if (batch < 1 || batch > h->max_batch) return fail(BLURR_ERR_INVALID, "blurr_llm_generate_ragged: batch out of range");
-    if (max_prompt_len < 1 || n_new < 1 || max_prompt_len + n_new > c.max_positions)
-        return fail(BLURR_ERR_INVALID, "blurr_llm_generate_ragged: max_prompt_len + n_new exceeds max_positions");
-    for (int b = 0; b < batch; ++b)
-        if (prompt_lens[b] < 1 || prompt_lens[b] > max_prompt_len)
-            return fail(BLURR_ERR_INVALID, "blurr_llm_generate_ragged: prompt_lens[" + std::to_string(b) + "] = " +
-                                               std::to_string(prompt_lens[b]) + " is outside 1.." + std::to_string(max_prompt_len));
-    if (out_logits != nullptr && n_new > kMaxKeptLogits)
-        return fail(BLURR_ERR_INVALID, "blurr_llm_generate_ragged: logits are kept for at most 16 new tokens");
-    return generate(h, cuda_stream, batch, max_prompt_len, inputs_embeds, prompt_lens, nullptr, n_new, out_ids, out_logits);
-}
-
-// HF's checks of the warpers' arguments (TemperatureLogitsWarper, TopKLogitsWarper, TopPLogitsWarper) on the host
-static int check_sampling(const char* fn, const blurr_llm_sampling* params, int rows) {
-    if (!params) return fail(BLURR_ERR_INVALID, std::string(fn) + ": params is null");
-    for (int b = 0; b < rows; ++b) {
-        const blurr_llm_sampling& p = params[b];
-        const std::string at = std::string(fn) + ": params[" + std::to_string(b) + "].";
-        if (!std::isfinite(p.temperature) || !(p.temperature > 0.0f))
-            return fail(BLURR_ERR_INVALID, at + "temperature = " + std::to_string(p.temperature) + " must be finite and > 0");
-        if (p.top_k < 0) return fail(BLURR_ERR_INVALID, at + "top_k = " + std::to_string(p.top_k) + " must be >= 0");
-        if (!std::isfinite(p.top_p) || p.top_p < 0.0f || p.top_p > 1.0f)
-            return fail(BLURR_ERR_INVALID, at + "top_p = " + std::to_string(p.top_p) + " must be in [0, 1]");
-    }
-    return 0;
-}
-
-extern "C" int blurr_llm_generate_sampled(blurr_llm_t* h, void* cuda_stream, int batch, int max_prompt_len, const void* inputs_embeds,
-                                          const int32_t* prompt_lens, const blurr_llm_sampling* params, int n_new, int64_t* out_ids,
-                                          void* out_logits) {
-    const char* fn = "blurr_llm_generate_sampled";
-    if (!h || !inputs_embeds || !out_ids) return fail(BLURR_ERR_INVALID, std::string(fn) + ": null argument");
-    if (!h->finalized) return fail(BLURR_ERR_STATE, std::string(fn) + ": call blurr_llm_finalize first");
-    const auto& c = h->cfg;
-    if (batch < 1 || batch > h->max_batch) return fail(BLURR_ERR_INVALID, std::string(fn) + ": batch out of range");
-    if (max_prompt_len < 1 || n_new < 1 || max_prompt_len + n_new > c.max_positions)
-        return fail(BLURR_ERR_INVALID, std::string(fn) + ": max_prompt_len + n_new exceeds max_positions");
-    if (prompt_lens)
-        for (int b = 0; b < batch; ++b)
-            if (prompt_lens[b] < 1 || prompt_lens[b] > max_prompt_len)
-                return fail(BLURR_ERR_INVALID, std::string(fn) + ": prompt_lens[" + std::to_string(b) + "] = " +
-                                                   std::to_string(prompt_lens[b]) + " is outside 1.." + std::to_string(max_prompt_len));
-    if (out_logits != nullptr && n_new > kMaxKeptLogits)
-        return fail(BLURR_ERR_INVALID, std::string(fn) + ": logits are kept for at most 16 new tokens");
-    if (const int rc = check_sampling(fn, params, batch)) return rc;
-    return generate(h, cuda_stream, batch, max_prompt_len, inputs_embeds, prompt_lens, params, n_new, out_ids, out_logits);
 }
 
 extern "C" int blurr_llm_sample(blurr_llm_t* h, void* cuda_stream, const void* logits, int rows, int ld, const blurr_llm_sampling* params,
@@ -632,8 +599,7 @@ extern "C" int blurr_llm_set_option(blurr_llm_t* h, const char* name, int64_t va
             if (!h->trace_buf) return fail(BLURR_ERR_CUDA, "trace buffer allocation failed");
         }
         h->trace = value != 0;
-        for (auto& kv : h->graphs) { cudaGraphExecDestroy(kv.second.exec); cudaGraphDestroy(kv.second.graph); }
-        h->graphs.clear();
+        drop_graphs(h);
     }
     else return fail(BLURR_ERR_INVALID, "blurr_llm_set_option: unknown option " + n);
     return 0;

@@ -191,26 +191,15 @@ class LlamaDecoder:
         logits = torch.empty((B, n_new, self.cfg.vocab), device=self.device, dtype=torch.bfloat16) if return_logits else None
         stream = torch.cuda.current_stream(self.device).cuda_stream
         out_logits = C.c_void_p(logits.data_ptr()) if logits is not None else None
-        if do_sample:
-            params = sampling_params(B, temperature, top_k, top_p, seed)
-            lens_p = None
-            if prompt_lens is not None:
-                lens = np.ascontiguousarray(torch.as_tensor(prompt_lens).cpu().numpy(), dtype=np.int32)
-                if lens.shape != (B,):
-                    raise ValueError(f"prompt_lens must hold one length per sequence ({B}), got shape {lens.shape}")
-                lens_p = lens.ctypes.data_as(C.POINTER(C.c_int32))
-            capi.check(self.lib.blurr_llm_generate_sampled(self.handle, C.c_void_p(stream), B, T, C.c_void_p(x.data_ptr()), lens_p,
-                                                           params, n_new, C.c_void_p(ids.data_ptr()), out_logits))
-        elif prompt_lens is None:
-            capi.check(self.lib.blurr_llm_generate(self.handle, C.c_void_p(stream), B, T, C.c_void_p(x.data_ptr()), n_new,
-                                                   C.c_void_p(ids.data_ptr()), out_logits))
-        else:
+        params = sampling_params(B, temperature, top_k, top_p, seed) if do_sample else None
+        lens_p = None
+        if prompt_lens is not None:
             lens = np.ascontiguousarray(torch.as_tensor(prompt_lens).cpu().numpy(), dtype=np.int32)
             if lens.shape != (B,):
                 raise ValueError(f"prompt_lens must hold one length per sequence ({B}), got shape {lens.shape}")
-            capi.check(self.lib.blurr_llm_generate_ragged(self.handle, C.c_void_p(stream), B, T, C.c_void_p(x.data_ptr()),
-                                                          lens.ctypes.data_as(C.POINTER(C.c_int32)), n_new,
-                                                          C.c_void_p(ids.data_ptr()), out_logits))
+            lens_p = lens.ctypes.data_as(C.POINTER(C.c_int32))
+        capi.check(self.lib.blurr_llm_generate(self.handle, C.c_void_p(stream), B, T, C.c_void_p(x.data_ptr()), lens_p, params,
+                                               n_new, C.c_void_p(ids.data_ptr()), out_logits))
         return (ids, logits) if return_logits else ids
 
     def sample(self, logits: torch.Tensor, temperature=1.0, top_k=50, top_p=1.0, seed=None, step: int = 0,

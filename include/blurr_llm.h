@@ -13,14 +13,15 @@
  * PARITY: pinned against transformers 5.5.0 `LlamaForCausalLM` (a library present in this image, not reference source);
  * against the reference itself it is UNPINNED (the remote code is neither vendored nor downloadable), see DESIGN.md.
  *
- * A batch may mix prompts of different lengths (blurr_llm_generate_ragged): each sequence's prompt sits at the front of
- * its rows, pads behind it, and its tokens are generated at its own positions, so each sequence gets what it would get
- * alone; one CUDA graph per batch shape serves every vector of lengths.
+ * blurr_llm_generate serves equal-length, ragged and sampled calls.  A batch may mix prompts of different lengths
+ * (prompt_lens): each sequence's prompt sits at the front of its rows, pads behind it, and its tokens are generated at its
+ * own positions, so each sequence gets what it would get alone; one CUDA graph per batch shape serves every vector of
+ * lengths.
  *
- * Sampled decoding (blurr_llm_generate_sampled) draws each token as transformers' `generate(do_sample=True)` does: the
- * fp32 logits go through TemperatureLogitsWarper, TopKLogitsWarper and TopPLogitsWarper, then softmax and one draw.  The
- * draw of sequence b at step i uses Philox4x32-10 with key = params[b].seed and counter = (i, 0, 0, 0), so it depends
- * on nothing but the seed, the step and the logits; the result is bitwise repeatable.
+ * Sampled decoding (params) draws each token as transformers' `generate(do_sample=True)` does: the fp32 logits go
+ * through TemperatureLogitsWarper, TopKLogitsWarper and TopPLogitsWarper, then softmax and one draw.  The draw of
+ * sequence b at step i uses Philox4x32-10 with key = params[b].seed and counter = (i, 0, 0, 0), so it depends on nothing
+ * but the seed, the step and the logits; the result is bitwise repeatable.
  *
  * All pointers are device pointers unless stated.  Errors: negative blurr_status (blurr_pi0.h), message from
  * blurr_last_error().  One handle per GPU and per host thread.  Weights are bf16.
@@ -49,7 +50,7 @@ typedef struct blurr_llm_config {
     int32_t max_positions;        /* KV-cache slots per sequence: prompt + generated tokens, <= 320 */
     float rms_eps;                /* 1e-6 (OpenVLA) / 1e-5 (Llama-2) */
 } blurr_llm_config;
-#define BLURR_LLM_ABI_VERSION 1
+#define BLURR_LLM_ABI_VERSION 2
 
 /* Per-sequence sampling parameters (HF names and rules):
  *   temperature  finite, > 0: scores * (1.0f / temperature) (ATen's fp32 reciprocal);
@@ -89,31 +90,24 @@ int blurr_llm_finalize(blurr_llm_t* h);
 /* rows[i] = embed_tokens[ids[i]]  (bf16 [n][hidden]) */
 int blurr_llm_embed(blurr_llm_t* h, void* cuda_stream, const int64_t* ids, int n, void* rows_out);
 
-/* Greedy generation.  inputs_embeds: bf16 [batch][prompt_len][hidden] (every sequence has the same length, no padding;
- * prompts of different lengths go through blurr_llm_generate_ragged).  Writes out_ids int64 [batch][n_new]; if out_logits
- * != NULL also the bf16 logits each token was chosen from, [batch][n_new][vocab] (n_new <= 16).  prompt_len + n_new <=
- * max_positions.  The whole call (prefill, n_new - 1 decode steps, argmax) is replayed as one CUDA graph per
- * (batch, prompt_len, n_new, logits). */
-int blurr_llm_generate(blurr_llm_t* h, void* cuda_stream, int batch, int prompt_len, const void* inputs_embeds, int n_new,
-                       int64_t* out_ids, void* out_logits);
-/* Greedy generation over prompts of different lengths, right-aligned: sequence b's prompt is rows 0 .. prompt_lens[b] - 1.
- * inputs_embeds: bf16 [batch][max_prompt_len][hidden]; rows t >= prompt_lens[b] are ignored (never influence any output:
- * they are zeroed on the device before the prefill, which runs over all max_prompt_len rows).
- * prompt_lens: HOST int32 [batch], 1 <= prompt_lens[b] <= max_prompt_len; max_prompt_len + n_new <= max_positions.
- * Token i of sequence b is generated at position prompt_lens[b] + i, so each sequence gets what it would get alone.
- * Outputs as blurr_llm_generate.  One CUDA graph per (batch, max_prompt_len, n_new, logits) serves every length vector:
- * the lengths are uploaded before the launch and read by the kernels at run time. */
-int blurr_llm_generate_ragged(blurr_llm_t* h, void* cuda_stream, int batch, int max_prompt_len, const void* inputs_embeds,
-                              const int32_t* prompt_lens, int n_new, int64_t* out_ids, void* out_logits);
-/* Sampled generation over equal (prompt_lens == NULL: every sequence is max_prompt_len rows) or ragged prompts (as
- * blurr_llm_generate_ragged).  params: HOST [batch], checked on the host (BLURR_ERR_INVALID for a bad value; the
- * handle keeps working).  Outputs as blurr_llm_generate; out_logits holds the raw logits each token was drawn from.
- * A row with no finite positive mass (all -inf / NaN, a +inf logit, or a scaled score that overflows) takes the greedy
- * argmax and sets a sticky error that blurr_llm_check reports.  One CUDA graph per (batch, max_prompt_len, n_new,
- * logits, ragged) serves every vector of seeds and parameters; a sampled call launches as many kernels as a greedy one. */
-int blurr_llm_generate_sampled(blurr_llm_t* h, void* cuda_stream, int batch, int max_prompt_len, const void* inputs_embeds,
-                               const int32_t* prompt_lens, const blurr_llm_sampling* params, int n_new, int64_t* out_ids,
-                               void* out_logits);
+/* Generation.  inputs_embeds: bf16 [batch][max_prompt_len][hidden]; max_prompt_len + n_new <= max_positions.
+ * prompt_lens: HOST int32 [batch] or NULL.  NULL: every sequence is max_prompt_len rows, no padding.  Otherwise
+ * 1 <= prompt_lens[b] <= max_prompt_len and sequence b's prompt is rows 0 .. prompt_lens[b] - 1; rows t >= prompt_lens[b]
+ * are ignored (never influence any output: they are zeroed on the device before the prefill, which runs over all
+ * max_prompt_len rows), and token i of sequence b is generated at position prompt_lens[b] + i, so each sequence gets what
+ * it would get alone.  A non-NULL prompt_lens takes this ragged schedule even when every length is max_prompt_len.
+ * params: HOST [batch] or NULL.  NULL: greedy argmax.  Otherwise each token is drawn with its sequence's parameters,
+ * checked on the host; a row with no finite positive mass (all -inf / NaN, a +inf logit, or a scaled score that
+ * overflows) takes the greedy argmax and sets a sticky error that blurr_llm_check reports.
+ * Writes out_ids int64 [batch][n_new]; if out_logits != NULL also the raw bf16 logits each token was chosen from,
+ * [batch][n_new][vocab] (n_new <= 16).  A bad argument returns BLURR_ERR_INVALID and the handle keeps working.
+ * The whole call (prefill, n_new - 1 decode steps, argmax or draw) is replayed as one CUDA graph per
+ * (batch, max_prompt_len, n_new, logits, ragged, sampled): lengths and parameters are uploaded before the launch and read
+ * by the kernels at run time, so one graph serves every vector of them; a sampled call launches as many kernels as a
+ * greedy one. */
+int blurr_llm_generate(blurr_llm_t* h, void* cuda_stream, int batch, int max_prompt_len, const void* inputs_embeds,
+                       const int32_t* prompt_lens, const blurr_llm_sampling* params, int n_new, int64_t* out_ids,
+                       void* out_logits);
 /* The sampler alone, on caller-made logits (usable before blurr_llm_finalize): logits bf16 [rows][ld], first `vocab`
  * columns used, rows <= max_batch, ld >= vocab; params HOST [rows]; `step` is the Philox counter.  Writes out_ids int64
  * [rows]; out_probs (may be NULL) fp32 [rows][vocab]: the probability each token was drawn with, 0 outside the kept set. */

@@ -1,4 +1,4 @@
-"""Host restatement of the sampled decoding of `blurr_llm_generate_sampled` / `blurr_llm_sample` (test-only).
+"""Host restatement of the sampled decoding of `blurr_llm_generate` (with `params`) / `blurr_llm_sample` (test-only).
 
 HF semantics (transformers 5.5 `generation/utils.py` `_sample`, `generation/logits_process.py`): the last logits row is
 cast to fp32, then `TemperatureLogitsWarper` (T != 1), `TopKLogitsWarper` (k != 0), `TopPLogitsWarper` (p < 1) with

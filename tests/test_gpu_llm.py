@@ -12,45 +12,10 @@ import pytest
 import torch
 
 from blurr_b200 import openvla
+from llama_helpers import hf_greedy, hf_llama
 
 pytestmark = pytest.mark.gpu
 DEV = "cuda"
-
-
-def _hf_model(cfg: openvla.LlamaShapedConfig, seed: int, stress: bool):
-    from transformers import LlamaConfig, LlamaForCausalLM
-    hc = LlamaConfig(hidden_size=cfg.hidden, intermediate_size=cfg.intermediate, num_hidden_layers=cfg.num_layers,
-                     num_attention_heads=cfg.num_heads, num_key_value_heads=cfg.num_kv_heads, head_dim=cfg.head_dim,
-                     vocab_size=cfg.vocab, max_position_embeddings=2048, rms_norm_eps=cfg.rms_eps, rope_theta=cfg.rope_theta,
-                     attn_implementation="eager", tie_word_embeddings=False)
-    torch.manual_seed(seed)
-    model = LlamaForCausalLM(hc).eval()
-    with torch.no_grad():
-        for name, p in model.named_parameters():
-            if "layernorm" in name or name.endswith("norm.weight"):
-                p.copy_(1.0 + 0.2 * torch.randn_like(p))                 # norms away from their init of 1
-            elif stress and ("q_proj" in name or "k_proj" in name):
-                p.mul_(6.0)                                              # peaked attention: RoPE and the mask matter
-            elif stress and ("embed_tokens" in name or "lm_head" in name):
-                p.mul_(4.0)
-    return model.to(torch.bfloat16).to(DEV)
-
-
-@torch.inference_mode()
-def _hf_greedy(model, inputs_embeds, n_new):
-    out = model(inputs_embeds=inputs_embeds, use_cache=True)
-    past = out.past_key_values
-    logits, ids = [], []
-    last = out.logits[:, -1, :]
-    for i in range(n_new):
-        logits.append(last)
-        tok = last.float().argmax(dim=-1)
-        ids.append(tok)
-        if i + 1 < n_new:
-            out = model(input_ids=tok[:, None], past_key_values=past, use_cache=True)
-            past = out.past_key_values
-            last = out.logits[:, -1, :]
-    return torch.stack(ids, dim=1), torch.stack(logits, dim=1)
 
 
 def _inv_freq(model):
@@ -77,12 +42,12 @@ def test_generate_matches_transformers_llama(hidden, heads, hd, inter, layers, v
     n_new = 7
     cfg = openvla.LlamaShapedConfig(num_layers=layers, hidden=hidden, num_heads=heads, num_kv_heads=heads, head_dim=hd,
                                     intermediate=inter, vocab=vocab, max_positions=prompt + n_new + 1, rms_eps=1e-6)
-    model = _hf_model(cfg, 0, stress)
+    model = hf_llama(cfg, 0, qk_scale=6.0 if stress else 1.0, head_scale=4.0 if stress else 1.0)
     dec = openvla.LlamaDecoder.from_state_dict(cfg, model.state_dict(), DEV, max_batch=batch, inv_freq=_inv_freq(model))
     g = torch.Generator(device=DEV)
     g.manual_seed(1)
     x = (torch.randn((batch, prompt, hidden), device=DEV, generator=g) * (1.0 if stress else 0.3)).to(torch.bfloat16)
-    ref_ids, ref_logits = _hf_greedy(model, x, n_new)
+    ref_ids, ref_logits = hf_greedy(model, x, n_new)
     ids, logits = dec.generate(x, n_new, return_logits=True)
     dec.check()
     ids2 = dec.generate(x, n_new)                      # graph replay, no logits

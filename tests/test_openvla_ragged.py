@@ -1,6 +1,6 @@
 """Prompts of different lengths in one batch on the OpenVLA path (`LlamaDecoder.generate(..., prompt_lens=...)`,
-`blurr_llm_generate_ragged`, `ragged_prompt_ids`, `build_prompt_embeds_ragged`, `OpenVlaPolicy.predict_action` with a
-list or an `attention_mask`).
+`blurr_llm_generate` with `prompt_lens`, `ragged_prompt_ids`, `build_prompt_embeds_ragged`, `OpenVlaPolicy.predict_action`
+with a list or an `attention_mask`).
 
 Layout: sequence b's prompt is rows 0 .. len_b - 1 of its T_max rows, pads after; its token i is generated at position
 len_b + i.  So every sequence must get what the model gives for that sequence alone.
@@ -19,6 +19,7 @@ import pytest
 import torch
 
 from blurr_b200 import capi, openvla
+from llama_helpers import Q01, Q99, hf_greedy, hf_llama, instructions, small_policy, synthetic_decoder
 
 DEV = "cuda"
 
@@ -107,42 +108,6 @@ def test_actions_take_per_row_statistics():
 # ---------------------------------------------------------------------------------------------------------------------
 # GPU: the decoder against transformers, sequence by sequence
 # ---------------------------------------------------------------------------------------------------------------------
-def _hf_model(cfg: openvla.LlamaShapedConfig, seed: int, stress: bool):
-    from transformers import LlamaConfig, LlamaForCausalLM
-    hc = LlamaConfig(hidden_size=cfg.hidden, intermediate_size=cfg.intermediate, num_hidden_layers=cfg.num_layers,
-                     num_attention_heads=cfg.num_heads, num_key_value_heads=cfg.num_kv_heads, head_dim=cfg.head_dim,
-                     vocab_size=cfg.vocab, max_position_embeddings=2048, rms_norm_eps=cfg.rms_eps, rope_theta=cfg.rope_theta,
-                     attn_implementation="eager", tie_word_embeddings=False)
-    torch.manual_seed(seed)
-    model = LlamaForCausalLM(hc).eval()
-    with torch.no_grad():
-        for name, p in model.named_parameters():
-            if "layernorm" in name or name.endswith("norm.weight"):
-                p.copy_(1.0 + 0.2 * torch.randn_like(p))                 # norms away from their init of 1
-            elif stress and ("q_proj" in name or "k_proj" in name):
-                p.mul_(6.0)                                              # peaked attention: RoPE and the mask matter
-            elif stress and ("embed_tokens" in name or "lm_head" in name):
-                p.mul_(4.0)
-    return model.to(torch.bfloat16).to(DEV)
-
-
-@torch.inference_mode()
-def _hf_greedy(model, inputs_embeds, n_new):
-    out = model(inputs_embeds=inputs_embeds, use_cache=True)
-    past = out.past_key_values
-    logits, ids = [], []
-    last = out.logits[:, -1, :]
-    for i in range(n_new):
-        logits.append(last)
-        tok = last.float().argmax(dim=-1)
-        ids.append(tok)
-        if i + 1 < n_new:
-            out = model(input_ids=tok[:, None], past_key_values=past, use_cache=True)
-            past = out.past_key_values
-            last = out.logits[:, -1, :]
-    return torch.stack(ids, dim=1), torch.stack(logits, dim=1)
-
-
 def _lens(batch, lo, hi, seed):
     return np.random.default_rng(seed).integers(lo, hi + 1, size=batch).astype(np.int32)
 
@@ -166,7 +131,7 @@ def test_ragged_generate_matches_transformers_per_sequence(hidden, heads, hd, in
     B, T = len(lens), int(lens.max())
     cfg = openvla.LlamaShapedConfig(num_layers=layers, hidden=hidden, num_heads=heads, num_kv_heads=heads, head_dim=hd,
                                     intermediate=inter, vocab=vocab, max_positions=T + n_new + 1, rms_eps=1e-6)
-    model = _hf_model(cfg, 0, stress)
+    model = hf_llama(cfg, 0, qk_scale=6.0 if stress else 1.0, head_scale=4.0 if stress else 1.0)
     dec = openvla.LlamaDecoder.from_state_dict(cfg, model.state_dict(), DEV, max_batch=B,
                                                inv_freq=model.model.rotary_emb.inv_freq.detach().float())
     g = torch.Generator(device=DEV).manual_seed(1)
@@ -176,7 +141,7 @@ def test_ragged_generate_matches_transformers_per_sequence(hidden, heads, hd, in
     assert torch.equal(dec.generate(x, n_new, prompt_lens=lens), ids)          # graph replay, no logits
     first_equal, worst = 0, 0.0
     for b in range(B):
-        ref_ids, ref_logits = _hf_greedy(model, x[b:b + 1, :lens[b]], n_new)
+        ref_ids, ref_logits = hf_greedy(model, x[b:b + 1, :lens[b]], n_new)
         scale = ref_logits.float().abs().max().item()
         for i in range(n_new):
             d = (logits[b, i].float() - ref_logits[0, i].float()).abs().max().item()
@@ -196,36 +161,10 @@ def test_ragged_generate_matches_transformers_per_sequence(hidden, heads, hd, in
 # ---------------------------------------------------------------------------------------------------------------------
 # GPU: bitwise properties (synthetic weights)
 # ---------------------------------------------------------------------------------------------------------------------
-SHAPES = {
-    # hidden, heads, head_dim, inter, layers, vocab, batch, T_max
-    "few": (256, 2, 128, 512, 2, 1000, 4, 8),
-    "mid": (512, 4, 128, 1408, 2, 1064, 3, 37),
-    "b32": (1280, 10, 128, 2560, 2, 1000, 32, 12),
-    "b32-fused": (512, 8, 64, 1024, 1, 300, 32, 6),
-}
-
-
-def _decoder(name, n_new=7):
-    hidden, heads, hd, inter, layers, vocab, B, T = SHAPES[name]
-    cfg = openvla.LlamaShapedConfig(num_layers=layers, hidden=hidden, num_heads=heads, num_kv_heads=heads, head_dim=hd,
-                                    intermediate=inter, vocab=vocab, max_positions=T + n_new + 1)
-    sd = openvla.synthetic_llama_state_dict(cfg, DEV, 0)
-    with torch.no_grad():
-        for k, v in sd.items():
-            if "q_proj" in k or "k_proj" in k:
-                v.mul_(8.0)                                              # peaked attention
-            if k.startswith("lm_head"):
-                v.mul_(4.0)
-    dec = openvla.LlamaDecoder.from_state_dict(cfg, sd, DEV, max_batch=B)
-    g = torch.Generator(device=DEV).manual_seed(7)
-    x = (torch.randn((B, T, hidden), device=DEV, generator=g) * 0.5).to(torch.bfloat16)
-    return dec, x
-
-
 @pytest.mark.gpu
 @pytest.mark.parametrize("name", ["few", "mid", "b32", "b32-fused"])
 def test_equal_lengths_through_prompt_lens_are_bitwise_the_plain_call(name):
-    dec, x = _decoder(name)
+    dec, x = synthetic_decoder(name)
     B, T = x.shape[:2]
     ids0, lg0 = dec.generate(x, 7, return_logits=True)
     ids1, lg1 = dec.generate(x, 7, return_logits=True, prompt_lens=[T] * B)
@@ -237,7 +176,7 @@ def test_equal_lengths_through_prompt_lens_are_bitwise_the_plain_call(name):
 @pytest.mark.gpu
 @pytest.mark.parametrize("name", ["few", "mid", "b32", "b32-fused"])
 def test_pad_rows_and_other_sequences_never_matter(name):
-    dec, x = _decoder(name)
+    dec, x = synthetic_decoder(name)
     B, T = x.shape[:2]
     lens = _lens(B, 1, T, 11)
     lens[0] = T
@@ -262,7 +201,7 @@ def test_pad_rows_and_other_sequences_never_matter(name):
 @pytest.mark.gpu
 @pytest.mark.parametrize("name", ["few", "b32", "b32-fused"])
 def test_graph_replay_with_new_lengths_equals_eager(name):
-    dec, x = _decoder(name)
+    dec, x = synthetic_decoder(name)
     B, T = x.shape[:2]
     lens_a, lens_b = _lens(B, 1, T, 21), _lens(B, 1, T, 22)
     dec.generate(x, 7, prompt_lens=lens_a)                   # captures the (B, T, 7) ragged graph
@@ -279,8 +218,8 @@ def test_graph_replay_with_new_lengths_equals_eager(name):
 
 
 @pytest.mark.gpu
-def test_rejected_ragged_calls_leave_the_handle_working():
-    dec, x = _decoder("few")
+def test_rejected_ragged_calls_and_null_prompt_lens():
+    dec, x = synthetic_decoder("few", n_new=17)                # room for 17 tokens: the kept-logits limit is reachable
     B, T = x.shape[:2]
     ok = dec.generate(x, 7, prompt_lens=[T] * B)
     bad = [
@@ -292,19 +231,22 @@ def test_rejected_ragged_calls_leave_the_handle_working():
         with pytest.raises(capi.BlurrError):
             dec.generate(x, 7, prompt_lens=lens)
     with pytest.raises(capi.BlurrError):                      # max_prompt_len + n_new > max_positions
-        dec.generate(x, 9, prompt_lens=[T] * B)
+        dec.generate(x, dec.cfg.max_positions - T + 1, prompt_lens=[T] * B)
+    with pytest.raises(capi.BlurrError, match="at most 16"):  # logits are kept for at most 16 tokens
+        dec.generate(x, 17, return_logits=True, prompt_lens=[T] * B)
     with pytest.raises(ValueError):                           # one length per sequence
         dec.generate(x, 7, prompt_lens=[T] * (B - 1))
     lib, stream = dec.lib, C.c_void_p(torch.cuda.current_stream().cuda_stream)
     out = torch.empty((B, 7), device=DEV, dtype=torch.int64)
     lens = (C.c_int32 * B)(*([T] * B))
-    with pytest.raises(capi.BlurrError):                      # null prompt_lens
-        capi.check(lib.blurr_llm_generate_ragged(dec.handle, stream, B, T, C.c_void_p(x.data_ptr()), None, 7,
-                                                 C.c_void_p(out.data_ptr()), None))
+    # NULL prompt_lens and NULL params: the equal-length greedy call
+    capi.check(lib.blurr_llm_generate(dec.handle, stream, B, T, C.c_void_p(x.data_ptr()), None, None, 7,
+                                      C.c_void_p(out.data_ptr()), None))
+    assert torch.equal(out, dec.generate(x, 7))
     for batch in (0, B + 1):                                  # batch out of range
         with pytest.raises(capi.BlurrError):
-            capi.check(lib.blurr_llm_generate_ragged(dec.handle, stream, batch, T, C.c_void_p(x.data_ptr()), lens, 7,
-                                                     C.c_void_p(out.data_ptr()), None))
+            capi.check(lib.blurr_llm_generate(dec.handle, stream, batch, T, C.c_void_p(x.data_ptr()), lens, None, 7,
+                                              C.c_void_p(out.data_ptr()), None))
     assert torch.equal(dec.generate(x, 7, prompt_lens=[T] * B), ok)
     dec.check()
     dec.close()
@@ -315,50 +257,16 @@ def test_rejected_ragged_calls_leave_the_handle_working():
 # ---------------------------------------------------------------------------------------------------------------------
 @pytest.fixture(scope="module")
 def policy():
-    """Shrunk towers (depth 3) and a 2-layer 4096-wide decoder, as in tests/test_openvla_preprocess.py."""
-    B = 4
-    dino = openvla.VitEncoder.synthetic(openvla.dinov2_large_reg4_config(depth=3), DEV, max_batch=B, seed=3)
-    sig = openvla.VitEncoder.synthetic(openvla.siglip_so400m_config(depth=3), DEV, max_batch=B, seed=4)
-    proj = openvla.MlpProjector([2176, 8704, 4096, 4096], DEV, max_rows=B * 256)
-    g = torch.Generator(device=DEV).manual_seed(5)
-    for i, (n_out, n_in) in enumerate(((8704, 2176), (4096, 8704), (4096, 4096))):
-        proj.set_layer(i, (torch.randn((n_out, n_in), device=DEV, generator=g) * 0.02).to(torch.bfloat16),
-                       (torch.randn(n_out, device=DEV, generator=g) * 0.02).to(torch.bfloat16))
-    backbone = openvla.FusedVisionBackbone(dino, sig, proj)
-    cfg = openvla.LlamaShapedConfig(num_layers=2)
-    sd = openvla.synthetic_llama_state_dict(cfg, DEV, 0)
-    with torch.no_grad():
-        sd["lm_head.weight"].mul_(8.0)                       # spread the logits: fewer near-ties between rows
-    dec = openvla.LlamaDecoder.from_state_dict(cfg, sd, DEV, max_batch=B)
-    pre = openvla.ImagePreprocessor(480, 640, device=DEV)
-    pol = openvla.OpenVlaPolicy(pre, backbone, dec)
-    px = (torch.rand((B, 6, 224, 224), device=DEV, generator=g) * 2 - 1).to(torch.bfloat16)
-    yield pol, px
-    torch.cuda.synchronize()
-    dec.check()
-    for m in (pre, dino, sig, proj, dec):
-        m.close()
+    yield from small_policy()
 
 
-def _instructions(lengths, seed):
-    g = torch.Generator().manual_seed(seed)
-    rows = []
-    for n in lengths:
-        r = torch.randint(3, 32000, (n,), generator=g)
-        r[0] = 1
-        rows.append(r)
-    return rows
-
-
-Q01 = np.array([-0.03, -0.04, -0.02, -0.1, -0.1, -0.2, 0.0])
-Q99 = np.array([0.03, 0.04, 0.03, 0.1, 0.1, 0.2, 1.0])
 MASK = np.array([True] * 6 + [False])
 
 
 @pytest.mark.gpu
 def test_policy_prompt_forms_agree_and_rows_match_batch_one(policy):
     pol, px = policy
-    rows = _instructions([14, 3, 25, 9], 0)
+    rows = instructions([14, 3, 25, 9], 0)
     act, ids = pol.predict_action_from_pixels(px, rows, Q01, Q99, MASK, return_token_ids=True)
     assert act.shape == (4, 7) and ids.shape == (4, 7)
     for left in (True, False):
@@ -397,7 +305,7 @@ def test_policy_prompt_forms_agree_and_rows_match_batch_one(policy):
 @pytest.mark.gpu
 def test_policy_equal_length_list_is_bitwise_the_tensor_call(policy):
     pol, px = policy
-    rows = _instructions([17] * 4, 1)
+    rows = instructions([17] * 4, 1)
     a0, i0 = pol.predict_action_from_pixels(px, torch.stack(rows).to(DEV), Q01, Q99, MASK, return_token_ids=True)
     a1, i1 = pol.predict_action_from_pixels(px, rows, Q01, Q99, MASK, return_token_ids=True)
     assert torch.equal(i0, i1) and torch.equal(a0, a1)
@@ -406,7 +314,7 @@ def test_policy_equal_length_list_is_bitwise_the_tensor_call(policy):
 @pytest.mark.gpu
 def test_policy_per_row_statistics(policy):
     pol, px = policy
-    rows = _instructions([6, 11, 2, 20], 2)
+    rows = instructions([6, 11, 2, 20], 2)
     q01 = np.stack([Q01 * (1 + b) for b in range(4)])
     q99 = np.stack([Q99 * (1 + 2 * b) for b in range(4)])
     mask = np.stack([MASK, ~MASK, MASK, np.ones(7, bool)])

@@ -1,5 +1,5 @@
 """Sampled decoding on the OpenVLA path (`LlamaDecoder.generate(..., do_sample=True)`, `LlamaDecoder.sample`,
-`blurr_llm_generate_sampled`, `blurr_llm_sample`, `OpenVlaPolicy.predict_action(..., do_sample=True)`).
+`blurr_llm_generate` with `params`, `blurr_llm_sample`, `OpenVlaPolicy.predict_action(..., do_sample=True)`).
 
 The reference semantics are transformers' `generate(do_sample=True)`: fp32 logits -> Temperature -> TopK -> TopP warpers
 -> softmax -> one draw; oracle/openvla_sampling_oracle.py restates them with the kernel's Philox draw.
@@ -26,6 +26,7 @@ import pytest
 import torch
 
 from blurr_b200 import capi, openvla
+from llama_helpers import Q01, Q99, hf_llama, instructions, small_policy, synthetic_decoder
 from oracle import openvla_sampling_oracle as orc
 
 DEV = "cuda"
@@ -278,23 +279,6 @@ def test_draw_distribution_chi_square(kind, T, k, p):
 # ---------------------------------------------------------------------------------------------------------------------
 # GPU: sampled generate end to end
 # ---------------------------------------------------------------------------------------------------------------------
-def _hf_model(cfg, seed):
-    from transformers import LlamaConfig, LlamaForCausalLM
-    hc = LlamaConfig(hidden_size=cfg.hidden, intermediate_size=cfg.intermediate, num_hidden_layers=cfg.num_layers,
-                     num_attention_heads=cfg.num_heads, num_key_value_heads=cfg.num_kv_heads, head_dim=cfg.head_dim,
-                     vocab_size=cfg.vocab, max_position_embeddings=2048, rms_norm_eps=cfg.rms_eps, rope_theta=cfg.rope_theta,
-                     attn_implementation="eager", tie_word_embeddings=False)
-    torch.manual_seed(seed)
-    model = LlamaForCausalLM(hc).eval()
-    with torch.no_grad():
-        for name, p in model.named_parameters():
-            if "layernorm" in name or name.endswith("norm.weight"):
-                p.copy_(1.0 + 0.2 * torch.randn_like(p))
-            elif "embed_tokens" in name or "lm_head" in name:
-                p.mul_(4.0)                                   # logits spread over a few units: peaked and flat rows
-    return model.to(torch.bfloat16).to(DEV)
-
-
 GEN_CASES = [
     # hidden, heads, head_dim, inter, layers, vocab, lengths
     pytest.param(256, 2, 128, 512, 2, 1000, [8, 1, 5, 3], id="few-token"),
@@ -313,7 +297,7 @@ def test_sampled_generate_against_the_oracle_and_transformers(hidden, heads, hd,
     B, T = len(lens), int(lens.max())
     cfg = openvla.LlamaShapedConfig(num_layers=layers, hidden=hidden, num_heads=heads, num_kv_heads=heads, head_dim=hd,
                                     intermediate=inter, vocab=vocab, max_positions=T + n_new + 1, rms_eps=1e-6)
-    model = _hf_model(cfg, 0)
+    model = hf_llama(cfg, 0, head_scale=4.0)                # logits spread over a few units: peaked and flat rows
     dec = openvla.LlamaDecoder.from_state_dict(cfg, model.state_dict(), DEV, max_batch=B,
                                                inv_freq=model.model.rotary_emb.inv_freq.detach().float())
     g = torch.Generator(device=DEV).manual_seed(1)
@@ -358,36 +342,10 @@ def test_sampled_generate_against_the_oracle_and_transformers(hidden, heads, hd,
     dec.close()
 
 
-SHAPES = {
-    # hidden, heads, head_dim, inter, layers, vocab, batch, T_max
-    "few": (256, 2, 128, 512, 2, 1000, 4, 8),
-    "mid": (512, 4, 128, 1408, 2, 1064, 3, 37),
-    "b32": (1280, 10, 128, 2560, 2, 1000, 32, 12),
-    "b32-fused": (512, 8, 64, 1024, 1, 300, 32, 6),
-}
-
-
-def _decoder(name, n_new=7):
-    hidden, heads, hd, inter, layers, vocab, B, T = SHAPES[name]
-    cfg = openvla.LlamaShapedConfig(num_layers=layers, hidden=hidden, num_heads=heads, num_kv_heads=heads, head_dim=hd,
-                                    intermediate=inter, vocab=vocab, max_positions=T + n_new + 1)
-    sd = openvla.synthetic_llama_state_dict(cfg, DEV, 0)
-    with torch.no_grad():
-        for k, v in sd.items():
-            if "q_proj" in k or "k_proj" in k:
-                v.mul_(8.0)
-            if k.startswith("lm_head"):
-                v.mul_(4.0)
-    dec = openvla.LlamaDecoder.from_state_dict(cfg, sd, DEV, max_batch=B)
-    g = torch.Generator(device=DEV).manual_seed(7)
-    x = (torch.randn((B, T, hidden), device=DEV, generator=g) * 0.5).to(torch.bfloat16)
-    return dec, x
-
-
 @pytest.mark.gpu
 @pytest.mark.parametrize("name", ["few", "b32", "b32-fused"])
 def test_sampled_graph_replay_equals_eager_and_repeats(name):
-    dec, x = _decoder(name)
+    dec, x = synthetic_decoder(name)
     B, T = x.shape[:2]
     greedy = dec.generate(x, 7)
     greedy_launches = dec.last_launch_count
@@ -413,7 +371,7 @@ def test_sampled_graph_replay_equals_eager_and_repeats(name):
 @pytest.mark.gpu
 @pytest.mark.parametrize("name", ["few", "mid", "b32-fused"])
 def test_a_rows_ids_depend_only_on_its_prompt_and_seed(name):
-    dec, x = _decoder(name)
+    dec, x = synthetic_decoder(name)
     B, T = x.shape[:2]
     seeds = [1000 + b for b in range(B)]
     kw = dict(do_sample=True, temperature=1.0, top_k=0, top_p=0.95)
@@ -444,7 +402,7 @@ def test_a_rows_ids_depend_only_on_its_prompt_and_seed(name):
 @pytest.mark.gpu
 @pytest.mark.parametrize("name", ["few", "mid", "b32", "b32-fused"])
 def test_top_k_one_is_greedy(name):
-    dec, x = _decoder(name)
+    dec, x = synthetic_decoder(name)
     ids_g, lg = dec.generate(x, 7, return_logits=True)
     ids_s = dec.generate(x, 7, do_sample=True, top_k=1, temperature=0.8, top_p=0.5, seed=3)
     for b in range(x.shape[0]):
@@ -458,8 +416,8 @@ def test_top_k_one_is_greedy(name):
 
 
 @pytest.mark.gpu
-def test_rejected_sampled_calls_leave_the_handle_working():
-    dec, x = _decoder("few")
+def test_rejected_sampled_calls_and_null_params():
+    dec, x = synthetic_decoder("few")
     B, T = x.shape[:2]
     ok = dec.generate(x, 7, do_sample=True, seed=4)
     lib, stream = dec.lib, C.c_void_p(torch.cuda.current_stream().cuda_stream)
@@ -476,23 +434,24 @@ def test_rejected_sampled_calls_leave_the_handle_working():
            dict(top_k=-1), dict(top_p=-0.5), dict(top_p=1.01), dict(top_p=float("nan"))]
     for kw in bad:
         with pytest.raises(capi.BlurrError):
-            capi.check(lib.blurr_llm_generate_sampled(dec.handle, stream, B, T, C.c_void_p(x.data_ptr()), None, params(**kw), 7,
-                                                      C.c_void_p(out.data_ptr()), None))
+            capi.check(lib.blurr_llm_generate(dec.handle, stream, B, T, C.c_void_p(x.data_ptr()), None, params(**kw), 7,
+                                              C.c_void_p(out.data_ptr()), None))
         with pytest.raises(capi.BlurrError):
             capi.check(lib.blurr_llm_sample(dec.handle, stream, C.c_void_p(x.data_ptr()), B, dec.cfg.vocab, params(**kw), 0,
                                             C.c_void_p(out.data_ptr()), None))
     good = params()
-    with pytest.raises(capi.BlurrError):                                        # null params
-        capi.check(lib.blurr_llm_generate_sampled(dec.handle, stream, B, T, C.c_void_p(x.data_ptr()), None, None, 7,
-                                                  C.c_void_p(out.data_ptr()), None))
+    # NULL params: the greedy call
+    capi.check(lib.blurr_llm_generate(dec.handle, stream, B, T, C.c_void_p(x.data_ptr()), None, None, 7, C.c_void_p(out.data_ptr()),
+                                      None))
+    assert torch.equal(out, dec.generate(x, 7))
     lens = (C.c_int32 * B)(*([0] + [T] * (B - 1)))
     with pytest.raises(capi.BlurrError):                                        # a zero prompt length
-        capi.check(lib.blurr_llm_generate_sampled(dec.handle, stream, B, T, C.c_void_p(x.data_ptr()), lens, good, 7,
-                                                  C.c_void_p(out.data_ptr()), None))
+        capi.check(lib.blurr_llm_generate(dec.handle, stream, B, T, C.c_void_p(x.data_ptr()), lens, good, 7,
+                                          C.c_void_p(out.data_ptr()), None))
     for batch in (0, B + 1):
         with pytest.raises(capi.BlurrError):
-            capi.check(lib.blurr_llm_generate_sampled(dec.handle, stream, batch, T, C.c_void_p(x.data_ptr()), None, good, 7,
-                                                      C.c_void_p(out.data_ptr()), None))
+            capi.check(lib.blurr_llm_generate(dec.handle, stream, batch, T, C.c_void_p(x.data_ptr()), None, good, 7,
+                                              C.c_void_p(out.data_ptr()), None))
     with pytest.raises(capi.BlurrError):                                        # max_prompt_len + n_new > max_positions
         dec.generate(x, 9, do_sample=True, seed=4)
     with pytest.raises(capi.BlurrError):                                        # rows > max_batch
@@ -511,50 +470,14 @@ def test_rejected_sampled_calls_leave_the_handle_working():
 # ---------------------------------------------------------------------------------------------------------------------
 @pytest.fixture(scope="module")
 def policy():
-    """Shrunk towers (depth 3) and a 2-layer 4096-wide decoder, as in tests/test_openvla_ragged.py."""
-    B = 4
-    dino = openvla.VitEncoder.synthetic(openvla.dinov2_large_reg4_config(depth=3), DEV, max_batch=B, seed=3)
-    sig = openvla.VitEncoder.synthetic(openvla.siglip_so400m_config(depth=3), DEV, max_batch=B, seed=4)
-    proj = openvla.MlpProjector([2176, 8704, 4096, 4096], DEV, max_rows=B * 256)
-    g = torch.Generator(device=DEV).manual_seed(5)
-    for i, (n_out, n_in) in enumerate(((8704, 2176), (4096, 8704), (4096, 4096))):
-        proj.set_layer(i, (torch.randn((n_out, n_in), device=DEV, generator=g) * 0.02).to(torch.bfloat16),
-                       (torch.randn(n_out, device=DEV, generator=g) * 0.02).to(torch.bfloat16))
-    backbone = openvla.FusedVisionBackbone(dino, sig, proj)
-    cfg = openvla.LlamaShapedConfig(num_layers=2)
-    sd = openvla.synthetic_llama_state_dict(cfg, DEV, 0)
-    with torch.no_grad():
-        sd["lm_head.weight"].mul_(8.0)
-    dec = openvla.LlamaDecoder.from_state_dict(cfg, sd, DEV, max_batch=B)
-    pre = openvla.ImagePreprocessor(480, 640, device=DEV)
-    pol = openvla.OpenVlaPolicy(pre, backbone, dec)
-    px = (torch.rand((B, 6, 224, 224), device=DEV, generator=g) * 2 - 1).to(torch.bfloat16)
-    yield pol, px
-    torch.cuda.synchronize()
-    dec.check()
-    for m in (pre, dino, sig, proj, dec):
-        m.close()
-
-
-Q01 = np.array([-0.03, -0.04, -0.02, -0.1, -0.1, -0.2, 0.0])
-Q99 = np.array([0.03, 0.04, 0.03, 0.1, 0.1, 0.2, 1.0])
-
-
-def _instructions(lengths, seed):
-    g = torch.Generator().manual_seed(seed)
-    rows = []
-    for n in lengths:
-        r = torch.randint(3, 32000, (n,), generator=g)
-        r[0] = 1
-        rows.append(r)
-    return rows
+    yield from small_policy()
 
 
 @pytest.mark.gpu
 def test_policy_sampling_is_repeatable_and_composes(policy):
     pol, px = policy
     dec = pol.decoder
-    rows = _instructions([12, 12, 12, 12], 0)
+    rows = instructions([12, 12, 12, 12], 0)
     ids_t = torch.stack(rows).to(DEV)
     kw = dict(do_sample=True, temperature=0.7, top_k=50, top_p=0.9, seed=11)
     a1, i1 = pol.predict_action_from_pixels(px, ids_t, Q01, Q99, return_token_ids=True, **kw)
@@ -589,7 +512,7 @@ def test_policy_sampling_is_repeatable_and_composes(policy):
 def test_policy_top_k_one_is_greedy_and_default_top_k_is_50(policy):
     pol, px = policy
     dec = pol.decoder
-    rows = _instructions([14, 3, 25, 9], 1)
+    rows = instructions([14, 3, 25, 9], 1)
     a_g, i_g = pol.predict_action_from_pixels(px, rows, Q01, Q99, return_token_ids=True)
     a_1, i_1 = pol.predict_action_from_pixels(px, rows, Q01, Q99, return_token_ids=True, do_sample=True, top_k=1, seed=2)
     assert torch.equal(i_1, i_g) and torch.equal(a_1, a_g)
