@@ -21,7 +21,7 @@ LIB_PATH = os.path.join(LIB_DIR, "libblurr_pi0.so")
 INCLUDE_DIR = os.path.join(os.path.dirname(PKG_DIR), "include")
 
 SOURCES = ["gemm_tc.cu", "norm_consumers.cu", "attention.cu", "attention_tc.cu", "misc_kernels.cu", "engine.cu",
-           "preprocess.cu", "llm_kernels.cu", "llm_engine.cu", "vit_engine.cu"]
+           "preprocess.cu", "llm_kernels.cu", "llm_engine.cu", "vit_engine.cu", "act_head.cu"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",
     "-lineinfo", "-O3", "-std=c++17",

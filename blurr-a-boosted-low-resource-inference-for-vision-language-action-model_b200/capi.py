@@ -64,6 +64,18 @@ class LlmSamplingC(C.Structure):
     _fields_ = [("seed", C.c_uint64), ("temperature", C.c_float), ("top_k", C.c_int32), ("top_p", C.c_float)]
 
 
+class ActHeadConfigC(C.Structure):
+    """`blurr_act_head_config` (include/blurr_act_head.h): 28 bytes, ln_eps at 24."""
+
+    _fields_ = [
+        ("abi_version", C.c_int32), ("input_dim", C.c_int32), ("action_dim", C.c_int32), ("chunk", C.c_int32),
+        ("hidden_dim", C.c_int32), ("num_blocks", C.c_int32), ("ln_eps", C.c_float),
+    ]
+
+
+ACT_HEAD_ABI_VERSION = 1
+
+
 class VitConfigC(C.Structure):
     """`blurr_vit_config` (include/blurr_vit.h)."""
 
@@ -149,6 +161,9 @@ _SIGNATURES = [
     ("blurr_llm_generate", C.c_int,
      [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.POINTER(C.c_int32), C.POINTER(LlmSamplingC), C.c_int, C.c_void_p,
       C.c_void_p]),
+    ("blurr_llm_forward_rows", C.c_int,
+     [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.POINTER(C.c_int32), C.POINTER(C.c_int32), C.POINTER(C.c_int32),
+      C.c_int, C.c_void_p]),
     ("blurr_llm_sample", C.c_int,
      [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.POINTER(LlmSamplingC), C.c_int, C.c_void_p, C.c_void_p]),
     ("blurr_llm_set_option", C.c_int, [C.c_void_p, C.c_char_p, C.c_int64]),
@@ -178,6 +193,17 @@ _SIGNATURES = [
      [C.c_int, C.c_int, C.POINTER(C.c_int32), C.POINTER(C.c_int32), C.c_int]),
 ]
 DECLARED_SYMBOLS = [s[0] for s in _SIGNATURES]
+# include/blurr_act_head.h (OpenVLA-OFT's action head), listed apart from the three headers above
+_ACT_HEAD_SIGNATURES = [
+    ("blurr_act_head_create", C.c_int, [C.POINTER(ActHeadConfigC), C.c_int, C.c_int, C.POINTER(C.c_void_p)]),
+    ("blurr_act_head_destroy", None, [C.c_void_p]),
+    ("blurr_act_head_set_weight", C.c_int, [C.c_void_p, C.c_char_p, C.c_void_p, C.POINTER(C.c_int64), C.c_int]),
+    ("blurr_act_head_finalize", C.c_int, [C.c_void_p]),
+    ("blurr_act_head_forward", C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]),
+    ("blurr_act_head_check", C.c_int, [C.c_void_p, C.c_void_p]),
+    ("blurr_act_head_last_launch_count", C.c_int64, [C.c_void_p]),
+]
+ACT_HEAD_SYMBOLS = [s[0] for s in _ACT_HEAD_SIGNATURES]
 
 _lib: Optional[C.CDLL] = None
 
@@ -195,7 +221,7 @@ def load_library(path: Optional[str] = None) -> C.CDLL:
         )
     lib = C.CDLL(p)
     lenient = bool(os.environ.get("BLURR_PI0_LIB_LENIENT"))      # tooling only: A/B against an older build
-    for name, restype, argtypes in _SIGNATURES:
+    for name, restype, argtypes in _SIGNATURES + _ACT_HEAD_SIGNATURES:
         if lenient and not hasattr(lib, name):
             continue
         fn = getattr(lib, name)          # AttributeError if the .so does not export it

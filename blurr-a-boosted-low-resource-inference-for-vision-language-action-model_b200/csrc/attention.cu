@@ -700,4 +700,64 @@ cudaError_t launch_mha_attention(cudaStream_t stream, const MhaAttnArgs& m, cons
     return cudaErrorInvalidValue;
 }
 
+// OFT's prefill (llm_engine.cu blurr_llm_forward_rows): causal over the prompt, bidirectional inside the action block,
+// per-sequence lengths and block starts read at run time, up to 384 keys.  A kernel of its own so that MODE 2's
+// instantiations above keep their code.
+template <int HD_PAD, int BM>
+__global__ void __launch_bounds__(kAttnThreads) attn_block_kernel(const AttnMmaArgs a, const int* seq_len, const int* block_start) {
+    extern __shared__ __align__(16) uint8_t smem_attn[];
+    trace_stamp(a.trace, 0);
+    pdl_wait();
+    pdl_trigger();
+    trace_stamp(a.trace, 1);
+    attn_mma_body<HD_PAD, BM, 3, kAttnMaxBlocksWide>(a, smem_attn, blockIdx.x, blockIdx.y, blockIdx.z, seq_len, block_start);
+    trace_stamp(a.trace, 2);
+}
+
+template <int HD_PAD, int BM>
+static cudaError_t launch_attn_block(cudaStream_t stream, const AttnMmaArgs& a, const int* seq_len, const int* block_start, int rows,
+                                     int heads, int batch) {
+    const size_t smem = attn_smem_bytes<HD_PAD, BM>(a.n_keys);      // 168 KB at head_dim 128, BM 64, 384 keys
+    static bool attr = false;
+    if (!attr) {
+        int dev = 0, optin = 0;
+        cudaError_t e = cudaGetDevice(&dev);
+        if (e == cudaSuccess) e = cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev);
+        if (e != cudaSuccess) return e;
+        if (static_cast<size_t>(optin) < kAttnSmemMax) return cudaErrorInvalidConfiguration;
+        e = cudaFuncSetAttribute(attn_block_kernel<HD_PAD, BM>, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(kAttnSmemMax));
+        if (e != cudaSuccess) return e;
+        attr = true;
+    }
+    if (smem > kAttnSmemMax) return cudaErrorInvalidValue;
+    dim3 grid((rows + BM - 1) / BM, heads, batch);
+    return launch_kernel(attn_block_kernel<HD_PAD, BM>, grid, dim3(kAttnThreads), smem, stream, a, seq_len, block_start);
+}
+
+cudaError_t launch_mha_block_attention(cudaStream_t stream, const MhaAttnArgs& m, const int* block_start) {
+    if (m.n_keys > kAttnMaxBlocksWide * kBK || m.n_kv_heads != m.n_heads || m.q_pos0 != 0 ||
+        m.n_keys != m.q_per_sample || m.seq_len == nullptr || block_start == nullptr)
+        return cudaErrorInvalidValue;
+    AttnMmaArgs a{};
+    const int width = m.n_heads * m.head_dim;
+    a.q = m.q; a.ldq = width; a.q_col0 = 0; a.q_per_sample = m.q_per_sample;
+    a.k = m.k_cache; a.ldk = width; a.k_col0 = 0; a.kv_per_sample = m.n_slots;
+    a.v = m.v_cache; a.ldv = width; a.v_col0 = 0;
+    a.out = m.out; a.ldo = width; a.o_col0 = 0;
+    a.hd = m.head_dim; a.head_stride_q = m.head_dim; a.head_stride_kv = m.head_dim; a.n_keys = m.n_keys;
+    a.scale = m.scale; a.mask = nullptr; a.q_row_offset = 0; a.trace = m.trace;
+    const int bm = attn_tile_rows(m.q_per_sample, m.n_heads, m.batch, 64);
+    const int* L = m.seq_len;
+    if (m.head_dim == 128) {
+        if (bm == 16) return launch_attn_block<128, 16>(stream, a, L, block_start, m.q_per_sample, m.n_heads, m.batch);
+        if (bm == 32) return launch_attn_block<128, 32>(stream, a, L, block_start, m.q_per_sample, m.n_heads, m.batch);
+        return launch_attn_block<128, 64>(stream, a, L, block_start, m.q_per_sample, m.n_heads, m.batch);
+    }
+    if (m.head_dim == 64) {
+        if (bm == 16) return launch_attn_block<64, 16>(stream, a, L, block_start, m.q_per_sample, m.n_heads, m.batch);
+        return launch_attn_block<64, 32>(stream, a, L, block_start, m.q_per_sample, m.n_heads, m.batch);
+    }
+    return cudaErrorInvalidValue;
+}
+
 }  // namespace blurr

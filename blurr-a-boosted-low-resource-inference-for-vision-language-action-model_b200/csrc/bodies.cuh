@@ -327,6 +327,7 @@ __device__ __forceinline__ void rope_kv_body(const RopeKvArgs& a, const int t, c
 static constexpr int kAttnThreads = 256;   // 8 warps per attention tile
 static constexpr int kBK = 64;             // keys per streamed block
 static constexpr int kAttnMaxBlocks = 5;   // up to 320 keys resident in shared memory
+static constexpr int kAttnMaxBlocksWide = 6;   // MODE 3 (block-bidirectional prefill): up to 384 keys
 
 __device__ __forceinline__ void attn_bar_sync() { __syncthreads(); }
 
@@ -357,10 +358,12 @@ __device__ __forceinline__ void load_rows_async(bf16* dst, const bf16* src, int 
 // as they land; the V blocks are requested into the same buffers as soon as the logits are done, so
 // their latency hides behind the softmax.
 // MODE: 0 = logits * scale (SigLIP), 1 = Gemma chain (1/16, soft-clamp, additive mask), 2 = logits * scale with the
-// causal mask computed from positions (Llama-style MHA: query row r sits at key position q_row_offset + r)
-template <int HD_PAD, int BM, int MODE>
+// causal mask computed from positions (Llama-style MHA: query row r sits at key position q_row_offset + r), 3 = MODE 2's
+// logits with a per-sequence rule read from `seq_len[b]` / `block_start[b]` (OFT's action block): query p sees key k iff
+// k < seq_len and (k <= p, or p >= block_start and k >= block_start).  MAXB: key blocks a row's softmax holds.
+template <int HD_PAD, int BM, int MODE, int MAXB = kAttnMaxBlocks>
 __device__ __forceinline__ void attn_mma_body(const AttnMmaArgs& a, uint8_t* smem_attn, const int qt, const int h,
-                                              const int b) {
+                                              const int b, const int* seq_len = nullptr, const int* block_start = nullptr) {
     // BM query rows per tile: 16 at batch 1 (most tiles, least latency), 32/64 for batched episodes
     // (K/V of a head are re-read once per tile, so larger tiles cut the L2 -> SM traffic)
     constexpr int WR = BM / 16;                 // row groups
@@ -374,7 +377,15 @@ __device__ __forceinline__ void attn_mma_body(const AttnMmaArgs& a, uint8_t* sme
     constexpr int LDS_MIN = WC * NP_PV * 16 > HD_PAD ? WC * NP_PV * 16 : HD_PAD;
     constexpr int LDS = LDS_MIN + 8;            // smem row stride (elements), conflict-free for ldmatrix
     // causal (MODE 2): keys past the tile's last query position are masked for every row - never load them
-    const int n_keys_tile = MODE == 2 ? min(a.n_keys, a.q_row_offset + qt * BM + BM) : a.n_keys;
+    int n_keys_tile = MODE == 2 ? min(a.n_keys, a.q_row_offset + qt * BM + BM) : a.n_keys;
+    int blk_len = 0, blk0 = 0;
+    if constexpr (MODE == 3) {
+        // keys past the sequence are never seen; a tile without a query in the action block needs the causal bound only
+        blk_len = max(1, min(seq_len[b], a.n_keys));           // the host validates both; never read out of range
+        blk0 = max(1, min(block_start[b], blk_len));
+        const int last_q = a.q_row_offset + qt * BM + BM - 1;
+        n_keys_tile = min(blk_len, last_q >= blk0 ? a.n_keys : last_q + 1);
+    }
     const int nkb = (n_keys_tile + kBK - 1) / kBK;
     const int ldl = nkb * kBK + 8;              // logit row stride (elements)
     bf16* Qs = reinterpret_cast<bf16*>(smem_attn);
@@ -479,6 +490,12 @@ __device__ __forceinline__ void attn_mma_body(const AttnMmaArgs& a, uint8_t* sme
                         if (kcol > qpos) s0 = -INFINITY;
                         if (kcol + 1 > qpos) s1 = -INFINITY;
                     }
+                    if constexpr (MODE == 3) {
+                        const int qpos = a.q_row_offset + q_row0 + r;
+                        const bool in_blk = qpos >= blk0;
+                        if (!(kcol < blk_len && (kcol <= qpos || (in_blk && kcol >= blk0)))) s0 = -INFINITY;
+                        if (!(kcol + 1 < blk_len && (kcol + 1 <= qpos || (in_blk && kcol + 1 >= blk0)))) s1 = -INFINITY;
+                    }
                 }
                 *reinterpret_cast<uint32_t*>(Ls + r * ldl + kcol) = pack_bf16x2(s0, s1);
             }
@@ -495,7 +512,7 @@ __device__ __forceinline__ void attn_mma_body(const AttnMmaArgs& a, uint8_t* sme
     // ---------------- softmax: fp32 over bf16 logits, result bf16 in place ----------------
     for (int rr = 0; rr < BM / 8; ++rr) {
         bf16* lrow = Ls + (warp * (BM / 8) + rr) * ldl;
-        constexpr int PER_LANE = kAttnMaxBlocks * kBK / 32;     // 10 logits per lane
+        constexpr int PER_LANE = MAXB * kBK / 32;               // 10 logits per lane (12 at 384 keys)
         float x[PER_LANE];
         float m = -INFINITY;
 #pragma unroll

@@ -187,6 +187,10 @@ struct MhaAttnArgs {
     const int* seq_len; int len_off;
 };
 struct RopeMhaArgs;
+// OFT's block-bidirectional prefill (attention.cu, up to 384 keys): q_per_sample == n_keys rows per sequence from position
+// 0; sequence b's query p sees key k iff k < seq_len[b] and (k <= p, or p >= block_start[b] and k >= block_start[b]).
+// a.seq_len and block_start are device arrays [batch], read at run time; block_start[b] == seq_len[b] is plain causal.
+cudaError_t launch_mha_block_attention(cudaStream_t stream, const MhaAttnArgs& a, const int* block_start);
 // decode steps of <= 2 waves of (sequence, head) CTAs can do the new token's RoPE + cache append themselves
 bool mha_decode_fuses_rope(const MhaAttnArgs& a);
 cudaError_t launch_mha_attention(cudaStream_t stream, const MhaAttnArgs& a, const RopeMhaArgs* fused_rope = nullptr);
@@ -213,6 +217,13 @@ cudaError_t launch_embed_rows(cudaStream_t stream, const int64_t* ids, int n, co
 // is seq_len[b] - 1 instead of `row`
 cudaError_t launch_gather_rows(cudaStream_t stream, const bf16* src, int batch, int rows_per_seq, int row, int width, bf16* dst,
                                const int* seq_len = nullptr);
+// dst[b][i] = src[b * rows_per_seq + row_start[b] + i] for i < n_rows (row_start: device [batch], read at run time)
+cudaError_t launch_gather_row_block(cudaStream_t stream, const bf16* src, int batch, int rows_per_seq, const int* row_start, int n_rows,
+                                    int width, bf16* dst);
+// tile-packed weight (gemm_tc.h) <- src rows [rows][cols]; destination row = r * row_mul + row_off (llm_engine.cu)
+cudaError_t launch_pack_rows(cudaStream_t stream, const bf16* src, int rows, int cols, bf16* dst, int row_mul, int row_off, int kb_total);
+// K slices of a few-token split-K GEMM over `tiles` weight tiles: as few, as full waves of 148 CTAs as possible (llm_engine.cu)
+int pick_splitk_waves(int tiles, int kb_total);
 // x[b][t][:] = 0 for seq_len[b] <= t < rows_per_seq: the pad rows of a ragged prompt batch (device lengths, read at run time)
 cudaError_t launch_zero_pad_rows(cudaStream_t stream, bf16* x, int batch, int rows_per_seq, int width, const int* seq_len);
 // ids[b] = argmax over logits[b][0..vocab) (lowest index among equal maxima, like torch.argmax on CPU)

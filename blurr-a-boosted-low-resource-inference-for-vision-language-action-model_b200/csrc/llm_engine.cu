@@ -54,6 +54,8 @@ constexpr int kTraceMax = 4096;
 constexpr int kMaxKeptLogits = 16;    // generated tokens whose logits blurr_llm_generate can return
 constexpr int kMidTokens = 288;       // up to here o / down run as chunked split-K (plan_mid_tokens)
 constexpr int kFewTokens = 32;        // at most this many token rows: split-K partials + consumers (weight streaming)
+constexpr int kGenerateMaxPositions = 320;     // generate's decode kernels hold a sequence's logits in sc[320]
+constexpr int kForwardMaxPositions = 384;      // blurr_llm_forward_rows: bodies.cuh kAttnMaxBlocksWide x kBK keys (MODE 3)
 
 struct Lin { bf16* w = nullptr; int Nw = 0, K = 0; };
 struct Layer { Lin qkv, o, gu, down; bf16 *in_ln = nullptr, *post_ln = nullptr; };
@@ -69,6 +71,14 @@ __global__ void llm_pack_rows_kernel(const bf16* __restrict__ src, int rows, int
 }
 
 }  // namespace
+
+namespace blurr {
+cudaError_t launch_pack_rows(cudaStream_t stream, const bf16* src, int rows, int cols, bf16* dst, int row_mul, int row_off, int kb_total) {
+    const size_t total = static_cast<size_t>(rows) * cols;
+    llm_pack_rows_kernel<<<static_cast<unsigned>((total + 255) / 256), 256, 0, stream>>>(src, rows, cols, dst, row_mul, row_off, kb_total);
+    return cudaGetLastError();
+}
+}  // namespace blurr
 
 struct blurr_llm {
     blurr_llm_config cfg{};
@@ -88,9 +98,11 @@ struct blurr_llm {
     int64_t *ids = nullptr, *out_ids = nullptr;
     int* d_err = nullptr;
     // per-row inputs the captured kernels read at replay, so one graph serves every vector of them: the prompt lengths of
-    // a ragged call (d_lens) and the sampling parameters of a sampled one (d_sampling).  h_stage is their pinned staging
-    // copy ([max_batch] parameters, then [max_batch] lengths), reused once `staged` says the last upload has left it.
-    int* d_lens = nullptr;
+    // a ragged call or sequence lengths of forward_rows (d_lens), forward_rows' block and row starts (d_blk, d_row0: the
+    // same allocation) and the sampling parameters of a sampled call (d_sampling).  h_stage is their pinned staging copy
+    // ([max_batch] parameters, then [max_batch] each of lengths, block starts, row starts), reused once `staged` says the
+    // last upload has left it.
+    int *d_lens = nullptr, *d_blk = nullptr, *d_row0 = nullptr;
     SampleParams* d_sampling = nullptr;
     unsigned char* h_stage = nullptr;
     cudaEvent_t staged = nullptr;
@@ -99,7 +111,8 @@ struct blurr_llm {
     bool finalized = false, use_graph = true;
     int64_t launches = 0, weight_bytes = 0;
     struct GraphEntry { cudaGraph_t graph; cudaGraphExec_t exec; int64_t launches; };
-    std::map<std::tuple<int, int, int, int, int, int>, GraphEntry> graphs;     // (batch, prompt_len, n_new, logits, ragged, sampled)
+    // (batch, prompt_len, n_new, logits, ragged, sampled, forward_rows); forward_rows: (batch, max_len, 0, 0, 0, 0, 1)
+    std::map<std::tuple<int, int, int, int, int, int, int>, GraphEntry> graphs;
     // in-graph timeline (option "trace"): every kernel stamps %globaltimer at entry / after its dependency wait / at exit
     bool trace = false;
     unsigned long long* trace_buf = nullptr;
@@ -143,8 +156,8 @@ extern "C" int blurr_llm_create(const blurr_llm_config* cfg, int device, int max
     if ((c.num_heads * c.head_dim) % 128 || c.hidden > 4096 * 2)
         return fail(BLURR_ERR_INVALID, "num_heads * head_dim must be a multiple of 128; hidden <= 8192");
     if (c.hidden > 4096) return fail(BLURR_ERR_INVALID, "the RMSNorm consumer covers rows of up to 4096 columns");
-    if (c.max_positions < 2 || c.max_positions > 320)
-        return fail(BLURR_ERR_INVALID, "max_positions must be in 2..320 (the attention keeps every key of a head in shared memory)");
+    if (c.max_positions < 2 || c.max_positions > kForwardMaxPositions)
+        return fail(BLURR_ERR_INVALID, "max_positions must be in 2..384 (the attention keeps every key of a head in shared memory)");
     if (max_batch > kFewTokens) return fail(BLURR_ERR_INVALID, "max_batch <= 32 (one decode step is a few-token GEMM)");
     int ndev = 0;
     if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0)
@@ -193,9 +206,10 @@ extern "C" int blurr_llm_create(const blurr_llm_config* cfg, int device, int max
     h->ids = static_cast<int64_t*>(dalloc(h, static_cast<size_t>(max_batch) * 8));
     h->out_ids = static_cast<int64_t*>(dalloc(h, static_cast<size_t>(max_batch) * c.max_positions * 8));
     h->d_err = static_cast<int*>(dalloc(h, 16));
-    h->d_lens = static_cast<int*>(dalloc(h, static_cast<size_t>(max_batch) * 4));
+    h->d_lens = static_cast<int*>(dalloc(h, static_cast<size_t>(max_batch) * 3 * 4));
+    if (h->d_lens) { h->d_blk = h->d_lens + max_batch; h->d_row0 = h->d_lens + 2 * max_batch; }
     h->d_sampling = static_cast<SampleParams*>(dalloc(h, static_cast<size_t>(max_batch) * sizeof(SampleParams)));
-    if (cudaMallocHost(&h->h_stage, static_cast<size_t>(max_batch) * (sizeof(SampleParams) + 4)) != cudaSuccess) h->h_stage = nullptr;
+    if (cudaMallocHost(&h->h_stage, static_cast<size_t>(max_batch) * (sizeof(SampleParams) + 3 * 4)) != cudaSuccess) h->h_stage = nullptr;
     if (cudaEventCreateWithFlags(&h->staged, cudaEventDisableTiming) != cudaSuccess) h->staged = nullptr;
     ok &= h->d_lens && h->d_sampling && h->h_stage && h->staged;
     ok &= h->embed && h->final_norm && h->IN && h->X && h->XN && h->Q && h->AO && h->HM && h->LIN && h->LAST && h->LOGITS &&
@@ -207,9 +221,7 @@ extern "C" int blurr_llm_create(const blurr_llm_config* cfg, int device, int max
 }
 
 static int pack(const bf16* src, int rows, int cols, Lin& L, int row_mul, int row_off) {
-    const size_t total = static_cast<size_t>(rows) * cols;
-    llm_pack_rows_kernel<<<static_cast<unsigned>((total + 255) / 256), 256>>>(src, rows, cols, L.w, row_mul, row_off, L.K / 64);
-    const cudaError_t e = cudaGetLastError();
+    const cudaError_t e = launch_pack_rows(nullptr, src, rows, cols, L.w, row_mul, row_off, L.K / 64);
     return e == cudaSuccess ? 0 : fail(BLURR_ERR_CUDA, std::string("weight repack: ") + cudaGetErrorString(e));
 }
 
@@ -292,10 +304,8 @@ extern "C" int blurr_llm_finalize(blurr_llm_t* h) {
     return 0;
 }
 
-namespace {
-
 // K slices of a few-token GEMM: tiles * S CTAs in as few, as full waves of 148 as possible (each slice >= 4 k-blocks)
-int pick_splitk(int tiles, int kb_total) {
+int blurr::pick_splitk_waves(int tiles, int kb_total) {
     int best_s = 1;
     double best = 0.0;
     for (int s = 1; s <= 16; ++s) {
@@ -306,6 +316,8 @@ int pick_splitk(int tiles, int kb_total) {
     }
     return best_s;
 }
+
+namespace {
 
 struct Run {
     blurr_llm* h;
@@ -330,7 +342,7 @@ struct Run {
         c.epi = epi; c.splitk = 1; c.glu_act = 1; c.w_static = 1;
         c.out = out; c.ldo = ldo;
         if (epi == EPI_PARTIAL) {
-            c.splitk = T <= kFewTokens ? pick_splitk(L.Nw / 128, (L.K + 63) / 64)
+            c.splitk = T <= kFewTokens ? pick_splitk_waves(L.Nw / 128, (L.K + 63) / 64)
                                        : gemm_plan_chunked_splitk(T, L.Nw, L.K, h->ws_floats, &c.bn_override);
             c.partial = h->ws;
         }
@@ -371,7 +383,8 @@ struct Run {
     // One decoder layer over B sequences x Tq new tokens at positions pos0..pos0+Tq-1 (modeling_llama.py LlamaDecoderLayer).
     // `lens` (decode of a ragged batch, Tq == 1): sequence b's token sits at position lens[b] + step - 1 instead and
     // attends lens[b] + step keys; pos0 is then the batch's largest position.
-    void layer(int l, int B, int Tq, int pos0, const bf16* next_norm, const int* lens = nullptr, int step = 0) {
+    // `blk` (forward_rows, pos0 == 0): the attention takes OFT's rule with lengths d_lens and block starts blk.
+    void layer(int l, int B, int Tq, int pos0, const bf16* next_norm, const int* lens = nullptr, int step = 0, const int* blk = nullptr) {
         const auto& c = h->cfg;
         Layer& L = h->layers[l];
         const int T = B * Tq, QW = c.num_heads * c.head_dim, KVW = c.num_kv_heads * c.head_dim;
@@ -392,13 +405,19 @@ struct Run {
         m.n_slots = c.max_positions; m.n_keys = pos0 + Tq; m.batch = B; m.n_heads = c.num_heads; m.n_kv_heads = c.num_kv_heads;
         m.head_dim = c.head_dim; m.scale = static_cast<float>(std::pow(static_cast<double>(c.head_dim), -0.5)); m.out = h->AO;
         m.seq_len = lens; m.len_off = step;
-        const bool fuse = few && Tq == 1 && mha_decode_fuses_rope(m);       // decode: RoPE + append inside the attention kernel
+        const bool fuse = blk == nullptr && few && Tq == 1 && mha_decode_fuses_rope(m);       // decode: RoPE + append inside the attention kernel
         if (!fuse) {
             r.trace = slot("rope_mha");
             if (!rc) launched(launch_rope_mha(st, r), "rope_mha");
         }
-        m.trace = slot(Tq == 1 ? (fuse ? "rope+mha_decode" : "mha_decode") : "mha_prefill");
-        if (!rc) launched(launch_mha_attention(st, m, fuse ? &r : nullptr), "mha_attention");
+        if (blk != nullptr) {
+            m.seq_len = h->d_lens; m.len_off = 0;
+            m.trace = slot("mha_block_prefill");
+            if (!rc) launched(launch_mha_block_attention(st, m, blk), "mha_block_attention");
+        } else {
+            m.trace = slot(Tq == 1 ? (fuse ? "rope+mha_decode" : "mha_decode") : "mha_prefill");
+            if (!rc) launched(launch_mha_attention(st, m, fuse ? &r : nullptr), "mha_attention");
+        }
         // o_proj + residual + post-attention norm
         s = gemm(L.o, h->AO, T, part ? EPI_PARTIAL : EPI_STORE, h->LIN, L.o.Nw);
         consumer(part ? s : 0, part ? nullptr : h->LIN, T, c.hidden, L.o.Nw, h->X, h->X, L.post_ln, h->XN);
@@ -439,15 +458,20 @@ struct Run {
 // `ragged`: sequence b's prompt is rows 0 .. d_lens[b] - 1 of its T rows; the rest are pads.  Prefill runs over all T rows
 // unchanged (pads come after the real rows, so the causal mask hides them from every real query); the pads are zeroed
 // first, the first token is read from row d_lens[b] - 1, and decode step i places sequence b's token at d_lens[b] + i - 1.
-void run_generate(Run& R, int B, int T, int n_new, bool keep_logits, bool ragged, bool sampled) {
+void reset_trace(Run& R) {
     blurr_llm* h = R.h;
-    const auto& c = h->cfg;
-    const int L = c.num_layers;
     if (h->trace && h->trace_buf) {
         h->trace_labels.clear();
         if (cudaMemsetAsync(h->trace_buf, 0xFF, static_cast<size_t>(kTraceMax) * 4 * sizeof(unsigned long long), R.st) != cudaSuccess)
             R.rc = fail(BLURR_ERR_CUDA, "trace reset failed");
     }
+}
+
+void run_generate(Run& R, int B, int T, int n_new, bool keep_logits, bool ragged, bool sampled) {
+    blurr_llm* h = R.h;
+    const auto& c = h->cfg;
+    const int L = c.num_layers;
+    reset_trace(R);
     const int* lens = ragged ? h->d_lens : nullptr;
     if (ragged && !R.rc) R.launched(launch_zero_pad_rows(R.st, h->IN, B, T, c.hidden, lens), "zero_pad_rows");
     // ---- prefill: X <- inputs_embeds, XN <- input norm of layer 0 ----
@@ -464,6 +488,57 @@ void run_generate(Run& R, int B, int T, int n_new, bool keep_logits, bool ragged
     }
 }
 
+// forward_rows: the prefill schedule over B x T rows with OFT's attention rule (lengths d_lens, block starts d_blk); pads
+// are zeroed first, and XN ends as the final norm's output of every row.
+void run_forward_rows(Run& R, int B, int T) {
+    blurr_llm* h = R.h;
+    const auto& c = h->cfg;
+    const int L = c.num_layers;
+    reset_trace(R);
+    if (!R.rc) R.launched(launch_zero_pad_rows(R.st, h->IN, B, T, c.hidden, h->d_lens), "zero_pad_rows");
+    R.consumer(0, nullptr, B * T, c.hidden, c.hidden, h->IN, h->X, h->layers[0].in_ln, h->XN);
+    for (int l = 0; l < L; ++l) R.layer(l, B, T, 0, l + 1 < L ? h->layers[l + 1].in_ln : h->final_norm, nullptr, 0, h->d_blk);
+}
+
+using GraphKey = std::tuple<int, int, int, int, int, int, int>;
+
+// Runs `body` on `st`: eagerly (option use_cuda_graph 0), or as the CUDA graph cached under `key`, captured on first use
+// after one warm run (attribute setup, tensor maps).  h->launches ends as the launch count of one run.
+template <typename Body>
+int run_graph(blurr_llm* h, cudaStream_t st, const GraphKey& key, Body body) {
+    h->launches = 0;
+    Run R{h, st};
+    if (!h->use_graph) {
+        body(R);
+        return R.rc;
+    }
+    auto it = h->graphs.find(key);
+    if (it == h->graphs.end()) {
+        body(R);
+        if (R.rc) return R.rc;
+        LLM_CUDA_TRY(cudaStreamSynchronize(st));
+        h->launches = 0;
+        cudaStream_t cs;
+        LLM_CUDA_TRY(cudaStreamCreateWithFlags(&cs, cudaStreamNonBlocking));
+        Run C{h, cs};
+        cudaError_t e = cudaStreamBeginCapture(cs, cudaStreamCaptureModeThreadLocal);
+        if (e != cudaSuccess) { cudaStreamDestroy(cs); return fail(BLURR_ERR_CUDA, "graph capture begin failed"); }
+        body(C);
+        cudaGraph_t g = nullptr;
+        e = cudaStreamEndCapture(cs, &g);
+        cudaStreamDestroy(cs);
+        if (C.rc) { if (g) cudaGraphDestroy(g); return C.rc; }
+        if (e != cudaSuccess || !g) return fail(BLURR_ERR_CUDA, std::string("graph capture failed: ") + cudaGetErrorString(e));
+        cudaGraphExec_t ex = nullptr;
+        e = cudaGraphInstantiate(&ex, g, 0);
+        if (e != cudaSuccess) { cudaGraphDestroy(g); return fail(BLURR_ERR_CUDA, std::string("graph instantiate failed: ") + cudaGetErrorString(e)); }
+        it = h->graphs.emplace(key, blurr_llm::GraphEntry{g, ex, h->launches}).first;
+    }
+    LLM_CUDA_TRY(cudaGraphLaunch(it->second.exec, st));
+    h->launches = it->second.launches;
+    return 0;
+}
+
 }  // namespace
 
 extern "C" int blurr_llm_embed(blurr_llm_t* h, void* cuda_stream, const int64_t* ids, int n, void* rows_out) {
@@ -475,20 +550,24 @@ extern "C" int blurr_llm_embed(blurr_llm_t* h, void* cuda_stream, const int64_t*
     return 0;
 }
 
-// Uploads the per-row inputs a graph reads at replay (host arrays of `rows` entries, either may be null) through the pinned
-// staging buffer, on `st` ahead of the launch.
-static int stage_rows(blurr_llm_t* h, cudaStream_t st, int rows, const int32_t* lens, const blurr_llm_sampling* params) {
-    if (!lens && !params) return 0;
+// Uploads the per-row inputs a graph reads at replay (host arrays of `rows` entries, any may be null) through the pinned
+// staging buffer, on `st` ahead of the launch: lengths -> d_lens, block starts -> d_blk, row starts -> d_row0.
+static int stage_rows(blurr_llm_t* h, cudaStream_t st, int rows, const int32_t* lens, const blurr_llm_sampling* params,
+                      const int32_t* blk = nullptr, const int32_t* row0 = nullptr) {
+    if (!lens && !params && !blk && !row0) return 0;
     LLM_CUDA_TRY(cudaEventSynchronize(h->staged));              // the previous upload has read the staging buffer
     unsigned char* stage_params = h->h_stage;
-    unsigned char* stage_lens = h->h_stage + static_cast<size_t>(h->max_batch) * sizeof(SampleParams);
     if (params) {
         memcpy(stage_params, params, static_cast<size_t>(rows) * sizeof(SampleParams));
         LLM_CUDA_TRY(cudaMemcpyAsync(h->d_sampling, stage_params, static_cast<size_t>(rows) * sizeof(SampleParams), cudaMemcpyHostToDevice, st));
     }
-    if (lens) {
-        memcpy(stage_lens, lens, static_cast<size_t>(rows) * 4);
-        LLM_CUDA_TRY(cudaMemcpyAsync(h->d_lens, stage_lens, static_cast<size_t>(rows) * 4, cudaMemcpyHostToDevice, st));
+    const int32_t* src[3] = {lens, blk, row0};
+    int* dst[3] = {h->d_lens, h->d_blk, h->d_row0};
+    for (int i = 0; i < 3; ++i) {
+        if (!src[i]) continue;
+        unsigned char* stage = h->h_stage + static_cast<size_t>(h->max_batch) * (sizeof(SampleParams) + 4 * i);
+        memcpy(stage, src[i], static_cast<size_t>(rows) * 4);
+        LLM_CUDA_TRY(cudaMemcpyAsync(dst[i], stage, static_cast<size_t>(rows) * 4, cudaMemcpyHostToDevice, st));
     }
     LLM_CUDA_TRY(cudaEventRecord(h->staged, st));
     return 0;
@@ -520,6 +599,8 @@ extern "C" int blurr_llm_generate(blurr_llm_t* h, void* cuda_stream, int batch, 
     if (batch < 1 || batch > h->max_batch) return fail(BLURR_ERR_INVALID, std::string(fn) + ": batch out of range");
     if (max_prompt_len < 1 || n_new < 1 || max_prompt_len + n_new > c.max_positions)
         return fail(BLURR_ERR_INVALID, std::string(fn) + ": max_prompt_len + n_new exceeds max_positions");
+    if (max_prompt_len + n_new > kGenerateMaxPositions)
+        return fail(BLURR_ERR_INVALID, std::string(fn) + ": max_prompt_len + n_new exceeds 320 (the decode attention's limit)");
     if (prompt_lens)
         for (int b = 0; b < batch; ++b)
             if (prompt_lens[b] < 1 || prompt_lens[b] > max_prompt_len)
@@ -535,41 +616,46 @@ extern "C" int blurr_llm_generate(blurr_llm_t* h, void* cuda_stream, int batch, 
     const bool sampled = params != nullptr;
     LLM_CUDA_TRY(cudaMemcpyAsync(h->IN, inputs_embeds, static_cast<size_t>(batch) * max_prompt_len * c.hidden * 2, cudaMemcpyDeviceToDevice, st));
     if (const int rc = stage_rows(h, st, batch, prompt_lens, params)) return rc;
-    h->launches = 0;
-    Run R{h, st};
-    if (!h->use_graph) {
-        run_generate(R, batch, max_prompt_len, n_new, keep, ragged, sampled);
-        if (R.rc) return R.rc;
-    } else {
-        const auto key = std::make_tuple(batch, max_prompt_len, n_new, keep ? 1 : 0, ragged ? 1 : 0, sampled ? 1 : 0);
-        auto it = h->graphs.find(key);
-        if (it == h->graphs.end()) {
-            run_generate(R, batch, max_prompt_len, n_new, keep, ragged, sampled);         // warm run: attribute setup, tensor maps
-            if (R.rc) return R.rc;
-            LLM_CUDA_TRY(cudaStreamSynchronize(st));
-            h->launches = 0;
-            cudaStream_t cs;
-            LLM_CUDA_TRY(cudaStreamCreateWithFlags(&cs, cudaStreamNonBlocking));
-            Run C{h, cs};
-            cudaError_t e = cudaStreamBeginCapture(cs, cudaStreamCaptureModeThreadLocal);
-            if (e != cudaSuccess) { cudaStreamDestroy(cs); return fail(BLURR_ERR_CUDA, "graph capture begin failed"); }
-            run_generate(C, batch, max_prompt_len, n_new, keep, ragged, sampled);
-            cudaGraph_t g = nullptr;
-            e = cudaStreamEndCapture(cs, &g);
-            cudaStreamDestroy(cs);
-            if (C.rc) { if (g) cudaGraphDestroy(g); return C.rc; }
-            if (e != cudaSuccess || !g) return fail(BLURR_ERR_CUDA, std::string("graph capture failed: ") + cudaGetErrorString(e));
-            cudaGraphExec_t ex = nullptr;
-            e = cudaGraphInstantiate(&ex, g, 0);
-            if (e != cudaSuccess) { cudaGraphDestroy(g); return fail(BLURR_ERR_CUDA, std::string("graph instantiate failed: ") + cudaGetErrorString(e)); }
-            it = h->graphs.emplace(key, blurr_llm::GraphEntry{g, ex, h->launches}).first;
-        }
-        LLM_CUDA_TRY(cudaGraphLaunch(it->second.exec, st));
-        h->launches = it->second.launches;
-    }
+    const GraphKey key = std::make_tuple(batch, max_prompt_len, n_new, keep ? 1 : 0, ragged ? 1 : 0, sampled ? 1 : 0, 0);
+    if (const int rc = run_graph(h, st, key, [&](Run& R) { run_generate(R, batch, max_prompt_len, n_new, keep, ragged, sampled); }))
+        return rc;
     LLM_CUDA_TRY(cudaMemcpyAsync(out_ids, h->out_ids, static_cast<size_t>(batch) * n_new * 8, cudaMemcpyDeviceToDevice, st));
     if (keep)
         LLM_CUDA_TRY(cudaMemcpyAsync(out_logits, h->LOGITS_ALL, static_cast<size_t>(batch) * n_new * c.vocab * 2, cudaMemcpyDeviceToDevice, st));
+    return 0;
+}
+
+extern "C" int blurr_llm_forward_rows(blurr_llm_t* h, void* cuda_stream, int batch, int max_len, const void* inputs_embeds,
+                                      const int32_t* seq_lens, const int32_t* block_starts, const int32_t* row_starts, int n_rows,
+                                      void* out_hidden) {
+    const char* fn = "blurr_llm_forward_rows";
+    if (!h || !inputs_embeds || !seq_lens || !block_starts || !row_starts || !out_hidden)
+        return fail(BLURR_ERR_INVALID, std::string(fn) + ": null argument");
+    if (!h->finalized) return fail(BLURR_ERR_STATE, std::string(fn) + ": call blurr_llm_finalize first");
+    const auto& c = h->cfg;
+    if (batch < 1 || batch > h->max_batch) return fail(BLURR_ERR_INVALID, std::string(fn) + ": batch out of range");
+    if (max_len < 1 || max_len > c.max_positions)
+        return fail(BLURR_ERR_INVALID, std::string(fn) + ": max_len must be in 1..max_positions (" + std::to_string(c.max_positions) + ")");
+    if (n_rows < 1 || n_rows > max_len) return fail(BLURR_ERR_INVALID, std::string(fn) + ": n_rows must be in 1..max_len");
+    for (int b = 0; b < batch; ++b) {
+        const std::string at = std::string(fn) + ": sequence " + std::to_string(b) + ": ";
+        if (seq_lens[b] < 1 || seq_lens[b] > max_len)
+            return fail(BLURR_ERR_INVALID, at + "seq_lens = " + std::to_string(seq_lens[b]) + " is outside 1.." + std::to_string(max_len));
+        if (block_starts[b] < 1 || block_starts[b] > seq_lens[b])
+            return fail(BLURR_ERR_INVALID, at + "block_starts = " + std::to_string(block_starts[b]) + " is outside 1..seq_lens");
+        if (row_starts[b] < 0 || row_starts[b] > seq_lens[b] - n_rows)
+            return fail(BLURR_ERR_INVALID, at + "rows " + std::to_string(row_starts[b]) + " + " + std::to_string(n_rows) +
+                                               " run past seq_lens = " + std::to_string(seq_lens[b]));
+    }
+    LLM_CUDA_TRY(cudaSetDevice(h->device));
+    cudaStream_t st = static_cast<cudaStream_t>(cuda_stream);
+    LLM_CUDA_TRY(cudaMemcpyAsync(h->IN, inputs_embeds, static_cast<size_t>(batch) * max_len * c.hidden * 2, cudaMemcpyDeviceToDevice, st));
+    if (const int rc = stage_rows(h, st, batch, seq_lens, nullptr, block_starts, row_starts)) return rc;
+    // the graph ends at XN; the rows go straight to the caller's buffer, so one graph serves every n_rows and out_hidden
+    const GraphKey key = std::make_tuple(batch, max_len, 0, 0, 0, 0, 1);
+    if (const int rc = run_graph(h, st, key, [&](Run& R) { run_forward_rows(R, batch, max_len); })) return rc;
+    LLM_CUDA_TRY(launch_gather_row_block(st, h->XN, batch, max_len, h->d_row0, n_rows, c.hidden, static_cast<bf16*>(out_hidden)));
+    ++h->launches;
     return 0;
 }
 

@@ -418,6 +418,25 @@ cudaError_t launch_gather_rows(cudaStream_t stream, const bf16* src, int batch, 
     return launch_kernel(gather_rows_kernel, dim3(batch), dim3(256), 0, stream, src, rows_per_seq, row, width, dst, seq_len);
 }
 
+// OFT's action rows: a block of n_rows consecutive rows per sequence, starting where the device array says.  One CTA per
+// (sequence, row), 16-byte copies.
+__global__ void __launch_bounds__(256) gather_row_block_kernel(const bf16* src, int rows_per_seq, const int* row_start, int width,
+                                                               bf16* dst) {
+    pdl_wait();
+    pdl_trigger();
+    const int b = blockIdx.y, i = blockIdx.x;
+    const int row = row_start[b] + i;           // the host validates row_start[b] + n_rows <= rows_per_seq
+    const uint4* s = reinterpret_cast<const uint4*>(src + (static_cast<size_t>(b) * rows_per_seq + row) * width);
+    uint4* d = reinterpret_cast<uint4*>(dst + (static_cast<size_t>(b) * gridDim.x + i) * width);
+    for (int j = threadIdx.x; j < width / 8; j += blockDim.x) d[j] = s[j];
+}
+
+cudaError_t launch_gather_row_block(cudaStream_t stream, const bf16* src, int batch, int rows_per_seq, const int* row_start, int n_rows,
+                                    int width, bf16* dst) {
+    if ((width & 7) || row_start == nullptr || n_rows < 1 || batch < 1) return cudaErrorInvalidValue;
+    return launch_kernel(gather_row_block_kernel, dim3(n_rows, batch), dim3(256), 0, stream, src, rows_per_seq, row_start, width, dst);
+}
+
 // Pad rows of a ragged prompt batch -> 0 before prefill.  The prefill attention multiplies whole key blocks by P, and a
 // masked key's P = 0 still turns a NaN / Inf value into NaN; with zero inputs every pad row stays a finite function of
 // its sequence's real rows, so nothing the caller left in the pads reaches a real row.  One CTA column per sequence.

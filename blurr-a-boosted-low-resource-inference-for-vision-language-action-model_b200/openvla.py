@@ -202,6 +202,32 @@ class LlamaDecoder:
                                                n_new, C.c_void_p(ids.data_ptr()), out_logits))
         return (ids, logits) if return_logits else ids
 
+    def forward_rows(self, inputs_embeds: torch.Tensor, seq_lens, block_starts, row_starts, n_rows: int) -> torch.Tensor:
+        """One forward pass without lm_head (OpenVLA-OFT's parallel decoding): inputs_embeds bf16 [B, T, hidden] on the
+        device, one int per sequence in `seq_lens` (1..T), `block_starts` (1..seq_lens[b]) and `row_starts` (0..
+        seq_lens[b] - n_rows) -> bf16 [B, n_rows, hidden]: rows row_starts[b] .. + n_rows - 1 of sequence b after the
+        final RMSNorm.  Query p of sequence b sees key k iff k < seq_lens[b] and (k <= p, or p >= block_starts[b] and
+        k >= block_starts[b]); block_starts[b] = seq_lens[b] is plain causal attention.  Rows past seq_lens[b] are pads
+        and never influence any output.  One CUDA graph per (B, T) serves every vector of lengths and starts."""
+        if inputs_embeds.dim() != 3 or inputs_embeds.shape[2] != self.cfg.hidden:
+            raise ValueError(f"inputs_embeds must be [B, T, {self.cfg.hidden}]")
+        if inputs_embeds.dtype != torch.bfloat16 or inputs_embeds.device.type != "cuda":
+            raise ValueError("inputs_embeds must be a bf16 CUDA tensor")
+        x = inputs_embeds.contiguous()
+        B, T = x.shape[0], x.shape[1]
+        arrs = []
+        for name, v in (("seq_lens", seq_lens), ("block_starts", block_starts), ("row_starts", row_starts)):
+            a = np.ascontiguousarray(torch.as_tensor(v).cpu().numpy(), dtype=np.int32)
+            if a.shape != (B,):
+                raise ValueError(f"{name} must hold one value per sequence ({B}), got shape {a.shape}")
+            arrs.append(a)
+        out = torch.empty((B, int(n_rows), self.cfg.hidden), device=self.device, dtype=torch.bfloat16)
+        stream = torch.cuda.current_stream(self.device).cuda_stream
+        ptrs = [a.ctypes.data_as(C.POINTER(C.c_int32)) for a in arrs]
+        capi.check(self.lib.blurr_llm_forward_rows(self.handle, C.c_void_p(stream), B, T, C.c_void_p(x.data_ptr()), *ptrs, int(n_rows),
+                                                   C.c_void_p(out.data_ptr())))
+        return out
+
     def sample(self, logits: torch.Tensor, temperature=1.0, top_k=50, top_p=1.0, seed=None, step: int = 0,
                return_probs: bool = False):
         """The device sampler alone: bf16 logits [rows, ld >= vocab] on the device (rows <= max_batch; the first vocab
@@ -250,6 +276,26 @@ class LlamaDecoder:
             pass
 
 
+def denormalize_actions(norm: np.ndarray, q01, q99, mask=None) -> np.ndarray:
+    """OpenVLA's de-normalisation: `0.5 * (a + 1) * (q99 - q01) + q01` where `mask`, `a` elsewhere, in float64.  q01 / q99
+    / mask broadcast against `norm` from the right."""
+    q01, q99 = np.asarray(q01, dtype=np.float64), np.asarray(q99, dtype=np.float64)
+    mask = np.ones_like(q01, dtype=bool) if mask is None else np.asarray(mask, dtype=bool)
+    return np.where(mask, 0.5 * (norm + 1) * (q99 - q01) + q01, norm)
+
+
+def denormalize_chunk(norm: np.ndarray, q01, q99, mask=None) -> np.ndarray:
+    """`denormalize_actions` on a chunk: norm [B, K, D] -> float64 [B, K, D]; q01 / q99 / mask are [D] (one dataset) or
+    [B, D] (one dataset's statistics per row), the same for every step of the chunk."""
+    q01, q99 = np.asarray(q01, dtype=np.float64), np.asarray(q99, dtype=np.float64)
+    m = None if mask is None else np.asarray(mask, dtype=bool)
+    if q01.ndim == 2:
+        q01, q99 = q01[:, None, :], q99[:, None, :]
+    if m is not None and m.ndim == 2:
+        m = m[:, None, :]
+    return denormalize_actions(np.asarray(norm, dtype=np.float64), q01, q99, m)
+
+
 class ActionDetokenizer:
     """OpenVLA's `predict_action` tail (public modeling_prismatic.py): the last `action_dim` generated ids ->
     `vocab_size - id` -> bin index -> bin centre on [-1, 1] -> de-normalised with the dataset's q01 / q99 where `mask`.
@@ -267,10 +313,7 @@ class ActionDetokenizer:
         return self.bin_centers[discretized]
 
     def actions(self, token_ids: np.ndarray, q01: np.ndarray, q99: np.ndarray, mask: Optional[np.ndarray] = None) -> np.ndarray:
-        norm = self.normalized(token_ids)
-        q01, q99 = np.asarray(q01, dtype=np.float64), np.asarray(q99, dtype=np.float64)
-        mask = np.ones_like(q01, dtype=bool) if mask is None else np.asarray(mask, dtype=bool)
-        return np.where(mask, 0.5 * (norm + 1) * (q99 - q01) + q01, norm)
+        return denormalize_actions(self.normalized(token_ids), q01, q99, mask)
 
 
 def build_prompt_embeds(decoder: LlamaDecoder, input_ids: torch.Tensor, patch_embeds: torch.Tensor) -> torch.Tensor:
@@ -768,3 +811,238 @@ class OpenVlaPolicy:
         `sampling_params` (None: drawn from torch's default generator)."""
         return self.predict_action_from_pixels(self.pixel_values(frames), input_ids, q01, q99, mask, return_token_ids,
                                                attention_mask, do_sample, temperature, top_k, top_p, seed)
+
+
+# ---------------------------------------------------------------------------------------------------------------------
+# OpenVLA-OFT: parallel decoding of action chunks (include/blurr_llm.h blurr_llm_forward_rows, include/blurr_act_head.h)
+# ---------------------------------------------------------------------------------------------------------------------
+@dataclass
+class OftConfig:
+    """OpenVLA-OFT's action chunking (Kim, Finn, Liang 2025): `chunk` actions of `action_dim` dimensions per call, one
+    empty action slot per value.  `bidirectional_actions`: the slots (and the stop token) attend to each other, as the
+    paper describes; False gives plain causal attention.  The head is `MLPResNet(head_num_blocks, action_dim * hidden,
+    head_hidden_dim, action_dim)`; `max_positions` is the decoder's (1 + 256 patches + prompt + 56 slots + stop)."""
+    chunk: int = 8
+    action_dim: int = 7
+    bidirectional_actions: bool = True
+    head_hidden_dim: int = 4096
+    head_num_blocks: int = 2
+    head_ln_eps: float = 1e-5
+    max_positions: int = 384
+    empty_token: int = 29871          # Llama-2's empty token after "Out:"
+    stop_token: int = 2               # </s>
+
+
+def openvla_oft_7b_config(oft: Optional[OftConfig] = None) -> LlamaShapedConfig:
+    """The OpenVLA-7B decoder with room for OFT's sequence (384 positions; `openvla_7b_config` keeps 320)."""
+    return LlamaShapedConfig(max_positions=(oft or OftConfig()).max_positions)
+
+
+@dataclass
+class OftLayout:
+    """Host-side layout of one OFT batch.  Sequence b is `[BOS] + P patches + ids[b, 1:text_lens[b]] + chunk * action_dim
+    zero rows + embed(stop)`, pads after it up to `max_len`."""
+    ids: torch.Tensor                  # int64 [B, S_max] on the host: row b's text_lens[b] tokens (29871 appended), pad id 0 after
+    text_lens: torch.Tensor            # int64 [B]: S_b, BOS included
+    seq_lens: np.ndarray               # int32 [B]: P + S_b + chunk * action_dim + 1
+    block_starts: np.ndarray           # int32 [B]: a0 = P + S_b (seq_lens with bidirectional_actions=False)
+    row_starts: np.ndarray             # int32 [B]: P + S_b - 1, the row before each action slot
+    max_len: int
+    n_rows: int                        # chunk * action_dim
+
+
+def oft_prompt_layout(input_ids, attention_mask: Optional[torch.Tensor] = None, n_patches: int = 256,
+                      cfg: Optional[OftConfig] = None) -> OftLayout:
+    """OFT's `predict_action` prompt for the three forms `ragged_prompt_ids` accepts ([B, S], a list of 1-D id tensors, or
+    [B, S] with a left- or right-padded `attention_mask`): a row whose last id is not `empty_token` (29871) gets it
+    appended; then the action slots, the stop token and the attention block follow.  Raises ValueError when a sequence
+    would need more than `cfg.max_positions` positions."""
+    cfg = cfg or OftConfig()
+    ids, lens = ragged_prompt_ids(input_ids, attention_mask)
+    ids, lens = ids.cpu(), lens.clone()
+    last = ids.gather(1, (lens - 1)[:, None])[:, 0]
+    add = last != cfg.empty_token
+    S = int((lens + add.to(torch.int64)).max())
+    out = torch.zeros((ids.shape[0], S), dtype=torch.int64)
+    out[:, :ids.shape[1]] = ids[:, :S]
+    rows = torch.arange(ids.shape[0])
+    out[rows[add], lens[add]] = cfg.empty_token
+    lens = lens + add.to(torch.int64)
+    n_rows = cfg.chunk * cfg.action_dim
+    a0 = (lens + n_patches).numpy().astype(np.int32)
+    seq = a0 + n_rows + 1
+    max_len = int(seq.max())
+    if max_len > cfg.max_positions:
+        raise ValueError(f"an OFT sequence needs {max_len} positions (patches {n_patches} + prompt {int(lens.max())} + "
+                         f"{n_rows} action slots + stop), more than max_positions = {cfg.max_positions}")
+    blk = a0.copy() if cfg.bidirectional_actions else seq.copy()
+    return OftLayout(ids=out, text_lens=lens, seq_lens=seq, block_starts=blk,
+                     row_starts=(a0 - 1).astype(np.int32), max_len=max_len, n_rows=n_rows)
+
+
+def build_oft_embeds(decoder: LlamaDecoder, layout: OftLayout, patch_embeds: torch.Tensor, stop_token: int = 2) -> torch.Tensor:
+    """bf16 [B, layout.max_len, hidden]: the prompt rows of `build_prompt_embeds` / `build_prompt_embeds_ragged`, then
+    chunk * action_dim zeroed slots and the stop token's embedding; zeros after it."""
+    x, _ = build_prompt_embeds_ragged(decoder, layout.ids.to(decoder.device), layout.text_lens, patch_embeds)
+    B, L, H = x.shape[0], layout.max_len, x.shape[2]
+    full = torch.zeros((B, L, H), device=x.device, dtype=x.dtype)
+    full[:, :x.shape[1]] = x
+    pos = torch.arange(L, device=x.device)[None, :]
+    a0 = torch.as_tensor(layout.row_starts + 1, device=x.device, dtype=torch.int64)[:, None]
+    stop_row = decoder.embed(torch.tensor([stop_token], device=x.device))[0]
+    full = torch.where((pos < a0)[..., None], full, torch.zeros((), device=x.device, dtype=x.dtype))
+    return torch.where((pos == a0 + layout.n_rows)[..., None], stop_row, full).contiguous()
+
+
+class L1RegressionHead:
+    """OpenVLA-OFT's `L1RegressionActionHead` on one B200 through `include/blurr_act_head.h`: the decoder's action rows
+    [B, chunk * action_dim, hidden] -> normalised actions fp32 [B, chunk, action_dim] (the module's bf16 output)."""
+
+    def __init__(self, cfg: OftConfig, input_dim: int, device, max_batch: int = 1):
+        self.lib = capi.load_library()
+        self.cfg, self.input_dim = cfg, int(input_dim)
+        self.device = torch.device(device)
+        self.max_batch = max_batch
+        self.handle = C.c_void_p()
+        c = capi.ActHeadConfigC(capi.ACT_HEAD_ABI_VERSION, self.input_dim, cfg.action_dim, cfg.chunk, cfg.head_hidden_dim,
+                                cfg.head_num_blocks, cfg.head_ln_eps)
+        index = self.device.index if self.device.index is not None else torch.cuda.current_device()
+        capi.check(self.lib.blurr_act_head_create(C.byref(c), index, max_batch, C.byref(self.handle)))
+
+    @classmethod
+    def from_state_dict(cls, cfg: OftConfig, state_dict: Dict[str, torch.Tensor], input_dim: int, device, max_batch: int = 1,
+                        prefix: str = "") -> "L1RegressionHead":
+        """`state_dict`: keys of OFT's `L1RegressionActionHead.state_dict()` ("model.fc1.weight", ...), optionally under
+        `prefix`."""
+        self = cls(cfg, input_dim, device, max_batch)
+        try:
+            for key, t in state_dict.items():
+                if prefix and not key.startswith(prefix):
+                    continue
+                self.set_weight(key[len(prefix):], t)
+            capi.check(self.lib.blurr_act_head_finalize(self.handle))
+        except Exception:
+            self.close()
+            raise
+        return self
+
+    @classmethod
+    def synthetic(cls, cfg: OftConfig, input_dim: int, device, max_batch: int = 1, seed: int = 0) -> "L1RegressionHead":
+        """Random-init head with nn.Linear's default init (uniform, bound 1 / sqrt(fan_in)) and LayerNorms at 1 / 0,
+        generated on the device (0.25 GB at OFT's widths)."""
+        return cls.from_state_dict(cfg, synthetic_act_head_state_dict(cfg, input_dim, device, seed), input_dim, device, max_batch)
+
+    def set_weight(self, name: str, tensor: torch.Tensor):
+        t = tensor.detach().to(device=self.device, dtype=torch.bfloat16).contiguous()
+        torch.cuda.current_stream(self.device).synchronize()
+        shape = (C.c_int64 * t.dim())(*t.shape)
+        capi.check(self.lib.blurr_act_head_set_weight(self.handle, name.encode(), C.c_void_p(t.data_ptr()), shape, t.dim()))
+
+    def forward(self, hidden_rows: torch.Tensor) -> torch.Tensor:
+        """hidden_rows bf16 [B, chunk * action_dim, input_dim] on the device -> fp32 [B, chunk, action_dim]."""
+        K, D = self.cfg.chunk, self.cfg.action_dim
+        if hidden_rows.dim() != 3 or tuple(hidden_rows.shape[1:]) != (K * D, self.input_dim):
+            raise ValueError(f"hidden_rows must be [B, {K * D}, {self.input_dim}]")
+        if hidden_rows.dtype != torch.bfloat16 or hidden_rows.device.type != "cuda":
+            raise ValueError("hidden_rows must be a bf16 CUDA tensor")
+        x = hidden_rows.contiguous()
+        B = x.shape[0]
+        out = torch.empty((B, K, D), device=self.device, dtype=torch.float32)
+        stream = torch.cuda.current_stream(self.device).cuda_stream
+        capi.check(self.lib.blurr_act_head_forward(self.handle, C.c_void_p(stream), B, C.c_void_p(x.data_ptr()),
+                                                   C.c_void_p(out.data_ptr())))
+        return out
+
+    def check(self):
+        capi.check(self.lib.blurr_act_head_check(self.handle, C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)))
+
+    @property
+    def last_launch_count(self) -> int:
+        return int(self.lib.blurr_act_head_last_launch_count(self.handle))
+
+    def close(self):
+        if self.handle:
+            self.lib.blurr_act_head_destroy(self.handle)
+            self.handle = C.c_void_p()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+
+def synthetic_act_head_state_dict(cfg: OftConfig, input_dim: int, device, seed: int = 0,
+                                  dtype=torch.bfloat16) -> Dict[str, torch.Tensor]:
+    """Random-init weights of `L1RegressionActionHead` with its state_dict keys, nn.Linear's default init."""
+    g = torch.Generator(device=device)
+    g.manual_seed(seed)
+    H, W, D = cfg.head_hidden_dim, cfg.action_dim * input_dim, cfg.action_dim
+
+    def u(shape, fan_in):
+        return ((torch.rand(shape, device=device, generator=g) * 2 - 1) / math.sqrt(fan_in)).to(dtype)
+
+    sd = {"model.layer_norm1.weight": torch.ones(W, device=device, dtype=dtype),
+          "model.layer_norm1.bias": torch.zeros(W, device=device, dtype=dtype),
+          "model.fc1.weight": u((H, W), W), "model.fc1.bias": u((H,), W)}
+    for i in range(cfg.head_num_blocks):
+        p = f"model.mlp_resnet_blocks.{i}.ffn."
+        sd[p + "0.weight"] = torch.ones(H, device=device, dtype=dtype)
+        sd[p + "0.bias"] = torch.zeros(H, device=device, dtype=dtype)
+        sd[p + "1.weight"] = u((H, H), H)
+        sd[p + "1.bias"] = u((H,), H)
+    sd["model.layer_norm2.weight"] = torch.ones(H, device=device, dtype=dtype)
+    sd["model.layer_norm2.bias"] = torch.zeros(H, device=device, dtype=dtype)
+    sd["model.fc2.weight"] = u((D, H), H)
+    sd["model.fc2.bias"] = u((D,), H)
+    return sd
+
+
+class OftPolicy:
+    """OpenVLA-OFT's `predict_action` with parallel decoding: device preprocessing -> DINOv2 + SigLIP towers ->
+    projector -> `[BOS] + patches + prompt + empty action slots + stop` -> one decoder pass (`forward_rows`) -> the
+    L1-regression head -> a whole chunk of de-normalised actions.  No decode loop: one call yields `chunk` actions."""
+
+    def __init__(self, preprocessor: ImagePreprocessor, backbone: FusedVisionBackbone, decoder: LlamaDecoder,
+                 head: L1RegressionHead, cfg: Optional[OftConfig] = None):
+        if preprocessor.n_norms != 2:
+            raise ValueError("the fused backbone needs two normalisations (DINOv2's, then SigLIP's)")
+        cfg = cfg or head.cfg
+        if (head.cfg.chunk, head.cfg.action_dim) != (cfg.chunk, cfg.action_dim) or head.input_dim != decoder.cfg.hidden:
+            raise ValueError("the head's chunk, action_dim and input width must match the config and the decoder")
+        self.preprocessor, self.backbone, self.decoder, self.head, self.cfg = preprocessor, backbone, decoder, head, cfg
+
+    def pixel_values(self, frames) -> torch.Tensor:
+        """uint8 frame(s) [H, W, 3] / [B, H, W, 3] -> bf16 [B, 6, 224, 224] (as `OpenVlaPolicy.pixel_values`)."""
+        f = torch.as_tensor(frames)
+        if f.dim() == 3:
+            f = f[None]
+        if not f.is_cuda:
+            f = f.to(self.preprocessor.device)
+        return self.preprocessor(f)
+
+    def action_rows(self, pixel_values: torch.Tensor, input_ids, attention_mask: Optional[torch.Tensor] = None) -> torch.Tensor:
+        """The decoder's final-normed rows in front of the action slots, bf16 [B, chunk * action_dim, hidden]."""
+        patch = self.backbone.forward(pixel_values[:, :3], pixel_values[:, 3:])
+        lay = oft_prompt_layout(input_ids, attention_mask, patch.shape[1], self.cfg)
+        if lay.max_len > self.decoder.cfg.max_positions:
+            raise ValueError(f"an OFT sequence needs {lay.max_len} positions; the decoder holds {self.decoder.cfg.max_positions}")
+        x = build_oft_embeds(self.decoder, lay, patch, self.cfg.stop_token)
+        return self.decoder.forward_rows(x, lay.seq_lens, lay.block_starts, lay.row_starts, lay.n_rows)
+
+    def predict_action_chunk_from_pixels(self, pixel_values: torch.Tensor, input_ids, q01, q99, mask=None,
+                                         attention_mask: Optional[torch.Tensor] = None, return_normalized: bool = False):
+        """The same as `predict_action_chunk`, from prepared bf16 pixel values [B, 6, 224, 224]."""
+        norm = self.head.forward(self.action_rows(pixel_values, input_ids, attention_mask))
+        actions = torch.from_numpy(denormalize_chunk(norm.cpu().numpy(), q01, q99, mask))
+        return (actions, norm) if return_normalized else actions
+
+    def predict_action_chunk(self, frames, input_ids, q01, q99, mask=None, attention_mask: Optional[torch.Tensor] = None,
+                             return_normalized: bool = False):
+        """frames: uint8 [H, W, 3] or [B, H, W, 3] RGB.  input_ids: [B, S] (first column BOS), a list of B 1-D id tensors,
+        or [B, S] with a left- or right-padded `attention_mask` (see `oft_prompt_layout`).  q01 / q99 / mask:
+        [action_dim] or [B, action_dim], applied to every step of the chunk.  Returns float64 actions
+        [B, chunk, action_dim] on the host (and, with `return_normalized`, the head's output fp32 [B, chunk, action_dim]
+        on the device)."""
+        return self.predict_action_chunk_from_pixels(self.pixel_values(frames), input_ids, q01, q99, mask, attention_mask,
+                                                     return_normalized)

@@ -47,7 +47,7 @@ typedef struct blurr_llm_config {
     int32_t head_dim;             /* 128 (or 64) */
     int32_t intermediate;         /* 11008, multiple of 64 */
     int32_t vocab;                /* 32064 (rows of embed_tokens / lm_head) */
-    int32_t max_positions;        /* KV-cache slots per sequence: prompt + generated tokens, <= 320 */
+    int32_t max_positions;        /* KV-cache slots per sequence, <= 384 (generate: prompt + generated tokens <= 320) */
     float rms_eps;                /* 1e-6 (OpenVLA) / 1e-5 (Llama-2) */
 } blurr_llm_config;
 #define BLURR_LLM_ABI_VERSION 2
@@ -90,7 +90,7 @@ int blurr_llm_finalize(blurr_llm_t* h);
 /* rows[i] = embed_tokens[ids[i]]  (bf16 [n][hidden]) */
 int blurr_llm_embed(blurr_llm_t* h, void* cuda_stream, const int64_t* ids, int n, void* rows_out);
 
-/* Generation.  inputs_embeds: bf16 [batch][max_prompt_len][hidden]; max_prompt_len + n_new <= max_positions.
+/* Generation.  inputs_embeds: bf16 [batch][max_prompt_len][hidden]; max_prompt_len + n_new <= min(max_positions, 320).
  * prompt_lens: HOST int32 [batch] or NULL.  NULL: every sequence is max_prompt_len rows, no padding.  Otherwise
  * 1 <= prompt_lens[b] <= max_prompt_len and sequence b's prompt is rows 0 .. prompt_lens[b] - 1; rows t >= prompt_lens[b]
  * are ignored (never influence any output: they are zeroed on the device before the prefill, which runs over all
@@ -108,6 +108,20 @@ int blurr_llm_embed(blurr_llm_t* h, void* cuda_stream, const int64_t* ids, int n
 int blurr_llm_generate(blurr_llm_t* h, void* cuda_stream, int batch, int max_prompt_len, const void* inputs_embeds,
                        const int32_t* prompt_lens, const blurr_llm_sampling* params, int n_new, int64_t* out_ids,
                        void* out_logits);
+/* One forward pass without lm_head, for OpenVLA-OFT's parallel decoding: the final-normed hidden rows of each sequence.
+ * inputs_embeds bf16 [batch][max_len][hidden]; seq_lens, block_starts, row_starts: HOST int32 [batch] with
+ * 1 <= seq_lens[b] <= max_len <= max_positions, 1 <= block_starts[b] <= seq_lens[b], 0 <= row_starts[b] and
+ * row_starts[b] + n_rows <= seq_lens[b].  Rows t >= seq_lens[b] are pads: zeroed on the device, they never influence any
+ * output.  Attention: query p of sequence b sees key k iff k < seq_lens[b] and (k <= p, or p >= block_starts[b] and
+ * k >= block_starts[b]): causal over the prompt, bidirectional inside the block [block_starts[b], seq_lens[b]);
+ * block_starts[b] == seq_lens[b] is plain causal attention.  Positions (RoPE) are 0..max_len-1 for every sequence.
+ * Writes out_hidden bf16 [batch][n_rows][hidden]: rows row_starts[b] .. + n_rows - 1 of sequence b after the final
+ * RMSNorm (transformers' LlamaModel.last_hidden_state).  Accepts up to 384 positions (blurr_llm_generate: 320).  The
+ * pass is replayed as one CUDA graph per (batch, max_len) whatever the lengths, starts and n_rows; the row copy to
+ * out_hidden is one more kernel after it.  A bad argument returns BLURR_ERR_INVALID and the handle keeps working. */
+int blurr_llm_forward_rows(blurr_llm_t* h, void* cuda_stream, int batch, int max_len, const void* inputs_embeds,
+                           const int32_t* seq_lens, const int32_t* block_starts, const int32_t* row_starts, int n_rows,
+                           void* out_hidden);
 /* The sampler alone, on caller-made logits (usable before blurr_llm_finalize): logits bf16 [rows][ld], first `vocab`
  * columns used, rows <= max_batch, ld >= vocab; params HOST [rows]; `step` is the Philox counter.  Writes out_ids int64
  * [rows]; out_probs (may be NULL) fp32 [rows][vocab]: the probability each token was drawn with, 0 outside the kept set. */
@@ -120,7 +134,7 @@ int blurr_llm_set_option(blurr_llm_t* h, const char* name, int64_t value);
 int blurr_llm_check(blurr_llm_t* h, void* cuda_stream);
 /* Text timeline of the last generate call under option "trace": one line per kernel, microseconds. */
 int blurr_llm_trace_report(blurr_llm_t* h, char* buf, size_t buf_bytes);
-/* Kernels launched by the last blurr_llm_generate call, and the weight bytes one decode step streams. */
+/* Kernels launched by the last blurr_llm_generate / blurr_llm_forward_rows call, and the weight bytes one decode step streams. */
 int64_t blurr_llm_last_launch_count(const blurr_llm_t* h);
 int64_t blurr_llm_weight_bytes_per_token(const blurr_llm_t* h);
 
