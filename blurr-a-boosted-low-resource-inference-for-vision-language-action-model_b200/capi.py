@@ -51,11 +51,11 @@ class LlmConfigC(C.Structure):
     _fields_ = [
         ("abi_version", C.c_int32), ("num_layers", C.c_int32), ("hidden", C.c_int32), ("num_heads", C.c_int32),
         ("num_kv_heads", C.c_int32), ("head_dim", C.c_int32), ("intermediate", C.c_int32), ("vocab", C.c_int32),
-        ("max_positions", C.c_int32), ("rms_eps", C.c_float),
+        ("max_positions", C.c_int32), ("rms_eps", C.c_float), ("long_forward", C.c_int32),
     ]
 
 
-LLM_ABI_VERSION = 2
+LLM_ABI_VERSION = 3
 
 
 class LlmSamplingC(C.Structure):

@@ -701,7 +701,7 @@ cudaError_t launch_mha_attention(cudaStream_t stream, const MhaAttnArgs& m, cons
 }
 
 // OFT's prefill (llm_engine.cu blurr_llm_forward_rows): causal over the prompt, bidirectional inside the action block,
-// per-sequence lengths and block starts read at run time, up to 384 keys.  A kernel of its own so that MODE 2's
+// per-sequence lengths and block starts read at run time, up to 384 keys resident.  A kernel of its own so that MODE 2's
 // instantiations above keep their code.
 template <int HD_PAD, int BM>
 __global__ void __launch_bounds__(kAttnThreads) attn_block_kernel(const AttnMmaArgs a, const int* seq_len, const int* block_start) {
@@ -734,8 +734,245 @@ static cudaError_t launch_attn_block(cudaStream_t stream, const AttnMmaArgs& a, 
     return launch_kernel(attn_block_kernel<HD_PAD, BM>, grid, dim3(kAttnThreads), smem, stream, a, seq_len, block_start);
 }
 
+// The same rule past 384 keys: K and V stream through a ring of kAttnStreamStages 64-key buffers instead of staying
+// resident, while the bf16 logits of the tile's whole key range stay in shared memory.  The rounding chain, the fp32
+// softmax over the whole row (lane striding c = lane + 32 i, the same summation order) and the key-block order of P.V
+// are attn_mma_body's, so a row's output equals the resident kernel's for any key count both can hold.  The softmax
+// reads the row from shared memory on each pass instead of holding up to 32 logits per lane in registers; expf is
+// recomputed on the last pass, which gives the same value.
+static constexpr int kAttnStreamStages = 3;
+static constexpr int kAttnStreamMaxBlocks = 16;     // 1024 keys
+
+template <int HD_PAD, int BM>
+__device__ __forceinline__ void attn_block_stream_body(const AttnMmaArgs& a, uint8_t* smem_attn, const int qt, const int h,
+                                                       const int b, const int* seq_len, const int* block_start) {
+    constexpr int S = kAttnStreamStages;
+    constexpr int WR = BM / 16;
+    constexpr int WC = (kAttnThreads / 32) / WR;
+    constexpr int KPW = kBK / WC;
+    constexpr int NT_S = KPW / 8;
+    constexpr int NT_ALL = HD_PAD / 8;
+    constexpr int NT_PV = (NT_ALL + WC - 1) / WC;
+    constexpr int NP_PV = (NT_PV + 1) / 2;
+    constexpr int CH = HD_PAD / 8;
+    constexpr int LDS_MIN = WC * NP_PV * 16 > HD_PAD ? WC * NP_PV * 16 : HD_PAD;
+    constexpr int LDS = LDS_MIN + 8;
+    const int blk_len = max(1, min(seq_len[b], a.n_keys));            // the host validates both; never read out of range
+    const int blk0 = max(1, min(block_start[b], blk_len));
+    const int last_q = a.q_row_offset + qt * BM + BM - 1;
+    const int n_keys_tile = min(blk_len, last_q >= blk0 ? a.n_keys : last_q + 1);
+    const int nkb = (n_keys_tile + kBK - 1) / kBK;
+    const int ldl = nkb * kBK + 8;
+    bf16* Qs = reinterpret_cast<bf16*>(smem_attn);
+    bf16* ring = Qs + BM * LDS;                 // S buffers of [64][LDS]
+    bf16* Ls = ring + S * kBK * LDS;            // [BM][ldl]
+
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const int wr = warp % WR, wc = warp / WR;
+    const int q_row0 = qt * BM;
+    const int n_rows_valid = a.q_per_sample;
+    const bf16* qbase = a.q + static_cast<size_t>(b) * a.q_per_sample * a.ldq + a.q_col0 + h * a.head_stride_q;
+    const bf16* kbase = a.k + static_cast<size_t>(b) * a.kv_per_sample * a.ldk + a.k_col0 + h * a.head_stride_kv;
+    const bf16* vbase = a.v + static_cast<size_t>(b) * a.kv_per_sample * a.ldv + a.v_col0 + h * a.head_stride_kv;
+
+    for (int idx = threadIdx.x; idx < BM * CH; idx += kAttnThreads) {
+        const int r = idx / CH, c = idx - r * CH;
+        const int row = q_row0 + r;
+        const bool valid = (row < n_rows_valid) && (c * 8 < a.hd);
+        cp_async_16(Qs + r * LDS + c * 8, valid ? qbase + static_cast<size_t>(row) * a.ldq + c * 8 : qbase, valid);
+    }
+    // one cp.async group per key block (empty past the last one); block kb lives in buffer kb % S.  S - 1 blocks are in
+    // flight ahead of the one being consumed; a buffer is refilled after the barrier that ends every warp's use of it.
+    for (int kb = 0; kb < S - 1; ++kb) {
+        if (kb < nkb) load_rows_async<LDS, CH>(ring + kb * kBK * LDS, kbase, a.ldk, kb * kBK, kBK, n_keys_tile, a.hd);
+        cp_async_commit();
+    }
+
+    // ---------------- phase S: logits = chain(Q K^T) -> Ls (bf16) ----------------
+    for (int kb = 0; kb < nkb; ++kb) {
+        cp_async_wait<S - 2>();
+        attn_bar_sync();
+        if (kb + S - 1 < nkb)
+            load_rows_async<LDS, CH>(ring + ((kb + S - 1) % S) * kBK * LDS, kbase, a.ldk, (kb + S - 1) * kBK, kBK, n_keys_tile, a.hd);
+        cp_async_commit();
+        const bf16* Kcur = ring + (kb % S) * kBK * LDS;
+
+        float acc[NT_S][4];
+#pragma unroll
+        for (int i = 0; i < NT_S; ++i)
+#pragma unroll
+            for (int j = 0; j < 4; ++j) acc[i][j] = 0.f;
+#pragma unroll
+        for (int kk = 0; kk < HD_PAD / 16; ++kk) {
+            uint32_t af[4];
+            ldmatrix_x4(af, smem_u32(Qs + (wr * 16 + (lane & 15)) * LDS + kk * 16 + (lane >> 4) * 8));
+            if (NT_S == 1) {
+                uint32_t bfr[2];
+                const int key = wc * KPW + (lane & 7);
+                ldmatrix_x2(bfr, smem_u32(Kcur + key * LDS + kk * 16 + ((lane >> 3) & 1) * 8));
+                mma_bf16_16816(acc[0], af, bfr[0], bfr[1]);
+            } else {
+#pragma unroll
+                for (int np = 0; np < NT_S / 2; ++np) {
+                    uint32_t bfr[4];
+                    const int mi = lane >> 3;
+                    const int key = wc * KPW + np * 16 + (mi >> 1) * 8 + (lane & 7);
+                    ldmatrix_x4(bfr, smem_u32(Kcur + key * LDS + kk * 16 + (mi & 1) * 8));
+                    mma_bf16_16816(acc[np * 2 + 0], af, bfr[0], bfr[1]);
+                    mma_bf16_16816(acc[np * 2 + (NT_S > 1 ? 1 : 0)], af, bfr[2], bfr[3]);
+                }
+            }
+        }
+#pragma unroll
+        for (int nt = 0; nt < NT_S; ++nt) {
+#pragma unroll
+            for (int half = 0; half < 2; ++half) {
+                const int r = wr * 16 + (lane >> 2) + half * 8;
+                const int kcol = kb * kBK + wc * KPW + nt * 8 + (lane & 3) * 2;
+                float s0 = bf16_round(acc[nt][half * 2 + 0]);
+                float s1 = bf16_round(acc[nt][half * 2 + 1]);
+                s0 = bf16_round(s0 * a.scale);
+                s1 = bf16_round(s1 * a.scale);
+                const int qpos = a.q_row_offset + q_row0 + r;
+                const bool in_blk = qpos >= blk0;
+                if (!(kcol < blk_len && (kcol <= qpos || (in_blk && kcol >= blk0)))) s0 = -INFINITY;
+                if (!(kcol + 1 < blk_len && (kcol + 1 <= qpos || (in_blk && kcol + 1 >= blk0)))) s1 = -INFINITY;
+                *reinterpret_cast<uint32_t*>(Ls + r * ldl + kcol) = pack_bf16x2(s0, s1);
+            }
+        }
+    }
+    attn_bar_sync();   // every warp is done with the K buffers; all logits are visible
+
+    for (int kb = 0; kb < S - 1; ++kb) {
+        if (kb < nkb) load_rows_async<LDS, CH>(ring + kb * kBK * LDS, vbase, a.ldv, kb * kBK, kBK, n_keys_tile, a.hd);
+        cp_async_commit();
+    }
+
+    // ---------------- softmax: fp32 over bf16 logits, result bf16 in place ----------------
+    const int n_it = (n_keys_tile + 31) / 32;
+    for (int rr = 0; rr < BM / 8; ++rr) {
+        bf16* lrow = Ls + (warp * (BM / 8) + rr) * ldl;
+        float m = -INFINITY;
+        for (int i = 0; i < n_it; ++i) {
+            const int c = lane + i * 32;
+            m = fmaxf(m, (c < n_keys_tile) ? bf2f(lrow[c]) : -INFINITY);
+        }
+        m = warp_max(m);
+        float sum = 0.f;
+        for (int i = 0; i < n_it; ++i) {
+            const int c = lane + i * 32;
+            sum += (c < n_keys_tile) ? expf(bf2f(lrow[c]) - m) : 0.f;
+        }
+        sum = warp_sum(sum);
+        for (int i = 0; i < nkb * (kBK / 32); ++i) {
+            const int c = lane + i * 32;
+            const float x = (c < n_keys_tile) ? expf(bf2f(lrow[c]) - m) : 0.f;
+            lrow[c] = f2bf(x / sum);
+        }
+    }
+
+    // ---------------- phase PV ----------------
+    float oacc[NP_PV * 2][4];
+#pragma unroll
+    for (int i = 0; i < NP_PV * 2; ++i)
+#pragma unroll
+        for (int j = 0; j < 4; ++j) oacc[i][j] = 0.f;
+    const int nt0 = wc * NT_PV;
+    for (int kb = 0; kb < nkb; ++kb) {
+        cp_async_wait<S - 2>();
+        attn_bar_sync();                        // (kb == 0: also publishes the probabilities)
+        if (kb + S - 1 < nkb)
+            load_rows_async<LDS, CH>(ring + ((kb + S - 1) % S) * kBK * LDS, vbase, a.ldv, (kb + S - 1) * kBK, kBK, n_keys_tile, a.hd);
+        cp_async_commit();
+        const bf16* Vcur = ring + (kb % S) * kBK * LDS;
+#pragma unroll
+        for (int kk = 0; kk < kBK / 16; ++kk) {
+            uint32_t af[4];
+            ldmatrix_x4(af, smem_u32(Ls + (wr * 16 + (lane & 15)) * ldl + kb * kBK + kk * 16 + (lane >> 4) * 8));
+#pragma unroll
+            for (int np = 0; np < NP_PV; ++np) {
+                if ((nt0 + np * 2) >= NT_ALL) continue;
+                uint32_t bfr[4];
+                const int mi = lane >> 3;
+                const int key = kk * 16 + (mi & 1) * 8 + (lane & 7);
+                const int dim = (nt0 + np * 2) * 8 + (mi >> 1) * 8;
+                ldmatrix_x4_trans(bfr, smem_u32(Vcur + key * LDS + dim));
+                mma_bf16_16816(oacc[np * 2 + 0], af, bfr[0], bfr[1]);
+                if (np * 2 + 1 < NT_PV && nt0 + np * 2 + 1 < NT_ALL)
+                    mma_bf16_16816(oacc[np * 2 + 1], af, bfr[2], bfr[3]);
+            }
+        }
+    }
+    cp_async_wait<0>();
+
+    bf16* obase = a.out + static_cast<size_t>(b) * a.q_per_sample * a.ldo + a.o_col0 + h * a.head_stride_q;
+#pragma unroll
+    for (int nt = 0; nt < NT_PV; ++nt) {
+#pragma unroll
+        for (int half = 0; half < 2; ++half) {
+            const int r = q_row0 + wr * 16 + (lane >> 2) + half * 8;
+            const int dim = (nt0 + nt) * 8 + (lane & 3) * 2;
+            if (r < n_rows_valid && dim < a.hd)
+                *reinterpret_cast<uint32_t*>(obase + static_cast<size_t>(r) * a.ldo + dim) =
+                    pack_bf16x2(oacc[nt][half * 2 + 0], oacc[nt][half * 2 + 1]);
+        }
+    }
+}
+
+template <int HD_PAD, int BM>
+inline size_t attn_stream_smem_bytes(int n_keys) {
+    constexpr int WC = (kAttnThreads / 32) / (BM / 16);
+    constexpr int NT_PV = (HD_PAD / 8 + WC - 1) / WC;
+    constexpr int NP_PV = (NT_PV + 1) / 2;
+    constexpr int LDS_MIN = WC * NP_PV * 16 > HD_PAD ? WC * NP_PV * 16 : HD_PAD;
+    constexpr int LDS = LDS_MIN + 8;
+    const int nkb = (n_keys + kBK - 1) / kBK;
+    return static_cast<size_t>(BM + kAttnStreamStages * kBK) * LDS * 2 + static_cast<size_t>(BM) * (nkb * kBK + 8) * 2;
+}
+
+template <int HD_PAD, int BM>
+__global__ void __launch_bounds__(kAttnThreads) attn_block_stream_kernel(const AttnMmaArgs a, const int* seq_len, const int* block_start) {
+    extern __shared__ __align__(16) uint8_t smem_attn[];
+    trace_stamp(a.trace, 0);
+    pdl_wait();
+    pdl_trigger();
+    trace_stamp(a.trace, 1);
+    attn_block_stream_body<HD_PAD, BM>(a, smem_attn, blockIdx.x, blockIdx.y, blockIdx.z, seq_len, block_start);
+    trace_stamp(a.trace, 2);
+}
+
+template <int HD_PAD, int BM>
+static cudaError_t launch_attn_block_stream(cudaStream_t stream, const AttnMmaArgs& a, const int* seq_len, const int* block_start,
+                                            int rows, int heads, int batch) {
+    const size_t smem = attn_stream_smem_bytes<HD_PAD, BM>(a.n_keys);     // 197 KB at head_dim 128, BM 64, 1024 keys
+    static bool attr = false;
+    if (!attr) {
+        int dev = 0, optin = 0;
+        cudaError_t e = cudaGetDevice(&dev);
+        if (e == cudaSuccess) e = cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev);
+        if (e != cudaSuccess) return e;
+        if (static_cast<size_t>(optin) < kAttnSmemMax) return cudaErrorInvalidConfiguration;
+        e = cudaFuncSetAttribute(attn_block_stream_kernel<HD_PAD, BM>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                 static_cast<int>(kAttnSmemMax));
+        if (e != cudaSuccess) return e;
+        attr = true;
+    }
+    if (smem > kAttnSmemMax) return cudaErrorInvalidValue;
+    dim3 grid((rows + BM - 1) / BM, heads, batch);
+    return launch_kernel(attn_block_stream_kernel<HD_PAD, BM>, grid, dim3(kAttnThreads), smem, stream, a, seq_len, block_start);
+}
+
+template <int HD_PAD, int BM>
+static cudaError_t launch_block_rule(bool stream_kv, cudaStream_t stream, const AttnMmaArgs& a, const int* seq_len,
+                                     const int* block_start, const MhaAttnArgs& m) {
+    return stream_kv ? launch_attn_block_stream<HD_PAD, BM>(stream, a, seq_len, block_start, m.q_per_sample, m.n_heads, m.batch)
+                     : launch_attn_block<HD_PAD, BM>(stream, a, seq_len, block_start, m.q_per_sample, m.n_heads, m.batch);
+}
+
+// Up to 384 keys every key block of a head stays resident in shared memory (attn_block_kernel); past that, up to 1024,
+// K and V stream through a ring (attn_block_stream_kernel).
 cudaError_t launch_mha_block_attention(cudaStream_t stream, const MhaAttnArgs& m, const int* block_start) {
-    if (m.n_keys > kAttnMaxBlocksWide * kBK || m.n_kv_heads != m.n_heads || m.q_pos0 != 0 ||
+    if (m.n_keys > kAttnStreamMaxBlocks * kBK || m.n_kv_heads != m.n_heads || m.q_pos0 != 0 ||
         m.n_keys != m.q_per_sample || m.seq_len == nullptr || block_start == nullptr)
         return cudaErrorInvalidValue;
     AttnMmaArgs a{};
@@ -748,14 +985,15 @@ cudaError_t launch_mha_block_attention(cudaStream_t stream, const MhaAttnArgs& m
     a.scale = m.scale; a.mask = nullptr; a.q_row_offset = 0; a.trace = m.trace;
     const int bm = attn_tile_rows(m.q_per_sample, m.n_heads, m.batch, 64);
     const int* L = m.seq_len;
+    const bool sk = m.n_keys > kAttnMaxBlocksWide * kBK;
     if (m.head_dim == 128) {
-        if (bm == 16) return launch_attn_block<128, 16>(stream, a, L, block_start, m.q_per_sample, m.n_heads, m.batch);
-        if (bm == 32) return launch_attn_block<128, 32>(stream, a, L, block_start, m.q_per_sample, m.n_heads, m.batch);
-        return launch_attn_block<128, 64>(stream, a, L, block_start, m.q_per_sample, m.n_heads, m.batch);
+        if (bm == 16) return launch_block_rule<128, 16>(sk, stream, a, L, block_start, m);
+        if (bm == 32) return launch_block_rule<128, 32>(sk, stream, a, L, block_start, m);
+        return launch_block_rule<128, 64>(sk, stream, a, L, block_start, m);
     }
     if (m.head_dim == 64) {
-        if (bm == 16) return launch_attn_block<64, 16>(stream, a, L, block_start, m.q_per_sample, m.n_heads, m.batch);
-        return launch_attn_block<64, 32>(stream, a, L, block_start, m.q_per_sample, m.n_heads, m.batch);
+        if (bm == 16) return launch_block_rule<64, 16>(sk, stream, a, L, block_start, m);
+        return launch_block_rule<64, 32>(sk, stream, a, L, block_start, m);
     }
     return cudaErrorInvalidValue;
 }

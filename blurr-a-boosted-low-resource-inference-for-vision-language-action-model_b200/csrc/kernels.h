@@ -187,7 +187,7 @@ struct MhaAttnArgs {
     const int* seq_len; int len_off;
 };
 struct RopeMhaArgs;
-// OFT's block-bidirectional prefill (attention.cu, up to 384 keys): q_per_sample == n_keys rows per sequence from position
+// OFT's block-bidirectional prefill (attention.cu, up to 1024 keys; K and V resident up to 384): q_per_sample == n_keys rows per sequence from position
 // 0; sequence b's query p sees key k iff k < seq_len[b] and (k <= p, or p >= block_start[b] and k >= block_start[b]).
 // a.seq_len and block_start are device arrays [batch], read at run time; block_start[b] == seq_len[b] is plain causal.
 cudaError_t launch_mha_block_attention(cudaStream_t stream, const MhaAttnArgs& a, const int* block_start);

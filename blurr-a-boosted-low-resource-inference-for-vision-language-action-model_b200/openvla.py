@@ -51,6 +51,7 @@ class LlamaShapedConfig:
     max_positions: int = 320      # 1 + 256 patches + prompt + 7 action tokens fits
     rms_eps: float = 1e-6
     rope_theta: float = 10000.0
+    long_forward: bool = False    # max_positions up to 1024 for forward_rows (384 without); generate stops at 320 either way
 
 
 def openvla_7b_config() -> LlamaShapedConfig:
@@ -125,7 +126,7 @@ class LlamaDecoder:
         self.max_batch = max_batch
         self.handle = C.c_void_p()
         c = capi.LlmConfigC(capi.LLM_ABI_VERSION, cfg.num_layers, cfg.hidden, cfg.num_heads, cfg.num_kv_heads, cfg.head_dim,
-                            cfg.intermediate, cfg.vocab, cfg.max_positions, cfg.rms_eps)
+                            cfg.intermediate, cfg.vocab, cfg.max_positions, cfg.rms_eps, int(cfg.long_forward))
         index = self.device.index if self.device.index is not None else torch.cuda.current_device()
         capi.check(self.lib.blurr_llm_create(C.byref(c), index, max_batch, C.byref(self.handle)))
 
@@ -821,7 +822,9 @@ class OftConfig:
     """OpenVLA-OFT's action chunking (Kim, Finn, Liang 2025): `chunk` actions of `action_dim` dimensions per call, one
     empty action slot per value.  `bidirectional_actions`: the slots (and the stop token) attend to each other, as the
     paper describes; False gives plain causal attention.  The head is `MLPResNet(head_num_blocks, action_dim * hidden,
-    head_hidden_dim, action_dim)`; `max_positions` is the decoder's (1 + 256 patches + prompt + 56 slots + stop)."""
+    head_hidden_dim, action_dim)`; `max_positions` is the decoder's (1 + patches + prompt + 56 slots + stop).
+    `num_images` cameras (third-person first, then the wrist camera) give 256 patch rows each; `use_proprio` appends
+    one projected row of the `proprio_dim`-wide robot state after them."""
     chunk: int = 8
     action_dim: int = 7
     bidirectional_actions: bool = True
@@ -831,11 +834,32 @@ class OftConfig:
     max_positions: int = 384
     empty_token: int = 29871          # Llama-2's empty token after "Out:"
     stop_token: int = 2               # </s>
+    num_images: int = 1
+    use_proprio: bool = False
+    proprio_dim: int = 8
+
+
+def oft_libero_config() -> OftConfig:
+    """OFT's LIBERO checkpoints: third-person and wrist cameras, 8-D proprioception, chunks of 8 x 7.  A sequence is
+    1 + 513 + prompt + 56 + 1 positions (about 605 with LIBERO's instructions); the decoder holds 640."""
+    return OftConfig(num_images=2, use_proprio=True, proprio_dim=8, chunk=8, action_dim=7, max_positions=640)
 
 
 def openvla_oft_7b_config(oft: Optional[OftConfig] = None) -> LlamaShapedConfig:
-    """The OpenVLA-7B decoder with room for OFT's sequence (384 positions; `openvla_7b_config` keeps 320)."""
-    return LlamaShapedConfig(max_positions=(oft or OftConfig()).max_positions)
+    """The OpenVLA-7B decoder with room for OFT's sequence (`oft.max_positions`, 384 by default; `openvla_7b_config`
+    keeps 320).  Past 384 positions the decoder is created with `long_forward`."""
+    n = (oft or OftConfig()).max_positions
+    return LlamaShapedConfig(max_positions=n, long_forward=n > 384)
+
+
+def normalize_proprio(state, q01, q99, mask=None) -> np.ndarray:
+    """OFT's BOUNDS_Q99 normalisation of the robot state, on the host in float64:
+    `clip(where(mask, 2 * (x - q01) / (q99 - q01 + 1e-8) - 1, x), -1, 1)`.  state [B, D] (or [D]); q01 / q99 / mask
+    [D] or [B, D]."""
+    x = np.asarray(state.detach().cpu() if isinstance(state, torch.Tensor) else state, dtype=np.float64)
+    lo, hi = np.asarray(q01, dtype=np.float64), np.asarray(q99, dtype=np.float64)
+    m = np.ones(lo.shape, dtype=bool) if mask is None else np.asarray(mask, dtype=bool)
+    return np.clip(np.where(m, 2 * (x - lo) / (hi - lo + 1e-8) - 1, x), -1.0, 1.0)
 
 
 @dataclass
@@ -998,51 +1022,176 @@ def synthetic_act_head_state_dict(cfg: OftConfig, input_dim: int, device, seed: 
     return sd
 
 
-class OftPolicy:
-    """OpenVLA-OFT's `predict_action` with parallel decoding: device preprocessing -> DINOv2 + SigLIP towers ->
-    projector -> `[BOS] + patches + prompt + empty action slots + stop` -> one decoder pass (`forward_rows`) -> the
-    L1-regression head -> a whole chunk of de-normalised actions.  No decode loop: one call yields `chunk` actions."""
+class ProprioProjector:
+    """OpenVLA-OFT's `ProprioProjector`: `fc1 (proprio_dim -> hidden) -> GELU (exact) -> fc2 (hidden -> hidden)`, on
+    the `MlpProjector` engine.  That engine takes inputs 64 columns wide, so the state is zero-padded to 64 columns and
+    fc1's weight to [hidden, 64]; the padded products are exact zeros, so the result is fc1's."""
 
-    def __init__(self, preprocessor: ImagePreprocessor, backbone: FusedVisionBackbone, decoder: LlamaDecoder,
-                 head: L1RegressionHead, cfg: Optional[OftConfig] = None):
-        if preprocessor.n_norms != 2:
-            raise ValueError("the fused backbone needs two normalisations (DINOv2's, then SigLIP's)")
+    K_PAD = 64
+
+    def __init__(self, proprio_dim: int, hidden: int, device, max_rows: int = 1):
+        if not 1 <= proprio_dim <= self.K_PAD:
+            raise ValueError(f"proprio_dim must be in 1..{self.K_PAD}")
+        self.proprio_dim, self.hidden = int(proprio_dim), int(hidden)
+        self.device = torch.device(device)
+        self.mlp = MlpProjector([self.K_PAD, self.hidden, self.hidden], device, max_rows)
+
+    @classmethod
+    def from_state_dict(cls, state_dict: Dict[str, torch.Tensor], device, max_rows: int = 1, prefix: str = "") -> "ProprioProjector":
+        """`state_dict`: keys of OFT's `ProprioProjector.state_dict()` ("fc1.weight", "fc1.bias", "fc2.weight",
+        "fc2.bias"), optionally under `prefix`."""
+        sd = {k[len(prefix):]: v for k, v in state_dict.items() if k.startswith(prefix)}
+        missing = {"fc1.weight", "fc1.bias", "fc2.weight", "fc2.bias"} - set(sd)
+        if missing:
+            raise ValueError(f"ProprioProjector.from_state_dict: missing {sorted(missing)}")
+        hidden, dim = sd["fc1.weight"].shape
+        self = cls(dim, hidden, device, max_rows)
+        try:
+            w1 = torch.zeros((hidden, cls.K_PAD), device=self.device, dtype=torch.bfloat16)
+            w1[:, :dim] = sd["fc1.weight"].to(device=self.device, dtype=torch.bfloat16)
+            self.mlp.set_layer(0, w1, sd["fc1.bias"])
+            self.mlp.set_layer(1, sd["fc2.weight"], sd["fc2.bias"])
+        except Exception:
+            self.close()
+            raise
+        return self
+
+    @classmethod
+    def synthetic(cls, proprio_dim: int, hidden: int, device, max_rows: int = 1, seed: int = 0) -> "ProprioProjector":
+        """Random-init projector with nn.Linear's default init (uniform, bound 1 / sqrt(fan_in))."""
+        g = torch.Generator(device=device)
+        g.manual_seed(seed)
+
+        def u(shape, fan_in):
+            return ((torch.rand(shape, device=device, generator=g) * 2 - 1) / math.sqrt(fan_in)).to(torch.bfloat16)
+
+        sd = {"fc1.weight": u((hidden, proprio_dim), proprio_dim), "fc1.bias": u((hidden,), proprio_dim),
+              "fc2.weight": u((hidden, hidden), hidden), "fc2.bias": u((hidden,), hidden)}
+        return cls.from_state_dict(sd, device, max_rows)
+
+    def forward(self, state: torch.Tensor) -> torch.Tensor:
+        """state [B, proprio_dim] (already normalised; cast to bf16 on the device) -> bf16 [B, hidden]."""
+        if state.dim() != 2 or state.shape[1] != self.proprio_dim:
+            raise ValueError(f"state must be [B, {self.proprio_dim}]")
+        x = torch.zeros((state.shape[0], self.K_PAD), device=self.device, dtype=torch.bfloat16)
+        x[:, :self.proprio_dim] = state.to(device=self.device, dtype=torch.bfloat16)
+        return self.mlp.forward(x)
+
+    def close(self):
+        self.mlp.close()
+
+
+class OftPolicy:
+    """OpenVLA-OFT's `predict_action` with parallel decoding: device preprocessing of each camera -> DINOv2 + SigLIP
+    towers -> projector (-> the proprio projector) -> `[BOS] + patches (+ proprio row) + prompt + empty action slots +
+    stop` -> one decoder pass (`forward_rows`) -> the L1-regression head -> a whole chunk of de-normalised actions.  No
+    decode loop: one call yields `chunk` actions.  `preprocessor` is one `ImagePreprocessor` per camera (a single one
+    for one camera); the towers need max_batch >= B * num_images."""
+
+    def __init__(self, preprocessor, backbone: FusedVisionBackbone, decoder: LlamaDecoder,
+                 head: L1RegressionHead, cfg: Optional[OftConfig] = None, proprio_projector: Optional[ProprioProjector] = None):
         cfg = cfg or head.cfg
+        pres = list(preprocessor) if isinstance(preprocessor, (list, tuple)) else [preprocessor]
+        if len(pres) != cfg.num_images:
+            raise ValueError(f"{len(pres)} preprocessors for {cfg.num_images} cameras")
+        for p in pres:
+            if p.n_norms != 2:
+                raise ValueError("the fused backbone needs two normalisations (DINOv2's, then SigLIP's)")
         if (head.cfg.chunk, head.cfg.action_dim) != (cfg.chunk, cfg.action_dim) or head.input_dim != decoder.cfg.hidden:
             raise ValueError("the head's chunk, action_dim and input width must match the config and the decoder")
-        self.preprocessor, self.backbone, self.decoder, self.head, self.cfg = preprocessor, backbone, decoder, head, cfg
+        if cfg.use_proprio and (proprio_projector is None or proprio_projector.proprio_dim != cfg.proprio_dim
+                                or proprio_projector.hidden != decoder.cfg.hidden):
+            raise ValueError("use_proprio needs a ProprioProjector of proprio_dim columns and the decoder's width")
+        self.preprocessors, self.preprocessor = pres, pres[0]
+        self.backbone, self.decoder, self.head, self.cfg = backbone, decoder, head, cfg
+        self.proprio_projector = proprio_projector if cfg.use_proprio else None
 
     def pixel_values(self, frames) -> torch.Tensor:
-        """uint8 frame(s) [H, W, 3] / [B, H, W, 3] -> bf16 [B, 6, 224, 224] (as `OpenVlaPolicy.pixel_values`)."""
-        f = torch.as_tensor(frames)
-        if f.dim() == 3:
-            f = f[None]
-        if not f.is_cuda:
-            f = f.to(self.preprocessor.device)
-        return self.preprocessor(f)
+        """uint8 frame(s) [H, W, 3] / [B, H, W, 3] (one camera), or a sequence of num_images such batches (one per
+        camera, in the config's order) -> bf16 [B, 6 * num_images, 224, 224]: each camera's `OpenVlaPolicy.pixel_values`
+        stacked along channels."""
+        n = self.cfg.num_images
+        per_cam = [frames] if n == 1 else list(frames) if isinstance(frames, (list, tuple)) else None
+        if per_cam is None or len(per_cam) != n:
+            raise ValueError(f"frames must be a sequence of {n} per-camera uint8 batches")
+        out = []
+        for pre, fr in zip(self.preprocessors, per_cam):
+            f = torch.as_tensor(fr)
+            if f.dim() == 3:
+                f = f[None]
+            if not f.is_cuda:
+                f = f.to(pre.device)
+            out.append(pre(f))
+        if len({o.shape[0] for o in out}) != 1:
+            raise ValueError("every camera needs the same batch size")
+        return out[0] if n == 1 else torch.cat(out, dim=1)
 
-    def action_rows(self, pixel_values: torch.Tensor, input_ids, attention_mask: Optional[torch.Tensor] = None) -> torch.Tensor:
+    def patch_embeds(self, pixel_values: torch.Tensor, proprio_state: Optional[torch.Tensor] = None) -> torch.Tensor:
+        """bf16 pixel values [B, 6 * num_images, 224, 224] (and the normalised state [B, proprio_dim]) -> the rows
+        between BOS and the prompt, bf16 [B, 256 * num_images (+ 1), hidden]: image i's patches at rows 256 i ..
+        (OFT's `torch.cat(all_patches, dim=1)`), then the projected state."""
+        n = self.cfg.num_images
+        if pixel_values.dim() != 4 or pixel_values.shape[1] != 6 * n:
+            raise ValueError(f"pixel_values must be [B, {6 * n}, H, W] ({n} camera(s) of 6 channels)")
+        B = pixel_values.shape[0]
+        px = pixel_values if n == 1 else pixel_values.reshape(B * n, 6, *pixel_values.shape[2:])
+        patch = self.backbone.forward(px[:, :3], px[:, 3:])
+        if n > 1:
+            patch = patch.reshape(B, n * patch.shape[1], patch.shape[2])
+        if self.proprio_projector is None:
+            return patch
+        if proprio_state is None or proprio_state.dim() != 2 or tuple(proprio_state.shape) != (B, self.cfg.proprio_dim):
+            raise ValueError(f"use_proprio needs a proprio state [{B}, {self.cfg.proprio_dim}]")
+        row = self.proprio_projector.forward(proprio_state)
+        return torch.cat([patch, row[:, None].to(patch.dtype)], dim=1)
+
+    def action_rows(self, pixel_values: torch.Tensor, input_ids, attention_mask: Optional[torch.Tensor] = None,
+                    proprio_state: Optional[torch.Tensor] = None) -> torch.Tensor:
         """The decoder's final-normed rows in front of the action slots, bf16 [B, chunk * action_dim, hidden]."""
-        patch = self.backbone.forward(pixel_values[:, :3], pixel_values[:, 3:])
+        patch = self.patch_embeds(pixel_values, proprio_state)
         lay = oft_prompt_layout(input_ids, attention_mask, patch.shape[1], self.cfg)
         if lay.max_len > self.decoder.cfg.max_positions:
             raise ValueError(f"an OFT sequence needs {lay.max_len} positions; the decoder holds {self.decoder.cfg.max_positions}")
         x = build_oft_embeds(self.decoder, lay, patch, self.cfg.stop_token)
         return self.decoder.forward_rows(x, lay.seq_lens, lay.block_starts, lay.row_starts, lay.n_rows)
 
+    def proprio_state(self, proprio, proprio_q01, proprio_q99, proprio_mask=None) -> Optional[torch.Tensor]:
+        """The raw robot state [B, proprio_dim] -> `normalize_proprio` on the host -> float32 -> bf16 on the device, as
+        OFT's `torch.Tensor(proprio).to(bfloat16)` (None when the config has no proprio)."""
+        if not self.cfg.use_proprio:
+            if proprio is not None:
+                raise ValueError("proprio given, but the config has use_proprio = False")
+            return None
+        if proprio is None or proprio_q01 is None or proprio_q99 is None:
+            raise ValueError("use_proprio needs proprio, proprio_q01 and proprio_q99")
+        p = np.asarray(proprio.detach().cpu() if isinstance(proprio, torch.Tensor) else proprio, dtype=np.float64)
+        if p.ndim == 1:
+            p = p[None]
+        if p.ndim != 2 or p.shape[1] != self.cfg.proprio_dim:
+            raise ValueError(f"proprio must be [B, {self.cfg.proprio_dim}], got shape {p.shape}")
+        x = normalize_proprio(p, proprio_q01, proprio_q99, proprio_mask)
+        return torch.from_numpy(x.astype(np.float32)).to(device=self.decoder.device, dtype=torch.bfloat16)
+
     def predict_action_chunk_from_pixels(self, pixel_values: torch.Tensor, input_ids, q01, q99, mask=None,
-                                         attention_mask: Optional[torch.Tensor] = None, return_normalized: bool = False):
-        """The same as `predict_action_chunk`, from prepared bf16 pixel values [B, 6, 224, 224]."""
-        norm = self.head.forward(self.action_rows(pixel_values, input_ids, attention_mask))
+                                         attention_mask: Optional[torch.Tensor] = None, return_normalized: bool = False,
+                                         proprio=None, proprio_q01=None, proprio_q99=None, proprio_mask=None):
+        """The same as `predict_action_chunk`, from prepared bf16 pixel values [B, 6 * num_images, 224, 224]."""
+        state = self.proprio_state(proprio, proprio_q01, proprio_q99, proprio_mask)
+        if state is not None and state.shape[0] != pixel_values.shape[0]:
+            raise ValueError("proprio must hold one state per sequence")
+        norm = self.head.forward(self.action_rows(pixel_values, input_ids, attention_mask, state))
         actions = torch.from_numpy(denormalize_chunk(norm.cpu().numpy(), q01, q99, mask))
         return (actions, norm) if return_normalized else actions
 
     def predict_action_chunk(self, frames, input_ids, q01, q99, mask=None, attention_mask: Optional[torch.Tensor] = None,
-                             return_normalized: bool = False):
-        """frames: uint8 [H, W, 3] or [B, H, W, 3] RGB.  input_ids: [B, S] (first column BOS), a list of B 1-D id tensors,
-        or [B, S] with a left- or right-padded `attention_mask` (see `oft_prompt_layout`).  q01 / q99 / mask:
-        [action_dim] or [B, action_dim], applied to every step of the chunk.  Returns float64 actions
-        [B, chunk, action_dim] on the host (and, with `return_normalized`, the head's output fp32 [B, chunk, action_dim]
-        on the device)."""
+                             return_normalized: bool = False, proprio=None, proprio_q01=None, proprio_q99=None,
+                             proprio_mask=None):
+        """frames: uint8 [H, W, 3] or [B, H, W, 3] RGB for one camera; with num_images > 1 a sequence of such batches,
+        one per camera (third-person first, then the wrist camera).  input_ids: [B, S] (first column BOS), a list of B
+        1-D id tensors, or [B, S] with a left- or right-padded `attention_mask` (see `oft_prompt_layout`).  q01 / q99 /
+        mask: [action_dim] or [B, action_dim], applied to every step of the chunk.  With `use_proprio`: `proprio` the
+        raw state [B, proprio_dim] and its dataset's `proprio_q01` / `proprio_q99` (/ `proprio_mask`), normalised by
+        `normalize_proprio`.  Returns float64 actions [B, chunk, action_dim] on the host (and, with
+        `return_normalized`, the head's output fp32 [B, chunk, action_dim] on the device)."""
         return self.predict_action_chunk_from_pixels(self.pixel_values(frames), input_ids, q01, q99, mask, attention_mask,
-                                                     return_normalized)
+                                                     return_normalized, proprio, proprio_q01, proprio_q99, proprio_mask)
