@@ -82,11 +82,11 @@ class VitConfigC(C.Structure):
     _fields_ = [
         ("abi_version", C.c_int32), ("num_layers", C.c_int32), ("hidden", C.c_int32), ("num_heads", C.c_int32),
         ("mlp_dim", C.c_int32), ("image_size", C.c_int32), ("patch_size", C.c_int32), ("num_prefix_tokens", C.c_int32),
-        ("use_layerscale", C.c_int32), ("gelu_erf", C.c_int32), ("ln_eps", C.c_float),
+        ("use_layerscale", C.c_int32), ("gelu_erf", C.c_int32), ("ln_eps", C.c_float), ("film_dim", C.c_int32),
     ]
 
 
-VIT_ABI_VERSION = 1
+VIT_ABI_VERSION = 2
 
 
 class Pi0InputsC(C.Structure):
@@ -177,6 +177,8 @@ _SIGNATURES = [
     ("blurr_vit_set_weight", C.c_int, [C.c_void_p, C.c_char_p, C.c_void_p, C.POINTER(C.c_int64), C.c_int]),
     ("blurr_vit_finalize", C.c_int, [C.c_void_p]),
     ("blurr_vit_forward", C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.POINTER(C.c_int64), C.c_void_p, C.c_int]),
+    ("blurr_vit_forward_film", C.c_int,
+     [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.POINTER(C.c_int64), C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_int]),
     ("blurr_vit_set_option", C.c_int, [C.c_void_p, C.c_char_p, C.c_int64]),
     ("blurr_vit_last_launch_count", C.c_int64, [C.c_void_p]),
     ("blurr_mlp_create", C.c_int, [C.POINTER(C.c_int32), C.c_int, C.c_int, C.c_int, C.POINTER(C.c_void_p)]),

@@ -105,7 +105,9 @@ __device__ __forceinline__ void consumer_prefetch(const ConsumerArgs& a, const i
     }
 }
 
-template <int VPT, int THREADS = kRowThreads, bool PRELOADED = false>
+// FILM: the FiLM step of the ViT towers (ConsumerArgs::film_gamma) - a compile-time variant, so that the instantiations
+// without it keep their code
+template <int VPT, int THREADS = kRowThreads, bool PRELOADED = false, bool FILM = false>
 __device__ __forceinline__ void consumer_body(const ConsumerArgs& a, const int t, const ConsumerRowIn<VPT>* pre = nullptr) {
     __shared__ float red[(THREADS + 31) / 32];
     const int nvec = a.N >> 2;
@@ -117,12 +119,18 @@ __device__ __forceinline__ void consumer_body(const ConsumerArgs& a, const int t
     const bool want_norm = a.norm_mode != NORM_NONE && a.xn_out != nullptr;
     const bool from_res = a.partial == nullptr && a.lin == nullptr;
     uint2 pf_add[VPT], pf_w[VPT], pf_b[VPT];
+    uint2 pf_fg[VPT], pf_fb[VPT];          // FiLM gamma / beta of the row's condition
 #pragma unroll
     for (int i = 0; i < VPT; ++i) {
         const int v = threadIdx.x + i * THREADS;
         pf_add[i] = make_uint2(0u, 0u); pf_w[i] = make_uint2(0u, 0u); pf_b[i] = make_uint2(0u, 0u);
         if (v >= nvec) continue;
         const int n = v << 2;
+        if constexpr (FILM) {
+            const size_t c = static_cast<size_t>(t / a.film_rows) * a.film_ld + n;
+            pf_fg[i] = __ldcg(reinterpret_cast<const uint2*>(a.film_gamma + c));
+            pf_fb[i] = __ldcg(reinterpret_cast<const uint2*>(a.film_beta + c));
+        }
         if (!PRELOADED || from_res) {
             if (from_res || a.add_mode == ADD_RESIDUAL) pf_add[i] = __ldcg(reinterpret_cast<const uint2*>(a.res + static_cast<size_t>(t) * a.ldr + n));
             else if (a.add_mode == ADD_POSEMB) pf_add[i] = __ldcg(reinterpret_cast<const uint2*>(a.pos + static_cast<size_t>(t % a.pos_rows) * a.N + n));
@@ -172,6 +180,14 @@ __device__ __forceinline__ void consumer_body(const ConsumerArgs& a, const int t
             }
         } else {
             val = unpack_bf16x4(pf_add[i]);
+        }
+        if constexpr (FILM) {
+            // torch's bf16 `x * (1 + gamma) + beta`: every operation rounded to bf16
+            const float4 g = unpack_bf16x4(pf_fg[i]), be = unpack_bf16x4(pf_fb[i]);
+            val = make_float4(bf16_round(bf16_round(val.x * bf16_round(1.0f + g.x)) + be.x),
+                              bf16_round(bf16_round(val.y * bf16_round(1.0f + g.y)) + be.y),
+                              bf16_round(bf16_round(val.z * bf16_round(1.0f + g.z)) + be.z),
+                              bf16_round(bf16_round(val.w * bf16_round(1.0f + g.w)) + be.w));
         }
         if (a.x_out != nullptr) store_bf16x4(a.x_out + static_cast<size_t>(to) * a.ldx + n, val);
         x[i] = val;

@@ -44,6 +44,11 @@ struct ConsumerArgs {
     // output row map (0 = identity): row t is written to row t + (t / row_group) * row_extra + row_offset of x_out / xn_out
     // (ViT prefix tokens: the 256 patch rows of sample b land behind that sample's cls / register rows)
     int row_group, row_extra, row_offset;
+    // FiLM (non-null film_gamma; 1024 or 1152 columns only): after the residual add, row t becomes
+    // bf16(bf16(x * bf16(1 + gamma[c])) + beta[c]) with c = t / film_rows, before x_out and the norm statistics
+    const bf16* film_gamma;  // [n_cond][film_ld]
+    const bf16* film_beta;   // [n_cond][film_ld]
+    int film_ld, film_rows;
 };
 cudaError_t launch_consumer(cudaStream_t stream, const ConsumerArgs& a);
 

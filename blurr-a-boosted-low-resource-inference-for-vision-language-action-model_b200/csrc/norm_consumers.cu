@@ -13,19 +13,19 @@
 
 namespace blurr {
 
-template <int VPT, int THREADS>
+template <int VPT, int THREADS, bool FILM = false>
 __global__ void __launch_bounds__(THREADS) consumer_kernel(const ConsumerArgs a) {
     trace_stamp(a.trace, 0);
     pdl_wait();
     pdl_trigger();     // only now: a successor that is resident earlier just holds SM resources while it waits (measured)
     trace_stamp(a.trace, 1);
-    consumer_body<VPT, THREADS>(a, blockIdx.x);
+    consumer_body<VPT, THREADS, false, FILM>(a, blockIdx.x);
     trace_stamp(a.trace, 2);
 }
 
 // Batched episodes, bf16 hand-off mode: a fixed grid streams the rows, every CTA fetching the inputs of its next
 // row before it reduces the current one (the one-row-per-CTA launch is latency-bound: 1.7-2.4 TB/s at 64 episodes).
-template <int VPT, int THREADS>
+template <int VPT, int THREADS, bool FILM = false>
 __global__ void __launch_bounds__(THREADS) consumer_stream_kernel(const ConsumerArgs a) {
     trace_stamp(a.trace, 0);
     pdl_wait();
@@ -37,7 +37,7 @@ __global__ void __launch_bounds__(THREADS) consumer_stream_kernel(const Consumer
     for (; t < a.T; t += gridDim.x) {
         const int tn = t + gridDim.x;
         if (tn < a.T) consumer_prefetch<VPT, THREADS>(a, tn, nxt);
-        consumer_body<VPT, THREADS, true>(a, t, &cur);
+        consumer_body<VPT, THREADS, true, FILM>(a, t, &cur);
         cur = nxt;
     }
     trace_stamp(a.trace, 2);
@@ -45,7 +45,22 @@ __global__ void __launch_bounds__(THREADS) consumer_stream_kernel(const Consumer
 
 static constexpr int kStreamMinRows = 2048;
 
+// FiLM consumers: the ViT towers' widths (DINOv2-L 1024, SigLIP-so400m 1152 columns) in the three regimes the towers
+// reach - split-K partials (<= 288 rows), the bf16 hand-off, and the streaming launch from kStreamMinRows rows
+static cudaError_t launch_film_consumer(cudaStream_t stream, const ConsumerArgs& a) {
+    if ((a.N != 4 * 256 && a.N != 4 * 288) || (a.ldp & 3) || (a.film_ld & 3) || a.film_rows < 1) return cudaErrorInvalidValue;
+    const bool wide = a.N == 4 * 288;
+    if (a.lin != nullptr && a.T >= kStreamMinRows && a.partial == nullptr) {
+        const int grid = 148 * 6;
+        if (wide) return launch_kernel(consumer_stream_kernel<1, 288, true>, dim3(grid), dim3(288), 0, stream, a);
+        return launch_kernel(consumer_stream_kernel<1, kRowThreads, true>, dim3(grid), dim3(kRowThreads), 0, stream, a);
+    }
+    if (wide) return launch_kernel(consumer_kernel<1, 288, true>, dim3(a.T), dim3(288), 0, stream, a);
+    return launch_kernel(consumer_kernel<1, kRowThreads, true>, dim3(a.T), dim3(kRowThreads), 0, stream, a);
+}
+
 cudaError_t launch_consumer(cudaStream_t stream, const ConsumerArgs& a) {
+    if (a.film_gamma != nullptr) return launch_film_consumer(stream, a);
     if (a.lin != nullptr && a.T >= kStreamMinRows && !(a.N & 3) && a.partial == nullptr) {
         const int grid = 148 * 6;
         if (a.N == 4 * 288) return launch_kernel(consumer_stream_kernel<1, 288>, dim3(grid), dim3(288), 0, stream, a);

@@ -3,6 +3,8 @@
 // patch tokens of the second-to-last block, and the 3-layer GELU projector.  A third client of the Pi-0 kernels: the
 // schedule is the one of the Pi-0 SigLIP tower (engine.cu run_vision) with three additions - prefix-token rows (the
 // consumer's output row map), LayerScale (the consumer's per-column scale) and the erf GELU flavour of the GEMM epilogue.
+// FiLM handles (film_dim > 0, OpenVLA-OFT's language conditioning) add one GEMM in front of the blocks - every block's
+// gamma and beta from the caller's conditioning rows - and the FiLM variant of the out-projection's consumer.
 #include "blurr_pi0.h"
 #include "blurr_vit.h"
 
@@ -129,6 +131,10 @@ struct blurr_vit {
     std::vector<void*> allocs;
     VLin patch;
     bf16 *pos = nullptr, *prefix = nullptr;
+    // FiLM: [layers * 2 * hidden][film_dim] tile-packed, block l's scale rows at 2 l hidden, its shift rows behind them;
+    // cond [max_batch][film_dim] (the caller's rows, copied in before the graph), film_out [max_batch][film.Nw]
+    VLin film;
+    bf16 *cond = nullptr, *film_out = nullptr;
     std::vector<VLayer> layers;
     bf16 *patches = nullptr, *X = nullptr, *XN = nullptr, *QKV = nullptr, *AO = nullptr, *HM = nullptr, *LINB = nullptr;
     float* ws = nullptr;
@@ -138,9 +144,9 @@ struct blurr_vit {
     bool finalized = false, use_graph = true;
     int64_t launches = 0;
     // blocks between the patch im2col (reads the caller's pixels) and the final row copy (writes the caller's buffer)
-    // only touch the handle's own buffers: one CUDA graph per batch size
+    // only touch the handle's own buffers: one CUDA graph per (batch size, images per condition; 0 without FiLM)
     struct GraphEntry { cudaGraph_t graph; cudaGraphExec_t exec; int64_t launches; };
-    std::map<int, GraphEntry> graphs;
+    std::map<std::pair<int, int>, GraphEntry> graphs;
 };
 
 extern "C" void blurr_vit_destroy(blurr_vit_t* h) {
@@ -163,6 +169,9 @@ extern "C" int blurr_vit_create(const blurr_vit_config* cfg, int device, int max
     const int hd = c.hidden / c.num_heads;
     if ((hd & 7) || hd > 80) return fail(BLURR_ERR_INVALID, "head_dim must be a multiple of 8 and <= 80");
     if (c.num_prefix_tokens < 0 || c.num_prefix_tokens > 16 || c.mlp_dim < 64) return fail(BLURR_ERR_INVALID, "bad prefix token count / mlp_dim");
+    if (c.film_dim < 0 || c.film_dim % 64 || c.film_dim > 8192) return fail(BLURR_ERR_INVALID, "film_dim must be 0 or a multiple of 64 (<= 8192)");
+    if (c.film_dim > 0 && c.hidden != 1024 && c.hidden != 1152)
+        return fail(BLURR_ERR_INVALID, "FiLM towers must be 1024 (DINOv2-L) or 1152 (SigLIP-so400m) wide");
     int ndev = 0;
     if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) return fail(BLURR_ERR_CUDA, "no CUDA device: the B200 path has no CPU fallback");
     if (device < 0 || device >= ndev) return fail(BLURR_ERR_INVALID, "bad device index");
@@ -188,6 +197,12 @@ extern "C" int blurr_vit_create(const blurr_vit_config* cfg, int device, int max
         L.ln1w = bufb(H); L.ln1b = bufb(H); L.ln2w = bufb(H); L.ln2b = bufb(H); L.ls1 = bufb(H); L.ls2 = bufb(H);
         ok &= L.ln1w && L.ln1b && L.ln2w && L.ln2b && L.ls1 && L.ls2;
     }
+    if (c.film_dim > 0) {
+        ok &= alloc_lin(h, h->film, c.num_layers * 2 * H, c.film_dim);
+        h->cond = bufb(static_cast<size_t>(max_batch) * c.film_dim);
+        h->film_out = bufb(static_cast<size_t>(max_batch) * h->film.Nw);
+        ok &= h->cond && h->film_out;
+    }
     const int mlp_pad = h->layers[0].fc1.Nw;
     h->patches = bufb(Tp * h->patch.K);
     h->X = bufb(T * H); h->XN = bufb(T * H); h->QKV = bufb(T * 3 * H); h->AO = bufb(T * H); h->HM = bufb(T * mlp_pad);
@@ -196,7 +211,8 @@ extern "C" int blurr_vit_create(const blurr_vit_config* cfg, int device, int max
     h->ws = static_cast<float*>(dalloc_in(h, h->ws_floats * 4));
     ok &= h->pos && h->prefix && h->patches && h->X && h->XN && h->QKV && h->AO && h->HM && h->LINB && h->ws;
     if (!ok) { blurr_vit_destroy(h); return fail(BLURR_ERR_CUDA, "blurr_vit_create: device allocation failed"); }
-    h->expected = 3 + (c.num_prefix_tokens > 0 ? 1 : 0) + static_cast<size_t>(c.num_layers) * (16 + (c.use_layerscale ? 2 : 0));
+    h->expected = 3 + (c.num_prefix_tokens > 0 ? 1 : 0) +
+                  static_cast<size_t>(c.num_layers) * (16 + (c.use_layerscale ? 2 : 0) + (c.film_dim > 0 ? 4 : 0));
     *out = h;
     return 0;
 }
@@ -253,6 +269,10 @@ extern "C" int blurr_vit_set_weight(blurr_vit_t* h, const char* key_c, const voi
             rc = pack_weight(src, H, c.mlp_dim, L.fc2, 0);          // K padded to fc1.Nw: the pad columns stay zero
         }
         else if (rest == "fc2.bias") rc = vec(L.fc2.bias, H);
+        else if (c.film_dim > 0 && (rest == "film_scale.weight" || rest == "film_shift.weight"))
+            rc = mat(h->film, (2 * l + (rest == "film_shift.weight" ? 1 : 0)) * H, H);
+        else if (c.film_dim > 0 && (rest == "film_scale.bias" || rest == "film_shift.bias"))
+            rc = vec(h->film.bias + static_cast<size_t>(2 * l + (rest == "film_shift.bias" ? 1 : 0)) * H, H);
         else return fail(BLURR_ERR_INVALID, "unknown key " + key);
     } else {
         return fail(BLURR_ERR_INVALID, "unknown key " + key);
@@ -273,13 +293,16 @@ extern "C" int blurr_vit_finalize(blurr_vit_t* h) {
     return 0;
 }
 
-// patch GEMM .. last block, on the handle's own buffers (graph-capturable)
-static void vit_body(blurr_vit* h, Launcher& R, int batch) {
+// patch GEMM .. last block, on the handle's own buffers (graph-capturable); FiLM handles: image i uses condition row
+// i / images_per_cond of h->cond
+static void vit_body(blurr_vit* h, Launcher& R, int batch, int images_per_cond) {
     const auto& c = h->cfg;
     cudaStream_t st = R.st;
     const int H = c.hidden, P = c.num_prefix_tokens, S = h->seq, NP = h->n_patches;
     const int T = batch * S, Tp = batch * NP;
     const int gelu = c.gelu_erf ? GELU_ERF : GELU_TANH;
+    // every block's gamma | beta of every condition row at once: bf16(cond W^T + b), as nn.Linear
+    if (c.film_dim > 0) R.gemm(h->film, h->cond, batch / images_per_cond, EPI_STORE, h->film_out, h->film.Nw, 0);
     {   // patch embedding + position embeddings -> the patch rows of X (behind each sample's prefix rows)
         ConsumerArgs a{};
         a.add_mode = ADD_POSEMB; a.pos = h->pos; a.pos_rows = NP;
@@ -306,6 +329,11 @@ static void vit_body(blurr_vit* h, Launcher& R, int batch) {
             a.add_mode = ADD_RESIDUAL; a.res = h->X; a.ldr = H; a.x_out = h->X; a.ldx = H;
             a.col_scale = c.use_layerscale ? L.ls1 : nullptr;
             a.norm_mode = NORM_LAYERNORM; a.norm_w = L.ln2w; a.norm_b = L.ln2b; a.eps = c.ln_eps; a.xn_out = h->XN; a.ldn = H;
+            if (c.film_dim > 0) {       // x = x * (1 + gamma) + beta between the attention and the MLP residual
+                a.film_gamma = h->film_out + static_cast<size_t>(2 * l) * H;
+                a.film_beta = a.film_gamma + H;
+                a.film_ld = h->film.Nw; a.film_rows = images_per_cond * S;
+            }
             R.linear_consumer(L.o, h->AO, T, a);
         }
         R.gemm(L.fc1, h->XN, T, EPI_GELU, h->HM, L.fc1.Nw, gelu);
@@ -322,27 +350,32 @@ static void vit_body(blurr_vit* h, Launcher& R, int batch) {
     }
 }
 
-extern "C" int blurr_vit_forward(blurr_vit_t* h, void* cuda_stream, int batch, const void* pixel_values, const int64_t strides[4],
-                                 void* out, int out_ld) {
-    if (!h || !pixel_values || !strides || !out) return fail(BLURR_ERR_INVALID, "blurr_vit_forward: null argument");
-    if (!h->finalized) return fail(BLURR_ERR_STATE, "blurr_vit_forward: call blurr_vit_finalize first");
-    if (batch < 1 || batch > h->max_batch) return fail(BLURR_ERR_INVALID, "blurr_vit_forward: batch out of range");
+// images_per_cond: 0 on handles without FiLM; cond is then unused
+static int vit_forward(blurr_vit* h, void* cuda_stream, int batch, const void* pixel_values, const int64_t strides[4],
+                       const void* cond, int cond_ld, int images_per_cond, void* out, int out_ld, const std::string& who) {
+    if (!h || !pixel_values || !strides || !out) return fail(BLURR_ERR_INVALID, who + ": null argument");
+    if (!h->finalized) return fail(BLURR_ERR_STATE, who + ": call blurr_vit_finalize first");
+    if (batch < 1 || batch > h->max_batch) return fail(BLURR_ERR_INVALID, who + ": batch out of range");
     const auto& c = h->cfg;
     const int H = c.hidden, P = c.num_prefix_tokens, S = h->seq, NP = h->n_patches;
-    if (out_ld < H || (out_ld & 7)) return fail(BLURR_ERR_INVALID, "blurr_vit_forward: out_ld must be >= hidden and a multiple of 8");
+    if (out_ld < H || (out_ld & 7)) return fail(BLURR_ERR_INVALID, who + ": out_ld must be >= hidden and a multiple of 8");
     VIT_CUDA_TRY(cudaSetDevice(h->device));
     cudaStream_t st = static_cast<cudaStream_t>(cuda_stream);
     h->launches = 0;
     Launcher R{st, h->ws, h->ws_floats, h->LINB, &h->launches};
+    if (images_per_cond > 0)        // the graph reads the handle's copy: one graph serves every condition
+        VIT_CUDA_TRY(cudaMemcpy2DAsync(h->cond, static_cast<size_t>(c.film_dim) * 2, cond, static_cast<size_t>(cond_ld) * 2,
+                                       static_cast<size_t>(c.film_dim) * 2, batch / images_per_cond, cudaMemcpyDeviceToDevice, st));
     R.launched(launch_im2col(st, static_cast<const bf16*>(pixel_values), strides[0], strides[1], strides[2], strides[3], batch,
                              h->patches, h->patch.K), "im2col");
     if (R.rc) return R.rc;
     if (!h->use_graph) {
-        vit_body(h, R, batch);
+        vit_body(h, R, batch, images_per_cond);
     } else {
-        auto it = h->graphs.find(batch);
+        const std::pair<int, int> key(batch, images_per_cond);
+        auto it = h->graphs.find(key);
         if (it == h->graphs.end()) {
-            vit_body(h, R, batch);                                   // warm run: attribute setup, tensor maps
+            vit_body(h, R, batch, images_per_cond);                                   // warm run: attribute setup, tensor maps
             if (R.rc) return R.rc;
             VIT_CUDA_TRY(cudaStreamSynchronize(st));
             int64_t captured = 0;
@@ -351,7 +384,7 @@ extern "C" int blurr_vit_forward(blurr_vit_t* h, void* cuda_stream, int batch, c
             Launcher C{cs, h->ws, h->ws_floats, h->LINB, &captured};
             cudaError_t e = cudaStreamBeginCapture(cs, cudaStreamCaptureModeThreadLocal);
             if (e != cudaSuccess) { cudaStreamDestroy(cs); return fail(BLURR_ERR_CUDA, "graph capture begin failed"); }
-            vit_body(h, C, batch);
+            vit_body(h, C, batch, images_per_cond);
             cudaGraph_t g = nullptr;
             e = cudaStreamEndCapture(cs, &g);
             cudaStreamDestroy(cs);
@@ -360,7 +393,7 @@ extern "C" int blurr_vit_forward(blurr_vit_t* h, void* cuda_stream, int batch, c
             cudaGraphExec_t ex = nullptr;
             e = cudaGraphInstantiate(&ex, g, 0);
             if (e != cudaSuccess) { cudaGraphDestroy(g); return fail(BLURR_ERR_CUDA, std::string("graph instantiate failed: ") + cudaGetErrorString(e)); }
-            it = h->graphs.emplace(batch, blurr_vit::GraphEntry{g, ex, captured}).first;
+            it = h->graphs.emplace(key, blurr_vit::GraphEntry{g, ex, captured}).first;
             h->launches = 1;                                         // the im2col of this call; the replay below adds the rest
         }
         VIT_CUDA_TRY(cudaGraphLaunch(it->second.exec, st));
@@ -368,6 +401,24 @@ extern "C" int blurr_vit_forward(blurr_vit_t* h, void* cuda_stream, int batch, c
     }
     if (!R.rc) R.launched(launch_copy_rows(st, h->X, batch, S, P, NP, H, H, static_cast<bf16*>(out), out_ld), "copy_rows");
     return R.rc;
+}
+
+extern "C" int blurr_vit_forward(blurr_vit_t* h, void* cuda_stream, int batch, const void* pixel_values, const int64_t strides[4],
+                                 void* out, int out_ld) {
+    if (h && h->cfg.film_dim > 0) return fail(BLURR_ERR_STATE, "blurr_vit_forward: a FiLM handle needs blurr_vit_forward_film");
+    return vit_forward(h, cuda_stream, batch, pixel_values, strides, nullptr, 0, 0, out, out_ld, "blurr_vit_forward");
+}
+
+extern "C" int blurr_vit_forward_film(blurr_vit_t* h, void* cuda_stream, int batch, const void* pixel_values, const int64_t strides[4],
+                                      const void* cond, int cond_ld, int images_per_cond, void* out, int out_ld) {
+    if (!h) return fail(BLURR_ERR_INVALID, "blurr_vit_forward_film: null handle");
+    if (h->cfg.film_dim == 0) return fail(BLURR_ERR_STATE, "blurr_vit_forward_film: the handle was created without FiLM (film_dim 0)");
+    if (!cond) return fail(BLURR_ERR_INVALID, "blurr_vit_forward_film: null cond");
+    if (cond_ld < h->cfg.film_dim) return fail(BLURR_ERR_INVALID, "blurr_vit_forward_film: cond_ld smaller than film_dim");
+    if (images_per_cond < 1 || batch % images_per_cond)
+        return fail(BLURR_ERR_INVALID, "blurr_vit_forward_film: images_per_cond must be >= 1 and divide batch");
+    return vit_forward(h, cuda_stream, batch, pixel_values, strides, cond, cond_ld, images_per_cond, out, out_ld,
+                       "blurr_vit_forward_film");
 }
 
 extern "C" int blurr_vit_set_option(blurr_vit_t* h, const char* name, int64_t value) {

@@ -31,7 +31,7 @@ from __future__ import annotations
 import ctypes as C
 import math
 from dataclasses import dataclass
-from typing import Dict, Optional, Sequence, Tuple, Union
+from typing import Dict, List, Optional, Sequence, Tuple, Union
 
 import numpy as np
 import torch
@@ -427,6 +427,7 @@ class VitShapedConfig:
     image_size: int = 224
     patch_size: int = 14
     ln_eps: float = 1e-6
+    film_dim: int = 0          # > 0: FiLM-conditioned blocks (OpenVLA-OFT's language conditioning), conditioning width
 
 
 def dinov2_large_reg4_config(depth: int = 24) -> VitShapedConfig:
@@ -450,7 +451,8 @@ class VitEncoder:
         self.max_batch = max_batch
         self.handle = C.c_void_p()
         c = capi.VitConfigC(capi.VIT_ABI_VERSION, cfg.num_layers, cfg.hidden, cfg.num_heads, cfg.mlp_dim, cfg.image_size,
-                            cfg.patch_size, cfg.num_prefix_tokens, int(cfg.use_layerscale), int(cfg.gelu_erf), cfg.ln_eps)
+                            cfg.patch_size, cfg.num_prefix_tokens, int(cfg.use_layerscale), int(cfg.gelu_erf), cfg.ln_eps,
+                            cfg.film_dim)
         index = self.device.index if self.device.index is not None else torch.cuda.current_device()
         capi.check(self.lib.blurr_vit_create(C.byref(c), index, max_batch, C.byref(self.handle)))
         self.n_patches = (cfg.image_size // cfg.patch_size) ** 2
@@ -467,15 +469,24 @@ class VitEncoder:
     def set_option(self, name: str, value: int):
         capi.check(self.lib.blurr_vit_set_option(self.handle, name.encode(), int(value)))
 
+    def _set_films(self, films: Optional[Dict[str, torch.Tensor]]):
+        """FiLM Linears from a state dict keyed like OFT's per-block pairs: "N.scale.weight|bias", "N.shift.weight|bias"."""
+        for l in range(self.cfg.num_layers if films is not None else 0):
+            for name in ("scale", "shift"):
+                self.set_weight(f"layers.{l}.film_{name}.weight", films[f"{l}.{name}.weight"])
+                self.set_weight(f"layers.{l}.film_{name}.bias", films[f"{l}.{name}.bias"])
+
     @classmethod
-    def from_hf_dinov2(cls, model, device, max_batch: int = 1, num_layers: Optional[int] = None) -> "VitEncoder":
-        """From a transformers `Dinov2WithRegistersModel` (image_size 224 so that its position embeddings are native)."""
+    def from_hf_dinov2(cls, model, device, max_batch: int = 1, num_layers: Optional[int] = None,
+                       films: Optional[Dict[str, torch.Tensor]] = None) -> "VitEncoder":
+        """From a transformers `Dinov2WithRegistersModel` (image_size 224 so that its position embeddings are native).
+        `films`: FiLM weights ("N.scale.weight" [hidden, film_dim], ...) for a FiLM tower."""
         hc = model.config
         depth = hc.num_hidden_layers
         cfg = VitShapedConfig(num_layers=num_layers or depth - 1, hidden=hc.hidden_size, num_heads=hc.num_attention_heads,
                               mlp_dim=int(hc.hidden_size * hc.mlp_ratio), num_prefix_tokens=1 + hc.num_register_tokens,
                               use_layerscale=True, gelu_erf=True, image_size=hc.image_size, patch_size=hc.patch_size,
-                              ln_eps=hc.layer_norm_eps)
+                              ln_eps=hc.layer_norm_eps, film_dim=films["0.scale.weight"].shape[1] if films else 0)
         self = cls(cfg, device, max_batch)
         sd = {k: v.to(torch.bfloat16) for k, v in model.state_dict().items()}
         e = "embeddings."
@@ -494,16 +505,19 @@ class VitEncoder:
                 self.set_weight(q + b + ".bias", sd[p + a + ".bias"])
             self.set_weight(q + "ls1", sd[p + "layer_scale1.lambda1"])
             self.set_weight(q + "ls2", sd[p + "layer_scale2.lambda1"])
+        self._set_films(films)
         self.finalize()
         return self
 
     @classmethod
-    def from_hf_siglip(cls, model, device, max_batch: int = 1, num_layers: Optional[int] = None) -> "VitEncoder":
-        """From a transformers `SiglipVisionModel`."""
+    def from_hf_siglip(cls, model, device, max_batch: int = 1, num_layers: Optional[int] = None,
+                       films: Optional[Dict[str, torch.Tensor]] = None) -> "VitEncoder":
+        """From a transformers `SiglipVisionModel` (`films` as in `from_hf_dinov2`)."""
         hc = model.config
         cfg = VitShapedConfig(num_layers=num_layers or hc.num_hidden_layers - 1, hidden=hc.hidden_size,
                               num_heads=hc.num_attention_heads, mlp_dim=hc.intermediate_size, image_size=hc.image_size,
-                              patch_size=hc.patch_size, ln_eps=hc.layer_norm_eps)
+                              patch_size=hc.patch_size, ln_eps=hc.layer_norm_eps,
+                              film_dim=films["0.scale.weight"].shape[1] if films else 0)
         self = cls(cfg, device, max_batch)
         sd = {k: v.to(torch.bfloat16) for k, v in model.state_dict().items()}
         e = "vision_model.embeddings."
@@ -517,12 +531,14 @@ class VitEncoder:
                          ("self_attn.out_proj", "o")):
                 self.set_weight(q + b + ".weight", sd[p + a + ".weight"])
                 self.set_weight(q + b + ".bias", sd[p + a + ".bias"])
+        self._set_films(films)
         self.finalize()
         return self
 
     @classmethod
     def synthetic(cls, cfg: VitShapedConfig, device, max_batch: int = 1, seed: int = 0) -> "VitEncoder":
-        """Random-init tower of the given shape (benchmarks)."""
+        """Random-init tower of the given shape (benchmarks).  With `film_dim` the FiLM Linears are drawn after every other
+        weight, so a FiLM tower shares its other weights with the plain tower of the same seed."""
         self = cls(cfg, device, max_batch)
         g = torch.Generator(device=device)
         g.manual_seed(seed)
@@ -549,22 +565,42 @@ class VitEncoder:
             if cfg.use_layerscale:
                 self.set_weight(q + "ls1", ones)
                 self.set_weight(q + "ls2", ones)
+        for l in range(cfg.num_layers if cfg.film_dim else 0):
+            for name in ("film_scale", "film_shift"):
+                self.set_weight(f"layers.{l}.{name}.weight", w(H, cfg.film_dim))
+                self.set_weight(f"layers.{l}.{name}.bias", w(H))
         self.finalize()
         return self
 
-    def forward(self, pixel_values: torch.Tensor, out: Optional[torch.Tensor] = None) -> torch.Tensor:
-        """pixel_values bf16 [B, 3, 224, 224] -> bf16 [B, n_patches, hidden] (or the first `hidden` columns of `out`)."""
+    def forward(self, pixel_values: torch.Tensor, out: Optional[torch.Tensor] = None, film_cond: Optional[torch.Tensor] = None,
+                images_per_cond: int = 1) -> torch.Tensor:
+        """pixel_values bf16 [B, 3, 224, 224] -> bf16 [B, n_patches, hidden] (or the first `hidden` columns of `out`).
+        FiLM towers (`cfg.film_dim` > 0) need `film_cond`, bf16 [B / images_per_cond, film_dim] on the device: image i
+        is conditioned on row i // images_per_cond."""
         if pixel_values.dtype != torch.bfloat16 or pixel_values.device.type != "cuda" or pixel_values.dim() != 4:
             raise ValueError("pixel_values must be a bf16 CUDA tensor [B, 3, H, W]")
         B = pixel_values.shape[0]
+        film = self.cfg.film_dim > 0
+        if film != (film_cond is not None):
+            raise ValueError("film_cond is required by a FiLM tower (film_dim > 0) and rejected by any other")
+        if film and (film_cond.dtype != torch.bfloat16 or film_cond.device.type != "cuda" or film_cond.dim() != 2
+                     or film_cond.shape[1] != self.cfg.film_dim or film_cond.stride(1) != 1
+                     or images_per_cond < 1 or film_cond.shape[0] * images_per_cond != B):
+            raise ValueError(f"film_cond must be a bf16 CUDA tensor [B / images_per_cond, {self.cfg.film_dim}] with "
+                             f"contiguous rows (B = {B}, images_per_cond = {images_per_cond})")
         if out is None:
             out = torch.empty((B, self.n_patches, self.cfg.hidden), device=self.device, dtype=torch.bfloat16)
         if out.stride(-1) != 1 or out.stride(0) != self.n_patches * out.stride(1):
             raise ValueError("out must be [B, n_patches, >= hidden] with contiguous rows")
         strides = (C.c_int64 * 4)(*pixel_values.stride())
         stream = torch.cuda.current_stream(self.device).cuda_stream
-        capi.check(self.lib.blurr_vit_forward(self.handle, C.c_void_p(stream), B, C.c_void_p(pixel_values.data_ptr()), strides,
-                                              C.c_void_p(out.data_ptr()), out.stride(1)))
+        if film:
+            capi.check(self.lib.blurr_vit_forward_film(self.handle, C.c_void_p(stream), B, C.c_void_p(pixel_values.data_ptr()),
+                                                       strides, C.c_void_p(film_cond.data_ptr()), film_cond.stride(0),
+                                                       images_per_cond, C.c_void_p(out.data_ptr()), out.stride(1)))
+        else:
+            capi.check(self.lib.blurr_vit_forward(self.handle, C.c_void_p(stream), B, C.c_void_p(pixel_values.data_ptr()),
+                                                  strides, C.c_void_p(out.data_ptr()), out.stride(1)))
         return out
 
     @property
@@ -635,22 +671,26 @@ class FusedVisionBackbone:
         # the two towers are independent chains of small, latency-bound kernels: run them side by side on two streams
         self._side = torch.cuda.Stream(device=dino.device) if concurrent else None
 
-    def forward(self, pixel_values_dino: torch.Tensor, pixel_values_siglip: torch.Tensor) -> torch.Tensor:
+    def forward(self, pixel_values_dino: torch.Tensor, pixel_values_siglip: torch.Tensor, film_cond: Optional[torch.Tensor] = None,
+                images_per_cond: int = 1) -> torch.Tensor:
+        """`film_cond` (FiLM towers only): bf16 [B / images_per_cond, film_dim], given to both towers."""
         B = pixel_values_dino.shape[0]
         feats = torch.empty((B, self.dino.n_patches, self.width), device=pixel_values_dino.device, dtype=torch.bfloat16)
         sig_out = feats[:, :, self.dino.cfg.hidden:]
         if self._side is None:
-            self.dino.forward(pixel_values_dino, out=feats)
-            self.siglip.forward(pixel_values_siglip, out=sig_out)
+            self.dino.forward(pixel_values_dino, out=feats, film_cond=film_cond, images_per_cond=images_per_cond)
+            self.siglip.forward(pixel_values_siglip, out=sig_out, film_cond=film_cond, images_per_cond=images_per_cond)
         else:
             cur = torch.cuda.current_stream(self.dino.device)
             self._side.wait_stream(cur)
             with torch.cuda.stream(self._side):
-                self.siglip.forward(pixel_values_siglip, out=sig_out)
-            self.dino.forward(pixel_values_dino, out=feats)
+                self.siglip.forward(pixel_values_siglip, out=sig_out, film_cond=film_cond, images_per_cond=images_per_cond)
+            self.dino.forward(pixel_values_dino, out=feats, film_cond=film_cond, images_per_cond=images_per_cond)
             cur.wait_stream(self._side)
             pixel_values_siglip.record_stream(self._side)
             feats.record_stream(self._side)
+            if film_cond is not None:
+                film_cond.record_stream(self._side)
         return self.projector.forward(feats)
 
 
@@ -824,7 +864,8 @@ class OftConfig:
     paper describes; False gives plain causal attention.  The head is `MLPResNet(head_num_blocks, action_dim * hidden,
     head_hidden_dim, action_dim)`; `max_positions` is the decoder's (1 + patches + prompt + 56 slots + stop).
     `num_images` cameras (third-person first, then the wrist camera) give 256 patch rows each; `use_proprio` appends
-    one projected row of the `proprio_dim`-wide robot state after them."""
+    one projected row of the `proprio_dim`-wide robot state after them.  `use_film`: the towers are FiLM-conditioned on
+    the averaged instruction embedding (`film_language_embedding`), OFT's "OFT+" form."""
     chunk: int = 8
     action_dim: int = 7
     bidirectional_actions: bool = True
@@ -837,6 +878,7 @@ class OftConfig:
     num_images: int = 1
     use_proprio: bool = False
     proprio_dim: int = 8
+    use_film: bool = False
 
 
 def oft_libero_config() -> OftConfig:
@@ -916,6 +958,22 @@ def build_oft_embeds(decoder: LlamaDecoder, layout: OftLayout, patch_embeds: tor
     stop_row = decoder.embed(torch.tensor([stop_token], device=x.device))[0]
     full = torch.where((pos < a0)[..., None], full, torch.zeros((), device=x.device, dtype=x.dtype))
     return torch.where((pos == a0 + layout.n_rows)[..., None], stop_row, full).contiguous()
+
+
+def film_language_rows(layout: OftLayout, stop_token: int = 2) -> List[torch.Tensor]:
+    """The token ids whose embeddings FiLM averages, one int64 tensor per sequence: `ids[b, :text_lens[b]]` (BOS, the
+    instruction, the appended 29871) and the stop token.  OFT embeds its whole input and drops the positions its action
+    mask marks; that mask is taken to cover the action placeholders only, so the stop token stays - a restatement choice
+    (OFT's own code is not available here, DESIGN.md 10).  The action slots and the pads are never averaged, so a sequence
+    of a ragged batch gets what it gets alone.  Everything that needs these rows calls this function."""
+    stop = torch.tensor([stop_token], dtype=torch.int64)
+    return [torch.cat([layout.ids[b, :int(layout.text_lens[b])], stop]) for b in range(layout.ids.shape[0])]
+
+
+def film_language_embedding(decoder: LlamaDecoder, layout: OftLayout, stop_token: int = 2) -> torch.Tensor:
+    """FiLM's language vector, bf16 [B, hidden] on the decoder's device: the mean of the embeddings of
+    `film_language_rows`, per sequence, as OFT's `language_embeddings.mean(dim=1)` (fp32 sum, one bf16 rounding)."""
+    return torch.cat([decoder.embed(r)[None].mean(dim=1) for r in film_language_rows(layout, stop_token)]).contiguous()
 
 
 class L1RegressionHead:
@@ -1102,6 +1160,11 @@ class OftPolicy:
         if cfg.use_proprio and (proprio_projector is None or proprio_projector.proprio_dim != cfg.proprio_dim
                                 or proprio_projector.hidden != decoder.cfg.hidden):
             raise ValueError("use_proprio needs a ProprioProjector of proprio_dim columns and the decoder's width")
+        film_dims = (backbone.dino.cfg.film_dim, backbone.siglip.cfg.film_dim)
+        if film_dims != ((decoder.cfg.hidden,) * 2 if cfg.use_film else (0, 0)):
+            raise ValueError(f"use_film = {cfg.use_film} needs towers with film_dim = "
+                             f"{decoder.cfg.hidden if cfg.use_film else 0} (the decoder's width with FiLM, 0 without); "
+                             f"they have {film_dims}")
         self.preprocessors, self.preprocessor = pres, pres[0]
         self.backbone, self.decoder, self.head, self.cfg = backbone, decoder, head, cfg
         self.proprio_projector = proprio_projector if cfg.use_proprio else None
@@ -1126,16 +1189,20 @@ class OftPolicy:
             raise ValueError("every camera needs the same batch size")
         return out[0] if n == 1 else torch.cat(out, dim=1)
 
-    def patch_embeds(self, pixel_values: torch.Tensor, proprio_state: Optional[torch.Tensor] = None) -> torch.Tensor:
+    def patch_embeds(self, pixel_values: torch.Tensor, proprio_state: Optional[torch.Tensor] = None,
+                     film_cond: Optional[torch.Tensor] = None) -> torch.Tensor:
         """bf16 pixel values [B, 6 * num_images, 224, 224] (and the normalised state [B, proprio_dim]) -> the rows
         between BOS and the prompt, bf16 [B, 256 * num_images (+ 1), hidden]: image i's patches at rows 256 i ..
-        (OFT's `torch.cat(all_patches, dim=1)`), then the projected state."""
+        (OFT's `torch.cat(all_patches, dim=1)`), then the projected state.  With `use_film`, `film_cond` is the language
+        vector [B, hidden] every camera of a sequence is conditioned on."""
         n = self.cfg.num_images
         if pixel_values.dim() != 4 or pixel_values.shape[1] != 6 * n:
             raise ValueError(f"pixel_values must be [B, {6 * n}, H, W] ({n} camera(s) of 6 channels)")
         B = pixel_values.shape[0]
         px = pixel_values if n == 1 else pixel_values.reshape(B * n, 6, *pixel_values.shape[2:])
-        patch = self.backbone.forward(px[:, :3], px[:, 3:])
+        if self.cfg.use_film and film_cond is None:
+            raise ValueError("use_film needs the language vector (film_language_embedding)")
+        patch = self.backbone.forward(px[:, :3], px[:, 3:], film_cond if self.cfg.use_film else None, images_per_cond=n)
         if n > 1:
             patch = patch.reshape(B, n * patch.shape[1], patch.shape[2])
         if self.proprio_projector is None:
@@ -1147,11 +1214,16 @@ class OftPolicy:
 
     def action_rows(self, pixel_values: torch.Tensor, input_ids, attention_mask: Optional[torch.Tensor] = None,
                     proprio_state: Optional[torch.Tensor] = None) -> torch.Tensor:
-        """The decoder's final-normed rows in front of the action slots, bf16 [B, chunk * action_dim, hidden]."""
-        patch = self.patch_embeds(pixel_values, proprio_state)
-        lay = oft_prompt_layout(input_ids, attention_mask, patch.shape[1], self.cfg)
+        """The decoder's final-normed rows in front of the action slots, bf16 [B, chunk * action_dim, hidden].  The layout
+        comes first: with `use_film` the towers need the language vector it defines."""
+        P = self.backbone.dino.n_patches * self.cfg.num_images + (1 if self.cfg.use_proprio else 0)
+        lay = oft_prompt_layout(input_ids, attention_mask, P, self.cfg)
         if lay.max_len > self.decoder.cfg.max_positions:
             raise ValueError(f"an OFT sequence needs {lay.max_len} positions; the decoder holds {self.decoder.cfg.max_positions}")
+        cond = film_language_embedding(self.decoder, lay, self.cfg.stop_token) if self.cfg.use_film else None
+        if cond is not None and cond.shape[0] != pixel_values.shape[0]:
+            raise ValueError("input_ids must hold one prompt per sequence of pixel_values")
+        patch = self.patch_embeds(pixel_values, proprio_state, cond)
         x = build_oft_embeds(self.decoder, lay, patch, self.cfg.stop_token)
         return self.decoder.forward_rows(x, lay.seq_lens, lay.block_starts, lay.row_starts, lay.n_rows)
 

@@ -14,6 +14,12 @@
  * (+ LayerScale) -> residual; output = the patch-token rows after the last block that was built.  All on the kernels of
  * the Pi-0 SigLIP tower (tcgen05 GEMMs, LayerNorm consumers, the attention kernels of csrc/attention.cu).
  * Device pointers unless stated; errors as in blurr_pi0.h.  bf16 weights.
+ *
+ * FiLM (film_dim > 0): OpenVLA-OFT's language conditioning of the towers (its "OFT+" form).  Every block that runs becomes
+ * x = x + LS1(attn(LN1(x)));  x = x * (1 + gamma) + beta;  x = x + LS2(MLP(LN2(x)))
+ * with gamma = film_scale(cond), beta = film_shift(cond) (nn.Linear(film_dim -> hidden) each, per block) and every
+ * operation rounded to bf16 as torch does; cls / register rows are conditioned too.  FiLM towers must be 1024 or 1152
+ * wide.  One GEMM per call produces every block's gamma and beta before the first block.
  */
 #ifndef BLURR_VIT_H_
 #define BLURR_VIT_H_
@@ -39,8 +45,9 @@ typedef struct blurr_vit_config {
     int32_t use_layerscale;       /* 1 (DINOv2) / 0 */
     int32_t gelu_erf;             /* 1: exact GELU (DINOv2), 0: tanh approximation (SigLIP) */
     float ln_eps;                 /* 1e-6 */
+    int32_t film_dim;             /* 0: no FiLM; else the conditioning width (OpenVLA-OFT: 4096), multiple of 64, <= 8192 */
 } blurr_vit_config;
-#define BLURR_VIT_ABI_VERSION 1
+#define BLURR_VIT_ABI_VERSION 2
 
 int blurr_vit_create(const blurr_vit_config* cfg, int device, int max_batch, blurr_vit_t** out);
 void blurr_vit_destroy(blurr_vit_t* h);
@@ -48,15 +55,21 @@ void blurr_vit_destroy(blurr_vit_t* h);
  * (position embeddings of the patch tokens), "prefix" [num_prefix_tokens][hidden] (the prefix rows as they enter block 0:
  * cls + its position embedding, then the register tokens), and per block N: "layers.N.ln1.weight|bias",
  * "layers.N.q|k|v|o.weight|bias", "layers.N.ls1" [hidden], "layers.N.ln2.weight|bias", "layers.N.fc1|fc2.weight|bias",
- * "layers.N.ls2" [hidden].  Tensors are copied and repacked. */
+ * "layers.N.ls2" [hidden]; with film_dim > 0 also "layers.N.film_scale.weight|bias" and "layers.N.film_shift.weight|bias"
+ * ([hidden][film_dim], [hidden]).  Tensors are copied and repacked. */
 int blurr_vit_set_weight(blurr_vit_t* h, const char* key, const void* dev_ptr, const int64_t* shape, int ndim);
 int blurr_vit_finalize(blurr_vit_t* h);
 /* pixel_values: bf16 [batch][3][image][image] with element strides (b, c, h, w).  Writes the patch-token features,
  * bf16 [batch * n_patches][out_ld], columns 0..hidden-1 of the rows starting at `out` (so two towers can fill the two
- * halves of one concatenated feature matrix). */
+ * halves of one concatenated feature matrix).  BLURR_ERR_STATE on a FiLM handle. */
 int blurr_vit_forward(blurr_vit_t* h, void* cuda_stream, int batch, const void* pixel_values, const int64_t strides[4],
                       void* out, int out_ld);
-/* Options: "use_cuda_graph" (default 1: the blocks replay as one CUDA graph per batch size). */
+/* FiLM handles only (BLURR_ERR_STATE otherwise): blurr_vit_forward, with image i conditioned on row i / images_per_cond
+ * of cond, bf16 [batch / images_per_cond][cond_ld] (cond_ld >= film_dim).  images_per_cond must divide batch.  cond is
+ * copied into the handle before the blocks run, so one CUDA graph per (batch, images_per_cond) serves every condition. */
+int blurr_vit_forward_film(blurr_vit_t* h, void* cuda_stream, int batch, const void* pixel_values, const int64_t strides[4],
+                           const void* cond, int cond_ld, int images_per_cond, void* out, int out_ld);
+/* Options: "use_cuda_graph" (default 1: the blocks replay as one CUDA graph per batch size and images_per_cond). */
 int blurr_vit_set_option(blurr_vit_t* h, const char* name, int64_t value);
 int64_t blurr_vit_last_launch_count(const blurr_vit_t* h);
 
