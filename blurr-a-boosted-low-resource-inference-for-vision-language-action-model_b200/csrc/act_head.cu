@@ -37,6 +37,7 @@ namespace {
 constexpr int kFewRows = 32;              // at most this many rows: split-K partials (weight streaming), as the decoder
 constexpr int kWideThreads = 512;
 constexpr int kWideVpt = 16;              // 4-column groups per thread: rows of up to 512 * 16 * 4 = 32768 columns
+constexpr int kWideSmemMaxCols = 65536;   // act_wide_layernorm_smem_kernel: the bf16 row in 128 KB of shared memory
 constexpr int kActThreads = 512;
 constexpr int kActVpt = 2;                // rows of up to 4096 columns
 
@@ -72,6 +73,44 @@ __global__ void __launch_bounds__(kWideThreads) act_wide_layernorm_kernel(const 
         const float4 ww = load_bf16x4(w + g * 4), bb = load_bf16x4(bias + g * 4);
         store_bf16x4(y + row + g * 4, make_float4((v[i].x - mean) * rstd * ww.x + bb.x, (v[i].y - mean) * rstd * ww.y + bb.y,
                                                   (v[i].z - mean) * rstd * ww.z + bb.z, (v[i].w - mean) * rstd * ww.w + bb.w));
+    }
+}
+
+// The same LayerNorm for rows past the register kernel's 32768 columns (ALOHA: 14 * 4096 = 57344), the bf16 row staged in
+// dynamic shared memory (N * 2 bytes) instead of registers.  Thread striding (g = tid + 512 i), the per-thread summation
+// order and the block reductions are act_wide_layernorm_kernel's, so a row both kernels could take gets the same result.
+__global__ void __launch_bounds__(kWideThreads) act_wide_layernorm_smem_kernel(const bf16* __restrict__ x, int N,
+                                                                               const bf16* __restrict__ w,
+                                                                               const bf16* __restrict__ bias, float eps,
+                                                                               bf16* __restrict__ y) {
+    extern __shared__ __align__(16) uint2 xs[];     // [N / 4]: four bf16 per entry
+    __shared__ float red[kWideThreads / 32];
+    pdl_wait();
+    pdl_trigger();
+    const size_t row = static_cast<size_t>(blockIdx.x) * N;
+    const int nvec = N >> 2;
+    float lsum = 0.f;
+    for (int g = threadIdx.x; g < nvec; g += kWideThreads) {
+        const uint2 u = __ldcg(reinterpret_cast<const uint2*>(x + row + g * 4));
+        xs[g] = u;
+        const float2 a = unpack_bf16x2(u.x), b = unpack_bf16x2(u.y);
+        lsum += (a.x + a.y) + (b.x + b.y);
+    }
+    const float mean = block_sum<kWideThreads>(lsum, red) / static_cast<float>(N);
+    float lvar = 0.f;
+    for (int g = threadIdx.x; g < nvec; g += kWideThreads) {        // each thread reads back only what it wrote
+        const uint2 u = xs[g];
+        const float2 a = unpack_bf16x2(u.x), b = unpack_bf16x2(u.y);
+        const float dx = a.x - mean, dy = a.y - mean, dz = b.x - mean, dw = b.y - mean;
+        lvar += (dx * dx + dy * dy) + (dz * dz + dw * dw);
+    }
+    const float rstd = rsqrtf(block_sum<kWideThreads>(lvar, red) / static_cast<float>(N) + eps);
+    for (int g = threadIdx.x; g < nvec; g += kWideThreads) {
+        const uint2 u = xs[g];
+        const float2 a = unpack_bf16x2(u.x), b = unpack_bf16x2(u.y);
+        const float4 ww = load_bf16x4(w + g * 4), bb = load_bf16x4(bias + g * 4);
+        store_bf16x4(y + row + g * 4, make_float4((a.x - mean) * rstd * ww.x + bb.x, (a.y - mean) * rstd * ww.y + bb.y,
+                                                  (b.x - mean) * rstd * ww.z + bb.z, (b.y - mean) * rstd * ww.w + bb.w));
     }
 }
 
@@ -212,8 +251,9 @@ extern "C" int blurr_act_head_create(const blurr_act_head_config* cfg, int devic
     if (c.input_dim < 1 || c.action_dim < 1 || c.chunk < 1 || c.num_blocks < 0 || !(c.ln_eps > 0.0f))
         return fail(BLURR_ERR_INVALID, "blurr_act_head_create: input_dim, action_dim, chunk >= 1, num_blocks >= 0, ln_eps > 0");
     const int64_t wide = static_cast<int64_t>(c.action_dim) * c.input_dim;
-    if (wide % 64 || wide > 4 * kWideThreads * kWideVpt)
-        return fail(BLURR_ERR_INVALID, "action_dim * input_dim must be a multiple of 64 and at most 32768 (one LayerNorm row in registers)");
+    if (wide % 64 || wide > kWideSmemMaxCols)
+        return fail(BLURR_ERR_INVALID, "action_dim * input_dim must be a multiple of 64 and at most 65536 (one LayerNorm row in "
+                                       "shared memory)");
     if (c.hidden_dim < 128 || c.hidden_dim % 128 || c.hidden_dim > 4 * kActThreads * kActVpt)
         return fail(BLURR_ERR_INVALID, "hidden_dim must be a multiple of 128 and at most 4096");
     if (static_cast<int64_t>(max_batch) * c.chunk > 4096) return fail(BLURR_ERR_INVALID, "max_batch * chunk must be at most 4096 rows");
@@ -226,6 +266,9 @@ extern "C" int blurr_act_head_create(const blurr_act_head_config* cfg, int devic
     if (prop.major != 10)
         return fail(BLURR_ERR_CUDA, "device is sm_" + std::to_string(prop.major) + std::to_string(prop.minor) + ": this library is built for sm_100a only");
     HEAD_CUDA_TRY(cudaSetDevice(device));
+    if (wide > 4 * kWideThreads * kWideVpt)
+        HEAD_CUDA_TRY(cudaFuncSetAttribute(act_wide_layernorm_smem_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                           kWideSmemMaxCols * 2));
     auto* h = new blurr_act_head();
     h->cfg = c; h->device = device; h->max_batch = max_batch; h->max_rows = max_batch * c.chunk;
     const size_t R = h->max_rows, W = static_cast<size_t>(wide), H = c.hidden_dim;
@@ -369,7 +412,10 @@ void run_head(HeadRun& R, int rows) {
     blurr_act_head* h = R.h;
     const auto& c = h->cfg;
     const int wide = c.action_dim * c.input_dim, nb = c.num_blocks;
-    R.launched(launch_kernel(act_wide_layernorm_kernel, dim3(rows), dim3(kWideThreads), 0, R.st, static_cast<const bf16*>(h->IN), wide,
+    // by width only: rows up to 32768 columns keep the register kernel
+    const bool in_regs = wide <= 4 * kWideThreads * kWideVpt;
+    R.launched(launch_kernel(in_regs ? act_wide_layernorm_kernel : act_wide_layernorm_smem_kernel, dim3(rows), dim3(kWideThreads),
+                             in_regs ? 0 : static_cast<size_t>(wide) * 2, R.st, static_cast<const bf16*>(h->IN), wide,
                              static_cast<const bf16*>(h->ln1_w), static_cast<const bf16*>(h->ln1_b), c.ln_eps, h->XN1),
                "act_wide_layernorm");
     int s = R.gemm(h->fc1, h->XN1, rows);

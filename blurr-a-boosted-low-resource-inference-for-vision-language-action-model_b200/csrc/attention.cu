@@ -741,7 +741,7 @@ static cudaError_t launch_attn_block(cudaStream_t stream, const AttnMmaArgs& a, 
 // reads the row from shared memory on each pass instead of holding up to 32 logits per lane in registers; expf is
 // recomputed on the last pass, which gives the same value.
 static constexpr int kAttnStreamStages = 3;
-static constexpr int kAttnStreamMaxBlocks = 16;     // 1024 keys
+static constexpr int kAttnStreamMaxBlocks = 32;     // 2048 keys (BM 32 at head_dim 128 past 1152 keys, see below)
 
 template <int HD_PAD, int BM>
 __device__ __forceinline__ void attn_block_stream_body(const AttnMmaArgs& a, uint8_t* smem_attn, const int qt, const int h,
@@ -969,7 +969,18 @@ static cudaError_t launch_block_rule(bool stream_kv, cudaStream_t stream, const 
                      : launch_attn_block<HD_PAD, BM>(stream, a, seq_len, block_start, m.q_per_sample, m.n_heads, m.batch);
 }
 
-// Up to 384 keys every key block of a head stays resident in shared memory (attn_block_kernel); past that, up to 1024,
+// The streamed kernel's logits grow with the key count (BM x n_keys bf16), so past 1152 keys at head_dim 128 a 64-row tile
+// no longer fits the opt-in limit: the tile is halved until it does (BM 32 holds 2048 keys at either head_dim).  A row's
+// output does not depend on BM (its own rounding chain, lane-strided softmax and key-block order of P.V), so this changes
+// speed only; up to 1152 keys BM is what attn_tile_rows picks.
+static int attn_stream_fit_rows(int hd, int bm, int n_keys) {
+    if (hd == 64) return bm > 32 ? 32 : bm;                         // head_dim 64 runs at most BM 32: 2048 keys fit
+    if (bm == 64 && attn_stream_smem_bytes<128, 64>(n_keys) > kAttnSmemMax) bm = 32;
+    if (bm == 32 && attn_stream_smem_bytes<128, 32>(n_keys) > kAttnSmemMax) bm = 16;
+    return bm;
+}
+
+// Up to 384 keys every key block of a head stays resident in shared memory (attn_block_kernel); past that, up to 2048,
 // K and V stream through a ring (attn_block_stream_kernel).
 cudaError_t launch_mha_block_attention(cudaStream_t stream, const MhaAttnArgs& m, const int* block_start) {
     if (m.n_keys > kAttnStreamMaxBlocks * kBK || m.n_kv_heads != m.n_heads || m.q_pos0 != 0 ||
@@ -983,9 +994,10 @@ cudaError_t launch_mha_block_attention(cudaStream_t stream, const MhaAttnArgs& m
     a.out = m.out; a.ldo = width; a.o_col0 = 0;
     a.hd = m.head_dim; a.head_stride_q = m.head_dim; a.head_stride_kv = m.head_dim; a.n_keys = m.n_keys;
     a.scale = m.scale; a.mask = nullptr; a.q_row_offset = 0; a.trace = m.trace;
-    const int bm = attn_tile_rows(m.q_per_sample, m.n_heads, m.batch, 64);
+    int bm = attn_tile_rows(m.q_per_sample, m.n_heads, m.batch, 64);
     const int* L = m.seq_len;
     const bool sk = m.n_keys > kAttnMaxBlocksWide * kBK;
+    if (sk) bm = attn_stream_fit_rows(m.head_dim, bm, m.n_keys);
     if (m.head_dim == 128) {
         if (bm == 16) return launch_block_rule<128, 16>(sk, stream, a, L, block_start, m);
         if (bm == 32) return launch_block_rule<128, 32>(sk, stream, a, L, block_start, m);

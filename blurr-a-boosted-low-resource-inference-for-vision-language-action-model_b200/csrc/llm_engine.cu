@@ -57,6 +57,7 @@ constexpr int kFewTokens = 32;        // at most this many token rows: split-K p
 constexpr int kGenerateMaxPositions = 320;     // generate's decode kernels hold a sequence's logits in sc[320]
 constexpr int kForwardMaxPositions = 384;      // long_forward 0: attn_block_kernel keeps every key block resident (6 x 64)
 constexpr int kLongForwardMaxPositions = 1024; // long_forward 1: attn_block_stream_kernel streams K/V (16 x 64 keys)
+constexpr int kLongerForwardMaxPositions = 2048;   // long_forward 2 (1025..2048): the same kernel, 32 x 64 keys (BM <= 32 past 1152)
 
 struct Lin { bf16* w = nullptr; int Nw = 0, K = 0; };
 struct Layer { Lin qkv, o, gu, down; bf16 *in_ln = nullptr, *post_ln = nullptr; };
@@ -157,10 +158,14 @@ extern "C" int blurr_llm_create(const blurr_llm_config* cfg, int device, int max
     if ((c.num_heads * c.head_dim) % 128 || c.hidden > 4096 * 2)
         return fail(BLURR_ERR_INVALID, "num_heads * head_dim must be a multiple of 128; hidden <= 8192");
     if (c.hidden > 4096) return fail(BLURR_ERR_INVALID, "the RMSNorm consumer covers rows of up to 4096 columns");
-    if (c.long_forward != 0 && c.long_forward != 1) return fail(BLURR_ERR_INVALID, "long_forward must be 0 or 1");
-    if (c.max_positions < 2 || c.max_positions > (c.long_forward ? kLongForwardMaxPositions : kForwardMaxPositions))
+    if (c.long_forward < 0 || c.long_forward > 2) return fail(BLURR_ERR_INVALID, "long_forward must be 0, 1 or 2");
+    if (c.long_forward == 2) {
+        if (c.max_positions <= kLongForwardMaxPositions || c.max_positions > kLongerForwardMaxPositions)
+            return fail(BLURR_ERR_INVALID, "max_positions must be in 1025..2048 with long_forward = 2 (up to 1024: long_forward = 1)");
+    } else if (c.max_positions < 2 || c.max_positions > (c.long_forward ? kLongForwardMaxPositions : kForwardMaxPositions)) {
         return fail(BLURR_ERR_INVALID, c.long_forward ? "max_positions must be in 2..1024 with long_forward"
                                                       : "max_positions must be in 2..384 (1024 with long_forward = 1)");
+    }
     if (max_batch > kFewTokens) return fail(BLURR_ERR_INVALID, "max_batch <= 32 (one decode step is a few-token GEMM)");
     int ndev = 0;
     if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0)

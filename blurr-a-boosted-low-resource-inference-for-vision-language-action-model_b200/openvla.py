@@ -51,7 +51,8 @@ class LlamaShapedConfig:
     max_positions: int = 320      # 1 + 256 patches + prompt + 7 action tokens fits
     rms_eps: float = 1e-6
     rope_theta: float = 10000.0
-    long_forward: bool = False    # max_positions up to 1024 for forward_rows (384 without); generate stops at 320 either way
+    long_forward: int = 0         # max_positions: 0 up to 384, 1 up to 1024 (True means 1), 2 in 1025..2048, for
+                                  # forward_rows; generate stops at 320 on every handle
 
 
 def openvla_7b_config() -> LlamaShapedConfig:
@@ -279,7 +280,8 @@ class LlamaDecoder:
 
 def denormalize_actions(norm: np.ndarray, q01, q99, mask=None) -> np.ndarray:
     """OpenVLA's de-normalisation: `0.5 * (a + 1) * (q99 - q01) + q01` where `mask`, `a` elsewhere, in float64.  q01 / q99
-    / mask broadcast against `norm` from the right."""
+    / mask broadcast against `norm` from the right.  OFT's BOUNDS statistics (ALOHA) go in as min / max in place of
+    q01 / q99.  No `+ 1e-8` is added to the range; whether OFT's own un-normalisation adds one is unpinned."""
     q01, q99 = np.asarray(q01, dtype=np.float64), np.asarray(q99, dtype=np.float64)
     mask = np.ones_like(q01, dtype=bool) if mask is None else np.asarray(mask, dtype=bool)
     return np.where(mask, 0.5 * (norm + 1) * (q99 - q01) + q01, norm)
@@ -863,7 +865,8 @@ class OftConfig:
     empty action slot per value.  `bidirectional_actions`: the slots (and the stop token) attend to each other, as the
     paper describes; False gives plain causal attention.  The head is `MLPResNet(head_num_blocks, action_dim * hidden,
     head_hidden_dim, action_dim)`; `max_positions` is the decoder's (1 + patches + prompt + 56 slots + stop).
-    `num_images` cameras (third-person first, then the wrist camera) give 256 patch rows each; `use_proprio` appends
+    `num_images` cameras (third-person first, then the wrist camera; ALOHA: top, left wrist, right wrist) give 256
+    patch rows each; `use_proprio` appends
     one projected row of the `proprio_dim`-wide robot state after them.  `use_film`: the towers are FiLM-conditioned on
     the averaged instruction embedding (`film_language_embedding`), OFT's "OFT+" form."""
     chunk: int = 8
@@ -887,17 +890,26 @@ def oft_libero_config() -> OftConfig:
     return OftConfig(num_images=2, use_proprio=True, proprio_dim=8, chunk=8, action_dim=7, max_positions=640)
 
 
+def oft_aloha_config() -> OftConfig:
+    """OFT's bimanual ALOHA checkpoints (OFT+): three cameras in the order top, left wrist, right wrist, 14-D
+    proprioception, chunks of 25 x 14 and FiLM.  P = 3 * 256 + 1 = 769 rows precede the prompt and 25 * 14 = 350 empty
+    slots and the stop token follow it, so a sequence is 769 + S + 350 + 1 = 1120 + S positions (S: the prompt with BOS
+    and 29871; about 1140-1150 with OpenVLA's template).  The decoder holds 1280, which allows S <= 160.  ALOHA
+    normalises with OFT's BOUNDS statistics (min / max): pass them where the LIBERO form passes q01 / q99."""
+    return OftConfig(num_images=3, use_proprio=True, proprio_dim=14, chunk=25, action_dim=14, use_film=True, max_positions=1280)
+
+
 def openvla_oft_7b_config(oft: Optional[OftConfig] = None) -> LlamaShapedConfig:
     """The OpenVLA-7B decoder with room for OFT's sequence (`oft.max_positions`, 384 by default; `openvla_7b_config`
-    keeps 320).  Past 384 positions the decoder is created with `long_forward`."""
+    keeps 320).  `long_forward` is 0 up to 384 positions, 1 up to 1024 and 2 beyond."""
     n = (oft or OftConfig()).max_positions
-    return LlamaShapedConfig(max_positions=n, long_forward=n > 384)
+    return LlamaShapedConfig(max_positions=n, long_forward=0 if n <= 384 else 1 if n <= 1024 else 2)
 
 
 def normalize_proprio(state, q01, q99, mask=None) -> np.ndarray:
     """OFT's BOUNDS_Q99 normalisation of the robot state, on the host in float64:
     `clip(where(mask, 2 * (x - q01) / (q99 - q01 + 1e-8) - 1, x), -1, 1)`.  state [B, D] (or [D]); q01 / q99 / mask
-    [D] or [B, D]."""
+    [D] or [B, D].  OFT's BOUNDS rule (ALOHA) is the same arithmetic on the dataset's min / max: pass them as q01 / q99."""
     x = np.asarray(state.detach().cpu() if isinstance(state, torch.Tensor) else state, dtype=np.float64)
     lo, hi = np.asarray(q01, dtype=np.float64), np.asarray(q99, dtype=np.float64)
     m = np.ones(lo.shape, dtype=bool) if mask is None else np.asarray(mask, dtype=bool)
@@ -1259,11 +1271,12 @@ class OftPolicy:
                              return_normalized: bool = False, proprio=None, proprio_q01=None, proprio_q99=None,
                              proprio_mask=None):
         """frames: uint8 [H, W, 3] or [B, H, W, 3] RGB for one camera; with num_images > 1 a sequence of such batches,
-        one per camera (third-person first, then the wrist camera).  input_ids: [B, S] (first column BOS), a list of B
+        one per camera (third-person first, then the wrist camera; ALOHA: top, left wrist, right wrist).  input_ids: [B, S] (first column BOS), a list of B
         1-D id tensors, or [B, S] with a left- or right-padded `attention_mask` (see `oft_prompt_layout`).  q01 / q99 /
         mask: [action_dim] or [B, action_dim], applied to every step of the chunk.  With `use_proprio`: `proprio` the
         raw state [B, proprio_dim] and its dataset's `proprio_q01` / `proprio_q99` (/ `proprio_mask`), normalised by
-        `normalize_proprio`.  Returns float64 actions [B, chunk, action_dim] on the host (and, with
+        `normalize_proprio`.  For ALOHA (BOUNDS statistics) pass the min / max in place of q01 / q99, for the actions
+        and the state alike.  Returns float64 actions [B, chunk, action_dim] on the host (and, with
         `return_normalized`, the head's output fp32 [B, chunk, action_dim] on the device)."""
         return self.predict_action_chunk_from_pixels(self.pixel_values(frames), input_ids, q01, q99, mask, attention_mask,
                                                      return_normalized, proprio, proprio_q01, proprio_q99, proprio_mask)

@@ -9,7 +9,8 @@
  *   num_blocks x: x = x + ReLU(Linear(hidden -> hidden)(LayerNorm(hidden)(x)));
  *   LayerNorm(hidden) -> Linear(hidden -> D).
  * Arithmetic as torch runs the bf16 module: LayerNorm in fp32 with bf16 output, Linear as bf16(acc + bias), ReLU and the
- * residual add in bf16.  PARITY: pinned against a torch restatement of the module (oracle/openvla_oft_oracle.py); against
+ * residual add in bf16.  The first LayerNorm keeps a row of up to 32768 columns in registers and a wider one (up to 65536,
+ * ALOHA's 14 * 4096 = 57344) in shared memory, with the same summation order.  PARITY: pinned against a torch restatement of the module (oracle/openvla_oft_oracle.py); against
  * the OFT repository's code it is UNPINNED (neither vendored nor downloadable), see DESIGN.md.
  *
  * All pointers are device pointers.  Errors: negative blurr_status (blurr_pi0.h), message from blurr_last_error().
@@ -30,8 +31,8 @@ typedef struct blurr_act_head blurr_act_head_t;
 typedef struct blurr_act_head_config {
     int32_t abi_version;          /* BLURR_ACT_HEAD_ABI_VERSION */
     int32_t input_dim;            /* H: the decoder's hidden width, 4096 */
-    int32_t action_dim;           /* D: 7; D * H is a multiple of 64 and at most 32768 */
-    int32_t chunk;                /* K: actions per chunk, 8 */
+    int32_t action_dim;           /* D: 7 (14 for ALOHA); D * H is a multiple of 64 and at most 65536 */
+    int32_t chunk;                /* K: actions per chunk, 8 (25 for ALOHA) */
     int32_t hidden_dim;           /* 4096, a multiple of 128, at most 4096 */
     int32_t num_blocks;           /* MLP-ResNet blocks, 2 */
     float ln_eps;                 /* nn.LayerNorm's 1e-5 */

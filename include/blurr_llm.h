@@ -47,11 +47,12 @@ typedef struct blurr_llm_config {
     int32_t head_dim;             /* 128 (or 64) */
     int32_t intermediate;         /* 11008, multiple of 64 */
     int32_t vocab;                /* 32064 (rows of embed_tokens / lm_head) */
-    int32_t max_positions;        /* KV-cache slots per sequence, <= 384, or <= 1024 with long_forward = 1 (generate:
-                                     prompt + generated tokens <= 320 on every handle) */
+    int32_t max_positions;        /* KV-cache slots per sequence, <= 384, or <= 1024 with long_forward = 1, or 1025..2048
+                                     with long_forward = 2 (generate: prompt + generated tokens <= 320 on every handle) */
     float rms_eps;                /* 1e-6 (OpenVLA) / 1e-5 (Llama-2) */
     int32_t long_forward;         /* 0: max_positions <= 384; 1: up to 1024 for blurr_llm_forward_rows (OFT's two-camera
-                                     sequences); any other value is rejected */
+                                     sequences); 2: 1025..2048 (OFT's three-camera ALOHA sequences); any other value is
+                                     rejected */
 } blurr_llm_config;
 #define BLURR_LLM_ABI_VERSION 3
 
@@ -119,9 +120,9 @@ int blurr_llm_generate(blurr_llm_t* h, void* cuda_stream, int batch, int max_pro
  * k >= block_starts[b]): causal over the prompt, bidirectional inside the block [block_starts[b], seq_lens[b]);
  * block_starts[b] == seq_lens[b] is plain causal attention.  Positions (RoPE) are 0..max_len-1 for every sequence.
  * Writes out_hidden bf16 [batch][n_rows][hidden]: rows row_starts[b] .. + n_rows - 1 of sequence b after the final
- * RMSNorm (transformers' LlamaModel.last_hidden_state).  Accepts up to max_positions: 384, or 1024 on a handle created
- * with long_forward = 1 (past 384 keys the attention streams K and V through shared memory with the same arithmetic;
- * blurr_llm_generate stops at 320).  The
+ * RMSNorm (transformers' LlamaModel.last_hidden_state).  Accepts up to max_positions: 384, 1024 on a handle created
+ * with long_forward = 1, or 2048 with long_forward = 2 (past 384 keys the attention streams K and V through shared memory
+ * with the same arithmetic; blurr_llm_generate stops at 320).  The
  * pass is replayed as one CUDA graph per (batch, max_len) whatever the lengths, starts and n_rows; the row copy to
  * out_hidden is one more kernel after it.  A bad argument returns BLURR_ERR_INVALID and the handle keeps working. */
 int blurr_llm_forward_rows(blurr_llm_t* h, void* cuda_stream, int batch, int max_len, const void* inputs_embeds,
